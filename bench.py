@@ -14,6 +14,10 @@ Timing: W warm-up ticks, then K ticks each bracketed by CUDA events on the launc
 L2 flush (a 256 MiB memset) between ticks; ms_per_step = mean event time, max over ranks.  The
 `e2e` number drives the same tick through ok_step_host with pinned HOST buffers (H2D actions, D2H
 obs/reward/done inside the timed region).
+
+`--dump-outputs DIR` writes the buffers the last timed tick left (observations, rewards, flags, poses, ...) as
+DIR/<name>.npy, so that two builds can be compared output for output on identical inputs.  At N GPUs it writes rank 0's
+slice of the population only.
 """
 from __future__ import annotations
 
@@ -328,6 +332,28 @@ def bind_to_gpu_numa_node(torch, local: int):
 
 
 PARITY_BUFS = ("pos_x", "pos_y", "rot", "crashed", "timed_out", "hit_seg", "hit_t", "obs", "reward", "fitness", "nearest_idx", "reset_pt")
+DUMP_BUFS = PARITY_BUFS + ("speed", "done")
+DUMP_BYTES = 60_000_000  # array data; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(env, directory, stream=None):
+    """--dump-outputs: the buffers a caller of the tick reads, as DIR/<name>.npy.  binary32 buffers as they are, flags as
+    float32 and indices as float64 (both exact).  A population whose buffers would exceed DUMP_BYTES is cut to a fixed,
+    seeded sample of agents, the same rows in every buffer; agent_index.npy then names those rows."""
+    arrays = {}
+    for name in DUMP_BUFS:
+        a = env.read(name, stream)
+        arrays[name] = a.astype(np.float64 if a.dtype.kind in "iu" and a.itemsize == 4 else np.float32)
+    rows = None
+    per_agent = sum(a.nbytes for a in arrays.values()) // env.n
+    if per_agent * env.n > DUMP_BYTES:
+        k = DUMP_BYTES // (per_agent + 8)
+        rows = np.sort(np.random.default_rng(SEED).choice(env.n, k, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a if rows is None else a[rows])
+    if rows is not None:
+        np.save(os.path.join(directory, "agent_index.npy"), rows.astype(np.float64))
 
 
 def shard_parity_check(ok, torch, dist, env, rank, n, ticks, local, mode, extra):
@@ -379,7 +405,13 @@ def main():
     ap.add_argument("--generation", type=int, default=100, help="N>1: ticks between two fitness exchanges (NCCL all-gather + ranking)")
     ap.add_argument("--no-numa", action="store_true", help="do not bind the rank to its GPU's NUMA node")
     ap.add_argument("--config5", action="store_true", help="also run BASELINE configs[4]'s shape: 1,048,576 agents per GPU + CMA-ES exchange")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the buffers of the last timed tick as DIR/<name>.npy (float32 / float64, at most 64 MB; rank 0's agents)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU arm's buffers: it needs --impl ours")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -498,6 +530,8 @@ def main():
     gather_ms = float(np.mean([a.elapsed_time(m) for a, _, m in gens])) if gens else 0.0
     ms_per_step = ms_tick + gen_ms * len(gens) / args.steps
     crashed_frac = float(env.read("crashed", sp).mean())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(env, args.dump_outputs, sp)
     step_base += args.steps
     # clock window: the timed region of a short run is a few ms; keep the same launches going (untimed) until the
     # sampler has seen >= 1 s of this workload
@@ -528,12 +562,14 @@ def main():
         cma_us = 1e3 * c0.elapsed_time(c1) / 20
 
     # ---- end-to-end arm: HOST buffers through ok_step_host ---------------------------------------
-    e2e_steps = max(10, min(args.steps, 200))
-    thr = ok.pinned_array((e2e_steps, n), np.float32)
-    steer = ok.pinned_array((e2e_steps, n), np.float32)
+    # as many timed ticks as the device-resident arm; the host action rows repeat after 200 ticks
+    e2e_steps = args.steps
+    rows = min(e2e_steps, 200)
+    thr = ok.pinned_array((max(rows, 3), n), np.float32)
+    steer = ok.pinned_array((max(rows, 3), n), np.float32)
     rng = np.random.default_rng(1234 + rank)
-    thr[:] = rng.random((e2e_steps, n), dtype=np.float32) * 100.0
-    steer[:] = rng.random((e2e_steps, n), dtype=np.float32) * 10.0 - 5.0
+    thr[:] = rng.random(thr.shape, dtype=np.float32) * 100.0
+    steer[:] = rng.random(steer.shape, dtype=np.float32) * 10.0 - 5.0
     obs = ok.pinned_array((n, N_RAYS), np.float32)
     rew = ok.pinned_array((n,), np.float32)
     done = ok.pinned_array((n,), np.uint8)
@@ -545,7 +581,7 @@ def main():
     e0.record(stream)
     tw = time.perf_counter()
     for i in range(e2e_steps):
-        env.step_host(thr[i], steer[i], obs, rew, done, sp)
+        env.step_host(thr[i % rows], steer[i % rows], obs, rew, done, sp)
     e1.record(stream)
     barrier()
     tw = time.perf_counter() - tw
@@ -562,7 +598,7 @@ def main():
         barrier()
         tq = time.perf_counter()
         for i in range(e2e_steps):
-            env.step_host(thr[i], steer[i], obs_q, rew, done, sp)
+            env.step_host(thr[i % rows], steer[i % rows], obs_q, rew, done, sp)
         barrier()
         q16_ms = 1e3 * (time.perf_counter() - tq) / e2e_steps
     except Exception as ex:  # an experiment build (OK_B200_LIB) without the entry point

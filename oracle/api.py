@@ -58,8 +58,9 @@ class OkoConfig(C.Structure):
 
 def build(force: bool = False) -> None:
     """Compile the checkers (``make -C oracle``).  Building the checker is not using it."""
+    ref = os.environ.get("OPENKITCHEN_REF")  # a checkout of the original project (see oracle/Makefile)
     if force or not os.path.exists(os.path.join(HERE, "liboracle.so")) or (
-        os.path.isdir("/root/reference/Environment") and not os.path.exists(os.path.join(HERE, "_ref", "libokref.so"))
+        ref and os.path.isdir(os.path.join(ref, "Environment")) and not os.path.exists(os.path.join(HERE, "_ref", "libokref.so"))
     ):
         subprocess.run(["make", "-C", HERE], check=True, capture_output=True)
 

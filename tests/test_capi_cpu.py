@@ -3,6 +3,7 @@ bit-identically to the reference on the host, and refuses loudly to compute with
 import ctypes as C
 import os
 import re
+import sys
 import zlib
 
 import numpy as np
@@ -110,17 +111,14 @@ def test_shim_and_pybind_build_and_fail_loudly_without_gpu(tmp_path):
     assert os.path.exists(os.path.join(lib, "libopenkitchen_shim.so"))
     csv = tmp_path / "Monza.csv"
     ok.write_track_csv("Monza", str(csv))
-    try:
-        ok.Env(device=0).close()
-        pytest.skip("a GPU is present: covered by tests/test_gpu_shim.py")
-    except ok.OkError:
-        pass
-    r = subprocess.run([os.path.join(lib, "ok_shim_example"), str(csv), "3", "2"], capture_output=True, text=True)
+    # the checks run in child processes that see no device, so that they also hold on a machine with a GPU
+    no_gpu = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    r = subprocess.run([os.path.join(lib, "ok_shim_example"), str(csv), "3", "2"], capture_output=True, text=True, env=no_gpu)
     assert r.returncode != 0 and "no CPU fallback" in r.stderr
-    import open_kitchen_pybind as okp
-
-    with pytest.raises(RuntimeError, match="no CPU fallback"):
-        okp.Environment(str(csv))
+    code = ("import open_kitchen_pybind as okp, sys\n"
+            "try:\n    okp.Environment(sys.argv[1])\nexcept RuntimeError as ex:\n    print(ex)\n    sys.exit(3)\n")
+    r = subprocess.run([sys.executable, "-c", code, str(csv)], cwd=ROOT, capture_output=True, text=True, env=no_gpu)
+    assert r.returncode == 3 and "no CPU fallback" in r.stdout, r.stdout + r.stderr
 
 
 def test_q16_observation_helpers_round_trip():

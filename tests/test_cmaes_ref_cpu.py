@@ -4,7 +4,7 @@
    unmodified CmaEsSolverTorch.cpp + Controller.cpp compiled against pip-torch's libtorch) on identical seeds --
    samples and every state tensor BIT FOR BIT, generation after generation (both call the same ATen kernels);
 2. the restatement == tests/golden/cmaes_ref.npz, minted from that library (tools/make_golden_cmaes.py), so the pin
-   also holds where /root/reference and the compiled library are absent;
+   also holds where the reference's sources and the compiled library are absent;
 3. the product (openkitchen_b200/cmaes.py: batched, binary64 partial sums) == the restatement to float32 rounding:
    the reference narrows its binary64 sums to float32 after every candidate, the product once (tolerances below)."""
 import os

@@ -1,6 +1,7 @@
 """CPU: the plain-C oracle (oracle/ok_oracle.c) against the golden vectors minted from the reference's
 own objects (tools/make_golden.py -> tests/golden/), and -- when oracle/_ref is built -- against
-those objects live.  Bit-exact on every buffer."""
+those objects live.  Bit-exact on every buffer.  traces_live.npz stores the result of the live comparisons' scenarios
+(see tools/make_golden.py for how it was minted), so that they are checked where the reference is absent too."""
 import os
 import sys
 import zlib
@@ -16,6 +17,9 @@ sys.path.insert(0, os.path.join(os.path.dirname(__file__), "..", "tools"))
 import make_golden as mg  # noqa: E402
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
+# a checkout of the original project (not part of this repository): its track CSVs, when present
+REF = os.environ.get("OPENKITCHEN_REF")
+REF_TRACKS = os.path.join(REF, "tracks") if REF else None
 
 
 @pytest.fixture(scope="module")
@@ -50,42 +54,58 @@ def test_oracle_traces_match_golden(name, traces_gold):
         assert same_bits(arr, traces_gold[key]).all(), key
 
 
-@pytest.mark.skipif(not have_ref(), reason="oracle/_ref not built (needs /root/reference)")
+@pytest.fixture(scope="module")
+def live_gold():
+    return np.load(os.path.join(GOLD, "traces_live.npz"))
+
+
+@pytest.mark.parametrize("name", list(mg.LIVE_SCENARIOS))
+def test_oracle_live_scenarios_match_golden(name, live_gold):
+    """the live comparisons below, against their stored result (tests/golden/traces_live.npz): every buffer, bit-exact"""
+    cps = mg.golden_checkpoints(name)
+    got = mg.run_live_scenario("port", name, cps)
+    assert len(got) == len(cps) * len(BUF) + 1
+    for key, arr in got.items():
+        assert same_bits(arr, live_gold[key]).all(), key
+    if name.startswith("offset"):
+        assert got[f"{name}/crashed_seen"][0], "nobody crashed: the changed threshold was never exercised"
+
+
+def _live_pair(name):
+    """LIVE_SCENARIOS[name] through the restatement and through the reference's objects: every buffer at every
+    checkpoint, bit-exact"""
+    a, b = mg.run_live_scenario("port", name), mg.run_live_scenario("reference", name)
+    assert a.keys() == b.keys()
+    for key in a:
+        assert same_bits(a[key], b[key]).all(), key
+    return a
+
+
+@pytest.mark.skipif(not have_ref(), reason="oracle/_ref not built (needs the original project's sources: OPENKITCHEN_REF)")
 @pytest.mark.parametrize("mode,reward", [(0, 1), (0, 2), (1, 7), (1, 5), (0, 4), (0, 3), (1, 6)])
 def test_oracle_vs_reference_objects_live(mode, reward):
-    names = ["Monza", "Zandvoort", "Spa"]
-    pair = []
-    for kind in ("port", "reference"):
-        o = Oracle(kind, movement_mode=mode, reward_mode=reward, auto_reset=1)
-        for nm in names:
-            o.add_track(ok.track_columns(nm))
-        tid = (np.arange(60) % 3).astype(np.int32)
-        o.alloc_agents(60, ok.ray_fan(15), tid)
-        pair.append(o)
-    a, b = pair
-    rng = np.random.default_rng(7)
-    idx = np.arange(60, dtype=np.int64)
-    pts = np.array([rng.integers(0, a.track_points(int(i % 3))) for i in idx], dtype=np.int32)
-    alpha = (rng.integers(10, 91, size=60) / np.float32(100)).astype(np.float32)
-    hoff = rng.integers(-90, 91, size=60).astype(np.float32)
-    for o in pair:
-        o.reset(idx, pts, alpha, hoff)
-    for step in range(150):
-        for o in pair:
-            o.fill_random_actions(step)
-            o.step()
-        if step % 25 == 0 or step == 149:
-            for name in BUF:
-                assert same_bits(a.buffer(name), b.buffer(name)).all(), (step, name)
+    _live_pair(f"live_m{mode}_r{reward}")  # Monza, Zandvoort, Spa; 60 agents, drawn reset points and offsets
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/tracks"), reason="reference CSVs not present")
+def test_track_csv_writer_round_trips_the_pack(tmp_path):
+    """write_track_csv re-emits every packed track so that strtof reads back the very same columns"""
+    o = Oracle("port")
+    for nm in ok.track_names():
+        t_pack = o.add_track(ok.track_columns(nm))
+        p = tmp_path / f"{nm}.csv"
+        ok.write_track_csv(nm, str(p))
+        t_rt = o.load_track_csv(str(p))
+        for a in ("x", "y", "w_right", "w_left", "segments"):
+            assert same_bits(o.track_array(t_pack, a), o.track_array(t_rt, a)).all(), (nm, a)
+
+
+@pytest.mark.skipif(not (REF_TRACKS and os.path.isdir(REF_TRACKS)), reason="the original project's track CSVs are not present (OPENKITCHEN_REF)")
 def test_track_pack_matches_reference_csvs(tmp_path):
     """the packed columns are exactly what strtof parses out of the reference's CSV files, and the
     CSV writer round-trips them"""
     o = Oracle("port")
     for nm in ok.track_names():
-        t_csv = o.load_track_csv(f"/root/reference/tracks/{nm}.csv")
+        t_csv = o.load_track_csv(os.path.join(REF_TRACKS, f"{nm}.csv"))
         t_pack = o.add_track(ok.track_columns(nm))
         p = tmp_path / f"{nm}.csv"
         ok.write_track_csv(nm, str(p))
@@ -96,7 +116,7 @@ def test_track_pack_matches_reference_csvs(tmp_path):
             assert same_bits(ref, o.track_array(t_rt, a)).all(), (nm, a)
 
 
-@pytest.mark.skipif(not have_ref(), reason="oracle/_ref not built (needs /root/reference)")
+@pytest.mark.skipif(not have_ref(), reason="oracle/_ref not built (needs the original project's sources: OPENKITCHEN_REF)")
 @pytest.mark.parametrize("mode", [0, 1])
 @pytest.mark.parametrize("offset", [3.0, -5.0])
 def test_oracle_vs_reference_objects_with_a_sensor_offset(mode, offset):
@@ -105,29 +125,5 @@ def test_oracle_vs_reference_objects_with_a_sensor_offset(mode, offset):
     and the standstill window are compile-time constants there: Agent.h:10-12, Environment.h:19-20) -- in the C restatement
     against the reference's own objects.  The GPU tests compare the CUDA path with the restatement on the same settings
     (tests/test_gpu_parity_gaps.py): this closes the chain CUDA == restatement == reference for them."""
-    names = ["Monza", "Sepang"]
-    cfg = dict(movement_mode=mode, reward_mode=1, auto_reset=1, sensor_offset=offset, collision_dist2=3.5)
-    pair = []
-    for kind in ("port", "reference"):
-        o = Oracle(kind, **cfg)
-        for nm in names:
-            o.add_track(ok.track_columns(nm))
-        o.alloc_agents(48, ok.ray_fan(9), (np.arange(48) % 2).astype(np.int32))
-        pair.append(o)
-    a, b = pair
-    rng = np.random.default_rng(11)
-    idx = np.arange(48, dtype=np.int64)
-    pts = np.array([rng.integers(0, a.track_points(int(i % 2))) for i in idx], dtype=np.int32)
-    for o in pair:
-        o.reset(idx, pts, None, None)
-    crashed_seen = False
-    ticks = 120 if mode == 0 else 400  # the acceleration mode's action set builds speed slowly
-    for step in range(ticks):
-        for o in pair:
-            o.fill_random_actions(step)
-            o.step()
-        if step % 20 == 0 or step == ticks - 1:
-            for name in BUF:
-                assert same_bits(a.buffer(name), b.buffer(name)).all(), (step, name)
-        crashed_seen = crashed_seen or bool(a.buffer("crashed").any())
-    assert crashed_seen, "nobody crashed: the changed threshold was never exercised"
+    name = f"offset_m{mode}_{offset:+g}"
+    assert _live_pair(name)[f"{name}/crashed_seen"][0], "nobody crashed: the changed threshold was never exercised"

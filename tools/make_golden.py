@@ -4,11 +4,20 @@ oracle/_ref/libokref.so = the unmodified reference Agent.cpp + RaceTrack.cpp dri
 oracle/ref_harness.cpp (see oracle/Makefile).  The reference ships no tests or fixtures of its own
 (SURVEY.md section 4), so these are the pins for the oracle and, through it, for the CUDA path.
 
-    python tools/make_golden.py            # needs /root/reference (build with `make -C oracle`)
+    OPENKITCHEN_REF=<checkout> make -C oracle && python tools/make_golden.py            # all three files
+    python tools/make_golden.py --live-from-port                                       # traces_live.npz only
 
 Contents
-  tracks.npz   per track: CRC32 of every RaceTrack / TrackSegments array + first/last rows
-  traces.npz   per scenario: full state + lidar buffers at a few checkpoints of a scripted rollout
+  tracks.npz        per track: CRC32 of every RaceTrack / TrackSegments array + first/last rows
+  traces.npz        per scenario: full state + lidar buffers at a few checkpoints of a scripted rollout
+  traces_live.npz   the same for LIVE_SCENARIOS: the reset draws, reward modes, sensor offsets and crash threshold of
+                    the live comparisons in tests/test_oracle_golden.py
+
+`--live-from-port` mints traces_live.npz from the C restatement (oracle/ok_oracle.c) instead of the reference's objects.
+It gives the same bits only while the restatement is unchanged since the live comparisons last passed against those
+objects on exactly these scenarios.  The committed traces_live.npz was minted that way from oracle/ok_oracle.c as of
+commit 07333d5, the version the live comparisons were run against the reference's objects with (the sensor-offset one
+was added after it, in 2d0850c); the file has not changed since.
 """
 import os
 import sys
@@ -39,6 +48,67 @@ SCENARIOS = {
 }
 
 
+# The live comparisons of tests/test_oracle_golden.py (restatement vs the reference's objects), as scenarios.
+# name: (tracks, n_agents, rays, config, ticks, checkpoints, seed of the reset draws, whether the lane offset and heading
+# offset are drawn too).  Agents are dealt round-robin over the tracks.
+LIVE_SCENARIOS = {}
+for _mode, _reward in [(0, 1), (0, 2), (1, 7), (1, 5), (0, 4), (0, 3), (1, 6)]:
+    LIVE_SCENARIOS[f"live_m{_mode}_r{_reward}"] = (
+        ["Monza", "Zandvoort", "Spa"], 60, 15, dict(movement_mode=_mode, reward_mode=_reward, auto_reset=1), 150,
+        [s for s in range(150) if s % 25 == 0 or s == 149], 7, True)
+for _mode in (0, 1):
+    for _offset in (3.0, -5.0):
+        _ticks = 120 if _mode == 0 else 400  # the acceleration mode's action set builds speed slowly
+        LIVE_SCENARIOS[f"offset_m{_mode}_{_offset:+g}"] = (
+            ["Monza", "Sepang"], 48, 9, dict(movement_mode=_mode, reward_mode=1, auto_reset=1, sensor_offset=_offset,
+                                             collision_dist2=3.5), _ticks,
+            [s for s in range(_ticks) if s % 20 == 0 or s == _ticks - 1], 11, False)
+
+
+def live_inputs(name):
+    """(tracks, n, fan, config, ticks, checkpoints, track ids, agent ids, reset points, lane offsets, heading offsets)"""
+    tracks, n, rays, cfg, ticks, cps, seed, offsets = LIVE_SCENARIOS[name]
+    tid = (np.arange(n) % len(tracks)).astype(np.int32)
+    pts_per = [len(ok.track_columns(t)[0]) for t in tracks]
+    rng = np.random.default_rng(seed)
+    idx = np.arange(n, dtype=np.int64)
+    pts = np.array([rng.integers(0, pts_per[t]) for t in tid], dtype=np.int32)
+    alpha = hoff = None
+    if offsets:
+        alpha = (rng.integers(10, 91, size=n) / np.float32(100)).astype(np.float32)
+        hoff = rng.integers(-90, 91, size=n).astype(np.float32)
+    return tracks, n, fan_of(rays), cfg, ticks, cps, tid, idx, pts, alpha, hoff
+
+
+def golden_checkpoints(name):
+    """the checkpoints traces_live.npz keeps (three per scenario, to stay under 1 MB): the second, the middle, the last"""
+    cps = LIVE_SCENARIOS[name][5]
+    return [cps[1], cps[len(cps) // 2], cps[-1]]
+
+
+def run_live_scenario(kind, name, checkpoints=None):
+    """LIVE_SCENARIOS[name] through the oracle `kind`: {"name/tick/buffer": array} at every checkpoint (or at
+    `checkpoints`), and "name/crashed_seen": whether any agent crashed on any tick"""
+    tracks, n, fan, cfg, ticks, cps, tid, idx, pts, alpha, hoff = live_inputs(name)
+    cps = cps if checkpoints is None else checkpoints
+    o = Oracle(kind, **cfg)
+    for t in tracks:
+        o.add_track(ok.track_columns(t))
+    o.alloc_agents(n, fan, tid)
+    o.reset(idx, pts, alpha, hoff)
+    out, crashed_seen = {}, False
+    for s in range(ticks):
+        o.fill_random_actions(s)
+        o.step()
+        crashed_seen = crashed_seen or bool(o.buffer("crashed").any())
+        if s in cps:
+            for b in BUF:
+                out[f"{name}/{s}/{b}"] = o.buffer(b).copy()
+    out[f"{name}/crashed_seen"] = np.array([crashed_seen])
+    o.close()
+    return out
+
+
 def fan_of(spec):
     return ok.ray_fan(spec) if np.isscalar(spec) else np.asarray(spec, dtype=np.float32)
 
@@ -63,7 +133,19 @@ def run_scenario(kind, name):
     return out
 
 
+def save(name, arrays):
+    path = os.path.join(ROOT, "tests", "golden", name)
+    np.savez_compressed(path, **arrays)
+    print(name, os.path.getsize(path), "bytes")
+
+
 def main():
+    live = {}
+    if "--live-from-port" in sys.argv[1:]:
+        for name in LIVE_SCENARIOS:
+            live.update(run_live_scenario("port", name, golden_checkpoints(name)))
+        save("traces_live.npz", live)
+        return
     ref = Oracle("reference")
     tr = {}
     for nm in ok.track_names():
@@ -74,14 +156,14 @@ def main():
             tr[f"{nm}/{a}/shape"] = np.array(arr.shape, dtype=np.int32)
             tr[f"{nm}/{a}/head"] = arr.reshape(arr.shape[0], -1)[:2].copy()
             tr[f"{nm}/{a}/tail"] = arr.reshape(arr.shape[0], -1)[-2:].copy()
-    os.makedirs(os.path.join(ROOT, "tests", "golden"), exist_ok=True)
-    np.savez_compressed(os.path.join(ROOT, "tests", "golden", "tracks.npz"), **tr)
+    save("tracks.npz", tr)
     traces = {}
     for name in SCENARIOS:
         traces.update(run_scenario("reference", name))
-    np.savez_compressed(os.path.join(ROOT, "tests", "golden", "traces.npz"), **traces)
-    for f in ("tracks.npz", "traces.npz"):
-        print(f, os.path.getsize(os.path.join(ROOT, "tests", "golden", f)), "bytes")
+    save("traces.npz", traces)
+    for name in LIVE_SCENARIOS:
+        live.update(run_live_scenario("reference", name, golden_checkpoints(name)))
+    save("traces_live.npz", live)
 
 
 if __name__ == "__main__":

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Mints tests/golden/cmaes_ref.npz from the reference's OWN CMA-ES solver and controller
 (oracle/_ref/libcmaes_ref.so = CmaEsSolverTorch.cpp + Controller.cpp compiled unchanged, oracle/Makefile).
-Run in the build container (needs /root/reference to have been compiled): python tools/make_golden_cmaes.py"""
+Needs a checkout of the original project:  OPENKITCHEN_REF=<checkout> make -C oracle && python tools/make_golden_cmaes.py"""
 import os
 import sys
 

@@ -1,13 +1,13 @@
 #!/usr/bin/env python
 """Pack the 23 TUMFTM racetrack-database centre lines the reference ships (tracks/*.csv) into one
-binary file so that the benchmark / tests have BASELINE.json's tracks on the GPU box, where
-/root/reference does not exist.
+binary file so that the benchmark / tests have BASELINE.json's tracks without a checkout of the
+original project.
 
 The pack stores the four raw CSV columns (x_m, y_m, w_tr_right_m, w_tr_left_m) as binary32 exactly
 as std::stof (strtof) parses them -- the parse goes through the oracle's strtof-based loader's
 twin below and is cross-checked against it in tests/test_tracks.py when the CSVs are present.
 
-Usage:  python tools/make_track_pack.py [/root/reference/tracks] [openkitchen_b200/data/tracks_f32.npz]
+Usage:  python tools/make_track_pack.py [$OPENKITCHEN_REF/tracks] [openkitchen_b200/data/tracks_f32.npz]
 """
 import ctypes
 import glob
@@ -35,7 +35,7 @@ def parse_csv(path):
 
 
 def main():
-    src = sys.argv[1] if len(sys.argv) > 1 else "/root/reference/tracks"
+    src = sys.argv[1] if len(sys.argv) > 1 else os.path.join(os.environ.get("OPENKITCHEN_REF", "."), "tracks")
     dst = sys.argv[2] if len(sys.argv) > 2 else os.path.join(os.path.dirname(__file__), "..", "openkitchen_b200", "data", "tracks_f32.npz")
     out = {}
     names = []
