@@ -1,5 +1,5 @@
 // ok_capi.cu -- implementation of the C ABI (include/openkitchen_b200.h) over the sm_100a kernels.
-// Host side of the product: owns device memory, builds the tile table, launches.  No CPU
+// Host side of the product: owns device memory, uploads the tilings (ok_schedule.hpp), launches.  No CPU
 // fallback exists: without a CUDA device every compute entry point returns OK_ERR_NO_DEVICE.
 #include "../../include/openkitchen_b200.h"
 
@@ -20,6 +20,7 @@
 #include <map>
 #include <sys/stat.h>
 #include <thread>
+#include <type_traits>
 #include <unistd.h>
 #include <memory>
 #include <mutex>
@@ -146,6 +147,110 @@ struct DeviceBlob
     }
 };
 
+namespace
+{
+// owners of the CUDA resources of an env: freed (destroyed) when the owner is reset or goes away
+struct CudaFree
+{
+    void operator()(void *p) const
+    {
+        cudaFree(p);
+    }
+};
+template <typename T> using DevPtr = std::unique_ptr<T, CudaFree>;
+struct StreamDestroy
+{
+    void operator()(cudaStream_t s) const
+    {
+        cudaStreamDestroy(s);
+    }
+};
+using Stream = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, StreamDestroy>;
+struct EventDestroy
+{
+    void operator()(cudaEvent_t ev) const
+    {
+        cudaEventDestroy(ev);
+    }
+};
+using Event = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, EventDestroy>;
+
+// replaces what `p` holds by `count` uninitialised elements of device memory (the old block is freed first)
+template <typename T> cudaError_t dev_alloc(DevPtr<T> &p, size_t count)
+{
+    p.reset();
+    T *raw = nullptr;
+    const cudaError_t rc = cudaMalloc(&raw, sizeof(T) * count);
+    p.reset(raw);
+    return rc;
+}
+
+cudaError_t make_stream(Stream &s)
+{
+    cudaStream_t raw = nullptr;
+    const cudaError_t rc = cudaStreamCreateWithFlags(&raw, cudaStreamNonBlocking);
+    s.reset(raw);
+    return rc;
+}
+
+cudaError_t make_event(Event &ev)
+{
+    cudaEvent_t raw = nullptr;
+    const cudaError_t rc = cudaEventCreateWithFlags(&raw, cudaEventDisableTiming);
+    ev.reset(raw);
+    return rc;
+}
+
+// a tiling in device memory: the table the kernel reads, its length, and the grid that runs it
+struct Schedule
+{
+    DevPtr<ok::Tile> d;
+    int32_t          n{0}, grid{0};
+};
+
+// cost feedback for the beam tiling (ok_balance_schedule): the kernel leaves every tile's ray-phase / other time in
+// d_tile_ns, and reweigh_runs re-cuts the tiles from them.  The table is allocated once, at `capacity` tiles, and
+// rewritten in place: a CUDA graph captured earlier keeps reading it.
+struct BeamFeedback
+{
+    std::vector<ok::TileRun> runs;
+    std::vector<ok::Tile>    tiles; // host copy of the beam schedule's table
+    bool                     weighted{false};
+    int32_t                  target{0}, capacity{0};
+    DevPtr<uint32_t>         d_tile_ns;
+    uint64_t                 launches{0};
+};
+
+// everything ok_alloc_agents creates for one population: ok_alloc_agents and free_agents replace it as a whole
+struct Agents
+{
+    DevPtr<uint8_t>  slab;
+    DevPtr<float>    ray_deg;
+    DevPtr<uint16_t> ray_order;
+    DevPtr<int32_t>  sched;
+    Schedule         tiles; // the grid-walk kernel's tiling
+    // the beam kernel's batches are not limited by per-ray scratch: its own batch size, tiling and grid
+    Schedule     beam;
+    BeamFeedback feedback;
+    DevPtr<ok::FirstTile> first_beam; // the first tile of every CTA with its track record (ok_kernels.cuh)
+    int32_t               first_capacity{0};
+    bool                  first_dirty{true};
+    // ok_step_host's tiling: several tiles per CTA, so that a tile's observations cross PCIe while the next one is computed
+    Schedule e2e;
+    Schedule q16; // ok_step_host_q16's tiling: half the bytes per tile, fewer and larger tiles pay
+    // ... with flusher CTAs (obs_flush_kernel) on SMs of their own
+    DevPtr<uint32_t> tile_flag;
+    // ok_step_host: device stage of the caller's two mapped action arrays, filled by the copy engine on act_stream next to
+    // the running kernel, + the word the stream sets to this launch's target when both copies have landed
+    DevPtr<float>    act_stage;
+    DevPtr<uint32_t> act_ready;
+    uint32_t         act_ready_target{0};
+    DevPtr<unsigned long long> stats; // ok_debug_stats: allocated on first use
+    DevPtr<unsigned long long> trace; // ok_debug_trace
+    int32_t                    trace_tiles{0};
+};
+} // namespace
+
 struct OkEnv
 {
     OkConfig               cfg{};
@@ -154,8 +259,8 @@ struct OkEnv
     size_t                 max_blob{0};
     std::vector<ok::Track> tracks;
     // device track arena
-    uint8_t      *d_arena{nullptr};
-    ok::TrackRef *d_track_refs{nullptr};
+    DevPtr<uint8_t>      d_arena;
+    DevPtr<ok::TrackRef> d_track_refs;
     size_t        arena_bytes{0};
     size_t        max_blob_used{0};
     bool          arena_dirty{true};
@@ -163,80 +268,36 @@ struct OkEnv
     std::vector<std::shared_ptr<const std::vector<uint8_t>>> beams;     // host copies (host-only envs, ok_beam_lookup)
     std::vector<std::shared_ptr<const struct DeviceBlob>>    beams_dev; // what the kernels read; shared between envs
     bool          arena_has_beams{false};
+    std::vector<ok::TrackRef> h_track_refs; // host copy of d_track_refs
     // agents
     int64_t              n_agents{0};
     int32_t              rays{0};
-    uint8_t             *d_slab{nullptr};
+    Agents               ag;
     void                *d_buf[OK_BUF_COUNT]{};
     size_t               buf_off[OK_BUF_COUNT]{}; // offsets of the buffers inside the slab
-    float               *d_ray_deg{nullptr};
-    ok::Tile            *d_tiles{nullptr};
-    int32_t              n_tiles{0};
     int32_t              batch_agents{0};
-    // the beam kernel's batches are not limited by per-ray scratch: its own batch size, tile table and grid
-    ok::Tile            *d_tiles_beam{nullptr};
-    int32_t              n_tiles_beam{0};
-    // cost feedback for the beam tiling (ok_balance_schedule): the kernel leaves every tile's ray-phase / other time here
-    struct TileRun
-    {
-        int32_t track;
-        int64_t begin, len, cap; // cap: most agents a tile of this run may hold
-        double  w;               // measured cost per agent (ns in the ray phase), 1 before any measurement
-        int64_t k;               // tiles
-    };
-    std::vector<TileRun>  beam_runs;
-    std::vector<ok::Tile> h_tiles_beam;
-    bool                  beam_launches_weighted{false};
-    int32_t               tiles_beam_target{0}, tiles_beam_capacity{0};
-    uint32_t             *d_tile_ns{nullptr};
-    std::vector<ok::TrackRef> h_track_refs;     // host copy of d_track_refs
-    ok::FirstTile            *d_first_beam{nullptr}; // the first tile of every CTA with its track record (ok_kernels.cuh)
-    int32_t                   first_capacity{0};
-    bool                      first_dirty{true};
-    uint64_t              beam_launches{0};
-    int                   auto_balance{1};
-    float                 balance_before{0.0f}, balance_after{0.0f}; // predicted slowest-tile / mean-tile cost of the last rebalancing
-    // ok_step_host's tiling: several tiles per CTA, so that a tile's observations cross PCIe while the next one is computed
-    ok::Tile            *d_tiles_e2e{nullptr};
-    int32_t              n_tiles_e2e{0}, grid_e2e{0};
-    ok::Tile            *d_tiles_q16{nullptr}; // ok_step_host_q16's tiling: half the bytes per tile, fewer and larger tiles pay
-    int32_t              n_tiles_q16{0}, grid_q16{0};
-    // ... with flusher CTAs (obs_flush_kernel) on SMs of their own: flags, epoch, the side stream and its fork / join events
+    int                  auto_balance{1};
+    float                balance_before{0.0f}, balance_after{0.0f}; // predicted slowest-tile / mean-tile cost of the last rebalancing
     int32_t              e2e_flushers{0};
-    uint32_t            *d_tile_flag{nullptr};
     uint32_t             flag_epoch{0};
-    // ok_step_host: device stage of the caller's two mapped action arrays, filled by the copy engine on act_stream next to
-    // the running kernel, + the word the stream sets to this launch's target when both copies have landed
-    float               *d_act_stage{nullptr};
-    uint32_t            *d_act_ready{nullptr};
-    uint32_t             act_ready_target{0};
-    cudaStream_t         act_stream{nullptr};
-    cudaEvent_t          ev_act{nullptr};
     bool                 act_stage_on{true}; // OK_ACT_STAGE=0: every tile reads the mapping (A/B)
     int                  actor_dyn_max{0};   // dynamic shared memory the fused actor + step kernel may use
-    unsigned long long  *d_counters{nullptr}; // ok_population_counters
-    cudaStream_t         flush_stream{nullptr};
-    cudaEvent_t          ev_fork{nullptr}, ev_join{nullptr};
     int32_t              batch_agents_beam{0};
-    int32_t              grid_beam{0};
     int32_t              ctas_per_sm_beam{1};
     bool                 beam_staged{true}; // which shape of the beam kernel this population runs (ok_kernels.cuh)
-    bool                 beam_seg{false};   // ... the segment-staged one (two CTAs per SM); implies beam_staged
-    int                  smem_per_sm{0}, smem_reserved{1024};
     int32_t              beam_block{1024};
-    uint16_t            *d_ray_order{nullptr};
-    int32_t             *d_sched{nullptr};
-    unsigned long long  *d_stats{nullptr}; // ok_debug_stats: allocated on first use
-    unsigned long long  *d_trace{nullptr}; // ok_debug_trace
-    int32_t              trace_tiles{0};
     int                  smem_optin{0};
     std::vector<int32_t> h_track_id;
-    // staging for the *_host entry points
-    uint8_t *d_stage{nullptr};
-    size_t   stage_bytes{0};
+    // created on first use, kept until ok_destroy
+    DevPtr<uint8_t>            d_stage; // staging for the *_host entry points
+    size_t                     stage_bytes{0};
+    DevPtr<unsigned long long> d_counters; // ok_population_counters
+    Stream                     act_stream; // ok_step_host's action copies
+    Event                      ev_act;
+    Stream                     flush_stream; // the flusher CTAs' side stream and its fork / join events
+    Event                      ev_fork, ev_join;
     // stats
     uint64_t launches{0};
-    int32_t  grid{0};
     size_t   smem{0}, smem_beam{0};
 };
 
@@ -255,47 +316,10 @@ size_t buffer_bytes(const OkEnv *e, int which)
 
 void free_agents(OkEnv *e)
 {
-    if (e->d_slab)
-        cudaFree(e->d_slab);
-    if (e->d_ray_deg)
-        cudaFree(e->d_ray_deg);
-    if (e->d_tiles)
-        cudaFree(e->d_tiles);
-    if (e->d_tiles_beam)
-        cudaFree(e->d_tiles_beam);
-    if (e->d_tiles_e2e)
-        cudaFree(e->d_tiles_e2e);
-    if (e->d_tiles_q16)
-        cudaFree(e->d_tiles_q16);
-    e->d_tiles_q16 = nullptr, e->n_tiles_q16 = 0;
-    if (e->d_tile_flag)
-        cudaFree(e->d_tile_flag);
-    e->d_tile_flag = nullptr;
-    if (e->d_act_stage)
-        cudaFree(e->d_act_stage);
-    if (e->d_act_ready)
-        cudaFree(e->d_act_ready);
-    e->d_act_stage = nullptr, e->d_act_ready = nullptr, e->act_ready_target = 0;
-    e->d_tiles_beam = nullptr, e->n_tiles_beam = 0, e->d_tiles_e2e = nullptr, e->n_tiles_e2e = 0;
-    if (e->d_tile_ns)
-        cudaFree(e->d_tile_ns);
-    if (e->d_first_beam)
-        cudaFree(e->d_first_beam);
-    e->d_first_beam = nullptr, e->first_capacity = 0, e->first_dirty = true;
-    e->d_tile_ns = nullptr, e->beam_launches = 0, e->beam_launches_weighted = false, e->beam_runs.clear(), e->h_tiles_beam.clear();
-    if (e->d_ray_order)
-        cudaFree(e->d_ray_order);
-    if (e->d_sched)
-        cudaFree(e->d_sched);
-    if (e->d_stats)
-        cudaFree(e->d_stats);
-    if (e->d_trace)
-        cudaFree(e->d_trace);
-    e->d_stats = nullptr, e->d_trace = nullptr, e->trace_tiles = 0;
-    e->d_slab = nullptr, e->d_ray_deg = nullptr, e->d_tiles = nullptr, e->d_ray_order = nullptr, e->d_sched = nullptr;
+    e->ag = Agents{};
     for (auto &b : e->d_buf)
         b = nullptr;
-    e->n_agents = 0, e->rays = 0, e->n_tiles = 0;
+    e->n_agents = 0, e->rays = 0;
 }
 
 // Beam tables are pure functions of (segments, cell, bins, range) and take ~0.1-1 s of host time per track.
@@ -545,11 +569,7 @@ int ensure_arena(OkEnv *e)
     const bool want_beams = e->cfg.raycast_mode == OK_RAYCAST_BEAM;
     if (!e->arena_dirty && (!want_beams || e->arena_has_beams))
         return OK_SUCCESS;
-    if (e->d_arena)
-        cudaFree(e->d_arena);
-    if (e->d_track_refs)
-        cudaFree(e->d_track_refs);
-    e->d_arena = nullptr, e->d_track_refs = nullptr;
+    e->d_arena.reset(), e->d_track_refs.reset();
     std::vector<ok::TrackRef> refs;
     size_t                    total = 0;
     e->max_blob_used                = 0;
@@ -629,12 +649,12 @@ int ensure_arena(OkEnv *e)
     std::vector<uint8_t> host(total, 0);
     for (size_t i = 0; i < e->tracks.size(); ++i)
         std::memcpy(host.data() + refs[i].offset, e->tracks[i].blob.data(), e->tracks[i].blob.size());
-    OK_CUDA(cudaMalloc(&e->d_arena, std::max<size_t>(total, 128)));
-    OK_CUDA(cudaMalloc(&e->d_track_refs, sizeof(ok::TrackRef) * std::max<size_t>(refs.size(), 1)));
-    OK_CUDA(cudaMemcpy(e->d_arena, host.data(), total, cudaMemcpyHostToDevice));
-    OK_CUDA(cudaMemcpy(e->d_track_refs, refs.data(), sizeof(ok::TrackRef) * refs.size(), cudaMemcpyHostToDevice));
-    e->h_track_refs = refs;
-    e->first_dirty  = true;
+    OK_CUDA(dev_alloc(e->d_arena, std::max<size_t>(total, 128)));
+    OK_CUDA(dev_alloc(e->d_track_refs, std::max<size_t>(refs.size(), 1)));
+    OK_CUDA(cudaMemcpy(e->d_arena.get(), host.data(), total, cudaMemcpyHostToDevice));
+    OK_CUDA(cudaMemcpy(e->d_track_refs.get(), refs.data(), sizeof(ok::TrackRef) * refs.size(), cudaMemcpyHostToDevice));
+    e->h_track_refs   = refs;
+    e->ag.first_dirty = true;
     e->arena_bytes = total;
     e->arena_dirty = false;
     return OK_SUCCESS;
@@ -670,20 +690,20 @@ ok::StepParams base_params(OkEnv *e)
     p.reset_pt  = static_cast<int32_t *>(e->d_buf[OK_BUF_RESET_PT]);
     p.start_x   = static_cast<float *>(e->d_buf[OK_BUF_START_X]);
     p.start_y   = static_cast<float *>(e->d_buf[OK_BUF_START_Y]);
-    p.ray_deg   = e->d_ray_deg;
-    p.arena     = e->d_arena;
-    p.tracks    = e->d_track_refs;
-    p.tiles     = e->d_tiles;
-    p.n_tiles   = e->n_tiles;
+    p.ray_deg   = e->ag.ray_deg.get();
+    p.arena     = e->d_arena.get();
+    p.tracks    = e->d_track_refs.get();
+    p.tiles     = e->ag.tiles.d.get();
+    p.n_tiles   = e->ag.tiles.n;
     p.n_agents  = e->n_agents;
     p.rays      = e->rays;
     p.batch_agents      = e->batch_agents;
     p.smem_blob_bytes   = static_cast<uint32_t>((e->max_blob_used + 127) / 128 * 128);
-    p.ray_order         = e->d_ray_order;
-    p.sched             = e->d_sched;
-    p.stats             = e->d_stats;
-    p.trace             = e->d_trace;
-    p.trace_tiles       = e->trace_tiles;
+    p.ray_order         = e->ag.ray_order.get();
+    p.sched             = e->ag.sched.get();
+    p.stats             = e->ag.stats.get();
+    p.trace             = e->ag.trace.get();
+    p.trace_tiles       = e->ag.trace_tiles;
     p.movement_mode     = e->cfg.movement_mode;
     p.reward_mode       = e->cfg.reward_mode;
     p.raycast_mode      = e->cfg.raycast_mode;
@@ -721,151 +741,73 @@ int arm_shared_memory_limit(OkEnv *e)
     OK_CUDA(cudaFuncGetAttributes(&fa, ok::step_kernel<ok::kBeamBlockStaged, true, true>));
     OK_CUDA(cudaFuncSetAttribute(ok::step_kernel<ok::kBeamBlockStaged, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  e->smem_optin - static_cast<int>(fa.sharedSizeBytes)));
-    OK_CUDA(ok::arm_step_segstaged(e->smem_optin));
     OK_CUDA(ok::arm_step_actor(e->smem_optin, &e->actor_dyn_max));
     return OK_SUCCESS;
 }
 
-// Cost-aware balanced tiling.  A tile of `count` agents of run r costs about c0 + w_r * count (c0: the thread-per-agent
-// phases and barriers, whatever the size; w_r: the ray phase, which differs from track to track by up to 15 %).  Tiles go
-// to the runs greedily -- one more for the run whose tiles are the most expensive -- which minimises the slowest tile;
-// every run is cut into equal parts, most expensive first (CTAs take tiles in list order).  With w = 1, c0 = 0 this is the
-// plain balanced tiling by agent count.
-std::vector<ok::Tile> cost_balanced_tiles(std::vector<OkEnv::TileRun> &runs, int64_t target, double c0, float *slowest_over_mean)
+// Uploads `tiles` as schedule `s`, in a table of room for `capacity` tiles (at least as many as there are), run by
+// `ctas` CTAs at most.
+int upload_schedule(Schedule &s, const std::vector<ok::Tile> &tiles, size_t capacity, int ctas)
 {
-    int64_t have = 0;
-    for (auto &r : runs)
-    {
-        r.k = std::max<int64_t>(1, (r.len + r.cap - 1) / r.cap);
-        have += r.k;
-    }
-    auto cost = [&](const OkEnv::TileRun &r) { return c0 + r.w * static_cast<double>((r.len + r.k - 1) / r.k); };
-    for (; have < target; ++have)
-    {
-        OkEnv::TileRun *best = nullptr;
-        for (auto &r : runs)
-            if (r.len > r.k && (!best || cost(r) > cost(*best)))
-                best = &r;
-        if (!best)
-            break;
-        best->k++;
-    }
-    struct Costed
-    {
-        ok::Tile t;
-        double   c;
-    };
-    std::vector<Costed> tiles;
-    double              sum = 0.0, worst = 0.0;
-    for (const auto &r : runs)
-        for (int64_t t = 0; t < r.k; ++t)
-        {
-            const int64_t b0 = r.begin + r.len * t / r.k, b1 = r.begin + r.len * (t + 1) / r.k;
-            if (b1 > b0)
-            {
-                const double c = c0 + r.w * static_cast<double>(b1 - b0);
-                tiles.push_back({{r.track, static_cast<int32_t>(b1 - b0), b0}, c});
-                sum += c, worst = std::max(worst, c);
-            }
-        }
-    std::stable_sort(tiles.begin(), tiles.end(), [](const Costed &a, const Costed &b) { return a.c > b.c; });
-    if (slowest_over_mean)
-        *slowest_over_mean = tiles.empty() ? 1.0f : static_cast<float>(worst * static_cast<double>(tiles.size()) / sum);
-    std::vector<ok::Tile> out;
-    out.reserve(tiles.size());
-    for (const auto &t : tiles)
-        out.push_back(t.t);
-    return out;
+    OK_CUDA(dev_alloc(s.d, std::max(capacity, tiles.size())));
+    OK_CUDA(cudaMemcpy(s.d.get(), tiles.data(), sizeof(ok::Tile) * tiles.size(), cudaMemcpyHostToDevice));
+    s.n    = static_cast<int32_t>(tiles.size());
+    s.grid = std::max(1, std::min(ctas, s.n));
+    return OK_SUCCESS;
 }
 
 // The CTAs' first tiles with their track records side by side (ok::FirstTile), rebuilt whenever the tiling or the arena
 // changes.  Synchronises `s`: a launch in flight may still read the old records.
 int upload_first_tiles(OkEnv *e, cudaStream_t s)
 {
-    const int32_t nf = std::min<int32_t>(e->grid_beam, static_cast<int32_t>(e->h_tiles_beam.size()));
+    Agents       &ag = e->ag;
+    const int32_t nf = std::min<int32_t>(ag.beam.grid, static_cast<int32_t>(ag.feedback.tiles.size()));
     if (nf <= 0 || e->h_track_refs.empty())
         return OK_SUCCESS;
     OK_CUDA(cudaStreamSynchronize(s));
-    if (nf > e->first_capacity)
+    if (nf > ag.first_capacity)
     {
-        if (e->d_first_beam)
-            cudaFree(e->d_first_beam);
-        e->d_first_beam = nullptr, e->first_capacity = 0;
-        OK_CUDA(cudaMalloc(&e->d_first_beam, sizeof(ok::FirstTile) * static_cast<size_t>(nf)));
-        e->first_capacity = nf;
+        ag.first_capacity = 0;
+        OK_CUDA(dev_alloc(ag.first_beam, static_cast<size_t>(nf)));
+        ag.first_capacity = nf;
     }
     std::vector<ok::FirstTile> first(static_cast<size_t>(nf));
     for (int32_t i = 0; i < nf; ++i)
     {
-        first[i].tile = e->h_tiles_beam[i];
-        first[i].ref  = e->h_track_refs[e->h_tiles_beam[i].track];
+        first[i].tile = ag.feedback.tiles[i];
+        first[i].ref  = e->h_track_refs[ag.feedback.tiles[i].track];
         std::memset(first[i].pad, 0, sizeof first[i].pad);
     }
-    OK_CUDA(cudaMemcpy(e->d_first_beam, first.data(), sizeof(ok::FirstTile) * first.size(), cudaMemcpyHostToDevice));
-    e->first_dirty = false;
+    OK_CUDA(cudaMemcpy(ag.first_beam.get(), first.data(), sizeof(ok::FirstTile) * first.size(), cudaMemcpyHostToDevice));
+    ag.first_dirty = false;
     return OK_SUCCESS;
 }
 
-// Re-cuts the beam tiling from the per-tile times the last launch on `s` left in d_tile_ns.  Results do not depend on the
-// tiling (tests/test_gpu_properties.py); only the finish times of the SMs do.  Synchronises `s`.
+// Re-cuts the beam tiling from the per-tile times the last launch on `s` left in d_tile_ns (ok::reweigh_runs), in place.
+// Results do not depend on the tiling (tests/test_gpu_properties.py); only the finish times of the SMs do.  Synchronises `s`.
 int rebalance_beam_tiles(OkEnv *e, cudaStream_t s)
 {
-    if (!e->d_tile_ns || e->h_tiles_beam.empty() || e->beam_runs.empty())
+    Agents       &ag = e->ag;
+    BeamFeedback &fb = ag.feedback;
+    if (!fb.d_tile_ns || fb.tiles.empty() || fb.runs.empty())
         return OK_SUCCESS;
     OK_CUDA(cudaStreamSynchronize(s));
-    std::vector<uint32_t> ns(2 * e->h_tiles_beam.size());
-    OK_CUDA(cudaMemcpy(ns.data(), e->d_tile_ns, sizeof(uint32_t) * ns.size(), cudaMemcpyDeviceToHost));
-    // per run: ns of ray phase per agent; c0: the median of what a tile spends outside the ray phase
-    std::vector<double>   ray_ns(e->beam_runs.size(), 0.0), agents(e->beam_runs.size(), 0.0);
-    std::vector<uint32_t> rest;
-    for (size_t i = 0; i < e->h_tiles_beam.size(); ++i)
-    {
-        if (ns[2 * i] == 0 || ns[2 * i] > 1000000000u) // never ran (or a wrapped timer): no information
-            continue;
-        const ok::Tile &t = e->h_tiles_beam[i];
-        for (size_t r = 0; r < e->beam_runs.size(); ++r)
-            if (t.begin >= e->beam_runs[r].begin && t.begin < e->beam_runs[r].begin + e->beam_runs[r].len)
-            {
-                ray_ns[r] += ns[2 * i], agents[r] += t.count;
-                break;
-            }
-        rest.push_back(ns[2 * i + 1]);
-    }
-    if (rest.size() * 2 < e->h_tiles_beam.size())
-        return OK_SUCCESS; // too few tiles measured
-    std::nth_element(rest.begin(), rest.begin() + rest.size() / 2, rest.end());
-    const double c0 = rest[rest.size() / 2];
-    double       w_sum = 0.0, a_sum = 0.0;
-    for (size_t r = 0; r < e->beam_runs.size(); ++r)
-        w_sum += ray_ns[r], a_sum += agents[r];
-    const double w_mean = a_sum > 0 ? w_sum / a_sum : 1.0;
-    // what the CURRENT tiling costs under the measured model (for the report)
-    {
-        double sum = 0.0, worst = 0.0;
-        for (size_t i = 0; i < e->h_tiles_beam.size(); ++i)
-        {
-            const double c = static_cast<double>(ns[2 * i]) + ns[2 * i + 1];
-            sum += c, worst = std::max(worst, c);
-        }
-        e->balance_before = sum > 0 ? static_cast<float>(worst * e->h_tiles_beam.size() / sum) : 1.0f;
-    }
-    for (size_t r = 0; r < e->beam_runs.size(); ++r)
-    { // the first measurement as it is; later ones damped, half way from the weight in use to the measured one
-        const double measured = agents[r] > 0 ? ray_ns[r] / agents[r] : w_mean;
-        e->beam_runs[r].w     = e->beam_launches_weighted ? 0.5 * (e->beam_runs[r].w + measured) : measured;
-    }
-    e->beam_launches_weighted = true;
-    std::vector<ok::Tile> tiles = cost_balanced_tiles(e->beam_runs, e->tiles_beam_target, c0, &e->balance_after);
-    if (tiles.empty() || static_cast<int32_t>(tiles.size()) > e->tiles_beam_capacity)
+    std::vector<uint32_t> ns(2 * fb.tiles.size());
+    OK_CUDA(cudaMemcpy(ns.data(), fb.d_tile_ns.get(), sizeof(uint32_t) * ns.size(), cudaMemcpyDeviceToHost));
+    ok::Reweighing rw;
+    if (!ok::reweigh_runs(fb.runs, fb.tiles, ns.data(), fb.weighted, fb.target, rw))
         return OK_SUCCESS;
-    OK_CUDA(cudaMemcpy(e->d_tiles_beam, tiles.data(), sizeof(ok::Tile) * tiles.size(), cudaMemcpyHostToDevice));
-    OK_CUDA(cudaMemset(e->d_tile_ns, 0, sizeof(uint32_t) * 2 * static_cast<size_t>(e->tiles_beam_capacity)));
-    e->h_tiles_beam = std::move(tiles);
-    e->first_dirty  = true;
-    e->n_tiles_beam = static_cast<int32_t>(e->h_tiles_beam.size());
-    e->grid_beam    = std::max(1, std::min(e->num_sms * e->ctas_per_sm_beam, e->n_tiles_beam));
+    e->balance_before = rw.balance_before, e->balance_after = rw.balance_after;
+    if (rw.tiles.empty() || static_cast<int32_t>(rw.tiles.size()) > fb.capacity)
+        return OK_SUCCESS;
+    OK_CUDA(cudaMemcpy(ag.beam.d.get(), rw.tiles.data(), sizeof(ok::Tile) * rw.tiles.size(), cudaMemcpyHostToDevice));
+    OK_CUDA(cudaMemset(fb.d_tile_ns.get(), 0, sizeof(uint32_t) * 2 * static_cast<size_t>(fb.capacity)));
+    fb.tiles       = std::move(rw.tiles);
+    ag.first_dirty = true;
+    ag.beam.n      = static_cast<int32_t>(fb.tiles.size());
+    ag.beam.grid   = std::max(1, std::min(e->num_sms * e->ctas_per_sm_beam, ag.beam.n));
     // at once, not at the next launch: a CUDA graph captured earlier reads both arrays at every replay, and they must agree
-    return e->d_first_beam ? upload_first_tiles(e, s) : OK_SUCCESS;
+    return ag.first_beam ? upload_first_tiles(e, s) : OK_SUCCESS;
 }
 
 // cuStreamWriteValue32 through the runtime's driver-entry-point lookup (the library does not link libcuda); nullptr if absent
@@ -891,14 +833,15 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
     int rc = ensure_arena(e);
     if (rc)
         return rc;
-    p.arena      = e->d_arena;
-    p.tracks     = e->d_track_refs;
+    p.arena      = e->d_arena.get();
+    p.tracks     = e->d_track_refs.get();
+    Agents &ag   = e->ag;
     if (e->cfg.raycast_mode == OK_RAYCAST_BEAM)
     {
-        const bool e2e = (p.host_obs || p.host_obs_q16) && e->d_tiles_e2e;
-        if (!e2e && e->auto_balance && e->d_tile_ns)
+        const bool e2e = (p.host_obs || p.host_obs_q16) && ag.e2e.d;
+        if (!e2e && e->auto_balance && ag.feedback.d_tile_ns)
         { // feedback tiling: re-cut the tiles from the measured tile times, a few times early on, then now and then
-            const uint64_t k = e->beam_launches++;
+            const uint64_t k = ag.feedback.launches++;
             if (k == 16 || k == 64 || k == 256 || (k & 4095) == 4095)
             {
                 cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
@@ -907,78 +850,75 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
                         return rc2;
             }
         }
-        p.tiles        = e->d_tiles_beam;
-        p.n_tiles      = e->n_tiles_beam;
+        p.tiles        = ag.beam.d.get();
+        p.n_tiles      = ag.beam.n;
         p.batch_agents = e->batch_agents_beam;
-        p.tile_ns      = e2e ? nullptr : e->d_tile_ns;
-        int grid       = e->grid_beam;
+        p.tile_ns      = e2e ? nullptr : ag.feedback.d_tile_ns.get();
+        int grid       = ag.beam.grid;
         p.first        = nullptr;
-        if (!e2e && !e->h_tiles_beam.empty())
+        if (!e2e && !ag.feedback.tiles.empty())
         { // the CTAs' first tiles with their track records side by side (rebuilt when the tiling or the arena changed)
-            if (e->first_dirty)
+            if (ag.first_dirty)
             {
                 cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
                 if (cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap == cudaStreamCaptureStatusNone)
                     if (int rc2 = upload_first_tiles(e, s))
                         return rc2;
             }
-            if (!e->first_dirty)
-                p.first = e->d_first_beam;
+            if (!ag.first_dirty)
+                p.first = ag.first_beam.get();
         }
         if (e2e)
         { // results stream to a host buffer: several tiles per CTA, each flushed while the next is computed
-            p.tiles   = e->d_tiles_e2e;
-            p.n_tiles = e->n_tiles_e2e;
-            grid      = e->grid_e2e;
-            if (p.host_obs_q16 && e->d_tiles_q16)
-                p.tiles = e->d_tiles_q16, p.n_tiles = e->n_tiles_q16, grid = e->grid_q16;
-            if (p.ext_host && e->d_act_stage && p.n_tiles > grid && e->act_stage_on && stream_write_value32())
+            const Schedule &sch = p.host_obs_q16 && ag.q16.d ? ag.q16 : ag.e2e;
+            p.tiles             = sch.d.get();
+            p.n_tiles           = sch.n;
+            grid                = sch.grid;
+            if (p.ext_host && ag.act_stage && p.n_tiles > grid && e->act_stage_on && stream_write_value32())
             { // tiles after a CTA's first read the actions from a device copy (StepParams::act_ready)
-                p.act_stage_thr    = e->d_act_stage;
-                p.act_stage_steer  = e->d_act_stage + e->n_agents;
-                p.act_ready        = e->d_act_ready;
-                p.act_ready_target = ++e->act_ready_target;
+                p.act_stage_thr    = ag.act_stage.get();
+                p.act_stage_steer  = ag.act_stage.get() + e->n_agents;
+                p.act_ready        = ag.act_ready.get();
+                p.act_ready_target = ++ag.act_ready_target;
             }
         }
-        const bool flushers = e2e && p.host_obs && e->e2e_flushers > 0 && e->d_tile_flag && e->beam_staged && !e->beam_seg;
+        const bool flushers = e2e && p.host_obs && e->e2e_flushers > 0 && ag.tile_flag && e->beam_staged;
         if (flushers)
         { // fork: the flusher CTAs start next to the step kernel, on the side stream
-            p.tile_flag  = e->d_tile_flag;
+            p.tile_flag  = ag.tile_flag.get();
             p.flag_epoch = ++e->flag_epoch;
-            OK_CUDA(cudaEventRecord(e->ev_fork, s));
-            OK_CUDA(cudaStreamWaitEvent(e->flush_stream, e->ev_fork, 0));
-            ok::obs_flush_kernel<<<e->e2e_flushers, 1024, 0, e->flush_stream>>>(e->d_tiles_e2e, e->n_tiles_e2e, e->d_tile_flag, p.flag_epoch,
-                                                                                static_cast<const float *>(e->d_buf[OK_BUF_OBS]), p.host_obs, e->rays);
+            OK_CUDA(cudaEventRecord(e->ev_fork.get(), s));
+            OK_CUDA(cudaStreamWaitEvent(e->flush_stream.get(), e->ev_fork.get(), 0));
+            ok::obs_flush_kernel<<<e->e2e_flushers, 1024, 0, e->flush_stream.get()>>>(ag.e2e.d.get(), ag.e2e.n, ag.tile_flag.get(), p.flag_epoch,
+                                                                                      static_cast<const float *>(e->d_buf[OK_BUF_OBS]), p.host_obs, e->rays);
             OK_CUDA(cudaGetLastError());
-            OK_CUDA(cudaEventRecord(e->ev_join, e->flush_stream));
+            OK_CUDA(cudaEventRecord(e->ev_join.get(), e->flush_stream.get()));
         }
         if (actor)
         { // the policy step as phase 0 of every tile (ok_ppo_actor_step): its weights sit behind the kernel's own shared memory
             p.actor_smem_off = static_cast<uint32_t>((e->smem_beam + 15) & ~static_cast<size_t>(15));
-            OK_CUDA(ok::launch_step_actor(p, *actor, e->grid_beam, p.actor_smem_off + actor_smem, s));
+            OK_CUDA(ok::launch_step_actor(p, *actor, ag.beam.grid, p.actor_smem_off + actor_smem, s));
         }
-        else if (e->beam_seg)
-            OK_CUDA(ok::launch_step_segstaged(p, grid, e->smem_beam, s));
         else if (e->beam_staged)
             ok::step_kernel<ok::kBeamBlockStaged, true, true><<<grid, ok::kBeamBlockStaged, e->smem_beam, s>>>(p, ok::NoActor{});
         else
-            OK_CUDA(ok::launch_step_unstaged(p, e->grid_beam, e->smem_beam, s));
+            OK_CUDA(ok::launch_step_unstaged(p, ag.beam.grid, e->smem_beam, s));
     }
     else
-        ok::step_kernel<kBlock, false><<<e->grid, kBlock, e->smem, s>>>(p, ok::NoActor{});
+        ok::step_kernel<kBlock, false><<<ag.tiles.grid, kBlock, e->smem, s>>>(p, ok::NoActor{});
     OK_CUDA(cudaGetLastError());
     if (p.act_ready)
     { // enqueued AFTER the launch: the kernel is already running its first tiles while the host issues these
         const size_t bytes = sizeof(float) * static_cast<size_t>(e->n_agents);
-        OK_CUDA(cudaMemcpyAsync(p.act_stage_thr, p.ext_thr, bytes, cudaMemcpyHostToDevice, e->act_stream));
-        OK_CUDA(cudaMemcpyAsync(p.act_stage_steer, p.ext_steer, bytes, cudaMemcpyHostToDevice, e->act_stream));
-        if (stream_write_value32()(e->act_stream, reinterpret_cast<CUdeviceptr>(e->d_act_ready), p.act_ready_target, 0) != CUDA_SUCCESS)
+        OK_CUDA(cudaMemcpyAsync(p.act_stage_thr, p.ext_thr, bytes, cudaMemcpyHostToDevice, e->act_stream.get()));
+        OK_CUDA(cudaMemcpyAsync(p.act_stage_steer, p.ext_steer, bytes, cudaMemcpyHostToDevice, e->act_stream.get()));
+        if (stream_write_value32()(e->act_stream.get(), reinterpret_cast<CUdeviceptr>(ag.act_ready.get()), p.act_ready_target, 0) != CUDA_SUCCESS)
             return fail(OK_ERR_CUDA, "cuStreamWriteValue32 failed");
-        OK_CUDA(cudaEventRecord(e->ev_act, e->act_stream));
-        OK_CUDA(cudaStreamWaitEvent(s, e->ev_act, 0)); // join: nothing of this tick outlives the caller's stream
+        OK_CUDA(cudaEventRecord(e->ev_act.get(), e->act_stream.get()));
+        OK_CUDA(cudaStreamWaitEvent(s, e->ev_act.get(), 0)); // join: nothing of this tick outlives the caller's stream
     }
     if (p.tile_flag) // join: the tick is complete when the last tile has reached the host
-        OK_CUDA(cudaStreamWaitEvent(s, e->ev_join, 0));
+        OK_CUDA(cudaStreamWaitEvent(s, e->ev_join.get(), 0));
     e->launches++;
     return OK_SUCCESS;
 }
@@ -1082,8 +1022,6 @@ int ok_create(const OkConfig *cfg, OkEnv **out)
         e->has_device = true;
         e->num_sms    = sms;
         e->smem_optin = optin;
-        cudaDeviceGetAttribute(&e->smem_per_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, c.device);
-        cudaDeviceGetAttribute(&e->smem_reserved, cudaDevAttrReservedSharedMemoryPerBlock, c.device);
         e->max_blob   = optin > 65536 ? static_cast<size_t>(optin) - 40960 : 0; // room for the batch scratch
     }
     else
@@ -1125,29 +1063,7 @@ void ok_destroy(OkEnv *e)
 {
     if (!e)
         return;
-    if (e->has_device)
-    {
-        DeviceGuard g(e->cfg.device);
-        free_agents(e);
-        if (e->d_arena)
-            cudaFree(e->d_arena);
-        if (e->d_track_refs)
-            cudaFree(e->d_track_refs);
-        if (e->d_stage)
-            cudaFree(e->d_stage);
-        if (e->flush_stream)
-            cudaStreamDestroy(e->flush_stream);
-        if (e->d_counters)
-            cudaFree(e->d_counters);
-        if (e->act_stream)
-            cudaStreamDestroy(e->act_stream);
-        if (e->ev_act)
-            cudaEventDestroy(e->ev_act);
-        if (e->ev_fork)
-            cudaEventDestroy(e->ev_fork);
-        if (e->ev_join)
-            cudaEventDestroy(e->ev_join);
-    }
+    DeviceGuard g(e->has_device ? e->cfg.device : -1); // the env's members free their device resources on that device
     delete e;
 }
 
@@ -1275,16 +1191,9 @@ namespace
 int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg, const int32_t *h_track_id)
 {
     NvtxRange range("ok_alloc_agents (tiling, buffers)");
-    e->n_agents = n;
-    e->rays     = rays;
-    // the segment-staged shape (two 512-thread CTAs per SM): populations that give every CTA a worthwhile tile, tracks
-    // whose segments leave room for at least 64 agent records in half an SM's shared memory
-    const int64_t seg_budget = static_cast<int64_t>(e->smem_per_sm) / ok::kBeamSegCtasPerSm - e->smem_reserved -
-                               ok::beam_static_smem(true, true) - 256;
-    auto seg_cap_of = [&](int32_t track) -> int64_t {
-        const int64_t sb = (static_cast<int64_t>(reinterpret_cast<const ok::TrackHeader *>(e->tracks[track].blob.data())->off_words) + 127) / 128 * 128;
-        return std::min<int64_t>({(seg_budget - sb) / static_cast<int64_t>(sizeof(ok::AgentRec)), ok::kBeamBlockSeg, 65535 / rays});
-    };
+    Agents   &ag = e->ag;
+    e->n_agents  = n;
+    e->rays      = rays;
     // batch = the agents a CTA keeps in flight: as many as fit behind the largest staged track
     {
         const size_t blob  = (e->max_blob_used + 127) / 128 * 128;
@@ -1310,26 +1219,12 @@ int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg,
         // 4,096 agents of 5 rays (a PPO rollout tick: 0.0289 vs 0.0300 ms, 0.0262 with the policy step fused in), behind at
         // 8,192 agents of 5 rays (0.0376 vs 0.0318 ms)
         e->beam_staged = n >= 2048 && n * rays > 24576;
-        e->beam_seg = false; // opt-in (OK_BEAM_KERNEL=segstaged): 1 % ahead at 65,536 agents with tiles of equal agent counts, but its tile times
-                             // depend on the CTA that shares the SM, so the feedback tiling gains nothing there (0.092 vs 0.085 ms per tick)
         if (const char *env = std::getenv("OK_BEAM_KERNEL"))
-        {
-            e->beam_staged = std::strcmp(env, "unstaged") != 0 && (std::strcmp(env, "staged") == 0 || std::strcmp(env, "segstaged") == 0 || e->beam_staged);
-            e->beam_seg    = std::strcmp(env, "segstaged") == 0 || (e->beam_seg && e->beam_staged && std::strcmp(env, "staged") != 0);
-        }
-        if (e->beam_seg)
-            for (size_t t = 0; t < e->tracks.size(); ++t)
-                if (seg_cap_of(static_cast<int32_t>(t)) < 64)
-                    e->beam_seg = false; // a track too large for half an SM: the one-CTA-per-SM shape stages whole blobs
-        e->beam_block = e->beam_seg ? ok::kBeamBlockSeg : (e->beam_staged ? ok::kBeamBlockStaged : ok::kBeamBlockUnstaged);
+            e->beam_staged = std::strcmp(env, "unstaged") != 0 && (std::strcmp(env, "staged") == 0 || e->beam_staged);
+        e->beam_block = e->beam_staged ? ok::kBeamBlockStaged : ok::kBeamBlockUnstaged;
         int64_t ab;
         int     capb;
-        if (e->beam_seg)
-        { // provisional: the tiling below sizes every track's tiles by what fits behind ITS segments
-            ab   = ok::kBeamBlockSeg;
-            capb = ok::kBeamBlockSeg;
-        }
-        else if (e->beam_staged)
+        if (e->beam_staged)
         { // one 1,024-thread CTA per SM behind the staged track: as many agents per tile as the shared memory behind the
           // largest track holds (the balanced tiling then sizes the tiles: about one per CTA and wave)
             ab   = static_cast<int64_t>((avail - ok::beam_static_smem(true)) / sizeof(ok::AgentRec));
@@ -1347,7 +1242,7 @@ int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg,
         if (!e->beam_staged) // small populations: spread over all SMs rather than filling a few tiles
             ab = std::min<int64_t>(ab, std::max<int64_t>(1, (n + e->num_sms - 1) / std::max(1, e->num_sms)));
         e->batch_agents_beam = static_cast<int32_t>(std::max<int64_t>(1, ab));
-        e->smem_beam         = ((e->beam_staged && !e->beam_seg) ? blob : 0) + ok::beam_smem_bytes(e->batch_agents_beam); // (segment-staged: set by the tiling)
+        e->smem_beam         = (e->beam_staged ? blob : 0) + ok::beam_smem_bytes(e->batch_agents_beam);
         // The limit is an attribute of the FUNCTION on this device, not of the env: it is raised to the opt-in maximum
         // (minus the kernel's static shared memory), so that envs of different sizes can interleave their launches.
         if (int rc = arm_shared_memory_limit(e))
@@ -1361,15 +1256,15 @@ int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg,
         offs[b] = total;
         total += (buffer_bytes(e, b) + 255) / 256 * 256;
     }
-    OK_CUDA(cudaMalloc(&e->d_slab, total));
-    OK_CUDA(cudaMemset(e->d_slab, 0, total));
+    OK_CUDA(dev_alloc(ag.slab, total));
+    OK_CUDA(cudaMemset(ag.slab.get(), 0, total));
     for (int b = 0; b < OK_BUF_COUNT; ++b)
     {
-        e->d_buf[b]   = e->d_slab + offs[b];
+        e->d_buf[b]   = ag.slab.get() + offs[b];
         e->buf_off[b] = offs[b];
     }
-    OK_CUDA(cudaMalloc(&e->d_ray_deg, sizeof(float) * rays));
-    OK_CUDA(cudaMemcpy(e->d_ray_deg, h_ray_deg, sizeof(float) * rays, cudaMemcpyHostToDevice));
+    OK_CUDA(dev_alloc(ag.ray_deg, static_cast<size_t>(rays)));
+    OK_CUDA(cudaMemcpy(ag.ray_deg.get(), h_ray_deg, sizeof(float) * rays, cudaMemcpyHostToDevice));
     e->h_track_id.assign(static_cast<size_t>(n), 0);
     if (h_track_id)
         std::copy(h_track_id, h_track_id + n, e->h_track_id.begin());
@@ -1383,101 +1278,30 @@ int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg,
             order[i] = static_cast<uint16_t>(i);
         std::stable_sort(order.begin(), order.end(),
                          [&](uint16_t x, uint16_t y) { return std::fabs(h_ray_deg[x]) < std::fabs(h_ray_deg[y]); });
-        OK_CUDA(cudaMalloc(&e->d_ray_order, sizeof(uint16_t) * rays));
-        OK_CUDA(cudaMemcpy(e->d_ray_order, order.data(), sizeof(uint16_t) * rays, cudaMemcpyHostToDevice));
-        OK_CUDA(cudaMalloc(&e->d_sched, sizeof(int32_t) * 512));
-        OK_CUDA(cudaMemset(e->d_sched, 0, sizeof(int32_t) * 512));
+        OK_CUDA(dev_alloc(ag.ray_order, static_cast<size_t>(rays)));
+        OK_CUDA(cudaMemcpy(ag.ray_order.get(), order.data(), sizeof(uint16_t) * rays, cudaMemcpyHostToDevice));
+        OK_CUDA(dev_alloc(ag.sched, 512));
+        OK_CUDA(cudaMemset(ag.sched.get(), 0, sizeof(int32_t) * 512));
     }
 
-    // tiles: maximal runs of one track, cut into batches.  Guided self-scheduling: CTAs pull tiles in
-    // list order, so full-size batches come first and a tail of quarter-size ones (about half a big
-    // batch per SM) evens out the finish.
-    auto build_tiles = [&](int big, int ctas, int tail_div, ok::Tile **d_out, int32_t *n_out) -> int {
-        // tail_div = 0: uniform tiles; otherwise the last tiles (about half a big batch per CTA) are 1 / tail_div the size
-        const int     small = std::max(1, big / std::max(1, tail_div));
-        const int64_t tail_agents = tail_div > 1 ? std::min<int64_t>(n / 2, static_cast<int64_t>(ctas) * big / 2) : 0;
-        std::vector<ok::Tile> tiles, tail;
-        for (int64_t i = 0; i < n;)
-        {
-            int64_t j = i;
-            while (j < n && e->h_track_id[j] == e->h_track_id[i])
-                ++j;
-            // this run's share of the small-tile tail
-            const int64_t run_tail = (j - i) * tail_agents / n;
-            const int64_t split    = j - run_tail;
-            for (int64_t b = i; b < j;)
-            {
-                const bool    in_tail = b >= split;
-                const int64_t lim     = in_tail ? j : split;
-                ok::Tile      t{};
-                t.track = e->h_track_id[i];
-                t.begin = b;
-                t.count = static_cast<int32_t>(std::min<int64_t>(in_tail ? small : big, lim - b));
-                (in_tail ? tail : tiles).push_back(t);
-                b += t.count;
-            }
-            i = j;
-        }
-        tiles.insert(tiles.end(), tail.begin(), tail.end());
-        *n_out = static_cast<int32_t>(tiles.size());
-        OK_CUDA(cudaMalloc(d_out, sizeof(ok::Tile) * tiles.size()));
-        OK_CUDA(cudaMemcpy(*d_out, tiles.data(), sizeof(ok::Tile) * tiles.size(), cudaMemcpyHostToDevice));
-        return OK_SUCCESS;
-    };
-    // Balanced tiling (staged beam kernel).  The kernel's cost per ray is nearly uniform, but a tile pays ~15 us of serial
-    // latency (thread-per-agent phases, second ray pass, barriers) whatever its size: the fewer, larger and more equal
-    // the tiles, the better.  Tiles = CTAs x waves, dealt to the track runs in proportion to their length, every run
-    // cut into equal parts, largest first.
-    size_t seg_smem_need = 0; // segment-staged shape: the most (segments + records) any tile of any tiling may need
-    // Balanced tiling (staged beam kernels).  The kernel's cost per ray is nearly uniform, but a tile pays ~15 us of serial
-    // latency (thread-per-agent phases, second ray pass, barriers) whatever its size: the fewer, larger and more equal
-    // the tiles, the better.  Tiles = CTAs x waves, dealt to the track runs in proportion to their length (and, once the
-    // kernel has reported tile times, to their measured cost: cost_balanced_tiles / rebalance_beam_tiles).
-    auto build_tiles_balanced = [&](int max_tile, int ctas, ok::Tile **d_out, int32_t *n_out, int min_waves = 1, bool feedback = false) -> int {
-        std::vector<OkEnv::TileRun> runs;
-        int64_t                     have = 0;
-        for (int64_t i = 0; i < n;)
-        {
-            int64_t j = i;
-            while (j < n && e->h_track_id[j] == e->h_track_id[i])
-                ++j;
-            // (segment-staged shape: a track's tiles are capped by what fits behind ITS segments)
-            const int64_t cap = e->beam_seg ? std::min<int64_t>(max_tile, seg_cap_of(e->h_track_id[i])) : max_tile;
-            runs.push_back({e->h_track_id[i], i, j - i, cap, 1.0, 0});
-            have += (j - i + cap - 1) / cap;
-            if (e->beam_seg)
-                seg_smem_need = std::max(seg_smem_need, (static_cast<size_t>(reinterpret_cast<const ok::TrackHeader *>(e->tracks[e->h_track_id[i]].blob.data())->off_words) + 127) / 128 * 128 +
-                                                            ok::beam_smem_bytes(static_cast<int>(std::min<int64_t>(cap, j - i))));
-            i = j;
-        }
-        const int64_t waves  = std::max<int64_t>({static_cast<int64_t>(min_waves), (n + static_cast<int64_t>(ctas) * max_tile - 1) / (static_cast<int64_t>(ctas) * max_tile),
-                                                  (have + ctas - 1) / ctas});
-        const int64_t target = static_cast<int64_t>(ctas) * waves;
-        std::vector<ok::Tile> tiles = cost_balanced_tiles(runs, target, 0.0, nullptr);
-        const size_t capacity = std::max<size_t>(tiles.size(), static_cast<size_t>(target));
-        *n_out = static_cast<int32_t>(tiles.size());
-        OK_CUDA(cudaMalloc(d_out, sizeof(ok::Tile) * capacity));
-        OK_CUDA(cudaMemcpy(*d_out, tiles.data(), sizeof(ok::Tile) * tiles.size(), cudaMemcpyHostToDevice));
-        if (feedback)
-        {
-            e->beam_runs = runs, e->h_tiles_beam = tiles, e->first_dirty = true;
-            e->tiles_beam_target = static_cast<int32_t>(target), e->tiles_beam_capacity = static_cast<int32_t>(capacity);
-            OK_CUDA(cudaMalloc(&e->d_tile_ns, sizeof(uint32_t) * 2 * capacity));
-            OK_CUDA(cudaMemset(e->d_tile_ns, 0, sizeof(uint32_t) * 2 * capacity));
-        }
-        return OK_SUCCESS;
+    // tilings (ok_schedule.hpp)
+    const int32_t *track_id = e->h_track_id.data();
+    // the balanced tiling of the beam kernel's batches over `ctas` CTAs, at least `waves` tiles per CTA; `runs` keeps the
+    // track runs with their tile counts
+    auto balanced = [&](int ctas, int waves, std::vector<ok::TileRun> &runs) {
+        runs = ok::track_runs(track_id, n, e->batch_agents_beam);
+        return ok::balanced_tiles(runs, e->batch_agents_beam, ctas, waves);
     };
     {
         int per_sm = 1;
         if (!e->beam_staged)
             OK_CUDA(ok::occupancy_step_unstaged(e->smem_beam, &per_sm));
-        if (e->beam_seg)
-            per_sm = ok::kBeamSegCtasPerSm;
         e->ctas_per_sm_beam = std::max(1, per_sm);
     }
-    if (int rc = build_tiles(e->batch_agents, e->num_sms, 4, &e->d_tiles, &e->n_tiles))
+    if (int rc = upload_schedule(ag.tiles, ok::guided_tiles(track_id, n, e->batch_agents, e->num_sms, 4), 0, e->num_sms))
         return rc;
     {
+        const int beam_ctas = e->num_sms * e->ctas_per_sm_beam;
         // the unstaged beam kernel's small tiles cost about the same serial latency whatever their size (the thread-per-
         // agent phases, the second ray pass): shrinking them further only adds tiles
         int tail_div = e->beam_staged ? -1 : 0; // -1: balanced tiling
@@ -1486,21 +1310,28 @@ int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg,
         int waves = 1; // balanced tiling: tiles per CTA (OK_BEAM_WAVES)
         if (const char *env = std::getenv("OK_BEAM_WAVES"))
             waves = std::max(1, std::atoi(env));
-        if (e->beam_seg)
-            tail_div = -1; // (the guided schedule knows nothing of the per-track tile caps of the segment-staged shape)
         e->auto_balance = 1; // OK_AUTO_BALANCE=0: keep the tiling by agent count
         if (const char *env = std::getenv("OK_AUTO_BALANCE"))
             e->auto_balance = std::atoi(env);
-        const int rc = tail_div < 0 ? build_tiles_balanced(e->batch_agents_beam, e->num_sms * e->ctas_per_sm_beam, &e->d_tiles_beam, &e->n_tiles_beam, waves, true)
-                                    : build_tiles(e->batch_agents_beam, e->num_sms * e->ctas_per_sm_beam, tail_div, &e->d_tiles_beam, &e->n_tiles_beam);
-        if (rc)
+        if (tail_div < 0)
+        { // the feedback tiling: its table is allocated once, with room for every re-cut (rebalance_beam_tiles)
+            BeamFeedback      &fb = ag.feedback;
+            ok::BalancedTiling bt = balanced(beam_ctas, waves, fb.runs);
+            const size_t capacity = std::max<size_t>(bt.tiles.size(), static_cast<size_t>(bt.target));
+            fb.tiles    = bt.tiles;
+            fb.target   = static_cast<int32_t>(bt.target);
+            fb.capacity = static_cast<int32_t>(capacity);
+            if (int rc = upload_schedule(ag.beam, bt.tiles, capacity, beam_ctas))
+                return rc;
+            OK_CUDA(dev_alloc(fb.d_tile_ns, 2 * capacity));
+            OK_CUDA(cudaMemset(fb.d_tile_ns.get(), 0, sizeof(uint32_t) * 2 * capacity));
+        }
+        else if (int rc = upload_schedule(ag.beam, ok::guided_tiles(track_id, n, e->batch_agents_beam, beam_ctas, tail_div), 0, beam_ctas))
             return rc;
     }
-    e->grid      = std::max(1, std::min(e->num_sms, e->n_tiles));
-    e->grid_beam = std::max(1, std::min(e->num_sms * e->ctas_per_sm_beam, e->n_tiles_beam));
     if (e->beam_staged)
-    { // the end-to-end tiling (see ok_step_host): OK_E2E_TILES tiles per CTA (default 4; 2 for the two-CTAs-per-SM shape)
-        int per_cta = e->beam_seg ? 2 : 4;
+    { // the end-to-end tiling (see ok_step_host): OK_E2E_TILES tiles per CTA (default 4)
+        int per_cta = 4;
         if (const char *env = std::getenv("OK_E2E_TILES"))
             per_cta = std::max(1, std::atoi(env));
         // OK_E2E_FLUSHERS = F > 0: F SMs are left to obs_flush_kernel, which moves finished tiles to the host while the
@@ -1508,54 +1339,43 @@ int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg,
         e->e2e_flushers = 0;
         if (const char *env = std::getenv("OK_E2E_FLUSHERS"))
             e->e2e_flushers = std::max(0, std::min(std::atoi(env), e->num_sms / 2));
-        if (e->beam_seg)
-            e->e2e_flushers = 0;
-        const int e2e_ctas = (e->num_sms - e->e2e_flushers) * e->ctas_per_sm_beam;
-        if (int rc = build_tiles_balanced(e->batch_agents_beam, e2e_ctas, &e->d_tiles_e2e, &e->n_tiles_e2e, per_cta))
+        std::vector<ok::TileRun> runs;
+        const int                e2e_ctas = (e->num_sms - e->e2e_flushers) * e->ctas_per_sm_beam;
+        const ok::BalancedTiling e2e      = balanced(e2e_ctas, per_cta, runs);
+        if (int rc = upload_schedule(ag.e2e, e2e.tiles, static_cast<size_t>(e2e.target), e2e_ctas))
             return rc;
-        e->grid_e2e = std::max(1, std::min(e2e_ctas, e->n_tiles_e2e));
         { // ok_step_host_q16: measured at the C3 shape 0.164 / 0.157 / 0.171 / 0.199 ms per tick with 2 / 3 / 4 / 6 tiles per CTA
-            int per_cta_q16 = e->beam_seg ? 2 : 3;
+            int per_cta_q16 = 3;
             if (const char *env = std::getenv("OK_E2E_TILES_Q16"))
                 per_cta_q16 = std::max(1, std::atoi(env));
             else if (std::getenv("OK_E2E_TILES"))
                 per_cta_q16 = per_cta;
-            const int q16_ctas = e->num_sms * e->ctas_per_sm_beam;
-            if (int rc = build_tiles_balanced(e->batch_agents_beam, q16_ctas, &e->d_tiles_q16, &e->n_tiles_q16, per_cta_q16))
+            const int                q16_ctas = e->num_sms * e->ctas_per_sm_beam;
+            const ok::BalancedTiling q16      = balanced(q16_ctas, per_cta_q16, runs);
+            if (int rc = upload_schedule(ag.q16, q16.tiles, static_cast<size_t>(q16.target), q16_ctas))
                 return rc;
-            e->grid_q16 = std::max(1, std::min(q16_ctas, e->n_tiles_q16));
         }
-        OK_CUDA(cudaMalloc(&e->d_act_stage, sizeof(float) * 2 * static_cast<size_t>(n)));
-        OK_CUDA(cudaMalloc(&e->d_act_ready, sizeof(uint32_t)));
-        OK_CUDA(cudaMemset(e->d_act_ready, 0, sizeof(uint32_t)));
-        e->act_ready_target = 0;
+        OK_CUDA(dev_alloc(ag.act_stage, 2 * static_cast<size_t>(n)));
+        OK_CUDA(dev_alloc(ag.act_ready, 1));
+        OK_CUDA(cudaMemset(ag.act_ready.get(), 0, sizeof(uint32_t)));
         if (!e->act_stream)
         {
-            OK_CUDA(cudaStreamCreateWithFlags(&e->act_stream, cudaStreamNonBlocking));
-            OK_CUDA(cudaEventCreateWithFlags(&e->ev_act, cudaEventDisableTiming));
+            OK_CUDA(make_stream(e->act_stream));
+            OK_CUDA(make_event(e->ev_act));
         }
         if (const char *env = std::getenv("OK_ACT_STAGE"))
             e->act_stage_on = std::atoi(env) != 0;
         if (e->e2e_flushers > 0)
         {
-            OK_CUDA(cudaMalloc(&e->d_tile_flag, sizeof(uint32_t) * static_cast<size_t>(e->n_tiles_e2e)));
-            OK_CUDA(cudaMemset(e->d_tile_flag, 0, sizeof(uint32_t) * static_cast<size_t>(e->n_tiles_e2e)));
+            OK_CUDA(dev_alloc(ag.tile_flag, static_cast<size_t>(ag.e2e.n)));
+            OK_CUDA(cudaMemset(ag.tile_flag.get(), 0, sizeof(uint32_t) * static_cast<size_t>(ag.e2e.n)));
             if (!e->flush_stream)
             {
-                OK_CUDA(cudaStreamCreateWithFlags(&e->flush_stream, cudaStreamNonBlocking));
-                OK_CUDA(cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming));
-                OK_CUDA(cudaEventCreateWithFlags(&e->ev_join, cudaEventDisableTiming));
+                OK_CUDA(make_stream(e->flush_stream));
+                OK_CUDA(make_event(e->ev_fork));
+                OK_CUDA(make_event(e->ev_join));
             }
         }
-    }
-    if (e->beam_seg)
-    { // both tilings are built: the launch's dynamic shared memory is the largest tile's need; two CTAs must fit an SM
-        e->smem_beam = seg_smem_need;
-        int per_sm   = 0;
-        OK_CUDA(ok::occupancy_step_segstaged(e->smem_beam, &per_sm));
-        if (per_sm < ok::kBeamSegCtasPerSm)
-            return fail(OK_ERR_CAPACITY, "segment-staged beam kernel: " + std::to_string(e->smem_beam) + " bytes of shared memory per CTA do not give " +
-                                             std::to_string(ok::kBeamSegCtasPerSm) + " CTAs per SM (set OK_BEAM_KERNEL=staged)");
     }
 
     // every agent starts where `Environment::resetAgent(agent, false)` puts it: RaceTrack::kStartingIdx
@@ -1617,16 +1437,14 @@ int ok_reset_agents_host(OkEnv *e, const int64_t *h_agent_idx, const int32_t *h_
     const size_t need = static_cast<size_t>(n) * (8 + 4 + 4 + 4) + 64;
     if (need > e->stage_bytes)
     {
-        if (e->d_stage)
-            cudaFree(e->d_stage);
-        e->d_stage = nullptr, e->stage_bytes = 0;
-        OK_CUDA(cudaMalloc(&e->d_stage, need));
+        e->stage_bytes = 0;
+        OK_CUDA(dev_alloc(e->d_stage, need));
         e->stage_bytes = need;
     }
-    int64_t *d_ai = reinterpret_cast<int64_t *>(e->d_stage);
-    int32_t *d_pt = reinterpret_cast<int32_t *>(e->d_stage + 8 * static_cast<size_t>(n));
-    float   *d_la = reinterpret_cast<float *>(e->d_stage + 12 * static_cast<size_t>(n));
-    float   *d_ho = reinterpret_cast<float *>(e->d_stage + 16 * static_cast<size_t>(n));
+    int64_t *d_ai = reinterpret_cast<int64_t *>(e->d_stage.get());
+    int32_t *d_pt = reinterpret_cast<int32_t *>(e->d_stage.get() + 8 * static_cast<size_t>(n));
+    float   *d_la = reinterpret_cast<float *>(e->d_stage.get() + 12 * static_cast<size_t>(n));
+    float   *d_ho = reinterpret_cast<float *>(e->d_stage.get() + 16 * static_cast<size_t>(n));
     if (h_agent_idx)
         OK_CUDA(cudaMemcpyAsync(d_ai, h_agent_idx, 8 * static_cast<size_t>(n), cudaMemcpyHostToDevice, s));
     OK_CUDA(cudaMemcpyAsync(d_pt, h_pt_idx, 4 * static_cast<size_t>(n), cudaMemcpyHostToDevice, s));
@@ -1877,8 +1695,8 @@ int ok_track_query(OkEnv *e, const float *d_x, const float *d_y, const int32_t *
     if (rc)
         return rc;
     ok::StepParams  p{};
-    p.arena  = e->d_arena;
-    p.tracks = e->d_track_refs;
+    p.arena  = e->d_arena.get();
+    p.tracks = e->d_track_refs.get();
     ok::QueryParams q{d_x, d_y, d_track, n, static_cast<int32_t>(e->tracks.size()), d_idx, d_lane, d_bound};
     const int       threads = 256;
     const int64_t   blocks  = (n * 32 + threads - 1) / threads;
@@ -2304,20 +2122,19 @@ int ok_debug_stats(OkEnv *e, uint64_t out[4], int32_t enable)
     if (out)
     {
         out[0] = out[1] = out[2] = out[3] = 0;
-        if (e->d_stats)
-            OK_CUDA(cudaMemcpy(out, e->d_stats, 32, cudaMemcpyDeviceToHost));
+        if (e->ag.stats)
+            OK_CUDA(cudaMemcpy(out, e->ag.stats.get(), 32, cudaMemcpyDeviceToHost));
     }
-    if (enable && !e->d_stats)
+    if (enable && !e->ag.stats)
     {
-        OK_CUDA(cudaMalloc(&e->d_stats, 32));
+        OK_CUDA(dev_alloc(e->ag.stats, 4));
     }
-    if (e->d_stats)
-        OK_CUDA(cudaMemset(e->d_stats, 0, 32));
-    if (!enable && e->d_stats)
+    if (e->ag.stats)
+        OK_CUDA(cudaMemset(e->ag.stats.get(), 0, 32));
+    if (!enable && e->ag.stats)
     {
         OK_CUDA(cudaDeviceSynchronize());
-        cudaFree(e->d_stats);
-        e->d_stats = nullptr;
+        e->ag.stats.reset();
     }
     return OK_SUCCESS;
 }
@@ -2331,9 +2148,6 @@ int ok_debug_violations(OkEnv *e, uint64_t *count, int32_t *checks_compiled_in)
     unsigned long long v = 0, u = 0;
     OK_CUDA(cudaMemcpyFromSymbol(&v, ok::g_violations, sizeof v));
     OK_CUDA(ok::violations_step_unstaged(&u));
-    unsigned long long w = 0;
-    OK_CUDA(ok::violations_step_segstaged(&w));
-    u += w;
     if (count)
         *count = v + u;
     if (checks_compiled_in)
@@ -2360,14 +2174,15 @@ int64_t ok_debug_tiles(OkEnv *e, int64_t *h_out, int64_t capacity)
     int rc = check_ready(e);
     if (rc)
         return rc;
-    if (e->cfg.raycast_mode != OK_RAYCAST_BEAM || !e->d_tiles_beam)
+    const Schedule &beam = e->ag.beam;
+    if (e->cfg.raycast_mode != OK_RAYCAST_BEAM || !beam.d)
         return 0;
     DeviceGuard           g(e->cfg.device);
-    std::vector<ok::Tile> tiles(static_cast<size_t>(e->n_tiles_beam));
-    OK_CUDA(cudaMemcpy(tiles.data(), e->d_tiles_beam, sizeof(ok::Tile) * tiles.size(), cudaMemcpyDeviceToHost));
-    for (int64_t i = 0; h_out && i < std::min<int64_t>(capacity, e->n_tiles_beam); ++i)
+    std::vector<ok::Tile> tiles(static_cast<size_t>(beam.n));
+    OK_CUDA(cudaMemcpy(tiles.data(), beam.d.get(), sizeof(ok::Tile) * tiles.size(), cudaMemcpyDeviceToHost));
+    for (int64_t i = 0; h_out && i < std::min<int64_t>(capacity, beam.n); ++i)
         h_out[3 * i] = tiles[i].track, h_out[3 * i + 1] = tiles[i].count, h_out[3 * i + 2] = tiles[i].begin;
-    return e->n_tiles_beam;
+    return beam.n;
 }
 
 int64_t ok_debug_trace(OkEnv *e, uint64_t *h_out, int64_t capacity_words, int32_t tiles_per_cta)
@@ -2376,26 +2191,24 @@ int64_t ok_debug_trace(OkEnv *e, uint64_t *h_out, int64_t capacity_words, int32_
     if (rc)
         return rc;
     DeviceGuard  g(e->cfg.device);
-    const size_t words = static_cast<size_t>(e->grid_beam) * static_cast<size_t>(std::max(e->trace_tiles, 0)) * 6;
+    Agents      &ag    = e->ag;
+    const size_t words = static_cast<size_t>(ag.beam.grid) * static_cast<size_t>(std::max(ag.trace_tiles, 0)) * 6;
     int64_t      got   = 0;
     OK_CUDA(cudaDeviceSynchronize());
-    if (h_out && e->d_trace && words)
+    if (h_out && ag.trace && words)
     {
         got = static_cast<int64_t>(std::min<size_t>(words, static_cast<size_t>(std::max<int64_t>(capacity_words, 0))));
-        OK_CUDA(cudaMemcpy(h_out, e->d_trace, 8 * static_cast<size_t>(got), cudaMemcpyDeviceToHost));
+        OK_CUDA(cudaMemcpy(h_out, ag.trace.get(), 8 * static_cast<size_t>(got), cudaMemcpyDeviceToHost));
     }
-    if (e->d_trace && tiles_per_cta != e->trace_tiles)
-    {
-        cudaFree(e->d_trace);
-        e->d_trace = nullptr, e->trace_tiles = 0;
-    }
+    if (ag.trace && tiles_per_cta != ag.trace_tiles)
+        ag.trace.reset(), ag.trace_tiles = 0;
     if (tiles_per_cta > 0)
     {
-        const size_t bytes = 8 * static_cast<size_t>(e->grid_beam) * tiles_per_cta * 6;
-        if (!e->d_trace)
-            OK_CUDA(cudaMalloc(&e->d_trace, bytes));
-        OK_CUDA(cudaMemset(e->d_trace, 0, bytes));
-        e->trace_tiles = tiles_per_cta;
+        const size_t words_new = static_cast<size_t>(ag.beam.grid) * tiles_per_cta * 6;
+        if (!ag.trace)
+            OK_CUDA(dev_alloc(ag.trace, words_new));
+        OK_CUDA(cudaMemset(ag.trace.get(), 0, 8 * words_new));
+        ag.trace_tiles = tiles_per_cta;
     }
     return got;
 }
@@ -2411,17 +2224,17 @@ int ok_population_counters(OkEnv *e, OkPopulationCounters *out, void *stream)
     DeviceGuard  g(e->cfg.device);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     if (!e->d_counters)
-        OK_CUDA(cudaMalloc(&e->d_counters, 4 * sizeof(unsigned long long)));
-    OK_CUDA(cudaMemsetAsync(e->d_counters, 0, 4 * sizeof(unsigned long long), s));
+        OK_CUDA(dev_alloc(e->d_counters, 4));
+    OK_CUDA(cudaMemsetAsync(e->d_counters.get(), 0, 4 * sizeof(unsigned long long), s));
     const int threads = 256;
     const int blocks  = static_cast<int>(std::min<int64_t>((e->n_agents + threads - 1) / threads, 4 * e->num_sms));
     ok::population_counters_kernel<<<blocks, threads, 0, s>>>(static_cast<const uint8_t *>(e->d_buf[OK_BUF_CRASHED]),
                                                                static_cast<const uint8_t *>(e->d_buf[OK_BUF_TIMED_OUT]),
-                                                               static_cast<const uint8_t *>(e->d_buf[OK_BUF_DONE]), e->n_agents, e->d_counters);
+                                                               static_cast<const uint8_t *>(e->d_buf[OK_BUF_DONE]), e->n_agents, e->d_counters.get());
     OK_CUDA(cudaGetLastError());
     e->launches++;
     unsigned long long h[4];
-    OK_CUDA(cudaMemcpyAsync(h, e->d_counters, sizeof h, cudaMemcpyDeviceToHost, s));
+    OK_CUDA(cudaMemcpyAsync(h, e->d_counters.get(), sizeof h, cudaMemcpyDeviceToHost, s));
     OK_CUDA(cudaStreamSynchronize(s));
     out->agents = static_cast<uint64_t>(e->n_agents);
     out->alive = h[0], out->crashed = h[1], out->timed_out = h[2], out->done = h[3];
@@ -2433,10 +2246,11 @@ int ok_launch_stats(const OkEnv *e, OkLaunchStats *out)
     if (!e || !out)
         return fail(OK_ERR_INVALID_ARG, "NULL argument");
     out->kernel_launches = e->launches;
-    out->grid_blocks     = e->cfg.raycast_mode == OK_RAYCAST_BEAM ? e->grid_beam : e->grid;
+    const Schedule &sch  = e->cfg.raycast_mode == OK_RAYCAST_BEAM ? e->ag.beam : e->ag.tiles;
+    out->grid_blocks     = sch.grid;
     out->block_threads   = e->cfg.raycast_mode == OK_RAYCAST_BEAM ? e->beam_block : kBlock;
     out->smem_bytes      = static_cast<int32_t>(e->cfg.raycast_mode == OK_RAYCAST_BEAM ? e->smem_beam : e->smem);
-    out->tiles           = e->cfg.raycast_mode == OK_RAYCAST_BEAM ? e->n_tiles_beam : e->n_tiles;
+    out->tiles           = sch.n;
     return OK_SUCCESS;
 }
 }

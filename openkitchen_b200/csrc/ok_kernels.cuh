@@ -26,6 +26,7 @@
 
 #include "ok_beam.hpp"
 #include "ok_math.cuh"
+#include "ok_schedule.hpp"
 #include "ok_track.hpp"
 
 #include <cfloat>
@@ -51,13 +52,6 @@ static __device__ unsigned long long g_violations = 0; // one per translation un
 #define OK_CHECK(cond) ((void)0)
 #endif
 
-struct Tile
-{
-    int32_t track;
-    int32_t count;
-    int64_t begin;
-};
-
 struct TrackRef
 {
     uint64_t offset;      // byte offset of the blob in the arena (128-byte aligned)
@@ -69,7 +63,7 @@ struct TrackRef
     float    bx0, by0, binv_h, bbin_scale, brb;
     int32_t  bnx, bny, bnb;
     uint32_t boff_rows, boff_entries, boff_items, bn_rows, bn_chunks;
-    uint32_t seg_bytes;   // header + segments (+ the null segment) = the blob's prefix up to the grid words, multiple of 16
+    uint32_t seg_bytes;   // header + segments (+ the null segment) = the blob's prefix up to the grid words; no kernel reads it
     // what a crashed agent's auto-reset needs of the blob's header (phase 1 reads the GLOBAL blob: one trip to memory less)
     int32_t  n_points;
     uint32_t off_points, off_headings, pad;
@@ -174,24 +168,6 @@ __device__ __forceinline__ TrackView make_view(const uint8_t *blob)
     v.widths   = reinterpret_cast<const float *>(blob + h->off_widths);
     v.headings = reinterpret_cast<const float *>(blob + h->off_headings);
     v.safe     = reinterpret_cast<const float *>(blob + h->off_safe);
-    v.n_pts = h->n_points, v.n_seg = h->n_segments, v.nx = h->grid_nx, v.ny = h->grid_ny;
-    v.gx0 = h->grid_x0, v.gy0 = h->grid_y0, v.cell = h->cell, v.inv_cell = h->inv_cell;
-    return v;
-}
-
-// the SEGMENT-STAGED shape: header + segments from the staged prefix of the blob, everything else from the global blob
-__device__ __forceinline__ TrackView make_view_split(const uint8_t *staged_prefix, const uint8_t *gblob)
-{
-    const TrackHeader *h = reinterpret_cast<const TrackHeader *>(staged_prefix);
-    TrackView          v;
-    v.seg      = reinterpret_cast<const float4 *>(staged_prefix + h->off_segments);
-    v.words    = reinterpret_cast<const uint2 *>(gblob + h->off_words);
-    v.starts   = reinterpret_cast<const uint32_t *>(gblob + h->off_starts);
-    v.items    = reinterpret_cast<const uint16_t *>(gblob + h->off_items);
-    v.pts      = reinterpret_cast<const float2 *>(gblob + h->off_points);
-    v.widths   = reinterpret_cast<const float *>(gblob + h->off_widths);
-    v.headings = reinterpret_cast<const float *>(gblob + h->off_headings);
-    v.safe     = reinterpret_cast<const float *>(gblob + h->off_safe);
     v.n_pts = h->n_points, v.n_seg = h->n_segments, v.nx = h->grid_nx, v.ny = h->grid_ny;
     v.gx0 = h->grid_x0, v.gy0 = h->grid_y0, v.cell = h->cell, v.inv_cell = h->inv_cell;
     return v;
@@ -1219,28 +1195,18 @@ constexpr int kUnitsPerRefill = OK_UNITS; // units of work a lane does between t
 #ifndef OK_BEAM_TILE
 #define OK_BEAM_TILE 64 // agents per tile of the unstaged beam kernel
 #endif
-//  * SEGMENT-STAGED (kStaged = true, kSegOnly = true): TWO 512-thread CTAs per SM, each behind its own track's header +
-//    SEGMENTS only (47-90 KB of the blob's 77-143 KB, the only part the narrow phase reads per candidate); centre line,
-//    widths, headings and the rarely walked grid come from the global blob.  Twice as many, half as large tiles: while
-//    one CTA sits in a thread-per-agent phase the SM's other CTA casts rays, and the tiles-per-track quantisation halves.
-#ifndef OK_BEAM_BLOCK_SEG
-#define OK_BEAM_BLOCK_SEG 512
-#endif
 constexpr int kBeamBlockStaged   = 1024;
 constexpr int kBeamBlockUnstaged = OK_BEAM_BLOCK;
-constexpr int kBeamBlockSeg      = OK_BEAM_BLOCK_SEG;
-constexpr int kBeamSegCtasPerSm  = 1024 / OK_BEAM_BLOCK_SEG; // 64 registers per thread fill the register file
 // capacity of the CTA's queue of rays pass A leaves to pass B.  Tile-local ray indices are 16 bits, so a beam tile holds
 // at most 65,535 rays (the host caps the batch); a full queue only costs speed (see pass A).
-__host__ __device__ constexpr int beam_pend_cap(bool staged, bool seg_only = false)
+__host__ __device__ constexpr int beam_pend_cap(bool staged)
 {
-    return (staged && !seg_only) ? 8192 : 2048;
+    return staged ? 8192 : 2048;
 }
 // static shared memory of the beam kernel besides the staged track and the agent records (host: batch sizing)
-__host__ __device__ constexpr int beam_static_smem(bool staged, bool seg_only = false)
+__host__ __device__ constexpr int beam_static_smem(bool staged)
 {
-    return (staged ? (seg_only ? kBeamBlockSeg : kBeamBlockStaged) : kBeamBlockUnstaged) * (16 + 8) + 2 * beam_pend_cap(staged, seg_only) +
-           4 * (beam_pend_cap(staged, seg_only) / 32) + 128;
+    return (staged ? kBeamBlockStaged : kBeamBlockUnstaged) * (16 + 8) + 2 * beam_pend_cap(staged) + 4 * (beam_pend_cap(staged) / 32) + 128;
 }
 
 __device__ __forceinline__ unsigned long long global_timer()
@@ -1454,14 +1420,13 @@ template <> struct ActorArg<true>
 // kActor (ok_ppo_actor_step): the PPO racers' policy step runs as phase 0 of every tile -- the tile's agents choose their
 // actions from last tick's observations (actor_agent) and the kinematics read them from the action buffers -- so that a
 // rollout tick is ONE launch: at a few thousand agents a tick is latency, and two kernels pay it twice.
-template <int kBlock, bool kBeam, bool kStaged = true, bool kSegOnly = false, bool kActor = false>
-__global__ void __launch_bounds__(kBlock, (kBeam && !kStaged) ? OK_BEAM_MIN_CTAS : (kSegOnly ? 1024 / kBlock : 1))
+template <int kBlock, bool kBeam, bool kStaged = true, bool kActor = false>
+__global__ void __launch_bounds__(kBlock, (kBeam && !kStaged) ? OK_BEAM_MIN_CTAS : 1)
     step_kernel(const StepParams p, const typename ActorArg<kActor>::type q)
 {
-    static_assert(!kSegOnly || (kBeam && kStaged), "the segment-staged shape is a beam kernel");
     static_assert(!kActor || kBeam, "the fused actor is built for the beam kernels");
-    constexpr bool kStage   = !kBeam || kStaged; // the track (kSegOnly: its header + segments) is staged in shared memory with one TMA bulk copy
-    constexpr int  kPendCap = beam_pend_cap(kStaged, kSegOnly);
+    constexpr bool kStage   = !kBeam || kStaged; // the track is staged in shared memory with one TMA bulk copy
+    constexpr int  kPendCap = beam_pend_cap(kStaged);
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ uint16_t                      s_order[kBeam ? 1 : 1024]; // pool order of the rays (p.ray_order)
     __shared__ __align__(8) uint64_t         bar;
@@ -1544,14 +1509,11 @@ __global__ void __launch_bounds__(kBlock, (kBeam && !kStaged) ? OK_BEAM_MIN_CTAS
         // the bulk copy of the track runs under phase 1, which reads no staged data; it is awaited before the rays
         const uint8_t *gblob   = p.arena + tr.offset;
         const bool     restage = kStage && tl.track != staged;
-        const uint32_t stage_bytes = kSegOnly ? tr.seg_bytes : tr.bytes;
-        if (kSegOnly) // the records follow THIS track's segments (tracks differ by a factor of two: a fixed offset would waste it)
-            recs = reinterpret_cast<AgentRec *>(smem + ((tr.seg_bytes + 127u) & ~127u));
         if (restage && tid == 0)
         {
             fence_proxy_async();
-            mbar_expect_tx(&bar, stage_bytes);
-            tma_bulk_g2s(blob, gblob, stage_bytes, &bar);
+            mbar_expect_tx(&bar, tr.bytes);
+            tma_bulk_g2s(blob, gblob, tr.bytes, &bar);
         }
         BeamView bv;
         bv.valid = false;
@@ -1599,8 +1561,8 @@ __global__ void __launch_bounds__(kBlock, (kBeam && !kStaged) ? OK_BEAM_MIN_CTAS
         OK_TRACE(2);
         if (kBeam && p.tile_ns && tid == 0)
             s_tns[1] = global_timer();
-        const uint8_t  *track    = (kStage && !kSegOnly) ? blob : gblob; // where this tile reads its (whole) track from
-        const TrackView tv       = kSegOnly ? make_view_split(blob, gblob) : make_view(track);
+        const uint8_t  *track    = kStage ? blob : gblob; // where this tile reads its track from
+        const TrackView tv       = make_view(track);
         const int64_t   ray_base = tl.begin * R; // global index of the batch's first ray
         if (!kBeam)
         {
@@ -2613,10 +2575,5 @@ cudaError_t launch_step_actor(const StepParams &p, const ActorParams &q, int gri
 cudaError_t arm_step_actor(int smem_optin, int *max_dynamic);
 cudaError_t occupancy_step_unstaged(size_t smem_bytes, int *ctas_per_sm);
 cudaError_t violations_step_unstaged(unsigned long long *count);
-// the segment-staged beam kernel's (ok_step_segstaged.cu)
-cudaError_t launch_step_segstaged(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
-cudaError_t arm_step_segstaged(int smem_optin);
-cudaError_t occupancy_step_segstaged(size_t smem_bytes, int *ctas_per_sm);
-cudaError_t violations_step_segstaged(unsigned long long *count);
 
 } // namespace ok

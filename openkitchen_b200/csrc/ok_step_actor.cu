@@ -10,7 +10,7 @@ namespace ok
 {
 cudaError_t launch_step_actor(const StepParams &p, const ActorParams &q, int grid, size_t smem_bytes, cudaStream_t stream)
 {
-    step_kernel<kBeamBlockUnstaged, true, false, false, true><<<grid, kBeamBlockUnstaged, smem_bytes, stream>>>(p, q);
+    step_kernel<kBeamBlockUnstaged, true, false, true><<<grid, kBeamBlockUnstaged, smem_bytes, stream>>>(p, q);
     return cudaGetLastError();
 }
 
@@ -19,10 +19,10 @@ cudaError_t launch_step_actor(const StepParams &p, const ActorParams &q, int gri
 cudaError_t arm_step_actor(int smem_optin, int *max_dynamic)
 {
     cudaFuncAttributes fa{};
-    cudaError_t        rc = cudaFuncGetAttributes(&fa, step_kernel<kBeamBlockUnstaged, true, false, false, true>);
+    cudaError_t        rc = cudaFuncGetAttributes(&fa, step_kernel<kBeamBlockUnstaged, true, false, true>);
     if (rc != cudaSuccess)
         return rc;
     *max_dynamic = smem_optin - static_cast<int>(fa.sharedSizeBytes);
-    return cudaFuncSetAttribute(step_kernel<kBeamBlockUnstaged, true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, *max_dynamic);
+    return cudaFuncSetAttribute(step_kernel<kBeamBlockUnstaged, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, *max_dynamic);
 }
 } // namespace ok

@@ -333,17 +333,17 @@ def test_host_step_q16_rejects_pageable_memory():
         env.step_host(None, None, q, None, None)
 
 
-@pytest.mark.parametrize("kernel", ["staged", "unstaged", "segstaged"])
+@pytest.mark.parametrize("kernel", ["staged", "unstaged"])
 @pytest.mark.parametrize("mode", [ok.MOVE_VELOCITY, ok.MOVE_ACCELERATION])
 def test_both_beam_kernel_shapes_match_the_oracle(monkeypatch, kernel, mode):
-    """The beam kernel has three shapes (staged: one 1,024-thread CTA per SM behind the TMA-staged track; segment-staged:
-    two 512-thread CTAs per SM behind the track's segments only; unstaged: several 256-thread CTAs per SM reading the
-    track from global memory) and the host picks one by population size.  Forced each way on the same small population
-    -- with a sensor offset, auto-reset and all 23 tracks -- all must be the oracle, bit for bit."""
+    """The beam kernel has two shapes (staged: one 1,024-thread CTA per SM behind the TMA-staged track; unstaged: several
+    256-thread CTAs per SM reading the track from global memory) and the host picks one by population size.  Forced each
+    way on the same small population -- with a sensor offset, auto-reset and all 23 tracks -- both must be the oracle, bit
+    for bit."""
     monkeypatch.setenv("OK_BEAM_KERNEL", kernel)
     names = ok.track_names()
     env, ora, tid = make_pair(names, 23 * 9, 32, movement_mode=mode, reward_mode=ok.REWARD_Q_PROGRESS, auto_reset=1, sensor_offset=2.5)
-    assert env.launch_stats().block_threads == {"staged": 1024, "segstaged": 512, "unstaged": 256}[kernel]
+    assert env.launch_stats().block_threads == {"staged": 1024, "unstaged": 256}[kernel]
     pts = spread_points(ora, tid)
     env.reset(None, pts)
     ora.reset(None, pts)

@@ -153,7 +153,7 @@ def test_discounted_return_kernel_is_the_reference_loop():
         assert torch.equal(torch.from_numpy(got).cuda(), ref)
 
 
-@pytest.mark.parametrize("kernel,n", [("staged", 4096), ("unstaged", 700), ("segstaged", 4096)])
+@pytest.mark.parametrize("kernel,n", [("staged", 4096), ("unstaged", 700)])
 def test_one_launch_tick_equals_the_two_launches(monkeypatch, kernel, n):
     """ok_ppo_actor_step (policy step fused into the step kernel) against ok_ppo_actor + ok_launch_step on twin envs: every
     rollout record and every env buffer, bit for bit, in the beam kernel shape that has a fused instantiation (unstaged) and

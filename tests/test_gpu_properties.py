@@ -91,7 +91,7 @@ def test_tile_schedules_give_the_same_bits(monkeypatch):
         assert np.array_equal(a.read(name).view(np.uint8), c.read(name).view(np.uint8)), f"quarter-size tail: {name}"
 
 
-@pytest.mark.parametrize("kernel", ["staged", "segstaged"])
+@pytest.mark.parametrize("kernel", ["staged"])
 def test_feedback_tiling_changes_the_schedule_not_the_bits(monkeypatch, kernel):
     """ok_balance_schedule re-cuts the tiles from the tile times the kernel measured (the library also does it on its own
     after the 16th and 64th launch): the tiling changes, tiles stay within their tracks and cover every agent once, and
