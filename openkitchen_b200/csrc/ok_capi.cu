@@ -5,6 +5,7 @@
 
 #include "ok_beam.hpp"
 #include "ok_kernels.cuh"
+#include "ok_step.cuh"
 #include "ok_track.hpp"
 
 #include <nvtx3/nvToolsExt.h> // header-only; ranges only with OK_NVTX=1
@@ -87,10 +88,6 @@ struct DeviceGuard
     }
 };
 
-#ifndef OK_BLOCK
-#define OK_BLOCK 1024
-#endif
-constexpr int kBlock = OK_BLOCK;
 constexpr int kMaxBatchAgents = 256;
 
 struct BufferDesc
@@ -232,7 +229,7 @@ struct Agents
     // the beam kernel's batches are not limited by per-ray scratch: its own batch size, tiling and grid
     Schedule     beam;
     BeamFeedback feedback;
-    DevPtr<ok::FirstTile> first_beam; // the first tile of every CTA with its track record (ok_kernels.cuh)
+    DevPtr<ok::FirstTile> first_beam; // the first tile of every CTA with its track record (ok_device.cuh)
     int32_t               first_capacity{0};
     bool                  first_dirty{true};
     // ok_step_host's tiling: several tiles per CTA, so that a tile's observations cross PCIe while the next one is computed
@@ -284,7 +281,7 @@ struct OkEnv
     int                  actor_dyn_max{0};   // dynamic shared memory the fused actor + step kernel may use
     int32_t              batch_agents_beam{0};
     int32_t              ctas_per_sm_beam{1};
-    bool                 beam_staged{true}; // which shape of the beam kernel this population runs (ok_kernels.cuh)
+    bool                 beam_staged{true}; // which shape of the beam kernel this population runs (ok_step.cuh)
     int32_t              beam_block{1024};
     int                  smem_optin{0};
     std::vector<int32_t> h_track_id;
@@ -731,16 +728,13 @@ int check_ready(OkEnv *e)
     return OK_SUCCESS;
 }
 
-// cudaFuncAttributeMaxDynamicSharedMemorySize of both step kernels = everything the device allows.  Idempotent.
+// cudaFuncAttributeMaxDynamicSharedMemorySize of the grid, staged and actor step kernels = everything the device allows.
+// Idempotent.
 int arm_shared_memory_limit(OkEnv *e)
 {
-    cudaFuncAttributes fa{};
-    OK_CUDA(cudaFuncGetAttributes(&fa, ok::step_kernel<kBlock, false>));
-    OK_CUDA(cudaFuncSetAttribute(ok::step_kernel<kBlock, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 e->smem_optin - static_cast<int>(fa.sharedSizeBytes)));
-    OK_CUDA(cudaFuncGetAttributes(&fa, ok::step_kernel<ok::kBeamBlockStaged, true, true>));
-    OK_CUDA(cudaFuncSetAttribute(ok::step_kernel<ok::kBeamBlockStaged, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 e->smem_optin - static_cast<int>(fa.sharedSizeBytes)));
+    int max_dynamic = 0;
+    OK_CUDA(ok::arm_step_grid(e->smem_optin, &max_dynamic));
+    OK_CUDA(ok::arm_step_staged(e->smem_optin, &max_dynamic));
     OK_CUDA(ok::arm_step_actor(e->smem_optin, &e->actor_dyn_max));
     return OK_SUCCESS;
 }
@@ -900,13 +894,12 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
             OK_CUDA(ok::launch_step_actor(p, *actor, ag.beam.grid, p.actor_smem_off + actor_smem, s));
         }
         else if (e->beam_staged)
-            ok::step_kernel<ok::kBeamBlockStaged, true, true><<<grid, ok::kBeamBlockStaged, e->smem_beam, s>>>(p, ok::NoActor{});
+            OK_CUDA(ok::launch_step_staged(p, grid, e->smem_beam, s));
         else
             OK_CUDA(ok::launch_step_unstaged(p, ag.beam.grid, e->smem_beam, s));
     }
     else
-        ok::step_kernel<kBlock, false><<<ag.tiles.grid, kBlock, e->smem, s>>>(p, ok::NoActor{});
-    OK_CUDA(cudaGetLastError());
+        OK_CUDA(ok::launch_step_grid(p, ag.tiles.grid, e->smem, s));
     if (p.act_ready)
     { // enqueued AFTER the launch: the kernel is already running its first tiles while the host issues these
         const size_t bytes = sizeof(float) * static_cast<size_t>(e->n_agents);
@@ -1213,7 +1206,7 @@ int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg,
         e->batch_agents = static_cast<int32_t>(a);
         e->smem         = blob + ok::batch_smem_bytes(e->batch_agents, rays);
         // beam kernel: one 64-byte record per agent; phases 1 / 4 run a thread per agent, so at most one block of agents.
-        // Which shape (ok_kernels.cuh): the staged one for throughput, the unstaged one when the population is too small
+        // Which shape (ok_step.cuh): the staged one for throughput, the unstaged one when the population is too small
         // to give every SM a worthwhile tile (OK_BEAM_KERNEL = staged | unstaged overrides).
         // measured (tools/bench_small.py, tools/bench_c4.py): the unstaged shape is ahead below ~2,000 agents of 32 rays, and at
         // 4,096 agents of 5 rays (a PPO rollout tick: 0.0289 vs 0.0300 ms, 0.0262 with the policy step fused in), behind at
@@ -1221,7 +1214,7 @@ int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg,
         e->beam_staged = n >= 2048 && n * rays > 24576;
         if (const char *env = std::getenv("OK_BEAM_KERNEL"))
             e->beam_staged = std::strcmp(env, "unstaged") != 0 && (std::strcmp(env, "staged") == 0 || e->beam_staged);
-        e->beam_block = e->beam_staged ? ok::kBeamBlockStaged : ok::kBeamBlockUnstaged;
+        e->beam_block = ok::beam_block(e->beam_staged);
         int64_t ab;
         int     capb;
         if (e->beam_staged)
@@ -2145,11 +2138,13 @@ int ok_debug_violations(OkEnv *e, uint64_t *count, int32_t *checks_compiled_in)
         return fail(OK_ERR_NO_DEVICE, "no device");
     DeviceGuard g(e->cfg.device);
     OK_CUDA(cudaDeviceSynchronize());
-    unsigned long long v = 0, u = 0;
-    OK_CUDA(cudaMemcpyFromSymbol(&v, ok::g_violations, sizeof v));
-    OK_CUDA(ok::violations_step_unstaged(&u));
+    unsigned long long staged = 0, unstaged = 0, actor = 0, grid = 0;
+    OK_CUDA(ok::violations_step_staged(&staged));
+    OK_CUDA(ok::violations_step_unstaged(&unstaged));
+    OK_CUDA(ok::violations_step_actor(&actor));
+    OK_CUDA(ok::violations_step_grid(&grid));
     if (count)
-        *count = v + u;
+        *count = staged + unstaged + actor + grid;
     if (checks_compiled_in)
         *checks_compiled_in = OK_CHECKED;
     return OK_SUCCESS;
@@ -2248,7 +2243,7 @@ int ok_launch_stats(const OkEnv *e, OkLaunchStats *out)
     out->kernel_launches = e->launches;
     const Schedule &sch  = e->cfg.raycast_mode == OK_RAYCAST_BEAM ? e->ag.beam : e->ag.tiles;
     out->grid_blocks     = sch.grid;
-    out->block_threads   = e->cfg.raycast_mode == OK_RAYCAST_BEAM ? e->beam_block : kBlock;
+    out->block_threads   = e->cfg.raycast_mode == OK_RAYCAST_BEAM ? e->beam_block : ok::kGridBlock;
     out->smem_bytes      = static_cast<int32_t>(e->cfg.raycast_mode == OK_RAYCAST_BEAM ? e->smem_beam : e->smem);
     out->tiles           = sch.n;
     return OK_SUCCESS;

@@ -1,22 +1,18 @@
-// ok_step_unstaged.cu -- the UNSTAGED shape of the beam kernel (ok_kernels.cuh: several 256-thread CTAs per SM, the track
-// read from global memory) in a translation unit of its own.  Sharing a unit with the staged shape made ptxas share the
-// out-of-line device functions (grid-walk fallback, literal predicate) between two kernels with different launch bounds
-// and address spaces, and the staged kernel -- the throughput path -- ran at 0.139 ms per tick instead of 0.095.
-#define OK_STEP_KERNEL_ONLY 1
-#include "ok_kernels.cuh"
+// ok_step_unstaged.cu -- the UNSTAGED shape of the beam kernel (ok_step.cuh: several 256-thread CTAs per SM, the track
+// read from global memory) in a translation unit of its own.
+#include "ok_step.cuh"
 
 namespace ok
 {
 cudaError_t launch_step_unstaged(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream)
 {
-    step_kernel<kBeamBlockUnstaged, true, false><<<grid, kBeamBlockUnstaged, smem_bytes, stream>>>(p, NoActor{});
+    beam_step_kernel<false><<<grid, kBeamBlockUnstaged, smem_bytes, stream>>>(p, NoActor{});
     return cudaGetLastError();
 }
 
 cudaError_t occupancy_step_unstaged(size_t smem_bytes, int *ctas_per_sm)
 {
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, step_kernel<kBeamBlockUnstaged, true, false>, kBeamBlockUnstaged,
-                                                         smem_bytes);
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, beam_step_kernel<false>, kBeamBlockUnstaged, smem_bytes);
 }
 
 cudaError_t violations_step_unstaged(unsigned long long *count)

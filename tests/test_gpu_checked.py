@@ -1,10 +1,12 @@
 """GPU: index self-checks.  With the product library this only asserts that the checks are compiled out; run through
 tools/checked_build.sh (OK_B200_LIB = a -DOK_CHECKED=1 build) the same workload range-checks every table row, chunk,
-segment, ray and agent index in the beam kernel and must count zero violations (the pool's compute-sanitizer is closed)."""
+segment, ray and agent index in the beam kernels and must count zero violations (the pool's compute-sanitizer is closed)."""
 import numpy as np
 import pytest
+import torch
 
 import openkitchen_b200 as ok
+from openkitchen_b200.rollout import FusedActorRollout
 
 pytestmark = pytest.mark.gpu
 
@@ -27,5 +29,27 @@ def test_no_index_leaves_its_array():
         count, compiled_in = env.debug_violations()
         assert count == 0, f"{count} out-of-range indices"
         env.close()
+    if not compiled_in:
+        assert ok.LIB_PATH.endswith("libopenkitchen_b200.so")
+
+
+def test_no_index_leaves_its_array_in_the_fused_actor_tick():
+    """The unstaged beam kernel with the PPO racers' policy step fused in (one launch per tick) has a self-check counter
+    of its own: a small population selects that shape."""
+    torch.manual_seed(0)
+    l1, l2 = torch.nn.Linear(5, 128).cuda(), torch.nn.Linear(128, 3).cuda()
+    table = torch.tensor([[60.0, 0.0], [30.0, 5.0], [30.0, -5.0]], device="cuda")
+    n = 300
+    env = ok.BatchEnv(["Monza", "Zandvoort"], n, rays=np.array([-70, -30, 0, 30, 70], dtype=np.float32),
+                      reward_mode=ok.REWARD_CONSTANT, auto_reset=1)
+    env.reset(None, torch.from_numpy((np.arange(n) * 53 % 600).astype(np.int32)).cuda())
+    env.cast_rays()
+    before = env.env.launch_stats().kernel_launches
+    FusedActorRollout(env, l1, l2, table, steps=40, sample=True, one_launch=True).run_eager()
+    torch.cuda.synchronize()
+    assert env.env.launch_stats().kernel_launches - before == 41  # one launch per tick: the fused kernel ran
+    count, compiled_in = env.env.debug_violations()
+    assert count == 0, f"{count} out-of-range indices"
+    env.close()
     if not compiled_in:
         assert ok.LIB_PATH.endswith("libopenkitchen_b200.so")

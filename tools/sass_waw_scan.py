@@ -4,7 +4,7 @@ the write has to wait for the load (write-after-write on the scoreboard), i.e. t
 issued.  Found this way: pass A's 128-bit table-entry load whose dead third word ptxas reused for a flag byte (12.6 % of all
 stall samples on one PRMT, DESIGN.md 7).  Predicated select patterns (load a default, overwrite it under a predicate) show up
 too and are harmless when the load is a shared-memory one.
-usage: python tools/sass_waw_scan.py openkitchen_b200/lib/libopenkitchen_b200.so step_kernelILi1024ELb1ELb1ELb0ELb0"""
+usage: python tools/sass_waw_scan.py openkitchen_b200/lib/libopenkitchen_b200.so beam_step_kernelILb1ELb0E"""
 import re,subprocess,sys
 lib=sys.argv[1]; pat=sys.argv[2]
 out=subprocess.run(["cuobjdump","-sass",lib],capture_output=True,text=True).stdout
