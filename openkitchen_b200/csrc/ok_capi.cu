@@ -1,9 +1,10 @@
 // ok_capi.cu -- implementation of the C ABI (include/openkitchen_b200.h) over the sm_100a kernels.
-// Host side of the product: owns device memory, uploads the tilings (ok_schedule.hpp), launches.  No CPU
-// fallback exists: without a CUDA device every compute entry point returns OK_ERR_NO_DEVICE.
+// Host side of the product: owns device memory, allocates and uploads what the sizing and tilings of ok_schedule.hpp
+// decide, asks ok_beam_cache.hpp for the beam tables, launches.  No CPU fallback exists: without a CUDA device every
+// compute entry point returns OK_ERR_NO_DEVICE.
 #include "../../include/openkitchen_b200.h"
 
-#include "ok_beam.hpp"
+#include "ok_beam_cache.hpp"
 #include "ok_kernels.cuh"
 #include "ok_step.cuh"
 #include "ok_track.hpp"
@@ -17,15 +18,10 @@
 #include <cstdlib>
 #include <cstring>
 #include <chrono>
-#include <fcntl.h>
-#include <map>
-#include <sys/stat.h>
-#include <thread>
-#include <type_traits>
-#include <unistd.h>
 #include <memory>
-#include <mutex>
+#include <optional>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 namespace
@@ -69,26 +65,7 @@ struct NvtxRange
     NvtxRange &operator=(const NvtxRange &) = delete;
 };
 
-struct DeviceGuard
-{
-    int  prev{-1};
-    bool active{false};
-    explicit DeviceGuard(int dev)
-    {
-        if (dev >= 0 && cudaGetDevice(&prev) == cudaSuccess && prev != dev)
-        {
-            cudaSetDevice(dev);
-            active = true;
-        }
-    }
-    ~DeviceGuard()
-    {
-        if (active)
-            cudaSetDevice(prev);
-    }
-};
-
-constexpr int kMaxBatchAgents = 256;
+using ok::DeviceGuard;
 
 struct BufferDesc
 {
@@ -121,31 +98,7 @@ size_t dtype_size(int32_t dt)
 {
     return dt == OK_DTYPE_U8 ? 1 : 4;
 }
-} // namespace
 
-// a beam table in device memory, shared by every env of the process on that device
-struct DeviceBlob
-{
-    uint8_t *ptr{nullptr};
-    size_t   bytes{0};
-    int      device{0};
-    DeviceBlob(uint8_t *p, size_t b, int d) : ptr(p), bytes(b), device(d)
-    {
-    }
-    DeviceBlob(const DeviceBlob &) = delete;
-    DeviceBlob &operator=(const DeviceBlob &) = delete;
-    ~DeviceBlob()
-    {
-        if (ptr)
-        {
-            DeviceGuard g(device);
-            cudaFree(ptr); // an error after the runtime has shut down is harmless
-        }
-    }
-};
-
-namespace
-{
 // owners of the CUDA resources of an env: freed (destroyed) when the owner is reset or goes away
 struct CudaFree
 {
@@ -205,6 +158,12 @@ struct Schedule
     int32_t          n{0}, grid{0};
 };
 
+// the grid of a tiling of `tiles` tiles run by `ctas` CTAs at most
+int32_t schedule_grid(int ctas, int32_t tiles)
+{
+    return std::max(1, std::min(ctas, tiles));
+}
+
 // cost feedback for the beam tiling (ok_balance_schedule): the kernel leaves every tile's ray-phase / other time in
 // d_tile_ns, and reweigh_runs re-cuts the tiles from them.  The table is allocated once, at `capacity` tiles, and
 // rewritten in place: a CUDA graph captured earlier keeps reading it.
@@ -221,6 +180,7 @@ struct BeamFeedback
 // everything ok_alloc_agents creates for one population: ok_alloc_agents and free_agents replace it as a whole
 struct Agents
 {
+    ok::Sizing       sizing; // kernel shapes, batch sizes and the knob-derived flags (ok_schedule.hpp)
     DevPtr<uint8_t>  slab;
     DevPtr<float>    ray_deg;
     DevPtr<uint16_t> ray_order;
@@ -262,8 +222,8 @@ struct OkEnv
     size_t        max_blob_used{0};
     bool          arena_dirty{true};
     // beam tables (OK_RAYCAST_BEAM): one blob per track in global memory
-    std::vector<std::shared_ptr<const std::vector<uint8_t>>> beams;     // host copies (host-only envs, ok_beam_lookup)
-    std::vector<std::shared_ptr<const struct DeviceBlob>>    beams_dev; // what the kernels read; shared between envs
+    std::vector<ok::HostTable>   beams;     // host copies (ok_beam_lookup)
+    std::vector<ok::DeviceTable> beams_dev; // what the kernels read; shared between envs
     bool          arena_has_beams{false};
     std::vector<ok::TrackRef> h_track_refs; // host copy of d_track_refs
     // agents
@@ -272,17 +232,9 @@ struct OkEnv
     Agents               ag;
     void                *d_buf[OK_BUF_COUNT]{};
     size_t               buf_off[OK_BUF_COUNT]{}; // offsets of the buffers inside the slab
-    int32_t              batch_agents{0};
-    int                  auto_balance{1};
     float                balance_before{0.0f}, balance_after{0.0f}; // predicted slowest-tile / mean-tile cost of the last rebalancing
-    int32_t              e2e_flushers{0};
     uint32_t             flag_epoch{0};
-    bool                 act_stage_on{true}; // OK_ACT_STAGE=0: every tile reads the mapping (A/B)
     int                  actor_dyn_max{0};   // dynamic shared memory the fused actor + step kernel may use
-    int32_t              batch_agents_beam{0};
-    int32_t              ctas_per_sm_beam{1};
-    bool                 beam_staged{true}; // which shape of the beam kernel this population runs (ok_step.cuh)
-    int32_t              beam_block{1024};
     int                  smem_optin{0};
     std::vector<int32_t> h_track_id;
     // created on first use, kept until ok_destroy
@@ -295,7 +247,6 @@ struct OkEnv
     Event                      ev_fork, ev_join;
     // stats
     uint64_t launches{0};
-    size_t   smem{0}, smem_beam{0};
 };
 
 namespace
@@ -319,248 +270,6 @@ void free_agents(OkEnv *e)
     e->n_agents = 0, e->rays = 0;
 }
 
-// Beam tables are pure functions of (segments, cell, bins, range) and take ~0.1-1 s of host time per track.
-// Two caches: one per process (envs over the same tracks share a table), and one on disk
-// ($OK_BEAM_CACHE_DIR, default $TMPDIR/openkitchen_b200-cache-<uid>; OK_BEAM_CACHE=0 disables it) so that the ranks
-// of one box -- which all need every table -- build each table once between them instead of once each.
-uint64_t fnv1a(const void *ptr, size_t n, uint64_t h = 1469598103934665603ull)
-{
-    const uint8_t *b = static_cast<const uint8_t *>(ptr);
-    for (size_t i = 0; i < n; ++i)
-        h = (h ^ b[i]) * 1099511628211ull;
-    return h;
-}
-
-std::string beam_cache_dir()
-{
-    if (const char *off = std::getenv("OK_BEAM_CACHE"))
-        if (std::atoi(off) == 0)
-            return "";
-    std::string dir;
-    if (const char *d = std::getenv("OK_BEAM_CACHE_DIR"))
-        dir = d;
-    else
-    {
-        const char *tmp = std::getenv("TMPDIR");
-        dir             = std::string(tmp && *tmp ? tmp : "/tmp") + "/openkitchen_b200-cache-" + std::to_string(getuid());
-    }
-    ::mkdir(dir.c_str(), 0700);
-    // the tables loaded from here steer device reads: only a real directory that belongs to this user and that nobody
-    // else can write is trusted; anything else (a planted directory or symlink in a shared /tmp) disables the cache
-    struct stat st
-    {
-    };
-    if (::lstat(dir.c_str(), &st) != 0 || !S_ISDIR(st.st_mode) || st.st_uid != getuid() || (st.st_mode & (S_IWGRP | S_IWOTH)))
-        return "";
-    return dir;
-}
-
-struct BeamFileHeader
-{
-    char     magic[8]; // "OKBEAM02"
-    uint64_t bytes, checksum;
-};
-
-bool beam_file_load(const std::string &path, std::vector<uint8_t> &blob, int32_t n_segments)
-{
-    FILE *f = std::fopen(path.c_str(), "rb");
-    if (!f)
-        return false;
-    BeamFileHeader h{};
-    bool           ok = std::fread(&h, sizeof h, 1, f) == 1 && std::memcmp(h.magic, "OKBEAM02", 8) == 0 && h.bytes >= sizeof(ok::BeamHeader) &&
-              h.bytes < (1ull << 32);
-    if (ok)
-    {
-        blob.resize(h.bytes);
-        ok = std::fread(blob.data(), 1, h.bytes, f) == h.bytes && fnv1a(blob.data(), blob.size()) == h.checksum;
-        // the kernels trust a table's indices: one that did not come from this process is checked structurally first
-        std::string why;
-        ok = ok && ok::beam_validate(blob, n_segments, why);
-    }
-    std::fclose(f);
-    if (!ok)
-        blob.clear();
-    return ok;
-}
-
-void beam_file_save(const std::string &path, const std::vector<uint8_t> &blob)
-{
-    const std::string tmp = path + ".tmp." + std::to_string(getpid());
-    FILE             *f   = std::fopen(tmp.c_str(), "wb");
-    if (!f)
-        return;
-    BeamFileHeader h{};
-    std::memcpy(h.magic, "OKBEAM02", 8);
-    h.bytes    = blob.size();
-    h.checksum = fnv1a(blob.data(), blob.size());
-    const bool ok = std::fwrite(&h, sizeof h, 1, f) == 1 && std::fwrite(blob.data(), 1, blob.size(), f) == blob.size();
-    std::fclose(f);
-    if (ok && std::rename(tmp.c_str(), path.c_str()) == 0)
-        return;
-    std::remove(tmp.c_str());
-}
-
-std::string beam_key(const ok::Track &t, const ok::BeamConfig &cfg)
-{
-    uint64_t h = fnv1a(t.segments.data(), t.segments.size() * sizeof(float));
-    h          = fnv1a(t.x.data(), t.x.size() * sizeof(float), h);
-    h          = fnv1a(t.y.data(), t.y.size() * sizeof(float), h);
-    h          = fnv1a(t.w_left.data(), t.w_left.size() * sizeof(float), h);
-    h          = fnv1a(t.w_right.data(), t.w_right.size() * sizeof(float), h);
-    char key[128];
-    std::snprintf(key, sizeof key, "v%d-%016llx-%zu-%g-%d-%g", ok::kBeamBuildVersion, static_cast<unsigned long long>(h),
-                  t.segments.size(), static_cast<double>(cfg.cell), cfg.bins, static_cast<double>(cfg.range));
-    return key;
-}
-
-std::mutex                                                          g_beam_mu;
-std::map<std::string, std::shared_ptr<const std::vector<uint8_t>>> g_beam_cache;
-
-std::shared_ptr<const std::vector<uint8_t>> beam_cached(const std::string &key)
-{
-    std::lock_guard<std::mutex> lock(g_beam_mu);
-    auto                        it = g_beam_cache.find(key);
-    return it == g_beam_cache.end() ? nullptr : it->second;
-}
-
-std::shared_ptr<const std::vector<uint8_t>> beam_remember(const std::string &key, std::shared_ptr<std::vector<uint8_t>> blob)
-{
-    std::lock_guard<std::mutex> lock(g_beam_mu);
-    size_t                      held = blob->size();
-    for (auto &kv : g_beam_cache)
-        held += kv.second->size();
-    if (held > (size_t{12} << 30)) // envs keep their own references; this only bounds what the cache itself pins
-        g_beam_cache.clear();
-    g_beam_cache[key] = blob;
-    return blob;
-}
-
-// `wait` = false: return nullptr (no error) when another process holds the track's build lock, so that the caller
-// can build other tracks in the meantime; `wait` = true: wait for that process's file, or build after a timeout.
-std::shared_ptr<const std::vector<uint8_t>> beam_table_for(const ok::Track &t, const ok::BeamConfig &cfg, bool wait, std::string &err)
-{
-    const std::string key = beam_key(t, cfg);
-    if (auto hit = beam_cached(key))
-        return hit;
-    auto              blob = std::make_shared<std::vector<uint8_t>>();
-    const std::string dir  = beam_cache_dir();
-    const std::string path = dir.empty() ? "" : dir + "/beam-" + key + ".bin", lock = path + ".lock";
-    bool              locked = false;
-    if (!path.empty())
-    {
-        if (beam_file_load(path, *blob, t.n_segments()))
-            return beam_remember(key, blob);
-        const int fd = ::open(lock.c_str(), O_CREAT | O_EXCL | O_WRONLY, 0600);
-        if (fd >= 0)
-        {
-            ::close(fd);
-            locked = true;
-        }
-        else
-        {
-            struct stat st
-            {
-            };
-            const bool stale = ::stat(lock.c_str(), &st) == 0 && std::time(nullptr) - st.st_mtime > 300;
-            if (stale)
-                std::remove(lock.c_str());
-            else if (!wait)
-                return nullptr; // someone else is building it
-            else
-                for (int i = 0; i < 2400 && ::stat(lock.c_str(), &st) == 0; ++i) // up to two minutes
-                {
-                    std::this_thread::sleep_for(std::chrono::milliseconds(50));
-                    if (beam_file_load(path, *blob, t.n_segments()))
-                        return beam_remember(key, blob);
-                }
-            if (beam_file_load(path, *blob, t.n_segments()))
-                return beam_remember(key, blob);
-        }
-    }
-    const bool built = ok::build_beam_table(t, cfg, *blob, err);
-    if (built && !path.empty())
-        beam_file_save(path, *blob);
-    if (locked)
-        std::remove(lock.c_str());
-    if (!built)
-    {
-        if (err.empty())
-            err = "beam table build failed";
-        return nullptr;
-    }
-    return beam_remember(key, blob);
-}
-
-// never destroyed: at process exit the CUDA runtime may already be gone when static destructors run
-std::map<std::string, std::shared_ptr<const DeviceBlob>> &g_beam_dev_cache = *new std::map<std::string, std::shared_ptr<const DeviceBlob>>();
-
-// The track's table in the memory of `device`: built there by the kernel builder (ok_beam_gpu.cu); OK_BEAM_BUILDER=cpu
-// (or a failure of the device builder) builds it on the host instead and uploads it.  `wait` as in beam_table_for.
-std::shared_ptr<const DeviceBlob> beam_device_table_for(const ok::Track &t, const ok::BeamConfig &cfg, int device, bool wait,
-                                                        std::string &err)
-{
-    const std::string key = beam_key(t, cfg) + "@" + std::to_string(device);
-    {
-        std::lock_guard<std::mutex> lock(g_beam_mu);
-        auto                        it = g_beam_dev_cache.find(key);
-        if (it != g_beam_dev_cache.end())
-            return it->second;
-    }
-    std::shared_ptr<const DeviceBlob> out;
-    const char                       *force = std::getenv("OK_BEAM_BUILDER");
-    if (!(force && std::strcmp(force, "cpu") == 0))
-    {
-        uint8_t    *d = nullptr;
-        size_t      bytes = 0;
-        std::string gerr;
-        if (ok::build_beam_table_device(t, cfg, device, &d, &bytes, gerr))
-            out = std::make_shared<DeviceBlob>(d, bytes, device);
-        else if (force && std::strcmp(force, "gpu") == 0)
-        {
-            err = "device builder: " + gerr;
-            return nullptr;
-        }
-    }
-    if (!out)
-    {
-        auto host = beam_table_for(t, cfg, wait, err);
-        if (!host)
-            return nullptr;
-        DeviceGuard g(device);
-        uint8_t    *d = nullptr;
-        if (cudaMalloc(reinterpret_cast<void **>(&d), host->size()) != cudaSuccess ||
-            cudaMemcpy(d, host->data(), host->size(), cudaMemcpyHostToDevice) != cudaSuccess)
-        {
-            err = std::string("beam table upload: ") + cudaGetErrorString(cudaGetLastError());
-            if (d)
-                cudaFree(d);
-            return nullptr;
-        }
-        out = std::make_shared<DeviceBlob>(d, host->size(), device);
-    }
-    std::lock_guard<std::mutex> lock(g_beam_mu);
-    size_t                      held = out->bytes;
-    for (auto &kv : g_beam_dev_cache)
-        held += kv.second->bytes;
-    if (held > (size_t{24} << 30)) // envs keep their own references; this only bounds what the cache itself pins
-        g_beam_dev_cache.clear();
-    g_beam_dev_cache[key] = out;
-    return out;
-}
-
-ok::BeamConfig beam_config(const OkEnv *e)
-{
-    ok::BeamConfig c;
-    c.cell  = e->cfg.beam_cell;
-    c.bins  = e->cfg.beam_bins;
-    c.range = 200.0f; // Agent::kSensorRange; a larger OkConfig::sensor_range stays exact through the grid walk
-    if (const char *env = std::getenv("OK_BEAM_THREADS"))
-        c.threads = std::atoi(env);
-    else if (const char *lws = std::getenv("LOCAL_WORLD_SIZE")) // torchrun: the ranks of a box share its cores
-        c.threads = std::max(1, static_cast<int>(std::thread::hardware_concurrency()) / std::max(1, std::atoi(lws)));
-    return c;
-}
-
 int ensure_arena(OkEnv *e)
 {
     const bool want_beams = e->cfg.raycast_mode == OK_RAYCAST_BEAM;
@@ -570,51 +279,11 @@ int ensure_arena(OkEnv *e)
     std::vector<ok::TrackRef> refs;
     size_t                    total = 0;
     e->max_blob_used                = 0;
-    e->beams_dev.resize(e->tracks.size());
-    const bool verbose = std::getenv("OK_BEAM_VERBOSE") != nullptr;
-    const auto t_0     = std::chrono::steady_clock::now();
     if (want_beams)
     {
-        { // the tables nobody has built yet in this process, all at once: the device builder pipelines them
-            const char *force = std::getenv("OK_BEAM_BUILDER");
-            std::vector<const ok::Track *> todo;
-            std::vector<std::string>       keys;
-            if (!(force && std::strcmp(force, "cpu") == 0))
-            {
-                std::lock_guard<std::mutex> lock(g_beam_mu);
-                for (size_t i = 0; i < e->tracks.size(); ++i)
-                {
-                    const std::string key = beam_key(e->tracks[i], beam_config(e)) + "@" + std::to_string(e->cfg.device);
-                    if (!e->beams_dev[i] && !g_beam_dev_cache.count(key) && std::find(keys.begin(), keys.end(), key) == keys.end())
-                        todo.push_back(&e->tracks[i]), keys.push_back(key);
-                }
-            }
-            if (todo.size() > 1)
-            {
-                std::vector<uint8_t *> blobs;
-                std::vector<size_t>    sizes;
-                ok::build_beam_tables_device(todo, beam_config(e), e->cfg.device, blobs, sizes);
-                std::lock_guard<std::mutex> lock(g_beam_mu);
-                for (size_t k = 0; k < todo.size(); ++k)
-                    if (blobs[k])
-                        g_beam_dev_cache[keys[k]] = std::make_shared<DeviceBlob>(blobs[k], sizes[k], e->cfg.device);
-            }
-        }
-        // (host-built tables only) first every table nobody else is building, then the ones other ranks were busy with
-        for (int pass = 0; pass < 2; ++pass)
-            for (size_t i = 0; i < e->tracks.size(); ++i)
-                if (!e->beams_dev[i])
-                {
-                    std::string err;
-                    e->beams_dev[i] = beam_device_table_for(e->tracks[i], beam_config(e), e->cfg.device, pass == 1, err);
-                    if (!e->beams_dev[i] && (pass == 1 || !err.empty()))
-                        return fail(OK_ERR_INVALID_ARG, "beam table: " + err);
-                }
-        const auto t_1 = std::chrono::steady_clock::now();
-        ok::beam_builder_release(); // the device builder's scratch pool (kept from track to track) is no longer needed
-        if (verbose)
-            std::fprintf(stderr, "[ensure_arena] tables %.1f ms, pool release %.1f ms\n", std::chrono::duration<double, std::milli>(t_1 - t_0).count(),
-                         std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_1).count());
+        std::string err;
+        if (int rc = ok::beam_device_tables(e->tracks, ok::beam_config(e->cfg.beam_cell, e->cfg.beam_bins), e->cfg.device, e->beams_dev, err))
+            return fail(rc, err);
     }
     for (size_t i = 0; i < e->tracks.size(); ++i)
     {
@@ -694,7 +363,7 @@ ok::StepParams base_params(OkEnv *e)
     p.n_tiles   = e->ag.tiles.n;
     p.n_agents  = e->n_agents;
     p.rays      = e->rays;
-    p.batch_agents      = e->batch_agents;
+    p.batch_agents      = e->ag.sizing.batch_agents;
     p.smem_blob_bytes   = static_cast<uint32_t>((e->max_blob_used + 127) / 128 * 128);
     p.ray_order         = e->ag.ray_order.get();
     p.sched             = e->ag.sched.get();
@@ -717,12 +386,21 @@ ok::StepParams base_params(OkEnv *e)
     return p;
 }
 
-int check_ready(OkEnv *e)
+// an env that can compute: not NULL and created with a device
+int check_device(const OkEnv *e)
 {
     if (!e)
         return fail(OK_ERR_INVALID_ARG, "env is NULL");
     if (!e->has_device)
         return fail(OK_ERR_NO_DEVICE, "this env was created without a CUDA device (device = -1): no compute entry point is available");
+    return OK_SUCCESS;
+}
+
+// ... with agents
+int check_ready(OkEnv *e)
+{
+    if (int rc = check_device(e))
+        return rc;
     if (e->n_agents <= 0)
         return fail(OK_ERR_STATE, "ok_alloc_agents has not been called");
     return OK_SUCCESS;
@@ -739,14 +417,13 @@ int arm_shared_memory_limit(OkEnv *e)
     return OK_SUCCESS;
 }
 
-// Uploads `tiles` as schedule `s`, in a table of room for `capacity` tiles (at least as many as there are), run by
-// `ctas` CTAs at most.
-int upload_schedule(Schedule &s, const std::vector<ok::Tile> &tiles, size_t capacity, int ctas)
+// Uploads tiling `t` as schedule `s`
+int upload_schedule(Schedule &s, const ok::Tiling &t)
 {
-    OK_CUDA(dev_alloc(s.d, std::max(capacity, tiles.size())));
-    OK_CUDA(cudaMemcpy(s.d.get(), tiles.data(), sizeof(ok::Tile) * tiles.size(), cudaMemcpyHostToDevice));
-    s.n    = static_cast<int32_t>(tiles.size());
-    s.grid = std::max(1, std::min(ctas, s.n));
+    OK_CUDA(dev_alloc(s.d, std::max(t.capacity, t.tiles.size())));
+    OK_CUDA(cudaMemcpy(s.d.get(), t.tiles.data(), sizeof(ok::Tile) * t.tiles.size(), cudaMemcpyHostToDevice));
+    s.n    = static_cast<int32_t>(t.tiles.size());
+    s.grid = schedule_grid(t.ctas, s.n);
     return OK_SUCCESS;
 }
 
@@ -799,7 +476,7 @@ int rebalance_beam_tiles(OkEnv *e, cudaStream_t s)
     fb.tiles       = std::move(rw.tiles);
     ag.first_dirty = true;
     ag.beam.n      = static_cast<int32_t>(fb.tiles.size());
-    ag.beam.grid   = std::max(1, std::min(e->num_sms * e->ctas_per_sm_beam, ag.beam.n));
+    ag.beam.grid   = schedule_grid(e->num_sms * ag.sizing.ctas_per_sm_beam, ag.beam.n);
     // at once, not at the next launch: a CUDA graph captured earlier reads both arrays at every replay, and they must agree
     return ag.first_beam ? upload_first_tiles(e, s) : OK_SUCCESS;
 }
@@ -833,7 +510,7 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
     if (e->cfg.raycast_mode == OK_RAYCAST_BEAM)
     {
         const bool e2e = (p.host_obs || p.host_obs_q16) && ag.e2e.d;
-        if (!e2e && e->auto_balance && ag.feedback.d_tile_ns)
+        if (!e2e && ag.sizing.auto_balance && ag.feedback.d_tile_ns)
         { // feedback tiling: re-cut the tiles from the measured tile times, a few times early on, then now and then
             const uint64_t k = ag.feedback.launches++;
             if (k == 16 || k == 64 || k == 256 || (k & 4095) == 4095)
@@ -846,7 +523,7 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
         }
         p.tiles        = ag.beam.d.get();
         p.n_tiles      = ag.beam.n;
-        p.batch_agents = e->batch_agents_beam;
+        p.batch_agents = ag.sizing.batch_agents_beam;
         p.tile_ns      = e2e ? nullptr : ag.feedback.d_tile_ns.get();
         int grid       = ag.beam.grid;
         p.first        = nullptr;
@@ -868,7 +545,7 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
             p.tiles             = sch.d.get();
             p.n_tiles           = sch.n;
             grid                = sch.grid;
-            if (p.ext_host && ag.act_stage && p.n_tiles > grid && e->act_stage_on && stream_write_value32())
+            if (p.ext_host && ag.act_stage && p.n_tiles > grid && ag.sizing.act_stage && stream_write_value32())
             { // tiles after a CTA's first read the actions from a device copy (StepParams::act_ready)
                 p.act_stage_thr    = ag.act_stage.get();
                 p.act_stage_steer  = ag.act_stage.get() + e->n_agents;
@@ -876,30 +553,30 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
                 p.act_ready_target = ++ag.act_ready_target;
             }
         }
-        const bool flushers = e2e && p.host_obs && e->e2e_flushers > 0 && ag.tile_flag && e->beam_staged;
+        const bool flushers = e2e && p.host_obs && ag.sizing.e2e_flushers > 0 && ag.tile_flag && ag.sizing.beam_staged;
         if (flushers)
         { // fork: the flusher CTAs start next to the step kernel, on the side stream
             p.tile_flag  = ag.tile_flag.get();
             p.flag_epoch = ++e->flag_epoch;
             OK_CUDA(cudaEventRecord(e->ev_fork.get(), s));
             OK_CUDA(cudaStreamWaitEvent(e->flush_stream.get(), e->ev_fork.get(), 0));
-            ok::obs_flush_kernel<<<e->e2e_flushers, 1024, 0, e->flush_stream.get()>>>(ag.e2e.d.get(), ag.e2e.n, ag.tile_flag.get(), p.flag_epoch,
-                                                                                      static_cast<const float *>(e->d_buf[OK_BUF_OBS]), p.host_obs, e->rays);
+            ok::obs_flush_kernel<<<ag.sizing.e2e_flushers, 1024, 0, e->flush_stream.get()>>>(ag.e2e.d.get(), ag.e2e.n, ag.tile_flag.get(), p.flag_epoch,
+                                                                                             static_cast<const float *>(e->d_buf[OK_BUF_OBS]), p.host_obs, e->rays);
             OK_CUDA(cudaGetLastError());
             OK_CUDA(cudaEventRecord(e->ev_join.get(), e->flush_stream.get()));
         }
         if (actor)
         { // the policy step as phase 0 of every tile (ok_ppo_actor_step): its weights sit behind the kernel's own shared memory
-            p.actor_smem_off = static_cast<uint32_t>((e->smem_beam + 15) & ~static_cast<size_t>(15));
+            p.actor_smem_off = static_cast<uint32_t>((ag.sizing.smem_beam + 15) & ~static_cast<size_t>(15));
             OK_CUDA(ok::launch_step_actor(p, *actor, ag.beam.grid, p.actor_smem_off + actor_smem, s));
         }
-        else if (e->beam_staged)
-            OK_CUDA(ok::launch_step_staged(p, grid, e->smem_beam, s));
+        else if (ag.sizing.beam_staged)
+            OK_CUDA(ok::launch_step_staged(p, grid, ag.sizing.smem_beam, s));
         else
-            OK_CUDA(ok::launch_step_unstaged(p, ag.beam.grid, e->smem_beam, s));
+            OK_CUDA(ok::launch_step_unstaged(p, ag.beam.grid, ag.sizing.smem_beam, s));
     }
     else
-        OK_CUDA(ok::launch_step_grid(p, ag.tiles.grid, e->smem, s));
+        OK_CUDA(ok::launch_step_grid(p, ag.tiles.grid, ag.sizing.smem, s));
     if (p.act_ready)
     { // enqueued AFTER the launch: the kernel is already running its first tiles while the host issues these
         const size_t bytes = sizeof(float) * static_cast<size_t>(e->n_agents);
@@ -932,6 +609,18 @@ template <typename T> T *pinned_alias(T *h)
         return nullptr;
     }
     return at.type == cudaMemoryTypeHost ? static_cast<T *>(at.devicePointer) : nullptr;
+}
+
+// the modes of an OkConfig (ok_create, ok_update_config)
+int check_modes(const OkConfig &c)
+{
+    if (c.movement_mode != OK_MOVE_VELOCITY && c.movement_mode != OK_MOVE_ACCELERATION)
+        return fail(OK_ERR_INVALID_ARG, "movement_mode must be VELOCITY or ACCELERATION");
+    if (c.reward_mode < OK_REWARD_NONE || c.reward_mode > OK_REWARD_LANE_CENTER)
+        return fail(OK_ERR_INVALID_ARG, "unknown reward_mode");
+    if (c.raycast_mode < OK_RAYCAST_GRID || c.raycast_mode > OK_RAYCAST_BEAM)
+        return fail(OK_ERR_INVALID_ARG, "unknown raycast_mode");
+    return OK_SUCCESS;
 }
 } // namespace
 
@@ -980,12 +669,8 @@ int ok_create(const OkConfig *cfg, OkEnv **out)
         c = *cfg;
     else
         ok_config_default(&c);
-    if (c.movement_mode != OK_MOVE_VELOCITY && c.movement_mode != OK_MOVE_ACCELERATION)
-        return fail(OK_ERR_INVALID_ARG, "movement_mode must be VELOCITY or ACCELERATION");
-    if (c.reward_mode < OK_REWARD_NONE || c.reward_mode > OK_REWARD_LANE_CENTER)
-        return fail(OK_ERR_INVALID_ARG, "unknown reward_mode");
-    if (c.raycast_mode < OK_RAYCAST_GRID || c.raycast_mode > OK_RAYCAST_BEAM)
-        return fail(OK_ERR_INVALID_ARG, "unknown raycast_mode");
+    if (int rc = check_modes(c))
+        return rc;
     if (!(c.grid_cell >= 1.0f && c.grid_cell <= 512.0f))
         return fail(OK_ERR_INVALID_ARG, "grid_cell must be in [1, 512] px");
     if (c.beam_cell == 0.0f)
@@ -1029,12 +714,8 @@ int ok_update_config(OkEnv *e, const OkConfig *cfg)
 {
     if (!e || !cfg)
         return fail(OK_ERR_INVALID_ARG, "NULL argument");
-    if (cfg->movement_mode != OK_MOVE_VELOCITY && cfg->movement_mode != OK_MOVE_ACCELERATION)
-        return fail(OK_ERR_INVALID_ARG, "movement_mode must be VELOCITY or ACCELERATION");
-    if (cfg->reward_mode < OK_REWARD_NONE || cfg->reward_mode > OK_REWARD_LANE_CENTER)
-        return fail(OK_ERR_INVALID_ARG, "unknown reward_mode");
-    if (cfg->raycast_mode < OK_RAYCAST_GRID || cfg->raycast_mode > OK_RAYCAST_BEAM)
-        return fail(OK_ERR_INVALID_ARG, "unknown raycast_mode");
+    if (int rc = check_modes(*cfg))
+        return rc;
     OkConfig c   = *cfg;
     c.device     = e->cfg.device;
     c.grid_cell  = e->cfg.grid_cell;
@@ -1138,10 +819,8 @@ int64_t ok_track_copy(const OkEnv *e, int32_t id, int32_t which, float *h_out, i
 
 int ok_alloc_agents(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg, const int32_t *h_track_id)
 {
-    if (!e)
-        return fail(OK_ERR_INVALID_ARG, "env is NULL");
-    if (!e->has_device)
-        return fail(OK_ERR_NO_DEVICE, "this env was created without a CUDA device (device = -1)");
+    if (int rc = check_device(e))
+        return rc;
     if (n <= 0 || rays <= 0 || !h_ray_deg)
         return fail(OK_ERR_INVALID_ARG, "n_agents and rays must be positive and ray angles given");
     if (rays > 1024)
@@ -1181,66 +860,57 @@ int ok_alloc_agents(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg, c
 
 namespace
 {
+// the environment variables of the sizing (ok::SizingKnobs), read at every ok_alloc_agents
+ok::SizingKnobs sizing_knobs()
+{
+    auto number = [](const char *name) {
+        const char *v = std::getenv(name);
+        return v ? std::optional<int>(std::atoi(v)) : std::nullopt;
+    };
+    ok::SizingKnobs k;
+    k.batch_agents = number("OK_BATCH_AGENTS");
+    if (const char *v = std::getenv("OK_BEAM_KERNEL"))
+        k.beam_kernel = std::strcmp(v, "staged") == 0     ? ok::SizingKnobs::BeamKernel::Staged
+                        : std::strcmp(v, "unstaged") == 0 ? ok::SizingKnobs::BeamKernel::Unstaged
+                                                          : ok::SizingKnobs::BeamKernel::Automatic;
+    k.beam_batch_agents = number("OK_BEAM_BATCH_AGENTS");
+    k.beam_tail         = number("OK_BEAM_TAIL");
+    k.beam_waves        = number("OK_BEAM_WAVES");
+    k.auto_balance      = number("OK_AUTO_BALANCE");
+    k.e2e_tiles         = number("OK_E2E_TILES");
+    k.e2e_tiles_q16     = number("OK_E2E_TILES_Q16");
+    k.e2e_flushers      = number("OK_E2E_FLUSHERS");
+    k.act_stage         = number("OK_ACT_STAGE");
+    return k;
+}
+
+// what the step kernels need of shared memory (ok_step.cuh), for ok::size_population
+ok::StepFootprint step_footprint()
+{
+    ok::StepFootprint fp;
+    fp.agent_rec           = sizeof(ok::AgentRec);
+    fp.grid_ray_bytes      = static_cast<int64_t>(ok::batch_smem_bytes(1, 1) - sizeof(ok::AgentRec));
+    fp.beam_static_staged  = ok::beam_static_smem(true);
+    fp.beam_block_staged   = ok::beam_block(true);
+    fp.beam_block_unstaged = ok::beam_block(false);
+    fp.beam_tile           = OK_BEAM_TILE;
+    return fp;
+}
+
 int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg, const int32_t *h_track_id)
 {
     NvtxRange range("ok_alloc_agents (tiling, buffers)");
     Agents   &ag = e->ag;
     e->n_agents  = n;
     e->rays      = rays;
-    // batch = the agents a CTA keeps in flight: as many as fit behind the largest staged track
-    {
-        const size_t blob  = (e->max_blob_used + 127) / 128 * 128;
-        const size_t avail = static_cast<size_t>(e->smem_optin) > blob + 4096 ? e->smem_optin - blob - 4096 : 0;
-        const size_t per   = ok::batch_smem_bytes(1, rays);
-        int64_t      a     = static_cast<int64_t>(avail / per);
-        if (avail < static_cast<size_t>(ok::beam_static_smem(true)) + 4096)
-            a = 0; // the beam kernel keeps per-thread scratch and its ray queue in static shared memory
-        int          cap   = kMaxBatchAgents;
-        if (const char *env = std::getenv("OK_BATCH_AGENTS"))
-            cap = std::max(1, std::atoi(env));
-        a = std::min<int64_t>(a, cap);
-        // small populations: spread over all SMs rather than filling a few batches
-        a = std::min<int64_t>(a, std::max<int64_t>(1, (n + e->num_sms - 1) / std::max(1, e->num_sms)));
-        if (a < 1)
-            return fail(OK_ERR_CAPACITY, "shared memory cannot hold one agent's rays next to the largest track");
-        e->batch_agents = static_cast<int32_t>(a);
-        e->smem         = blob + ok::batch_smem_bytes(e->batch_agents, rays);
-        // beam kernel: one 64-byte record per agent; phases 1 / 4 run a thread per agent, so at most one block of agents.
-        // Which shape (ok_step.cuh): the staged one for throughput, the unstaged one when the population is too small
-        // to give every SM a worthwhile tile (OK_BEAM_KERNEL = staged | unstaged overrides).
-        // measured (tools/bench_small.py, tools/bench_c4.py): the unstaged shape is ahead below ~2,000 agents of 32 rays, and at
-        // 4,096 agents of 5 rays (a PPO rollout tick: 0.0289 vs 0.0300 ms, 0.0262 with the policy step fused in), behind at
-        // 8,192 agents of 5 rays (0.0376 vs 0.0318 ms)
-        e->beam_staged = n >= 2048 && n * rays > 24576;
-        if (const char *env = std::getenv("OK_BEAM_KERNEL"))
-            e->beam_staged = std::strcmp(env, "unstaged") != 0 && (std::strcmp(env, "staged") == 0 || e->beam_staged);
-        e->beam_block = ok::beam_block(e->beam_staged);
-        int64_t ab;
-        int     capb;
-        if (e->beam_staged)
-        { // one 1,024-thread CTA per SM behind the staged track: as many agents per tile as the shared memory behind the
-          // largest track holds (the balanced tiling then sizes the tiles: about one per CTA and wave)
-            ab   = static_cast<int64_t>((avail - ok::beam_static_smem(true)) / sizeof(ok::AgentRec));
-            capb = e->beam_block;
-        }
-        else
-        { // several small CTAs per SM, nothing staged: small tiles, the SM's other CTAs hide a tile's serial phases
-            ab   = e->beam_block;
-            capb = OK_BEAM_TILE;
-        }
-        ab = std::min<int64_t>(ab, 65535 / rays); // tile-local ray indices are 16 bits (the kernel's ray queue)
-        if (const char *env = std::getenv("OK_BEAM_BATCH_AGENTS"))
-            capb = std::max(1, std::atoi(env));
-        ab = std::min<int64_t>({ab, capb, e->beam_block});
-        if (!e->beam_staged) // small populations: spread over all SMs rather than filling a few tiles
-            ab = std::min<int64_t>(ab, std::max<int64_t>(1, (n + e->num_sms - 1) / std::max(1, e->num_sms)));
-        e->batch_agents_beam = static_cast<int32_t>(std::max<int64_t>(1, ab));
-        e->smem_beam         = (e->beam_staged ? blob : 0) + ok::beam_smem_bytes(e->batch_agents_beam);
-        // The limit is an attribute of the FUNCTION on this device, not of the env: it is raised to the opt-in maximum
-        // (minus the kernel's static shared memory), so that envs of different sizes can interleave their launches.
-        if (int rc = arm_shared_memory_limit(e))
-            return rc;
-    }
+    const ok::SizingKnobs knobs = sizing_knobs();
+    std::string           err;
+    if (!ok::size_population(n, rays, e->num_sms, e->smem_optin, e->max_blob_used, step_footprint(), knobs, ag.sizing, err))
+        return fail(OK_ERR_CAPACITY, err);
+    // The limit is an attribute of the FUNCTION on this device, not of the env: it is raised to the opt-in maximum
+    // (minus the kernel's static shared memory), so that envs of different sizes can interleave their launches.
+    if (int rc = arm_shared_memory_limit(e))
+        return rc;
 
     // one slab, 256-byte aligned sub-buffers
     size_t offs[OK_BUF_COUNT], total = 0;
@@ -1278,76 +948,34 @@ int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg,
     }
 
     // tilings (ok_schedule.hpp)
-    const int32_t *track_id = e->h_track_id.data();
-    // the balanced tiling of the beam kernel's batches over `ctas` CTAs, at least `waves` tiles per CTA; `runs` keeps the
-    // track runs with their tile counts
-    auto balanced = [&](int ctas, int waves, std::vector<ok::TileRun> &runs) {
-        runs = ok::track_runs(track_id, n, e->batch_agents_beam);
-        return ok::balanced_tiles(runs, e->batch_agents_beam, ctas, waves);
-    };
     {
         int per_sm = 1;
-        if (!e->beam_staged)
-            OK_CUDA(ok::occupancy_step_unstaged(e->smem_beam, &per_sm));
-        e->ctas_per_sm_beam = std::max(1, per_sm);
+        if (!ag.sizing.beam_staged)
+            OK_CUDA(ok::occupancy_step_unstaged(ag.sizing.smem_beam, &per_sm));
+        ag.sizing.ctas_per_sm_beam = std::max(1, per_sm);
     }
-    if (int rc = upload_schedule(ag.tiles, ok::guided_tiles(track_id, n, e->batch_agents, e->num_sms, 4), 0, e->num_sms))
+    ok::PopulationTilings tilings = ok::tile_population(e->h_track_id.data(), n, ag.sizing, e->num_sms, knobs);
+    ag.sizing.e2e_flushers        = tilings.e2e_flushers;
+    if (int rc = upload_schedule(ag.tiles, tilings.grid))
         return rc;
-    {
-        const int beam_ctas = e->num_sms * e->ctas_per_sm_beam;
-        // the unstaged beam kernel's small tiles cost about the same serial latency whatever their size (the thread-per-
-        // agent phases, the second ray pass): shrinking them further only adds tiles
-        int tail_div = e->beam_staged ? -1 : 0; // -1: balanced tiling
-        if (const char *env = std::getenv("OK_BEAM_TAIL"))
-            tail_div = std::atoi(env);
-        int waves = 1; // balanced tiling: tiles per CTA (OK_BEAM_WAVES)
-        if (const char *env = std::getenv("OK_BEAM_WAVES"))
-            waves = std::max(1, std::atoi(env));
-        e->auto_balance = 1; // OK_AUTO_BALANCE=0: keep the tiling by agent count
-        if (const char *env = std::getenv("OK_AUTO_BALANCE"))
-            e->auto_balance = std::atoi(env);
-        if (tail_div < 0)
-        { // the feedback tiling: its table is allocated once, with room for every re-cut (rebalance_beam_tiles)
-            BeamFeedback      &fb = ag.feedback;
-            ok::BalancedTiling bt = balanced(beam_ctas, waves, fb.runs);
-            const size_t capacity = std::max<size_t>(bt.tiles.size(), static_cast<size_t>(bt.target));
-            fb.tiles    = bt.tiles;
-            fb.target   = static_cast<int32_t>(bt.target);
-            fb.capacity = static_cast<int32_t>(capacity);
-            if (int rc = upload_schedule(ag.beam, bt.tiles, capacity, beam_ctas))
-                return rc;
-            OK_CUDA(dev_alloc(fb.d_tile_ns, 2 * capacity));
-            OK_CUDA(cudaMemset(fb.d_tile_ns.get(), 0, sizeof(uint32_t) * 2 * capacity));
-        }
-        else if (int rc = upload_schedule(ag.beam, ok::guided_tiles(track_id, n, e->batch_agents_beam, beam_ctas, tail_div), 0, beam_ctas))
-            return rc;
+    if (int rc = upload_schedule(ag.beam, tilings.beam))
+        return rc;
+    if (tilings.feedback)
+    { // the feedback tiling: its table has room for every re-cut (rebalance_beam_tiles)
+        BeamFeedback &fb = ag.feedback;
+        fb.runs          = std::move(tilings.runs);
+        fb.tiles         = std::move(tilings.beam.tiles);
+        fb.target        = static_cast<int32_t>(tilings.target);
+        fb.capacity      = static_cast<int32_t>(tilings.beam.capacity);
+        OK_CUDA(dev_alloc(fb.d_tile_ns, 2 * tilings.beam.capacity));
+        OK_CUDA(cudaMemset(fb.d_tile_ns.get(), 0, sizeof(uint32_t) * 2 * tilings.beam.capacity));
     }
-    if (e->beam_staged)
-    { // the end-to-end tiling (see ok_step_host): OK_E2E_TILES tiles per CTA (default 4)
-        int per_cta = 4;
-        if (const char *env = std::getenv("OK_E2E_TILES"))
-            per_cta = std::max(1, std::atoi(env));
-        // OK_E2E_FLUSHERS = F > 0: F SMs are left to obs_flush_kernel, which moves finished tiles to the host while the
-        // step kernel's CTAs carry on
-        e->e2e_flushers = 0;
-        if (const char *env = std::getenv("OK_E2E_FLUSHERS"))
-            e->e2e_flushers = std::max(0, std::min(std::atoi(env), e->num_sms / 2));
-        std::vector<ok::TileRun> runs;
-        const int                e2e_ctas = (e->num_sms - e->e2e_flushers) * e->ctas_per_sm_beam;
-        const ok::BalancedTiling e2e      = balanced(e2e_ctas, per_cta, runs);
-        if (int rc = upload_schedule(ag.e2e, e2e.tiles, static_cast<size_t>(e2e.target), e2e_ctas))
+    if (ag.sizing.beam_staged)
+    { // the end-to-end tilings (see ok_step_host), the action stage and the flushers' flags
+        if (int rc = upload_schedule(ag.e2e, tilings.e2e))
             return rc;
-        { // ok_step_host_q16: measured at the C3 shape 0.164 / 0.157 / 0.171 / 0.199 ms per tick with 2 / 3 / 4 / 6 tiles per CTA
-            int per_cta_q16 = 3;
-            if (const char *env = std::getenv("OK_E2E_TILES_Q16"))
-                per_cta_q16 = std::max(1, std::atoi(env));
-            else if (std::getenv("OK_E2E_TILES"))
-                per_cta_q16 = per_cta;
-            const int                q16_ctas = e->num_sms * e->ctas_per_sm_beam;
-            const ok::BalancedTiling q16      = balanced(q16_ctas, per_cta_q16, runs);
-            if (int rc = upload_schedule(ag.q16, q16.tiles, static_cast<size_t>(q16.target), q16_ctas))
-                return rc;
-        }
+        if (int rc = upload_schedule(ag.q16, tilings.q16))
+            return rc;
         OK_CUDA(dev_alloc(ag.act_stage, 2 * static_cast<size_t>(n)));
         OK_CUDA(dev_alloc(ag.act_ready, 1));
         OK_CUDA(cudaMemset(ag.act_ready.get(), 0, sizeof(uint32_t)));
@@ -1356,9 +984,7 @@ int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg,
             OK_CUDA(make_stream(e->act_stream));
             OK_CUDA(make_event(e->ev_act));
         }
-        if (const char *env = std::getenv("OK_ACT_STAGE"))
-            e->act_stage_on = std::atoi(env) != 0;
-        if (e->e2e_flushers > 0)
+        if (ag.sizing.e2e_flushers > 0)
         {
             OK_CUDA(dev_alloc(ag.tile_flag, static_cast<size_t>(ag.e2e.n)));
             OK_CUDA(cudaMemset(ag.tile_flag.get(), 0, sizeof(uint32_t) * static_cast<size_t>(ag.e2e.n)));
@@ -1629,11 +1255,11 @@ int ok_ppo_actor_step(OkEnv *e, const OkActorIO *io, uint64_t step, uint32_t see
     if (rc)
         return rc;
     DeviceGuard  g(e->cfg.device);
-    const size_t wbytes = actor_weight_bytes(q, e->rays) + sizeof(float) * 2 * static_cast<size_t>(e->batch_agents_beam); // + the tile's chosen actions
+    const size_t wbytes = actor_weight_bytes(q, e->rays) + sizeof(float) * 2 * static_cast<size_t>(e->ag.sizing.batch_agents_beam); // + the tile's chosen actions
     // one launch when the env runs the unstaged beam kernel (the shape of small populations, where a tick is latency) and the
     // weights fit behind its shared memory; otherwise the same tick as two launches
-    const bool fused = q.act && e->cfg.raycast_mode == OK_RAYCAST_BEAM && !e->beam_staged &&
-                       ((e->smem_beam + 15) & ~static_cast<size_t>(15)) + wbytes <= static_cast<size_t>(std::max(0, e->actor_dyn_max));
+    const bool fused = q.act && e->cfg.raycast_mode == OK_RAYCAST_BEAM && !e->ag.sizing.beam_staged &&
+                       ((e->ag.sizing.smem_beam + 15) & ~static_cast<size_t>(15)) + wbytes <= static_cast<size_t>(std::max(0, e->actor_dyn_max));
     if (!fused)
     {
         if (!skip)
@@ -1651,10 +1277,8 @@ int ok_ppo_actor_step(OkEnv *e, const OkActorIO *io, uint64_t step, uint32_t see
 int ok_discounted_returns(OkEnv *e, const float *d_rewards, const uint8_t *d_done, float *d_out, int32_t steps, int64_t n,
                           float gamma, void *stream)
 {
-    if (!e)
-        return fail(OK_ERR_INVALID_ARG, "env is NULL");
-    if (!e->has_device)
-        return fail(OK_ERR_NO_DEVICE, "this env was created without a CUDA device (device = -1)");
+    if (int rc = check_device(e))
+        return rc;
     if (!d_rewards || !d_out || steps < 0 || n < 0)
         return fail(OK_ERR_INVALID_ARG, "bad arguments");
     if (steps == 0 || n == 0)
@@ -1671,10 +1295,8 @@ int ok_discounted_returns(OkEnv *e, const float *d_rewards, const uint8_t *d_don
 int ok_track_query(OkEnv *e, const float *d_x, const float *d_y, const int32_t *d_track, int64_t n, int32_t *d_idx,
                    float *d_lane, float *d_bound, void *stream)
 {
-    if (!e)
-        return fail(OK_ERR_INVALID_ARG, "env is NULL");
-    if (!e->has_device)
-        return fail(OK_ERR_NO_DEVICE, "this env was created without a CUDA device (device = -1)");
+    if (int rc = check_device(e))
+        return rc;
     if (e->tracks.empty())
         return fail(OK_ERR_STATE, "no track has been added");
     if (n <= 0)
@@ -1702,10 +1324,8 @@ int ok_track_query(OkEnv *e, const float *d_x, const float *d_y, const int32_t *
 int ok_track_query_host(OkEnv *e, const float *h_x, const float *h_y, const int32_t *h_track, int64_t n, int32_t *h_idx,
                         float *h_lane, float *h_bound, void *stream)
 {
-    if (!e)
-        return fail(OK_ERR_INVALID_ARG, "env is NULL");
-    if (!e->has_device)
-        return fail(OK_ERR_NO_DEVICE, "this env was created without a CUDA device (device = -1)");
+    if (int rc = check_device(e))
+        return rc;
     if (n <= 0)
         return OK_SUCCESS;
     if (!h_x || !h_y)
@@ -1986,21 +1606,9 @@ static int host_beam(OkEnv *e, int32_t id)
     if (e->beams[id])
         return OK_SUCCESS;
     std::string err;
-    if (e->has_device)
-    { // the table the kernels use, copied back
-        auto dev = beam_device_table_for(e->tracks[id], beam_config(e), e->cfg.device, true, err);
-        if (!dev)
-            return fail(OK_ERR_INVALID_ARG, "beam table: " + err);
-        auto        host = std::make_shared<std::vector<uint8_t>>(dev->bytes);
-        DeviceGuard g(e->cfg.device);
-        OK_CUDA(cudaMemcpy(host->data(), dev->ptr, dev->bytes, cudaMemcpyDeviceToHost));
-        e->beams[id] = host;
-        return OK_SUCCESS;
-    }
-    e->beams[id] = beam_table_for(e->tracks[id], beam_config(e), true, err);
-    if (!e->beams[id])
-        return fail(OK_ERR_INVALID_ARG, "beam table: " + err);
-    return OK_SUCCESS;
+    const int   rc = ok::beam_host_table(e->tracks[id], ok::beam_config(e->cfg.beam_cell, e->cfg.beam_bins), e->has_device ? e->cfg.device : -1,
+                                         e->beams[id], err);
+    return rc ? fail(rc, err) : OK_SUCCESS;
 }
 
 int32_t ok_beam_lookup(OkEnv *e, int32_t id, float x, float y, float angle, uint16_t *h_items, int32_t capacity,
@@ -2028,10 +1636,7 @@ int32_t ok_beam_lookup_ex(OkEnv *e, int32_t id, float x, float y, float angle, u
 
 void ok_release_caches(void)
 {
-    std::lock_guard<std::mutex> lock(g_beam_mu);
-    g_beam_cache.clear();
-    g_beam_dev_cache.clear(); // tables still referenced by live envs stay alive until those envs are destroyed
-    ok::beam_builder_release();
+    ok::beam_release_caches();
 }
 
 int64_t ok_beam_table_bytes(OkEnv *e, int32_t id)
@@ -2243,8 +1848,8 @@ int ok_launch_stats(const OkEnv *e, OkLaunchStats *out)
     out->kernel_launches = e->launches;
     const Schedule &sch  = e->cfg.raycast_mode == OK_RAYCAST_BEAM ? e->ag.beam : e->ag.tiles;
     out->grid_blocks     = sch.grid;
-    out->block_threads   = e->cfg.raycast_mode == OK_RAYCAST_BEAM ? e->beam_block : ok::kGridBlock;
-    out->smem_bytes      = static_cast<int32_t>(e->cfg.raycast_mode == OK_RAYCAST_BEAM ? e->smem_beam : e->smem);
+    out->block_threads   = e->cfg.raycast_mode == OK_RAYCAST_BEAM ? e->ag.sizing.beam_block : ok::kGridBlock;
+    out->smem_bytes      = static_cast<int32_t>(e->cfg.raycast_mode == OK_RAYCAST_BEAM ? e->ag.sizing.smem_beam : e->ag.sizing.smem);
     out->tiles           = sch.n;
     return OK_SUCCESS;
 }

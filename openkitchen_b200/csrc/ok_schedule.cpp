@@ -1,4 +1,4 @@
-// ok_schedule.cpp -- tilings of the agent range (ok_schedule.hpp)
+// ok_schedule.cpp -- sizing of a population and tilings of the agent range (ok_schedule.hpp)
 #include "ok_schedule.hpp"
 
 #include <algorithm>
@@ -151,6 +151,106 @@ bool reweigh_runs(std::vector<TileRun> &runs, const std::vector<Tile> &tiles, co
     weighted  = true;
     out.tiles = cost_balanced_tiles(runs, target, c0, &out.balance_after);
     return true;
+}
+
+bool size_population(int64_t n, int32_t rays, int num_sms, int smem_optin, size_t max_blob, const StepFootprint &fp,
+                     const SizingKnobs &knobs, Sizing &out, std::string &err)
+{
+    out = Sizing{};
+    // small populations: spread over all SMs rather than filling a few batches
+    const int64_t spread = std::max<int64_t>(1, (n + num_sms - 1) / std::max(1, num_sms));
+    // grid kernel: batch = the agents a CTA keeps in flight, as many as fit behind the largest staged track
+    const size_t blob  = (max_blob + 127) / 128 * 128;
+    const size_t avail = static_cast<size_t>(smem_optin) > blob + 4096 ? smem_optin - blob - 4096 : 0;
+    const size_t per   = static_cast<size_t>(fp.agent_rec + fp.grid_ray_bytes * rays);
+    int64_t      a     = static_cast<int64_t>(avail / per);
+    if (avail < static_cast<size_t>(fp.beam_static_staged) + 4096)
+        a = 0; // the beam kernel keeps per-thread scratch and its ray queue in static shared memory
+    a = std::min<int64_t>(a, knobs.batch_agents ? std::max(1, *knobs.batch_agents) : 256);
+    a = std::min<int64_t>(a, spread);
+    if (a < 1)
+    {
+        err = "shared memory cannot hold one agent's rays next to the largest track";
+        return false;
+    }
+    out.batch_agents = static_cast<int32_t>(a);
+    out.smem         = blob + static_cast<size_t>(a) * per;
+    // beam kernel: one AgentRec per agent; phases 1 / 4 run a thread per agent, so at most one block of agents.
+    // Which shape (ok_step.cuh): the staged one for throughput, the unstaged one when the population is too small
+    // to give every SM a worthwhile tile.
+    // measured (tools/bench_small.py, tools/bench_c4.py): the unstaged shape is ahead below ~2,000 agents of 32 rays, and at
+    // 4,096 agents of 5 rays (a PPO rollout tick: 0.0289 vs 0.0300 ms, 0.0262 with the policy step fused in), behind at
+    // 8,192 agents of 5 rays (0.0376 vs 0.0318 ms)
+    out.beam_staged = knobs.beam_kernel == SizingKnobs::BeamKernel::Automatic ? n >= 2048 && n * rays > 24576
+                                                                                : knobs.beam_kernel == SizingKnobs::BeamKernel::Staged;
+    out.beam_block = out.beam_staged ? fp.beam_block_staged : fp.beam_block_unstaged;
+    int64_t ab;
+    int64_t capb;
+    if (out.beam_staged)
+    { // one 1,024-thread CTA per SM behind the staged track: as many agents per tile as the shared memory behind the
+      // largest track holds (the balanced tiling then sizes the tiles: about one per CTA and wave)
+        ab   = static_cast<int64_t>((avail - static_cast<size_t>(fp.beam_static_staged)) / static_cast<size_t>(fp.agent_rec));
+        capb = out.beam_block;
+    }
+    else
+    { // several small CTAs per SM, nothing staged: small tiles, the SM's other CTAs hide a tile's serial phases
+        ab   = out.beam_block;
+        capb = fp.beam_tile;
+    }
+    ab = std::min<int64_t>(ab, 65535 / rays); // tile-local ray indices are 16 bits (the kernel's ray queue)
+    if (knobs.beam_batch_agents)
+        capb = std::max(1, *knobs.beam_batch_agents);
+    ab = std::min<int64_t>({ab, capb, out.beam_block});
+    if (!out.beam_staged)
+        ab = std::min<int64_t>(ab, spread);
+    out.batch_agents_beam = static_cast<int32_t>(std::max<int64_t>(1, ab));
+    // beam_smem_bytes: the records, rounded up to 16 bytes
+    out.smem_beam = (out.beam_staged ? blob : 0) + (static_cast<size_t>(out.batch_agents_beam * fp.agent_rec) + 15u) / 16u * 16u;
+    out.auto_balance = knobs.auto_balance.value_or(1) != 0;
+    out.act_stage    = knobs.act_stage.value_or(1) != 0;
+    return true;
+}
+
+PopulationTilings tile_population(const int32_t *track_id, int64_t n, const Sizing &s, int num_sms, const SizingKnobs &knobs)
+{
+    PopulationTilings out;
+    out.grid = {guided_tiles(track_id, n, s.batch_agents, num_sms, 4), 0, num_sms};
+    // the balanced tiling of the beam kernel's batches over `ctas` CTAs, at least `waves` tiles per CTA; `runs` keeps the
+    // track runs with their tile counts
+    auto balanced = [&](int ctas, int waves, std::vector<TileRun> &runs) {
+        runs = track_runs(track_id, n, s.batch_agents_beam);
+        return balanced_tiles(runs, s.batch_agents_beam, ctas, waves);
+    };
+    const int beam_ctas = num_sms * s.ctas_per_sm_beam;
+    // the unstaged beam kernel's small tiles cost about the same serial latency whatever their size (the thread-per-
+    // agent phases, the second ray pass): shrinking them further only adds tiles
+    const int tail_div = knobs.beam_tail.value_or(s.beam_staged ? -1 : 0); // -1: balanced tiling
+    if (tail_div < 0)
+    { // the feedback tiling: its table is allocated once, with room for every re-cut (rebalance_beam_tiles)
+        BalancedTiling bt = balanced(beam_ctas, std::max(1, knobs.beam_waves.value_or(1)), out.runs);
+        out.feedback      = true;
+        out.target        = bt.target;
+        out.beam          = {std::move(bt.tiles), 0, beam_ctas};
+        out.beam.capacity = std::max<size_t>(out.beam.tiles.size(), static_cast<size_t>(bt.target));
+    }
+    else
+        out.beam = {guided_tiles(track_id, n, s.batch_agents_beam, beam_ctas, tail_div), 0, beam_ctas};
+    if (s.beam_staged)
+    { // the end-to-end tilings (see ok_step_host).  OK_E2E_FLUSHERS = F > 0: F SMs are left to obs_flush_kernel, which
+      // moves finished tiles to the host while the step kernel's CTAs carry on
+        const int per_cta = std::max(1, knobs.e2e_tiles.value_or(4));
+        out.e2e_flushers  = std::max(0, std::min(knobs.e2e_flushers.value_or(0), num_sms / 2));
+        const int e2e_ctas = (num_sms - out.e2e_flushers) * s.ctas_per_sm_beam;
+        std::vector<TileRun> runs;
+        BalancedTiling       e2e = balanced(e2e_ctas, per_cta, runs);
+        out.e2e                  = {std::move(e2e.tiles), static_cast<size_t>(e2e.target), e2e_ctas};
+        // ok_step_host_q16: measured at the C3 shape 0.164 / 0.157 / 0.171 / 0.199 ms per tick with 2 / 3 / 4 / 6 tiles per CTA
+        const int      per_cta_q16 = knobs.e2e_tiles_q16 ? std::max(1, *knobs.e2e_tiles_q16) : knobs.e2e_tiles ? per_cta : 3;
+        const int      q16_ctas    = num_sms * s.ctas_per_sm_beam;
+        BalancedTiling q16         = balanced(q16_ctas, per_cta_q16, runs);
+        out.q16                    = {std::move(q16.tiles), static_cast<size_t>(q16.target), q16_ctas};
+    }
+    return out;
 }
 
 } // namespace ok

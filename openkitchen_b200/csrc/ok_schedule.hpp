@@ -1,9 +1,12 @@
-// ok_schedule.hpp -- how the agent range is cut into tiles (batches of same-track agents that the CTAs of the step kernel
-// pull in list order).  Host-only and free of CUDA: every decision here is a pure function of host data, and
-// ok_capi.cu uploads the result.
+// ok_schedule.hpp -- how large a population's batches are and which kernel shape runs it, and how the agent range is cut
+// into tiles (batches of same-track agents that the CTAs of the step kernel pull in list order).  Host-only and free of
+// CUDA: every decision here is a pure function of host data, and ok_capi.cu allocates and uploads the result.
 #pragma once
 
+#include <cstddef>
 #include <cstdint>
+#include <optional>
+#include <string>
 #include <vector>
 
 namespace ok
@@ -64,5 +67,81 @@ struct Reweighing
 };
 bool reweigh_runs(std::vector<TileRun> &runs, const std::vector<Tile> &tiles, const uint32_t *ns, bool &weighted, int64_t target,
                   Reweighing &out);
+
+// ---- sizing of a population (ok_alloc_agents) ---------------------------------------------------------------------------
+
+// The environment variables that steer the sizing, as ok_capi.cu reads them at every ok_alloc_agents (unset: empty).  Their
+// defaults and bounds are applied here.
+struct SizingKnobs
+{
+    enum class BeamKernel
+    {
+        Automatic,
+        Staged,
+        Unstaged
+    };
+    std::optional<int> batch_agents;                   // OK_BATCH_AGENTS: cap on the grid kernel's batch (default 256)
+    BeamKernel         beam_kernel{BeamKernel::Automatic}; // OK_BEAM_KERNEL = staged | unstaged (anything else: automatic)
+    std::optional<int> beam_batch_agents;              // OK_BEAM_BATCH_AGENTS: cap on the beam kernel's tile
+    std::optional<int> beam_tail;                      // OK_BEAM_TAIL: guided beam tiling with this tail divisor
+    std::optional<int> beam_waves;                     // OK_BEAM_WAVES: balanced tiling, tiles per CTA (default 1)
+    std::optional<int> auto_balance;                   // OK_AUTO_BALANCE=0: keep the tiling by agent count
+    std::optional<int> e2e_tiles;                      // OK_E2E_TILES: ok_step_host tiles per CTA (default 4)
+    std::optional<int> e2e_tiles_q16;                  // OK_E2E_TILES_Q16: ok_step_host_q16's (default 3, or OK_E2E_TILES)
+    std::optional<int> e2e_flushers;                   // OK_E2E_FLUSHERS: SMs left to obs_flush_kernel (at most half)
+    std::optional<int> act_stage;                      // OK_ACT_STAGE=0: every tile reads the mapped actions
+};
+
+// What the step kernels need of shared memory, as plain numbers (ok_capi.cu fills it from ok_step.cuh)
+struct StepFootprint
+{
+    int64_t agent_rec;          // sizeof(AgentRec): one per agent of a batch or tile
+    int64_t grid_ray_bytes;     // batch_smem_bytes: bytes per ray of an agent of the grid kernel's batch
+    int64_t beam_static_staged; // beam_static_smem(true)
+    int32_t beam_block_staged, beam_block_unstaged; // beam_block(true / false)
+    int32_t beam_tile;          // OK_BEAM_TILE: agents per tile of the unstaged beam kernel
+};
+
+// How a population runs: the kernel shapes and batch sizes (size_population), the unstaged beam kernel's occupancy
+// (queried by the caller), the flusher count (tile_population) and the knob-derived flags.
+struct Sizing
+{
+    int32_t batch_agents{0}; // the grid kernel's batch
+    size_t  smem{0};         // ... and its dynamic shared memory
+    bool    beam_staged{false};
+    int32_t beam_block{0};
+    int32_t batch_agents_beam{0};
+    size_t  smem_beam{0};
+    int32_t ctas_per_sm_beam{1};
+    int32_t e2e_flushers{0};
+    bool    auto_balance{true};
+    bool    act_stage{true};
+};
+
+// Stage 1: the shape of a population of n agents x rays behind tracks of up to max_blob bytes, on a device of num_sms SMs
+// and smem_optin bytes of shared memory per block.  False (with err) when shared memory cannot hold one agent's rays.
+bool size_population(int64_t n, int32_t rays, int num_sms, int smem_optin, size_t max_blob, const StepFootprint &fp,
+                     const SizingKnobs &knobs, Sizing &out, std::string &err);
+
+// a tiling as it is uploaded: the table, room for `capacity` tiles (at least as many as there are), run by `ctas` CTAs at most
+struct Tiling
+{
+    std::vector<Tile> tiles;
+    size_t            capacity{0};
+    int               ctas{0};
+};
+
+// Stage 2: every tiling of the population (track_id[0, n)) that s describes, s.ctas_per_sm_beam included.
+struct PopulationTilings
+{
+    Tiling grid; // guided, the grid kernel's
+    Tiling beam;
+    bool   feedback{false};      // beam is the feedback tiling: re-cut from measured tile times (reweigh_runs) ...
+    std::vector<TileRun> runs;   // ... of these runs ...
+    int64_t              target{0}; // ... into this many tiles
+    Tiling  e2e, q16;            // ok_step_host's and ok_step_host_q16's (staged beam kernel only)
+    int32_t e2e_flushers{0};
+};
+PopulationTilings tile_population(const int32_t *track_id, int64_t n, const Sizing &s, int num_sms, const SizingKnobs &knobs);
 
 } // namespace ok

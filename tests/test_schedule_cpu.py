@@ -1,9 +1,11 @@
-"""CPU: the tilings of the agent range (openkitchen_b200/csrc/ok_schedule.cpp), compiled with g++ next to a small C
-wrapper and driven through ctypes.  Guided and balanced tilings must partition the agents into same-track tiles within
-their caps; the cost-balanced tiling must minimise the slowest tile; the feedback model must ignore what carries no
-information and damp what it learns."""
+"""CPU: the sizing of a population and the tilings of the agent range (openkitchen_b200/csrc/ok_schedule.cpp), compiled
+with g++ next to a small C wrapper and driven through ctypes.  Guided and balanced tilings must partition the agents into
+same-track tiles within their caps; the cost-balanced tiling must minimise the slowest tile; the feedback model must
+ignore what carries no information and damp what it learns.  The sizing must choose the kernel shape and the tilings the
+library chose on a B200 (tests/golden/sizing_plans.json, tools/make_golden_sizing.py) and keep its rules."""
 import ctypes as C
 import itertools
+import json
 import os
 import subprocess
 
@@ -14,6 +16,8 @@ CSRC = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))),
 
 WRAPPER = r'''
 #include "ok_schedule.hpp"
+#include <climits>
+#include <cstdio>
 #include <cstring>
 
 namespace {
@@ -30,6 +34,27 @@ std::vector<ok::TileRun> runs_of(int64_t n_runs, const int32_t *track, const int
     for (int64_t r = 0; r < n_runs; ++r)
         runs.push_back({track[r], begin[r], len[r], cap[r], w[r], 0});
     return runs;
+}
+// k[10]: the knobs in SizingKnobs order, INT_MIN = unset; k[1] (OK_BEAM_KERNEL): 0 automatic, 1 staged, 2 unstaged
+ok::SizingKnobs knobs_of(const int *k)
+{
+    auto opt = [](int v) { return v == INT_MIN ? std::optional<int>() : std::optional<int>(v); };
+    ok::SizingKnobs s;
+    s.batch_agents      = opt(k[0]);
+    s.beam_kernel       = static_cast<ok::SizingKnobs::BeamKernel>(k[1] == INT_MIN ? 0 : k[1]);
+    s.beam_batch_agents = opt(k[2]);
+    s.beam_tail         = opt(k[3]);
+    s.beam_waves        = opt(k[4]);
+    s.auto_balance      = opt(k[5]);
+    s.e2e_tiles         = opt(k[6]);
+    s.e2e_tiles_q16     = opt(k[7]);
+    s.e2e_flushers      = opt(k[8]);
+    s.act_stage         = opt(k[9]);
+    return s;
+}
+ok::StepFootprint footprint_of(const int64_t *f)
+{
+    return {f[0], f[1], f[2], static_cast<int32_t>(f[3]), static_cast<int32_t>(f[4]), static_cast<int32_t>(f[5])};
 }
 } // namespace
 
@@ -75,6 +100,42 @@ int64_t sch_reweigh(int64_t n_runs, const int32_t *track, const int64_t *begin, 
     balance[0] = rw.balance_before, balance[1] = rw.balance_after;
     return put(rw.tiles, out, out_cap);
 }
+
+// dev: num_sms, smem_optin, max_blob.  shape[8]: batch_agents, smem, beam_staged, beam_block, batch_agents_beam, smem_beam,
+// auto_balance, act_stage.  Returns 0, or -1 with the error in err.
+int sch_size(int64_t n, int rays, const int64_t *dev, const int64_t *fp, const int *knobs, int64_t *shape, char *err, int err_cap)
+{
+    ok::Sizing  s;
+    std::string why;
+    if (!ok::size_population(n, rays, static_cast<int>(dev[0]), static_cast<int>(dev[1]), static_cast<size_t>(dev[2]), footprint_of(fp),
+                             knobs_of(knobs), s, why))
+    {
+        std::snprintf(err, err_cap, "%s", why.c_str());
+        return -1;
+    }
+    const int64_t v[8] = {s.batch_agents, static_cast<int64_t>(s.smem), s.beam_staged, s.beam_block, s.batch_agents_beam,
+                          static_cast<int64_t>(s.smem_beam), s.auto_balance, s.act_stage};
+    std::memcpy(shape, v, sizeof v);
+    return 0;
+}
+
+// tiling `which` (0 grid, 1 beam, 2 e2e, 3 q16) of the population sized as sch_size does, with `ctas_per_sm` unstaged beam
+// CTAs per SM.  info[5]: the tiling's ctas and capacity, feedback, target, e2e_flushers.
+int64_t sch_tiling(const int32_t *track_id, int64_t n, int rays, const int64_t *dev, const int64_t *fp, const int *knobs, int ctas_per_sm,
+                   int which, int64_t *out, int64_t cap, int64_t *info)
+{
+    ok::Sizing  s;
+    std::string why;
+    if (!ok::size_population(n, rays, static_cast<int>(dev[0]), static_cast<int>(dev[1]), static_cast<size_t>(dev[2]), footprint_of(fp),
+                             knobs_of(knobs), s, why))
+        return -1;
+    s.ctas_per_sm_beam          = s.beam_staged ? 1 : ctas_per_sm;
+    const ok::PopulationTilings t = ok::tile_population(track_id, n, s, static_cast<int>(dev[0]), knobs_of(knobs));
+    const ok::Tiling           &r = which == 0 ? t.grid : which == 1 ? t.beam : which == 2 ? t.e2e : t.q16;
+    const int64_t               v[5] = {r.ctas, static_cast<int64_t>(r.capacity), t.feedback, t.target, t.e2e_flushers};
+    std::memcpy(info, v, sizeof v);
+    return put(r.tiles, out, cap);
+}
 }
 '''
 
@@ -94,6 +155,9 @@ def lib(tmp_path_factory):
     L.sch_balanced.argtypes = [_P, C.c_int64, C.c_int64, C.c_int, C.c_int, _P, C.c_int64, _P]
     L.sch_cost_balanced.argtypes = [C.c_int64, _P, _P, _P, _P, _P, C.c_int64, C.c_double, _P, C.c_int64, _P]
     L.sch_reweigh.argtypes = [C.c_int64, _P, _P, _P, _P, _P, C.c_int64, _P, _P, _P, C.c_int64, _P, C.c_int64, _P]
+    L.sch_size.restype, L.sch_tiling.restype = C.c_int, C.c_int64
+    L.sch_size.argtypes = [C.c_int64, C.c_int, _P, _P, _P, _P, C.c_char_p, C.c_int]
+    L.sch_tiling.argtypes = [_P, C.c_int64, C.c_int, _P, _P, _P, C.c_int, C.c_int, _P, C.c_int64, _P]
     return L
 
 
@@ -328,3 +392,131 @@ def test_reweigh_needs_half_the_tiles_measured(lib):
     ns[len(tiles) // 2, 0] = 9 * tiles[len(tiles) // 2, 1]  # exactly half
     new, weighted, _ = reweigh(lib, runs, tiles, ns, False, target)
     assert new is not None and weighted
+
+
+# ---- sizing of a population -----------------------------------------------------------------------------------------
+
+# the step kernels' footprint (ok_step.cuh, ok_device.cuh): sizeof(AgentRec), batch_smem_bytes' bytes per ray,
+# beam_static_smem(true), beam_block(true), beam_block(false), OK_BEAM_TILE
+FOOTPRINT = np.array([64, 8, 42112, 1024, 256, 64], np.int64)
+# occupancy of the unstaged beam kernel (256 threads, 64 registers): the plan "bench-unstaged" runs 592 = 148 x 4 CTAs
+UNSTAGED_CTAS_PER_SM = 4
+KNOBS = ["OK_BATCH_AGENTS", "OK_BEAM_KERNEL", "OK_BEAM_BATCH_AGENTS", "OK_BEAM_TAIL", "OK_BEAM_WAVES", "OK_AUTO_BALANCE",
+         "OK_E2E_TILES", "OK_E2E_TILES_Q16", "OK_E2E_FLUSHERS", "OK_ACT_STAGE"]
+UNSET = -(2 ** 31)
+SHAPE = ["batch_agents", "smem", "beam_staged", "beam_block", "batch_agents_beam", "smem_beam", "auto_balance", "act_stage"]
+with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "sizing_plans.json")) as _f:
+    GOLDEN = json.load(_f)
+B200 = GOLDEN["device"]
+
+
+def knob_array(knobs):
+    """the variables as ok_capi.cu reads them (atoi; OK_BEAM_KERNEL by name)"""
+    def value(k, v):
+        if k == "OK_BEAM_KERNEL":
+            return {"staged": 1, "unstaged": 2}.get(v, 0)
+        return int(v)
+    return np.array([value(k, knobs[k]) if k in knobs else UNSET for k in KNOBS], np.int32)
+
+
+def device(num_sms=None, smem_optin=None, max_blob=None):
+    return np.array([num_sms or B200["num_sms"], smem_optin or B200["smem_optin"], max_blob or B200["max_blob"]], np.int64)
+
+
+def size(lib, n, rays, knobs=None, **dev):
+    shape, err = np.zeros(len(SHAPE), np.int64), C.create_string_buffer(256)
+    if lib.sch_size(n, rays, _p(device(**dev)), _p(FOOTPRINT), _p(knob_array(knobs or {})), _p(shape), err, 256) != 0:
+        return err.value.decode()
+    return dict(zip(SHAPE, shape.tolist()))
+
+
+TILINGS = {"grid": 0, "beam": 1, "e2e": 2, "q16": 3}
+
+
+def tiling(lib, tid, rays, which, knobs=None, ctas_per_sm=UNSTAGED_CTAS_PER_SM, **dev):
+    out, info = np.zeros((len(tid), 3), np.int64), np.zeros(5, np.int64)
+    k = lib.sch_tiling(_p(tid), len(tid), rays, _p(device(**dev)), _p(FOOTPRINT), _p(knob_array(knobs or {})), ctas_per_sm,
+                       TILINGS[which], _p(out), len(tid), _p(info))
+    assert k >= 0
+    return out[:k], dict(zip(["ctas", "capacity", "feedback", "target", "flushers"], info.tolist()))
+
+
+def golden_tid(n):
+    return (np.arange(n) * 23 // n).astype(np.int32)  # tools/make_golden_sizing.py: 23 tracks, contiguous
+
+
+@pytest.mark.parametrize("name", list(GOLDEN["plans"]))
+def test_plan_is_the_one_chosen_on_b200(lib, name):
+    """launch_stats() and debug_tiles() of the library right after alloc_agents, minted on a B200"""
+    p = GOLDEN["plans"][name]
+    shape = size(lib, p["n"], p["rays"], p["knobs"])
+    which = "beam" if p["raycast"] == "beam" else "grid"
+    tiles, info = tiling(lib, golden_tid(p["n"]), p["rays"], which, p["knobs"])
+    grid = max(1, min(info["ctas"], len(tiles)))  # ok_capi.cu: schedule_grid
+    if which == "beam":
+        assert (grid, shape["beam_block"], shape["smem_beam"], len(tiles)) == (p["grid"], p["block"], p["smem"], p["tiles"])
+        assert np.array_equal(tiles, np.asarray(p["debug_tiles"], np.int64).reshape(-1, 3))
+    else:
+        assert (grid, 1024, shape["smem"], len(tiles)) == (p["grid"], p["block"], p["smem"], p["tiles"])
+
+
+E2E_SHAPES = [
+    pytest.param(65536, 32, {}, id="bench"),
+    pytest.param(65536, 32, {"OK_E2E_FLUSHERS": "8"}, id="flushers8"),
+    pytest.param(65536, 32, {"OK_E2E_FLUSHERS": "500"}, id="flushers-capped"),
+    pytest.param(300, 32, {"OK_BEAM_KERNEL": "staged", "OK_E2E_TILES": "6"}, id="300-staged"),
+    pytest.param(8192, 5, {"OK_BEAM_BATCH_AGENTS": "40", "OK_E2E_TILES_Q16": "2"}, id="8192x5"),
+]
+
+
+@pytest.mark.parametrize("n,rays,knobs", E2E_SHAPES)
+def test_e2e_tilings_partition_the_agents_over_their_ctas(lib, n, rays, knobs):
+    tid = golden_tid(n)
+    shape = size(lib, n, rays, knobs)
+    assert shape["beam_staged"] == 1
+    flushers = min(int(knobs.get("OK_E2E_FLUSHERS", 0)), B200["num_sms"] // 2)
+    for which, ctas in [("e2e", B200["num_sms"] - flushers), ("q16", B200["num_sms"])]:
+        tiles, info = tiling(lib, tid, rays, which, knobs)
+        check_partition(tiles, tid, shape["batch_agents_beam"])
+        assert info["flushers"] == flushers and info["ctas"] == ctas
+        assert info["capacity"] % ctas == 0 and len(tiles) <= info["capacity"]  # capacity: the balanced tiling's target
+
+
+@pytest.mark.parametrize("knobs,e2e,q16", [({}, 4, 3), ({"OK_E2E_TILES": "6"}, 6, 6), ({"OK_E2E_TILES_Q16": "2"}, 4, 2),
+                                           ({"OK_E2E_TILES": "6", "OK_E2E_TILES_Q16": "2"}, 6, 2), ({"OK_E2E_TILES": "0"}, 1, 1)])
+def test_q16_tiles_follow_e2e_tiles_only_when_unset(lib, knobs, e2e, q16):
+    tid = golden_tid(65536)  # the bench population: one tile per CTA and wave
+    for which, per_cta in [("e2e", e2e), ("q16", q16)]:
+        tiles, info = tiling(lib, tid, 32, which, knobs)
+        assert info["capacity"] == per_cta * B200["num_sms"] and len(tiles) == info["capacity"]
+
+
+def test_unstaged_population_has_no_e2e_tiling_and_a_guided_beam_tiling(lib):
+    tid = golden_tid(300)
+    assert size(lib, 300, 32)["beam_staged"] == 0
+    assert len(tiling(lib, tid, 32, "e2e")[0]) == 0 and len(tiling(lib, tid, 32, "q16")[0]) == 0
+    tiles, info = tiling(lib, tid, 32, "beam")
+    assert not info["feedback"] and info["ctas"] == B200["num_sms"] * UNSTAGED_CTAS_PER_SM and info["capacity"] == 0
+
+
+def test_knob_flags_and_caps(lib):
+    bench = size(lib, 65536, 32)
+    assert bench["auto_balance"] == 1 and bench["act_stage"] == 1
+    off = size(lib, 65536, 32, {"OK_AUTO_BALANCE": "0", "OK_ACT_STAGE": "0"})
+    assert off["auto_balance"] == 0 and off["act_stage"] == 0
+    # OK_BATCH_AGENTS limits only the grid kernel's batch
+    capped = size(lib, 65536, 32, {"OK_BATCH_AGENTS": "7"})
+    assert capped["batch_agents"] == 7 and capped["batch_agents_beam"] == bench["batch_agents_beam"]
+    # tile-local ray indices are 16 bits: at most 65535 / rays agents per beam tile
+    assert size(lib, 65536, 1024, {"OK_BEAM_KERNEL": "staged"})["batch_agents_beam"] == 65535 // 1024
+
+
+@pytest.mark.parametrize("kernel", ["staged", "unstaged"])
+def test_too_little_shared_memory_is_a_capacity_error(lib, kernel):
+    """in both shapes, the beam kernel's static shared memory and 4 KB must fit next to the largest track (rounded up to
+    128 bytes) and its own 4 KB"""
+    blob = 146784
+    need = (blob + 127) // 128 * 128 + 4096 + int(FOOTPRINT[2]) + 4096
+    err = size(lib, 300, 32, {"OK_BEAM_KERNEL": kernel}, smem_optin=need - 1, max_blob=blob)
+    assert err == "shared memory cannot hold one agent's rays next to the largest track"
+    assert size(lib, 300, 32, {"OK_BEAM_KERNEL": kernel}, smem_optin=need, max_blob=blob)["batch_agents"] >= 1
