@@ -214,6 +214,33 @@ int ok_track_query(OkEnv *env, const float *d_x, const float *d_y, const int32_t
 int ok_track_query_host(OkEnv *env, const float *h_x, const float *h_y, const int32_t *h_track_id, int64_t n,
                         int32_t *h_nearest_idx, float *h_dist_lane_center, float *h_dist_boundary, void *stream);
 
+/* Lidar scans at arbitrary poses, with no agent state read or written (CollisionChecker::checkCollision's pack + kernel
+ * + unpack, CollisionChecker.cu:115-172, for poses that are not agents).  Pose k = (x[k], y[k], rot[k]) on track
+ * track_id[k] (NULL = track 0; out-of-range ids are clamped as in ok_track_query) casts the fan ray_deg[rays], angles in
+ * degrees relative to the heading, 1 <= rays <= 1024.  ray_deg NULL = the env's fan from ok_alloc_agents, and then rays
+ * must be ok_num_rays(env).  Uses the env's live OkConfig (sensor_range, sensor_offset, collision_dist2, raycast_mode);
+ * every output is bit for bit what ok_cast_rays writes for an agent at that pose whose crash flag is clear, in the layout
+ * of the agent buffer of the same name; every output is nullable.  crashed is the strict test min_dist2 <
+ * collision_dist2.  Needs tracks only, not agents.  The first call of an env may build the track arena (in beam mode also
+ * the device tables) synchronously; if that is still to do while `stream` is capturing, the call fails with OK_ERR_STATE:
+ * call once outside the capture, later calls can be captured.  n == 0 is a no-op. */
+typedef struct OkLidarQuery {
+    const float   *x, *y, *rot;        /* f32[n]: Agent::pos_, rot_ (degrees) */
+    const int32_t *track_id;           /* i32[n] or NULL */
+    int64_t        n;
+    const float   *ray_deg;            /* f32[rays] or NULL */
+    int32_t        rays, reserved;
+    float         *hit_abs, *hit_rel;  /* f32[n,R,2]: OK_BUF_HIT_ABS, OK_BUF_HIT_REL */
+    float         *obs, *hit_t;        /* f32[n,R] */
+    int32_t       *hit_seg;            /* i32[n,R], -1 = none */
+    float         *min_dist2;          /* f32[n] */
+    uint8_t       *crashed;            /* u8[n]: min_dist2 < collision_dist2 */
+} OkLidarQuery;
+/* device pointers; asynchronous on `stream` */
+int ok_lidar_query(OkEnv *env, const OkLidarQuery *q, void *stream);
+/* the same with HOST pointers (ray_deg included), staged through the env's staging buffer; synchronises `stream` */
+int ok_lidar_query_host(OkEnv *env, const OkLidarQuery *q, void *stream);
+
 /* The EvolutionaryRacer policy for the whole population (SURVEY.md 8f, N2): GeneticAgent::updateAction +
  * Network::infer (EvolutionaryRacer/GeneticAgent.hpp:37-50, Network.hpp:119-155).  Agent i has its own weights
  * d_w1[i] (f32 [R+2][hidden], inputs speed/100, normalizeAngleDeg(rot)/360, hits/200) and d_w2[i] (f32 [hidden][6]);

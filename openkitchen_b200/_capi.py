@@ -100,6 +100,17 @@ class OkActorIO(C.Structure):
     ]
 
 
+class OkLidarQuery(C.Structure):
+    _fields_ = [
+        ("x", C.c_void_p), ("y", C.c_void_p), ("rot", C.c_void_p), ("track_id", C.c_void_p),
+        ("n", C.c_int64),
+        ("ray_deg", C.c_void_p),
+        ("rays", C.c_int32), ("reserved", C.c_int32),
+        ("hit_abs", C.c_void_p), ("hit_rel", C.c_void_p), ("obs", C.c_void_p), ("hit_t", C.c_void_p),
+        ("hit_seg", C.c_void_p), ("min_dist2", C.c_void_p), ("crashed", C.c_void_p),
+    ]
+
+
 # every symbol include/openkitchen_b200.h declares: (restype, argtypes)
 _P = C.c_void_p
 SIGNATURES = {
@@ -154,6 +165,8 @@ SIGNATURES = {
     "ok_discounted_returns": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.c_int64, C.c_float, _P]),
     "ok_track_query": (C.c_int, [_P, _P, _P, _P, C.c_int64, _P, _P, _P, _P]),
     "ok_track_query_host": (C.c_int, [_P, _P, _P, _P, C.c_int64, _P, _P, _P, _P]),
+    "ok_lidar_query": (C.c_int, [_P, C.POINTER(OkLidarQuery), _P]),
+    "ok_lidar_query_host": (C.c_int, [_P, C.POINTER(OkLidarQuery), _P]),
     "ok_pcie_probe": (C.c_int, [C.c_int32, C.c_size_t, C.c_int32, C.c_int32, C.POINTER(C.c_double)]),
 }
 

@@ -13,7 +13,9 @@ import torch
 
 from . import _capi
 from .dlpack import DeviceBuffer
-from .env import Env, ray_fan, track_names
+from .env import LIDAR_OUTPUTS, Env, ray_fan, track_names
+
+_TORCH_DTYPES = {np.float32: torch.float32, np.int32: torch.int32, np.uint8: torch.uint8}
 
 
 class BatchEnv:
@@ -97,6 +99,41 @@ class BatchEnv:
     def cast_rays(self):
         self.env.cast_rays(self._stream())
         return self.obs
+
+    def lidar(self, x, y, rot, track_id=None, rays=None, outputs=None) -> dict:
+        """Lidar scans at arbitrary poses, with no agent state read or written (ok_lidar_query): what ``cast_rays`` would
+        give agents at these poses with their crash flags clear.  x, y, rot: f32[n] (rot in degrees); track_id: i32[n] or
+        None (track 0).  rays: None (this env's fan), a count or angles, as in the constructor.  outputs: names to compute
+        (default all of obs, hits, hit_points, hit_seg, hit_t, min_dist2, crashed).  Returns fresh tensors keyed by those
+        names, computed on torch's current stream with no host synchronisation."""
+        names = list(LIDAR_OUTPUTS) if outputs is None else list(outputs)
+        unknown = [nm for nm in names if nm not in LIDAR_OUTPUTS]
+        if unknown:
+            raise ValueError(f"unknown lidar outputs {unknown}; expected some of {list(LIDAR_OUTPUTS)}")
+        n = int(torch.as_tensor(x).numel())
+        if any(torch.as_tensor(a).dim() != 1 for a in (x, y, rot)) or any(int(torch.as_tensor(a).numel()) != n for a in (y, rot)):
+            raise ValueError("x, y and rot must be 1-d tensors of one length")
+        if track_id is not None and int(torch.as_tensor(track_id).numel()) != n:
+            raise ValueError("track_id must have one entry per pose")
+        x, y, rot = (torch.as_tensor(a).to(self.device, torch.float32).contiguous() for a in (x, y, rot))
+        tid = None if track_id is None else torch.as_tensor(track_id).to(self.device, torch.int32).contiguous()
+        fan = None if rays is None else self._fan(rays)
+        r = self.n_rays if fan is None else int(fan.numel())
+        out = {nm: torch.empty(LIDAR_OUTPUTS[nm][2](n, r), device=self.device, dtype=_TORCH_DTYPES[LIDAR_OUTPUTS[nm][1]])
+               for nm in names}
+        self.env.lidar_query_device(x.data_ptr(), y.data_ptr(), rot.data_ptr(), n, None if tid is None else tid.data_ptr(),
+                                    None if fan is None else fan.data_ptr(), r, self._stream(),
+                                    **{LIDAR_OUTPUTS[nm][0]: t.data_ptr() for nm, t in out.items()})
+        return out
+
+    def _fan(self, rays) -> torch.Tensor:
+        """a ray fan as a device tensor, kept per distinct fan: the upload happens once, later queries do not wait for it"""
+        a = ray_fan(rays) if np.isscalar(rays) else np.ascontiguousarray(torch.as_tensor(rays).cpu().numpy(), dtype=np.float32)
+        key = a.tobytes()
+        fans = self.__dict__.setdefault("_fans", {})
+        if key not in fans:
+            fans[key] = torch.from_numpy(a.copy()).to(self.device)
+        return fans[key]
 
     # ---- resets ----------------------------------------------------------------------------
     def reset(self, agents=None, pt_idx=None, lane_alpha=None, heading_off=None):

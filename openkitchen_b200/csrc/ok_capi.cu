@@ -6,6 +6,7 @@
 
 #include "ok_beam_cache.hpp"
 #include "ok_kernels.cuh"
+#include "ok_lidar_query.cuh"
 #include "ok_step.cuh"
 #include "ok_track.hpp"
 
@@ -1366,6 +1367,136 @@ int ok_track_query_host(OkEnv *e, const float *h_x, const float *h_y, const int3
 } // extern "C"
 namespace
 {
+// the argument checks both lidar entry points make before touching the device
+int check_lidar_query(OkEnv *e, const OkLidarQuery *q)
+{
+    if (int rc = check_device(e))
+        return rc;
+    if (!q)
+        return fail(OK_ERR_INVALID_ARG, "query is NULL");
+    if (e->tracks.empty())
+        return fail(OK_ERR_STATE, "no track has been added");
+    if (!q->ray_deg)
+    {
+        if (e->n_agents <= 0)
+            return fail(OK_ERR_STATE, "ray_deg is NULL and ok_alloc_agents has not been called: there is no fan to use");
+        if (q->rays != e->rays)
+            return fail(OK_ERR_INVALID_ARG, "with ray_deg NULL, rays must be the env's ray count");
+    }
+    else if (q->rays < 1 || q->rays > 1024)
+        return fail(OK_ERR_INVALID_ARG, "rays must be in 1..1024");
+    if (q->n < 0)
+        return fail(OK_ERR_INVALID_ARG, "n < 0");
+    if (q->n > 0 && (!q->x || !q->y || !q->rot))
+        return fail(OK_ERR_INVALID_ARG, "pose arrays are NULL");
+    return OK_SUCCESS;
+}
+} // namespace
+extern "C"
+{
+int ok_lidar_query(OkEnv *e, const OkLidarQuery *q, void *stream)
+{
+    if (int rc = check_lidar_query(e, q))
+        return rc;
+    if (q->n == 0)
+        return OK_SUCCESS;
+    DeviceGuard  g(e->cfg.device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    // the arena (and in beam mode the device tables) may still have to be built, with synchronous copies: never inside a
+    // stream capture
+    if (e->arena_dirty || (e->cfg.raycast_mode == OK_RAYCAST_BEAM && !e->arena_has_beams))
+    {
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        const cudaError_t       err = cudaStreamIsCapturing(s, &cap);
+        if (err != cudaSuccess)
+            cudaGetLastError();
+        if (err != cudaSuccess || cap != cudaStreamCaptureStatusNone)
+            return fail(OK_ERR_STATE, "ok_lidar_query: the track arena is not built yet and the stream is capturing; call once outside the capture");
+        if (int rc = ensure_arena(e))
+            return rc;
+    }
+    ok::LidarQueryParams p{};
+    p.x = q->x, p.y = q->y, p.rot = q->rot, p.track = q->track_id, p.n = q->n;
+    p.ray_deg  = q->ray_deg ? q->ray_deg : e->ag.ray_deg.get();
+    p.rays     = q->rays;
+    p.n_tracks = static_cast<int32_t>(e->tracks.size());
+    p.arena    = e->d_arena.get();
+    p.tracks   = e->d_track_refs.get();
+    p.hit_abs = q->hit_abs, p.hit_rel = q->hit_rel, p.obs = q->obs, p.hit_t = q->hit_t, p.hit_seg = q->hit_seg;
+    p.min_dist2 = q->min_dist2, p.crashed = q->crashed;
+    p.sensor_range    = e->cfg.sensor_range;
+    p.sensor_offset   = e->cfg.sensor_offset;
+    p.collision_dist2 = e->cfg.collision_dist2;
+    p.raycast_mode    = e->cfg.raycast_mode;
+    OK_CUDA(ok::launch_lidar_query(p, s));
+    e->launches++;
+    return OK_SUCCESS;
+}
+
+int ok_lidar_query_host(OkEnv *e, const OkLidarQuery *hq, void *stream)
+{
+    if (int rc = check_lidar_query(e, hq))
+        return rc;
+    if (hq->n == 0)
+        return OK_SUCCESS;
+    DeviceGuard  g(e->cfg.device);
+    cudaStream_t s  = static_cast<cudaStream_t>(stream);
+    const size_t n  = static_cast<size_t>(hq->n), nr = n * static_cast<size_t>(hq->rays);
+    // one region of the env's staging buffer per array the call moves, 256-byte aligned
+    struct Region
+    {
+        const void *h_in;
+        void       *h_out;
+        size_t      bytes, off;
+    };
+    Region regions[] = {
+        {hq->x, nullptr, 4 * n, 0},           {hq->y, nullptr, 4 * n, 0},         {hq->rot, nullptr, 4 * n, 0},
+        {hq->track_id, nullptr, 4 * n, 0},    {hq->ray_deg, nullptr, 4 * static_cast<size_t>(hq->rays), 0},
+        {nullptr, hq->hit_abs, 8 * nr, 0},    {nullptr, hq->hit_rel, 8 * nr, 0},  {nullptr, hq->obs, 4 * nr, 0},
+        {nullptr, hq->hit_t, 4 * nr, 0},      {nullptr, hq->hit_seg, 4 * nr, 0},  {nullptr, hq->min_dist2, 4 * n, 0},
+        {nullptr, hq->crashed, n, 0},
+    };
+    size_t need = 0;
+    for (Region &r : regions)
+        if (r.h_in || r.h_out)
+        {
+            r.off = need;
+            need += (r.bytes + 255) / 256 * 256;
+        }
+    if (need > e->stage_bytes)
+    {
+        e->stage_bytes = 0;
+        OK_CUDA(dev_alloc(e->d_stage, need));
+        e->stage_bytes = need;
+    }
+    void *d[sizeof regions / sizeof regions[0]];
+    for (size_t i = 0; i < sizeof regions / sizeof regions[0]; ++i)
+    {
+        d[i] = (regions[i].h_in || regions[i].h_out) ? e->d_stage.get() + regions[i].off : nullptr;
+        if (regions[i].h_in)
+            OK_CUDA(cudaMemcpyAsync(d[i], regions[i].h_in, regions[i].bytes, cudaMemcpyHostToDevice, s));
+    }
+    OkLidarQuery dq = *hq;
+    dq.x = static_cast<const float *>(d[0]), dq.y = static_cast<const float *>(d[1]), dq.rot = static_cast<const float *>(d[2]);
+    dq.track_id = static_cast<const int32_t *>(d[3]), dq.ray_deg = static_cast<const float *>(d[4]);
+    dq.hit_abs = static_cast<float *>(d[5]), dq.hit_rel = static_cast<float *>(d[6]), dq.obs = static_cast<float *>(d[7]);
+    dq.hit_t = static_cast<float *>(d[8]), dq.hit_seg = static_cast<int32_t *>(d[9]), dq.min_dist2 = static_cast<float *>(d[10]);
+    dq.crashed = static_cast<uint8_t *>(d[11]);
+    if (int rc = ok_lidar_query(e, &dq, stream))
+    {
+        cudaStreamSynchronize(s); // the uploads above still read the caller's arrays
+        return rc;
+    }
+    for (size_t i = 0; i < sizeof regions / sizeof regions[0]; ++i)
+        if (regions[i].h_out)
+            OK_CUDA(cudaMemcpyAsync(regions[i].h_out, d[i], regions[i].bytes, cudaMemcpyDeviceToHost, s));
+    OK_CUDA(cudaStreamSynchronize(s));
+    return OK_SUCCESS;
+}
+
+} // extern "C"
+namespace
+{
 // ok_step_host / ok_step_host_q16: `h_obs` is float[N][R], or uint16_t[N][R] when `q16`
 int step_host_impl(OkEnv *e, const float *h_thr, const float *h_steer, void *h_obs_any, const bool q16, float *h_reward, uint8_t *h_done,
                    void *stream)
@@ -1743,13 +1874,14 @@ int ok_debug_violations(OkEnv *e, uint64_t *count, int32_t *checks_compiled_in)
         return fail(OK_ERR_NO_DEVICE, "no device");
     DeviceGuard g(e->cfg.device);
     OK_CUDA(cudaDeviceSynchronize());
-    unsigned long long staged = 0, unstaged = 0, actor = 0, grid = 0;
+    unsigned long long staged = 0, unstaged = 0, actor = 0, grid = 0, lidar = 0;
     OK_CUDA(ok::violations_step_staged(&staged));
     OK_CUDA(ok::violations_step_unstaged(&unstaged));
     OK_CUDA(ok::violations_step_actor(&actor));
     OK_CUDA(ok::violations_step_grid(&grid));
+    OK_CUDA(ok::violations_lidar_query(&lidar));
     if (count)
-        *count = staged + unstaged + actor + grid;
+        *count = staged + unstaged + actor + grid + lidar;
     if (checks_compiled_in)
         *checks_compiled_in = OK_CHECKED;
     return OK_SUCCESS;

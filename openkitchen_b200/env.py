@@ -57,6 +57,28 @@ def ray_fan(n_rays: int) -> np.ndarray:
     return (np.float32(-70.0) + (i * np.float32(140.0)) / np.float32(n_rays - 1)).astype(np.float32)
 
 
+# the outputs of a lidar query, by their BatchEnv names: (OkLidarQuery field, numpy dtype, shape for (poses, rays))
+LIDAR_OUTPUTS = {
+    "obs": ("obs", np.float32, lambda n, r: (n, r)),
+    "hits": ("hit_rel", np.float32, lambda n, r: (n, r, 2)),
+    "hit_points": ("hit_abs", np.float32, lambda n, r: (n, r, 2)),
+    "hit_seg": ("hit_seg", np.int32, lambda n, r: (n, r)),
+    "hit_t": ("hit_t", np.float32, lambda n, r: (n, r)),
+    "min_dist2": ("min_dist2", np.float32, lambda n, r: (n,)),
+    "crashed": ("crashed", np.uint8, lambda n, r: (n,)),
+}
+
+
+def _pose_arrays(x, y, rot, track_id=None):
+    """x, y, rot as contiguous binary32 vectors of one length (and track_id of that length); raises ValueError otherwise"""
+    x, y, rot = (np.ascontiguousarray(a, dtype=np.float32) for a in (x, y, rot))
+    if x.ndim != 1 or x.shape != y.shape or x.shape != rot.shape:
+        raise ValueError("x, y and rot must be 1-d arrays of one length")
+    if track_id is not None and np.shape(track_id) != x.shape:
+        raise ValueError("track_id must have one entry per pose")
+    return x, y, rot
+
+
 class Env:
     """Owns one ``OkEnv``.  ``device=-1`` builds a host-only env (tracks can be built and inspected)."""
 
@@ -254,6 +276,33 @@ class Env:
     def track_query_device(self, d_x, d_y, d_track_id, n, d_idx=None, d_lane=None, d_bound=None, stream=None):
         """device-pointer form (asynchronous on `stream`)"""
         check(self.lib.ok_track_query(self.h, d_x, d_y, d_track_id, n, d_idx, d_lane, d_bound, stream))
+
+    def lidar_query(self, x, y, rot, track_id=None, ray_deg=None, stream=None) -> dict:
+        """Lidar scans at arbitrary poses (host arrays), with no agent state read or written: what ok_cast_rays would give
+        agents at these poses with their crash flags clear.  ray_deg None = the fan of alloc_agents.  Returns a dict keyed
+        by the BatchEnv names (see LIDAR_OUTPUTS); synchronises `stream`."""
+        x, y, rot = _pose_arrays(x, y, rot, track_id)
+        t = None if track_id is None else np.ascontiguousarray(track_id, dtype=np.int32)
+        fan = None if ray_deg is None else np.ascontiguousarray(ray_deg, dtype=np.float32).reshape(-1)
+        n, rays = len(x), (self.rays if fan is None else len(fan))
+        out = {name: np.empty(shape(n, rays), dtype=dt) for name, (_, dt, shape) in LIDAR_OUTPUTS.items()}
+        q = _capi.OkLidarQuery(x=_vp(x), y=_vp(y), rot=_vp(rot), track_id=_vp(t), n=n, ray_deg=_vp(fan), rays=rays)
+        for name, (field, _, _) in LIDAR_OUTPUTS.items():
+            setattr(q, field, _vp(out[name]))
+        check(self.lib.ok_lidar_query_host(self.h, C.byref(q), stream))
+        return out
+
+    def lidar_query_device(self, d_x, d_y, d_rot, n: int, d_track_id=None, d_ray_deg=None, rays=None, stream=None, **d_out):
+        """device-pointer form of lidar_query (asynchronous on `stream`): d_out maps the C field names (hit_abs, hit_rel,
+        obs, hit_t, hit_seg, min_dist2, crashed) to device pointers; absent outputs are not computed.  rays None = the
+        env's ray count."""
+        fields = {f for f, _, _ in LIDAR_OUTPUTS.values()}
+        unknown = set(d_out) - fields
+        if unknown:
+            raise ValueError(f"unknown lidar outputs {sorted(unknown)}; expected some of {sorted(fields)}")
+        q = _capi.OkLidarQuery(x=d_x, y=d_y, rot=d_rot, track_id=d_track_id, n=n, ray_deg=d_ray_deg,
+                               rays=self.rays if rays is None else rays, **d_out)
+        check(self.lib.ok_lidar_query(self.h, C.byref(q), stream))
 
     def sync(self, stream=None):
         check(self.lib.ok_sync(self.h, stream))
