@@ -415,10 +415,10 @@ bool beam_lookup(const std::vector<uint8_t> &blob, float x, float y, float angle
     const int32_t bin = static_cast<int32_t>(std::floor(angle * h.bin_scale)) & (h.nb - 1);
     uint32_t      e[4];
     std::memcpy(e, blob.data() + h.off_entries + 16 * (static_cast<size_t>(row) * h.nb + bin), 16);
-    const uint32_t dq = e[3] & 0xfffu, d1q = (e[3] >> 12) & 0xfffu, n_rest = e[3] >> 24;
-    d_out             = dq == kBeamDistFull ? h.rb : static_cast<float>(dq) * (1.0f / kBeamDistScale);
+    const uint32_t n_rest = beam_meta_rest(e[3]);
+    d_out                 = beam_meta_d(e[3], h.rb);
     if (d1_out)
-        *d1_out = n_rest ? static_cast<float>(d1q) * (1.0f / kBeamDistScale) : d_out;
+        *d1_out = n_rest ? beam_meta_d1(e[3], h.rb) : d_out;
     if ((h.tag >> 16) != kBeamFormat)
         return false;
     const uint16_t null_seg = static_cast<uint16_t>(h.tag & 0xffffu); // padding value: the blob's null segment
@@ -474,7 +474,7 @@ bool beam_validate(const std::vector<uint8_t> &blob, int32_t n_segments, std::st
         if ((e[0] & 0xffffu) > static_cast<uint32_t>(n_segments) || (e[0] >> 16) > static_cast<uint32_t>(n_segments) ||
             (e[1] & 0xffffu) > static_cast<uint32_t>(n_segments) || (e[1] >> 16) > static_cast<uint32_t>(n_segments))
             return bad("inline segment index");
-        const uint32_t n_rest = e[3] >> 24;
+        const uint32_t n_rest = beam_meta_rest(e[3]);
         if (n_rest && static_cast<uint64_t>(e[2]) + n_rest > h.n_chunks)
             return bad("chunk range");
     }

@@ -79,6 +79,20 @@ OK_BEAM_HD uint32_t beam_pack_meta(double d, double d1, bool full, uint32_t n_re
     const uint32_t d1q = static_cast<uint32_t>(q1 < 0.0 ? 0.0 : (q1 > 4094.0 ? 4094.0 : q1));
     return dq | (d1q << 12) | (n_rest << 24);
 }
+// the fields of a meta word w: chunks of the rest, d, d1 (rb = the table's completeness distance of full lists)
+OK_BEAM_HD uint32_t beam_meta_rest(uint32_t w)
+{
+    return w >> 24;
+}
+OK_BEAM_HD float beam_meta_d(uint32_t w, float rb)
+{
+    const uint32_t q = w & 0xfffu;
+    return q == kBeamDistFull ? rb : static_cast<float>(q) * (1.0f / kBeamDistScale);
+}
+OK_BEAM_HD float beam_meta_d1(uint32_t w, float rb)
+{
+    return beam_meta_d(w >> 12, rb);
+}
 
 struct BeamConfig
 {

@@ -4,6 +4,7 @@
 // PPO racers' policy step (actor_agent).
 #pragma once
 
+#include "../../include/openkitchen_b200.h" // OK_RAYCAST_GRID / BRUTE / BEAM
 #include "ok_beam.hpp"
 #include "ok_math.cuh"
 #include "ok_schedule.hpp"
@@ -636,8 +637,36 @@ __device__ __forceinline__ uint32_t obs_q16(const float ob)
     return __float2uint_rn(fmul(fminf(fmaxf(ob, 0.0f), 1.0f), 65535.0f));
 }
 
-// hit point, unpack (CollisionChecker.cu:68-69,152-165) and the per-ray outputs of ray `gi`, whose nearest
-// segment is `seg` (-1 = none); returns the squared norm of the relative hit
+// The lidar's geometry, shared by agent_pre, finish_ray and the lidar query kernel.  (ox, oy) = the lidar origin, (rc, rs)
+// = cos / sin of the heading, (dx, dy) = a ray's direction.
+// lidar origin, CollisionChecker.cu:121-124
+__device__ __forceinline__ float2 lidar_origin(const float x, const float y, const float rc, const float rs, const float offset)
+{
+    return make_float2(fadd(x, fmul(offset, rc)), fadd(y, fmul(offset, rs)));
+}
+// hit point (CollisionChecker.cu:68-69)
+__device__ __forceinline__ float2 ray_hit(const float ox, const float oy, const float dx, const float dy, const float t)
+{
+    return make_float2(fadd(ox, fmul(t, dx)), fadd(oy, fmul(t, dy)));
+}
+// unpack (CollisionChecker.cu:152-165): the hit in the lidar's frame and its squared norm.  By reference, so that
+// finish_ray reads its record's fields where they are used: read up front, they changed the step kernels' schedule.
+__device__ __forceinline__ float2 ray_rel(const float &ox, const float &oy, const float &rc, const float &rs, const float2 hit, float &sq)
+{
+    const float xt = fsub(hit.x, ox), yt = fsub(hit.y, oy);
+    float2      rel;
+    rel.x = fsub(fmul(xt, rc), fmul(yt, rs));
+    rel.y = fadd(fmul(xt, rs), fmul(yt, rc));
+    sq    = fadd(fmul(rel.x, rel.x), fmul(rel.y, rel.y));
+    return rel;
+}
+__device__ __forceinline__ float ray_obs(const float sq, const float range)
+{
+    return __fdiv_rn(__fsqrt_rn(sq), range);
+}
+
+// hit point, unpack and the per-ray outputs of ray `gi`, whose nearest segment is `seg` (-1 = none); returns the squared
+// norm of the relative hit
 // t_known != 0: the winner's exact t is already at hand (the beam key holds it; a zero is recomputed because the
 // key does not keep its sign)
 // kGrid (the grid kernel's phase 3): phase 2 has already stored the hit index, and the per-ray host mirrors are stored
@@ -654,20 +683,16 @@ __device__ __forceinline__ float finish_ray(const StepParams &p, const float4 *s
         if (!kGrid)
             p.hit_seg[gi] = seg;
         p.hit_t[gi]   = t;
-        hit.x         = fadd(rec.ox, fmul(t, dx));
-        hit.y         = fadd(rec.oy, fmul(t, dy));
+        hit           = ray_hit(rec.ox, rec.oy, dx, dy, t);
         reinterpret_cast<float2 *>(p.hit_abs)[gi] = hit;
     }
     else
         hit = reinterpret_cast<const float2 *>(p.hit_abs)[gi]; // stale hit of a crashed agent
     OK_CHECK(gi >= 0 && seg >= -1);
-    const float xt = fsub(hit.x, rec.ox), yt = fsub(hit.y, rec.oy);
-    float2      rel;
-    rel.x          = fsub(fmul(xt, rec.rc), fmul(yt, rec.rs));
-    rel.y          = fadd(fmul(xt, rec.rs), fmul(yt, rec.rc));
-    const float sq = fadd(fmul(rel.x, rel.x), fmul(rel.y, rel.y));
+    float        sq;
+    const float2 rel = ray_rel(rec.ox, rec.oy, rec.rc, rec.rs, hit, sq);
     reinterpret_cast<float2 *>(p.hit_rel)[gi] = rel;
-    const float ob = __fdiv_rn(__fsqrt_rn(sq), p.sensor_range);
+    const float ob = ray_obs(sq, p.sensor_range);
     p.obs[gi]      = ob;
     if (kGrid && p.host_obs)
         p.host_obs[gi] = ob;
@@ -821,13 +846,12 @@ __device__ __forceinline__ AgentRec agent_pre(const StepParams &p, const uint8_t
         p.x[a] = x, p.y[a] = y, p.rot[a] = rot, p.speed[a] = speed, p.accel[a] = accel;
         p.timed_out[a] = timed_out;
     }
-    // lidar origin, CollisionChecker.cu:121-124
     float rs = hs, rc = hc;
     if (!have_sc)
         sincosf(fmul(OK_DEG2RAD, rot), rs, rc);
-    AgentRec rec;
-    rec.ox = fadd(x, fmul(p.sensor_offset, rc));
-    rec.oy = fadd(y, fmul(p.sensor_offset, rs));
+    AgentRec     rec;
+    const float2 o = lidar_origin(x, y, rc, rs, p.sensor_offset);
+    rec.ox = o.x, rec.oy = o.y;
     rec.rc = rc, rec.rs = rs, rec.rot = rot, rec.x = x, rec.y = y, rec.rx = rx, rec.ry = ry;
     rec.min_d2_bits = __float_as_int(fmul(p.sensor_range, p.sensor_range));
     rec.flags       = flags | (crashed ? kFlagCrashed : 0u) | (timed_out ? kFlagTimedOut : 0u);

@@ -8,12 +8,12 @@
 // poses; for R > 32 a pose takes consecutive warps of one CTA (and a thread loops when R > kLidarBlock).  min_dist2 and
 // the crash flag are reduced in registers and shared memory and stored once per pose.
 //
-// Every output is bit for bit what ok_cast_rays writes for an agent at the same pose with no crash flag set: lidar origin
-// as agent_pre computes it, the beam kernel's per-ray decision (inline chunk, rest chunks, grid walk), finish_ray's
-// arithmetic and agent_post's strict crash test.  The rest chunks of a warp's undecided rays are dealt across its lanes
-// as process_full deals them (the beam kernel first gathers its undecided rays into full warps; here they stay where
-// they are).  The decision rule is restated here, not shared with the beam kernel: tests/test_gpu_lidar_query.py ties
-// the two copies together bit for bit.
+// Every output is bit for bit what ok_cast_rays writes for an agent at the same pose with no crash flag set.  The lidar
+// origin, the beam decision (beam_settles, beam_walk_rest), the table's meta word and result key, and the ray outputs
+// (ray_hit, ray_rel, ray_obs) are the step kernels' own helpers.  This kernel's own parts are its dealing loop and its
+// per-pose reductions: the rest chunks of a warp's undecided rays are dealt across its lanes as process_full deals them,
+// but the rays stay where they are (the beam kernel first gathers them into full warps); tests/test_gpu_lidar_query.py
+// checks those parts against ok_cast_rays bit for bit.
 #include "ok_lidar_query.cuh"
 #include "ok_step.cuh"
 
@@ -73,14 +73,14 @@ __global__ void __launch_bounds__(kLidarBlock, kLidarMinCtas) lidar_query_kernel
         const float x = q.x[k], y = q.y[k], rot = q.rot[k];
         float       rs, rc;
         sincosf(fmul(OK_DEG2RAD, rot), rs, rc);
-        LidarPose ps;
-        ps.ox = fadd(x, fmul(q.sensor_offset, rc));
-        ps.oy = fadd(y, fmul(q.sensor_offset, rs));
+        LidarPose    ps;
+        const float2 o = lidar_origin(x, y, rc, rs, q.sensor_offset);
+        ps.ox = o.x, ps.oy = o.y;
         ps.rc = rc, ps.rs = rs, ps.rot = rot, ps.track = t, ps.pad = 0;
         const TrackRef &tr = q.tracks[t];
         BeamView        bv;
         bv.valid = false;
-        if (q.raycast_mode == kLidarBeam && tr.has_beam)
+        if (q.raycast_mode == OK_RAYCAST_BEAM && tr.has_beam)
             bv = make_beam_view(tr);
         ps.row      = beam_row(bv, ps.ox, ps.oy);
         s_pose[tid] = ps;
@@ -98,7 +98,7 @@ __global__ void __launch_bounds__(kLidarBlock, kLidarMinCtas) lidar_query_kernel
     const TrackView tv   = make_view(blob);
     BeamView        bv;
     bv.valid = false;
-    if (q.raycast_mode == kLidarBeam && tr.has_beam)
+    if (q.raycast_mode == OK_RAYCAST_BEAM && tr.has_beam)
         bv = make_beam_view(tr);
     const unsigned long long key_none = (static_cast<unsigned long long>(__float_as_uint(q.sensor_range)) << 32) | 0x80000000ull;
     float                    m        = __int_as_float(0x7f800000);
@@ -115,7 +115,7 @@ __global__ void __launch_bounds__(kLidarBlock, kLidarMinCtas) lidar_query_kernel
         }
         int   seg     = -1;
         float t_known = 0.0f; // the winner's exact t when a beam key holds it (0 = recompute it)
-        if (q.raycast_mode == kLidarBeam)
+        if (q.raycast_mode == OK_RAYCAST_BEAM)
         { // the beam kernel's decision: pass A's inline chunk, process_full's rest chunks, the grid walk
             const bool         cov = has && ps.row >= 0 && fabsf(ang) < kBeamMaxAngle;
             uint4              ent = make_uint4(0u, 0u, 0u, 0u);
@@ -125,23 +125,14 @@ __global__ void __launch_bounds__(kLidarBlock, kLidarMinCtas) lidar_query_kernel
                 const int bin = __float2int_rd(fmul(ang, bv.bin_scale)) & (bv.nb - 1);
                 OK_CHECK(static_cast<uint32_t>(ps.row) < bv.n_rows);
                 ent = __ldg(bv.entries + static_cast<size_t>(ps.row) * bv.nb + bin);
-                OK_CHECK((ent.w >> 24) == 0 || ent.z + (ent.w >> 24) <= bv.n_chunks);
+                OK_CHECK(beam_meta_rest(ent.w) == 0 || ent.z + beam_meta_rest(ent.w) <= bv.n_chunks);
                 key = beam_chunk_key(tv.seg, ent.x, ent.y, ps.ox, ps.oy, dx, dy, q.sensor_range, key_none, tv.n_seg);
             }
-            // d1: up to there the inline four are the only contenders (pass A's test)
-            const bool     undecided =
-                has && !(cov && __uint_as_float(static_cast<uint32_t>(key >> 32)) <= beam_meta_dist((ent.w >> 12) & 0xfffu, bv.rb) - kBeamSlack);
-            const uint32_t nch = (undecided && cov) ? (ent.w >> 24) : 0u; // chunks of the rest of the list
+            const bool     undecided = has && !beam_settles(cov, key, beam_meta_d1(ent.w, bv.rb));
+            const uint32_t nch       = (undecided && cov) ? beam_meta_rest(ent.w) : 0u; // chunks of the rest of the list
             if (__any_sync(0xffffffffu, nch > 0))
             { // process_full's dealing: chunk j of the warp's rest chunks goes to lane j % 32, results meet in a shared key
-                uint32_t inc = nch;
-#pragma unroll
-                for (int o = 1; o < 32; o <<= 1)
-                {
-                    const uint32_t v = __shfl_up_sync(0xffffffffu, inc, o);
-                    if (lane >= o)
-                        inc += v;
-                }
+                const uint32_t inc   = warp_inclusive_scan(nch, lane);
                 const uint32_t total = __shfl_sync(0xffffffffu, inc, 31);
                 s_wray[tid]  = make_float4(ps.ox, ps.oy, dx, dy);
                 s_wkey[tid]  = key;
@@ -153,22 +144,15 @@ __global__ void __launch_bounds__(kLidarBlock, kLidarMinCtas) lidar_query_kernel
                 for (uint32_t base = 0; base < total; base += 32)
                 {
                     const uint32_t j     = base + lane;
-                    int            owner = 0; // the lane whose prefix range contains j
-#pragma unroll
-                    for (int s2 = 16; s2 > 0; s2 >>= 1)
-                    {
-                        const uint32_t v = __shfl_sync(0xffffffffu, inc, owner + s2 - 1);
-                        if (v <= j)
-                            owner += s2;
-                    }
+                    const int      owner = w0 + chunk_owner(inc, j);
                     if (j < total)
                     {
-                        const uint2               it = __ldg(s_wchk[w0 + owner] + j);
-                        const float4              ry = s_wray[w0 + owner];
-                        unsigned long long *const kp = s_wkey + w0 + owner;
+                        const uint2               it = __ldg(s_wchk[owner] + j);
+                        const float4              ry = s_wray[owner];
+                        unsigned long long *const kp = s_wkey + owner;
                         // the ray's incumbent exact t (already in the key) bounds what is worth a division
-                        const float              mt = __uint_as_float(reinterpret_cast<const uint32_t *>(kp)[1]);
-                        const unsigned long long kc = beam_chunk_key(s_wseg[w0 + owner], it.x, it.y, ry.x, ry.y, ry.z, ry.w, mt, ~0ull, s_wnseg[w0 + owner]);
+                        const unsigned long long kc =
+                            beam_chunk_key(s_wseg[owner], it.x, it.y, ry.x, ry.y, ry.z, ry.w, beam_key_t_at(kp), ~0ull, s_wnseg[owner]);
                         if (kc != ~0ull)
                             atomicMin(kp, kc);
                     }
@@ -177,20 +161,16 @@ __global__ void __launch_bounds__(kLidarBlock, kLidarMinCtas) lidar_query_kernel
                 key = s_wkey[tid];
                 __syncwarp(); // the next round rewrites the warp's slots
             }
-            const float min_t = __uint_as_float(static_cast<uint32_t>(key >> 32));
-            seg               = static_cast<int>(0x7fffffffu - static_cast<uint32_t>(key));
-            t_known           = min_t; // the key holds the exact t of its segment, or the sensor range when nothing was hit
-            if (undecided)
+            const float d_eff = beam_meta_d(ent.w, bv.rb);
+            seg               = beam_key_seg(key);
+            t_known           = beam_key_t(key); // the key holds the exact t of its segment
+            if (undecided && !beam_settles(cov, key, d_eff))
             {
-                const float d_eff = beam_meta_dist(ent.w & 0xfffu, bv.rb);
-                if (!(cov && min_t <= d_eff - kBeamSlack))
-                { // everything nearer than d_eff - 1 is settled, the grid walk covers the rest
-                    seg     = beam_walk_fallback(blob, ps.ox, ps.oy, dx, dy, q.sensor_range, cov ? fmaxf(d_eff - 1.0f, 0.0f) : 0.0f, seg, min_t);
-                    t_known = 0.0f;
-                }
+                seg     = beam_walk_rest(blob, ps.ox, ps.oy, dx, dy, q.sensor_range, cov, d_eff, key);
+                t_known = 0.0f;
             }
         }
-        else if (has && q.raycast_mode == kLidarGrid)
+        else if (has && q.raycast_mode == OK_RAYCAST_GRID)
         {
             RayWalk w;
             if (walk_begin(tv, w, ps.ox, ps.oy, dx, dy, q.sensor_range))
@@ -207,16 +187,11 @@ __global__ void __launch_bounds__(kLidarBlock, kLidarMinCtas) lidar_query_kernel
             continue; // (uniform loop: nothing below is warp-collective)
         OK_CHECK(seg >= -1 && seg < tv.n_seg);
         const int64_t gi = k * R + r;
-        // finish_ray: hit point, unpack (CollisionChecker.cu:68-69,152-165)
-        const float t = seg >= 0 ? (t_known != 0.0f ? t_known : exact_t(tv.seg[seg], ps.ox, ps.oy, dx, dy)) : q.sensor_range;
-        float2      hit;
-        hit.x          = fadd(ps.ox, fmul(t, dx));
-        hit.y          = fadd(ps.oy, fmul(t, dy));
-        const float xt = fsub(hit.x, ps.ox), yt = fsub(hit.y, ps.oy);
-        float2      rel;
-        rel.x          = fsub(fmul(xt, ps.rc), fmul(yt, ps.rs));
-        rel.y          = fadd(fmul(xt, ps.rs), fmul(yt, ps.rc));
-        const float sq = fadd(fmul(rel.x, rel.x), fmul(rel.y, rel.y));
+        // finish_ray's outputs, each only if asked for
+        const float  t   = seg >= 0 ? (t_known != 0.0f ? t_known : exact_t(tv.seg[seg], ps.ox, ps.oy, dx, dy)) : q.sensor_range;
+        const float2 hit = ray_hit(ps.ox, ps.oy, dx, dy, t);
+        float        sq;
+        const float2 rel = ray_rel(ps.ox, ps.oy, ps.rc, ps.rs, hit, sq);
         if (q.hit_seg)
             q.hit_seg[gi] = seg;
         if (q.hit_t)
@@ -226,7 +201,7 @@ __global__ void __launch_bounds__(kLidarBlock, kLidarMinCtas) lidar_query_kernel
         if (q.hit_rel)
             reinterpret_cast<float2 *>(q.hit_rel)[gi] = rel;
         if (q.obs)
-            q.obs[gi] = __fdiv_rn(__fsqrt_rn(sq), q.sensor_range);
+            q.obs[gi] = ray_obs(sq, q.sensor_range);
         // min_dist2 of CollisionChecker.cu:150,162-165: `if (sq < min) min = sq` skips NaN
         if (sq == sq)
             m = fminf(m, sq);

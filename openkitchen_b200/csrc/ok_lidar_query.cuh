@@ -6,14 +6,6 @@
 
 namespace ok
 {
-// OkRaycastMode's values
-enum : int32_t
-{
-    kLidarGrid  = 0,
-    kLidarBrute = 1,
-    kLidarBeam  = 2
-};
-
 struct LidarQueryParams
 {
     const float   *x, *y, *rot; // f32[n]: pose (rot in degrees)
@@ -30,7 +22,7 @@ struct LidarQueryParams
     float   *min_dist2;         // f32[n]
     uint8_t *crashed;           // u8[n]: min_dist2 < collision_dist2
     float    sensor_range, sensor_offset, collision_dist2;
-    int32_t  raycast_mode;
+    int32_t  raycast_mode;      // OkRaycastMode
 };
 
 constexpr int kLidarBlock = 256;

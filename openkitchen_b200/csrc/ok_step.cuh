@@ -69,6 +69,21 @@ __device__ __forceinline__ unsigned long long beam_key(float t, int idx)
     const uint32_t tb = (t == 0.0f) ? 0u : __float_as_uint(t);
     return (static_cast<unsigned long long>(tb) << 32) | static_cast<uint32_t>(0x7fffffff - idx);
 }
+// a key's exact t and segment (-1 = none)
+__device__ __forceinline__ float beam_key_t(const unsigned long long key)
+{
+    return __uint_as_float(static_cast<uint32_t>(key >> 32));
+}
+__device__ __forceinline__ int beam_key_seg(const unsigned long long key)
+{
+    return static_cast<int>(0x7fffffffu - static_cast<uint32_t>(key));
+}
+// the incumbent exact t of the key at `kp` (shared memory), while the rest chunks of its ray are being dealt: the high
+// word alone, one 32-bit load
+__device__ __forceinline__ float beam_key_t_at(const unsigned long long *kp)
+{
+    return __uint_as_float(reinterpret_cast<const uint32_t *>(kp)[1]);
+}
 
 // One candidate, written without branches (a warp's lanes hold unrelated rays, so every branch here would be
 // taken by a few lanes while the others wait) and free of dependences on the other candidates of the chunk, so
@@ -174,11 +189,6 @@ __device__ __forceinline__ unsigned long long beam_chunk_key(const float4 *segs,
     return key;
 }
 
-__device__ __forceinline__ float beam_meta_dist(const uint32_t q, const float rb)
-{ // 12-bit distance field of an entry's meta word (ok_beam.hpp): 1/16 px, all ones = complete up to rb
-    return q == kBeamDistFull ? rb : static_cast<float>(q) * (1.0f / kBeamDistScale);
-}
-
 // The rare ray a beam list cannot decide: uniform-grid walk from t_start with the best listed hit (best, min_t)
 // as the incumbent.  Out of line on purpose: the walk's state would otherwise count against the registers of
 // the hot loop around the call.
@@ -198,6 +208,51 @@ static __device__ __noinline__ int beam_walk_fallback(const uint8_t *blob, float
     {
     }
     return w.best;
+}
+
+// The beam decision of one ray, whose cell is covered (`cov`) by a table entry, and whose key holds its best listed hit
+// (the exact t, or the sensor range when nothing was hit).  Is that hit final?  Only if it lies within the distance d up
+// to which the listed candidates are the only contenders, less the slack: d1 after the entry's inline chunk (the
+// list's completeness distance when it has no rest), d after the rest chunks.
+__device__ __forceinline__ bool beam_settles(const bool cov, const unsigned long long key, const float d)
+{
+    return cov && (beam_key_t(key) <= d - kBeamSlack);
+}
+// A ray the whole list does not settle: everything nearer than d - 1 is settled, the grid walk covers the rest with the
+// listed hit as the incumbent.  Returns the segment.
+__device__ __forceinline__ int beam_walk_rest(const uint8_t *blob, const float ox, const float oy, const float dx, const float dy,
+                                              const float range, const bool cov, const float d, const unsigned long long key)
+{
+    return beam_walk_fallback(blob, ox, oy, dx, dy, range, cov ? fmaxf(d - 1.0f, 0.0f) : 0.0f, beam_key_seg(key), beam_key_t(key));
+}
+
+// Dealing a warp's rest chunks across its lanes (warp-collective): each lane's chunk count is scanned, and chunk j of the
+// warp belongs to the lane whose prefix range holds it.
+// `lane` is the caller's: a second read of threadIdx.x here loses the range the kernel's launch bounds give the first,
+// and the step kernels' shared-memory addressing grows.
+__device__ __forceinline__ uint32_t warp_inclusive_scan(uint32_t v, const int lane)
+{
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1)
+    {
+        const uint32_t u = __shfl_up_sync(0xffffffffu, v, o);
+        if (lane >= o)
+            v += u;
+    }
+    return v;
+}
+// the owner of chunk j: a shuffle binary search over the lanes' inclusive prefix sums `inc`
+__device__ __forceinline__ int chunk_owner(const uint32_t inc, const uint32_t j)
+{
+    int owner = 0;
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1)
+    {
+        const uint32_t v = __shfl_sync(0xffffffffu, inc, owner + s - 1);
+        if (v <= j)
+            owner += s;
+    }
+    return owner;
 }
 
 // beam mode: AgentRec only (the per-thread scratch is static shared memory)
@@ -525,7 +580,7 @@ __global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN
                         const uint2 c4 = __ldg(reinterpret_cast<const uint2 *>(ep));
                         ent            = make_uint4(c4.x, c4.y, 0u, __ldg(reinterpret_cast<const uint32_t *>(ep) + 3));
                     }
-                    OK_CHECK(!need_rest || (ent.w >> 24) == 0 || ent.z + (ent.w >> 24) <= bv.n_chunks);
+                    OK_CHECK(!need_rest || beam_meta_rest(ent.w) == 0 || ent.z + beam_meta_rest(ent.w) <= bv.n_chunks);
                     cov           = true;
                 }
             }
@@ -546,29 +601,14 @@ __global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN
             unsigned long long key0 = key_none;
             if (cov)
                 key0 = beam_chunk_key(tv.seg, ent.x, ent.y, rox, roy, dx, dy, p.sensor_range, key_none, tv.n_seg);
-            w_key[lane]        = key0;
-            const uint32_t nch = cov ? (ent.w >> 24) : 0u; // chunks of the rest of the list
-            uint32_t       inc = nch;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1)
-            {
-                const uint32_t v = __shfl_up_sync(0xffffffffu, inc, o);
-                if (lane >= o)
-                    inc += v;
-            }
+            w_key[lane]          = key0;
+            const uint32_t nch   = cov ? beam_meta_rest(ent.w) : 0u; // chunks of the rest of the list
+            const uint32_t inc   = warp_inclusive_scan(nch, lane);
             const uint32_t total = __shfl_sync(0xffffffffu, inc, 31);
             const uint32_t first = ent.z - (inc - nch); // chunk j of the warp's rest chunks is chunk (first + j) of the table
             __syncwarp();
-            // chunk j belongs to the lane `owner` whose prefix range contains j
             auto find_chunk = [&](uint32_t j, int &owner) -> uint32_t {
-                owner = 0;
-#pragma unroll
-                for (int s2 = 16; s2 > 0; s2 >>= 1)
-                {
-                    const uint32_t v = __shfl_sync(0xffffffffu, inc, owner + s2 - 1);
-                    if (v <= j)
-                        owner += s2;
-                }
+                owner = chunk_owner(inc, j);
                 return __shfl_sync(0xffffffffu, first, owner) + j;
             };
             int   owner = 0;
@@ -599,8 +639,8 @@ __global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN
                     const float4        ray = w_ray[owner];
                     unsigned long long *key = w_key + owner;
                     // the ray's incumbent exact t (already in the key) bounds what is worth a division
-                    const float              m = __uint_as_float(reinterpret_cast<const uint32_t *>(key)[1]);
-                    const unsigned long long k = beam_chunk_key(tv.seg, it.x, it.y, ray.x, ray.y, ray.z, ray.w, m, ~0ull, tv.n_seg);
+                    const unsigned long long k =
+                        beam_chunk_key(tv.seg, it.x, it.y, ray.x, ray.y, ray.z, ray.w, beam_key_t_at(key), ~0ull, tv.n_seg);
                     if (k != ~0ull)
                         atomicMin(key, k);
                 }
@@ -612,14 +652,12 @@ __global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN
             {
                 const AgentRec          &rec   = recs[al];
                 const unsigned long long key   = w_key[lane];
-                int                      best  = static_cast<int>(0x7fffffffu - static_cast<uint32_t>(key));
-                const float              min_t = __uint_as_float(static_cast<uint32_t>(key >> 32));
-                const float              d_eff = beam_meta_dist(ent.w & 0xfffu, ld_hot(s_hot.rb));
-                float t_known = min_t; // the key holds the exact t of `best`
-                if (active && !(cov && min_t <= d_eff - kBeamSlack))
-                { // undecided: everything nearer than d_eff - 1 is settled, the grid walk covers the rest
-                    best = beam_walk_fallback(track, rec.ox, rec.oy, dx, dy, p.sensor_range,
-                                              cov ? fmaxf(d_eff - 1.0f, 0.0f) : 0.0f, best, min_t);
+                int                      best  = beam_key_seg(key);
+                const float              d_eff = beam_meta_d(ent.w, ld_hot(s_hot.rb));
+                float t_known = beam_key_t(key); // the key holds the exact t of `best`
+                if (active && !beam_settles(cov, key, d_eff))
+                {
+                    best    = beam_walk_rest(track, rec.ox, rec.oy, dx, dy, p.sensor_range, cov, d_eff, key);
                     t_known = 0.0f;
                     if (p.stats)
                         atomicAdd(p.stats + 2, 1ull);
@@ -661,16 +699,11 @@ __global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN
             unsigned long long key = key_none;
             if (cov)
                 key = beam_chunk_key(tv.seg, ent.x, ent.y, rec.ox, rec.oy, dx, dy, p.sensor_range, key_none, tv.n_seg);
-            const float min_t = __uint_as_float(static_cast<uint32_t>(key >> 32));
-            // d1: up to there the inline four are the only contenders (= the list's completeness distance when it
-            // has no rest).  The key holds the exact t of its segment, or the sensor range when nothing was hit.
-            const float d1      = beam_meta_dist((ent.w >> 12) & 0xfffu, ld_hot(s_hot.rb));
-            const bool  settled = cov && (min_t <= d1 - kBeamSlack);
-            const bool  queue   = has && active && !settled;
-            float       sq      = inf;
+            const bool settled = beam_settles(cov, key, beam_meta_d1(ent.w, ld_hot(s_hot.rb)));
+            const bool queue   = has && active && !settled;
+            float      sq      = inf;
             if (has && !queue)
-                sq = finish_ray<false>(p, tv.seg, rec, ray_base + q, dx, dy, static_cast<int>(0x7fffffffu - static_cast<uint32_t>(key)),
-                                min_t);
+                sq = finish_ray<false>(p, tv.seg, rec, ray_base + q, dx, dy, beam_key_seg(key), beam_key_t(key));
             const unsigned qm = __ballot_sync(0xffffffffu, queue);
             if (qm)
             { // warp-aggregated append to the CTA's queue of undecided rays

@@ -93,7 +93,7 @@ __global__ void __launch_bounds__(kGridBlock, 1) grid_step_kernel(const StepPara
         // (one shared-memory atomic per ray), so the long rays of the heavy tail do not hold 31 lanes hostage.
         // The pool is ordered ray-major with the fan's centre rays first (p.ray_order): those are the long ones.
         // =====================================================================================
-        if (p.raycast_mode == 0)
+        if (p.raycast_mode == OK_RAYCAST_GRID)
         {
             // No warp-level primitive in this loop on purpose: every lane fetches and retires on its own
             // (one shared-memory atomic per ray), so nothing depends on the lanes of a warp being converged
