@@ -241,6 +241,42 @@ int ok_lidar_query(OkEnv *env, const OkLidarQuery *q, void *stream);
 /* the same with HOST pointers (ray_deg included), staged through the env's staging buffer; synchronises `stream` */
 int ok_lidar_query_host(OkEnv *env, const OkLidarQuery *q, void *stream);
 
+/* Bird's-eye-view rasters at arbitrary poses, with no agent state read or written: the observation of the apps that read
+ * the screen (ScreenGrabber), as a semantic image with an exact definition instead of raylib's RGB frame.
+ * Regions: the four boundary polylines LI, LO, RI, RO (ok_track_copy), each closed by the edge from its last point to its
+ * first -- the segments the lidar hits.  inside(L, p) is the even-odd (PNPOLY) rule over the edges (i, j = i - 1 cyclic)
+ * of loop L: flip when (y_i > p_y) != (y_j > p_y) and p_x < ((x_j - x_i) * (p_y - y_i)) / (y_j - y_i) + x_i, in binary32,
+ * every operation rounded in that order, no contraction.  k(p) = the sum over the four loops; the pixel's class is
+ * OK_BEV_LANE for k == 2, OK_BEV_WALL for odd k (the 3 px band between an inner and an outer bound), OK_BEV_OFF for k == 0
+ * or 4 (outside the track, or the infield).  Where an offset polyline folds on itself at a tight corner (most tracks have
+ * such folds), the even-odd rule decides the class of the small pocket inside the fold; the lidar sees the same segments.
+ * Sample points: pose k = (x[k], y[k], rot[k] degrees) on track track_id[k] (NULL = track 0; out-of-range ids are clamped
+ * as in ok_track_query); pixel (r, c) of the height x width image is the point
+ *   (rs, rc) = sincosf(kDeg2Rad * rot);  f = (0.5f*(H-1) - r) * scale + ahead;  l = (c - 0.5f*(W-1)) * scale;
+ *   px = x + (f*rc - l*rs);  py = y + (f*rs + l*rc)
+ * in binary32, rounded in that order: row 0 is ahead, column 0 on the agent's left (window y points down, so the right
+ * is (-sin, cos), the ray at +90 degrees); rot = -90 gives a crop aligned with the window.  A NaN coordinate is OFF.
+ * `scale` is track px per image pixel, `ahead` shifts the image forward.  The position is pos_, without the sensor
+ * offset; raycast_mode does not matter.  Needs tracks only, not agents.  The first call after a track was added builds a
+ * device table (per track, edge lists over 2 px bands of y) synchronously; if that is still to do while `stream` is
+ * capturing, the call fails with OK_ERR_STATE: call once outside the capture, later calls can be captured.  n == 0 is a
+ * no-op. */
+#define OK_BEV_OFF 0
+#define OK_BEV_WALL 1
+#define OK_BEV_LANE 2
+typedef struct OkBevQuery {
+    const float   *x, *y, *rot;  /* f32[n]: Agent::pos_, rot_ (degrees) */
+    const int32_t *track_id;     /* i32[n] or NULL (track 0) */
+    int64_t        n;
+    int32_t        height, width; /* 1..1024 each */
+    float          scale, ahead;  /* scale finite and > 0; ahead finite */
+    uint8_t       *out;          /* u8[n][height][width], row-major */
+} OkBevQuery;
+/* device pointers; asynchronous on `stream` */
+int ok_bev_query(OkEnv *env, const OkBevQuery *q, void *stream);
+/* the same with HOST pointers, staged through the env's staging buffer; synchronises `stream` */
+int ok_bev_query_host(OkEnv *env, const OkBevQuery *q, void *stream);
+
 /* The EvolutionaryRacer policy for the whole population (SURVEY.md 8f, N2): GeneticAgent::updateAction +
  * Network::infer (EvolutionaryRacer/GeneticAgent.hpp:37-50, Network.hpp:119-155).  Agent i has its own weights
  * d_w1[i] (f32 [R+2][hidden], inputs speed/100, normalizeAngleDeg(rot)/360, hits/200) and d_w2[i] (f32 [hidden][6]);

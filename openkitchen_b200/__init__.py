@@ -4,6 +4,9 @@ Only what the hot path needs: ``csrc/`` (sm_100a kernels + the C ABI of include/
 this ctypes front-end, the drop-in C++ shim (``shim/``) and the pybind module (``pybind/``).
 """
 from ._capi import (  # noqa: F401
+    BEV_LANE,
+    BEV_OFF,
+    BEV_WALL,
     BUF,
     BUFFERS,
     LIB_PATH,

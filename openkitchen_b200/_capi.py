@@ -18,6 +18,7 @@ MOVE_VELOCITY, MOVE_ACCELERATION = 0, 1
 REWARD_NONE, REWARD_Q_PROGRESS, REWARD_CMAES_PROGRESS, REWARD_CONSTANT = 0, 1, 2, 3
 REWARD_DISPLACEMENT, REWARD_MIN_RAY, REWARD_TRACK_INDEX, REWARD_LANE_CENTER = 4, 5, 6, 7
 RAYCAST_GRID, RAYCAST_BRUTE, RAYCAST_BEAM = 0, 1, 2
+BEV_OFF, BEV_WALL, BEV_LANE = 0, 1, 2
 
 BUFFERS = [
     "pos_x", "pos_y", "rot", "speed", "accel", "act_throttle", "act_steer",
@@ -111,6 +112,16 @@ class OkLidarQuery(C.Structure):
     ]
 
 
+class OkBevQuery(C.Structure):
+    _fields_ = [
+        ("x", C.c_void_p), ("y", C.c_void_p), ("rot", C.c_void_p), ("track_id", C.c_void_p),
+        ("n", C.c_int64),
+        ("height", C.c_int32), ("width", C.c_int32),
+        ("scale", C.c_float), ("ahead", C.c_float),
+        ("out", C.c_void_p),
+    ]
+
+
 # every symbol include/openkitchen_b200.h declares: (restype, argtypes)
 _P = C.c_void_p
 SIGNATURES = {
@@ -167,6 +178,8 @@ SIGNATURES = {
     "ok_track_query_host": (C.c_int, [_P, _P, _P, _P, C.c_int64, _P, _P, _P, _P]),
     "ok_lidar_query": (C.c_int, [_P, C.POINTER(OkLidarQuery), _P]),
     "ok_lidar_query_host": (C.c_int, [_P, C.POINTER(OkLidarQuery), _P]),
+    "ok_bev_query": (C.c_int, [_P, C.POINTER(OkBevQuery), _P]),
+    "ok_bev_query_host": (C.c_int, [_P, C.POINTER(OkBevQuery), _P]),
     "ok_pcie_probe": (C.c_int, [C.c_int32, C.c_size_t, C.c_int32, C.c_int32, C.POINTER(C.c_double)]),
 }
 

@@ -13,7 +13,7 @@ import torch
 
 from . import _capi
 from .dlpack import DeviceBuffer
-from .env import LIDAR_OUTPUTS, Env, ray_fan, track_names
+from .env import LIDAR_OUTPUTS, Env, _bev_shape, ray_fan, track_names
 
 _TORCH_DTYPES = {np.float32: torch.float32, np.int32: torch.int32, np.uint8: torch.uint8}
 
@@ -124,6 +124,32 @@ class BatchEnv:
         self.env.lidar_query_device(x.data_ptr(), y.data_ptr(), rot.data_ptr(), n, None if tid is None else tid.data_ptr(),
                                     None if fan is None else fan.data_ptr(), r, self._stream(),
                                     **{LIDAR_OUTPUTS[nm][0]: t.data_ptr() for nm, t in out.items()})
+        return out
+
+    def bev(self, height: int = 64, width: int = 64, scale: float = 1.0, ahead: float = 0.0, x=None, y=None, rot=None,
+            track_id=None) -> torch.Tensor:
+        """Bird's-eye-view rasters (ok_bev_query): u8[n, height, width] of ok.BEV_OFF / BEV_WALL / BEV_LANE around each
+        pose, row 0 ahead, column 0 on the left, `scale` track px per image pixel, the image shifted `ahead` px forward.
+        The poses default to the population's own pos_x / pos_y / rot / track_id; x, y, rot: f32[n] (rot in degrees),
+        track_id: i32[n] or None (track 0 for explicit poses).  Returns a fresh tensor, computed on torch's current stream
+        with no host synchronisation."""
+        height, width, scale, ahead = _bev_shape(height, width, scale, ahead)
+        if x is None and y is None and rot is None:
+            x, y, rot = self.pos_x, self.pos_y, self.rot
+            if track_id is None:
+                track_id = self._views["track_id"]
+        elif x is None or y is None or rot is None:
+            raise ValueError("pass all of x, y and rot, or none of them")
+        n = int(torch.as_tensor(x).numel())
+        if any(torch.as_tensor(a).dim() != 1 for a in (x, y, rot)) or any(int(torch.as_tensor(a).numel()) != n for a in (y, rot)):
+            raise ValueError("x, y and rot must be 1-d tensors of one length")
+        if track_id is not None and int(torch.as_tensor(track_id).numel()) != n:
+            raise ValueError("track_id must have one entry per pose")
+        x, y, rot = (torch.as_tensor(a).to(self.device, torch.float32).contiguous() for a in (x, y, rot))
+        tid = None if track_id is None else torch.as_tensor(track_id).to(self.device, torch.int32).contiguous()
+        out = torch.empty((n, height, width), device=self.device, dtype=torch.uint8)
+        self.env.bev_query_device(x.data_ptr(), y.data_ptr(), rot.data_ptr(), n, height, width, scale, out.data_ptr(), ahead,
+                                  None if tid is None else tid.data_ptr(), self._stream())
         return out
 
     def _fan(self, rays) -> torch.Tensor:

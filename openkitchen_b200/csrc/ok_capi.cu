@@ -5,6 +5,7 @@
 #include "../../include/openkitchen_b200.h"
 
 #include "ok_beam_cache.hpp"
+#include "ok_bev.cuh"
 #include "ok_kernels.cuh"
 #include "ok_lidar_query.cuh"
 #include "ok_step.cuh"
@@ -227,6 +228,10 @@ struct OkEnv
     std::vector<ok::DeviceTable> beams_dev; // what the kernels read; shared between envs
     bool          arena_has_beams{false};
     std::vector<ok::TrackRef> h_track_refs; // host copy of d_track_refs
+    // bird's-eye-view band table (ok_bev_query): its own allocation, built on first use for the first bev_tracks tracks
+    DevPtr<uint8_t>  d_bev;
+    ok::BevTableView bev_view{};
+    size_t           bev_tracks{0};
     // agents
     int64_t              n_agents{0};
     int32_t              rays{0};
@@ -1497,6 +1502,119 @@ int ok_lidar_query_host(OkEnv *e, const OkLidarQuery *hq, void *stream)
 } // extern "C"
 namespace
 {
+// the argument checks both bird's-eye-view entry points make before touching the device
+int check_bev_query(OkEnv *e, const OkBevQuery *q)
+{
+    if (int rc = check_device(e))
+        return rc;
+    if (!q)
+        return fail(OK_ERR_INVALID_ARG, "query is NULL");
+    if (e->tracks.empty())
+        return fail(OK_ERR_STATE, "no track has been added");
+    if (q->height < 1 || q->height > 1024 || q->width < 1 || q->width > 1024)
+        return fail(OK_ERR_INVALID_ARG, "height and width must be in 1..1024");
+    if (!(std::isfinite(q->scale) && q->scale > 0.0f))
+        return fail(OK_ERR_INVALID_ARG, "scale must be finite and > 0");
+    if (!std::isfinite(q->ahead))
+        return fail(OK_ERR_INVALID_ARG, "ahead must be finite");
+    if (q->n < 0)
+        return fail(OK_ERR_INVALID_ARG, "n < 0");
+    // one launch: at most 2^31 - 1 CTAs of ok::kBevBlock threads, ok::kBevBytes output bytes each
+    if (q->n > (int64_t{2147483647} - 1) * ok::kBevBlock * ok::kBevBytes / (int64_t{q->height} * q->width))
+        return fail(OK_ERR_INVALID_ARG, "too many pixels for one launch");
+    if (q->n > 0 && (!q->x || !q->y || !q->rot))
+        return fail(OK_ERR_INVALID_ARG, "pose arrays are NULL");
+    if (q->n > 0 && !q->out)
+        return fail(OK_ERR_INVALID_ARG, "out is NULL");
+    return OK_SUCCESS;
+}
+} // namespace
+extern "C"
+{
+int ok_bev_query(OkEnv *e, const OkBevQuery *q, void *stream)
+{
+    if (int rc = check_bev_query(e, q))
+        return rc;
+    if (q->n == 0)
+        return OK_SUCCESS;
+    DeviceGuard  g(e->cfg.device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    // the band table is built (with a synchronous upload) for the tracks added so far: never inside a stream capture
+    if (e->bev_tracks != e->tracks.size())
+    {
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        const cudaError_t       err = cudaStreamIsCapturing(s, &cap);
+        if (err != cudaSuccess)
+            cudaGetLastError();
+        if (err != cudaSuccess || cap != cudaStreamCaptureStatusNone)
+            return fail(OK_ERR_STATE, "ok_bev_query: the band table is not built yet and the stream is capturing; call once outside the capture");
+        ok::BevTableHost h;
+        ok::build_bev_table(e->tracks, h);
+        e->bev_tracks = 0;
+        OK_CUDA(dev_alloc(e->d_bev, h.bytes.size()));
+        OK_CUDA(cudaMemcpy(e->d_bev.get(), h.bytes.data(), h.bytes.size(), cudaMemcpyHostToDevice));
+        const uint8_t *base = e->d_bev.get();
+        e->bev_view.tracks    = reinterpret_cast<const ok::BevTrack *>(base);
+        e->bev_view.starts    = reinterpret_cast<const uint32_t *>(base + h.off_starts);
+        e->bev_view.a         = reinterpret_cast<const float4 *>(base + h.off_a);
+        e->bev_view.b         = reinterpret_cast<const float2 *>(base + h.off_b);
+        e->bev_view.n_starts  = static_cast<uint32_t>((h.off_a - h.off_starts) / sizeof(uint32_t));
+        e->bev_view.n_entries = static_cast<uint32_t>(h.entries);
+        e->bev_tracks         = e->tracks.size();
+    }
+    ok::BevQueryParams p{};
+    p.x = q->x, p.y = q->y, p.rot = q->rot, p.track = q->track_id, p.n = q->n;
+    p.height = q->height, p.width = q->width, p.scale = q->scale, p.ahead = q->ahead, p.out = q->out;
+    p.n_tracks = static_cast<int32_t>(e->tracks.size());
+    p.table    = e->bev_view;
+    OK_CUDA(ok::launch_bev_query(p, s));
+    e->launches++;
+    return OK_SUCCESS;
+}
+
+int ok_bev_query_host(OkEnv *e, const OkBevQuery *hq, void *stream)
+{
+    if (int rc = check_bev_query(e, hq))
+        return rc;
+    if (hq->n == 0)
+        return OK_SUCCESS;
+    DeviceGuard  g(e->cfg.device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const size_t n = static_cast<size_t>(hq->n);
+    const size_t out_bytes = n * static_cast<size_t>(hq->height) * static_cast<size_t>(hq->width);
+    // x, y, rot, track_id, out: one region each of the env's staging buffer, 256-byte aligned
+    const size_t r4 = (4 * n + 255) / 256 * 256;
+    const size_t need = 4 * r4 + out_bytes;
+    if (need > e->stage_bytes)
+    {
+        e->stage_bytes = 0;
+        OK_CUDA(dev_alloc(e->d_stage, need));
+        e->stage_bytes = need;
+    }
+    uint8_t   *d  = e->d_stage.get();
+    OkBevQuery dq = *hq;
+    dq.x = reinterpret_cast<const float *>(d), dq.y = reinterpret_cast<const float *>(d + r4);
+    dq.rot      = reinterpret_cast<const float *>(d + 2 * r4);
+    dq.track_id = hq->track_id ? reinterpret_cast<const int32_t *>(d + 3 * r4) : nullptr;
+    dq.out      = d + 4 * r4;
+    OK_CUDA(cudaMemcpyAsync(d, hq->x, 4 * n, cudaMemcpyHostToDevice, s));
+    OK_CUDA(cudaMemcpyAsync(d + r4, hq->y, 4 * n, cudaMemcpyHostToDevice, s));
+    OK_CUDA(cudaMemcpyAsync(d + 2 * r4, hq->rot, 4 * n, cudaMemcpyHostToDevice, s));
+    if (hq->track_id)
+        OK_CUDA(cudaMemcpyAsync(d + 3 * r4, hq->track_id, 4 * n, cudaMemcpyHostToDevice, s));
+    if (int rc = ok_bev_query(e, &dq, stream))
+    {
+        cudaStreamSynchronize(s); // the uploads above still read the caller's arrays
+        return rc;
+    }
+    OK_CUDA(cudaMemcpyAsync(hq->out, dq.out, out_bytes, cudaMemcpyDeviceToHost, s));
+    OK_CUDA(cudaStreamSynchronize(s));
+    return OK_SUCCESS;
+}
+
+} // extern "C"
+namespace
+{
 // ok_step_host / ok_step_host_q16: `h_obs` is float[N][R], or uint16_t[N][R] when `q16`
 int step_host_impl(OkEnv *e, const float *h_thr, const float *h_steer, void *h_obs_any, const bool q16, float *h_reward, uint8_t *h_done,
                    void *stream)
@@ -1874,14 +1992,15 @@ int ok_debug_violations(OkEnv *e, uint64_t *count, int32_t *checks_compiled_in)
         return fail(OK_ERR_NO_DEVICE, "no device");
     DeviceGuard g(e->cfg.device);
     OK_CUDA(cudaDeviceSynchronize());
-    unsigned long long staged = 0, unstaged = 0, actor = 0, grid = 0, lidar = 0;
+    unsigned long long staged = 0, unstaged = 0, actor = 0, grid = 0, lidar = 0, bev = 0;
     OK_CUDA(ok::violations_step_staged(&staged));
     OK_CUDA(ok::violations_step_unstaged(&unstaged));
     OK_CUDA(ok::violations_step_actor(&actor));
     OK_CUDA(ok::violations_step_grid(&grid));
     OK_CUDA(ok::violations_lidar_query(&lidar));
+    OK_CUDA(ok::violations_bev(&bev));
     if (count)
-        *count = staged + unstaged + actor + grid + lidar;
+        *count = staged + unstaged + actor + grid + lidar + bev;
     if (checks_compiled_in)
         *checks_compiled_in = OK_CHECKED;
     return OK_SUCCESS;

@@ -32,6 +32,10 @@ __device__ __forceinline__ float fmul(float a, float b)
 {
     return __fmul_rn(a, b);
 }
+__device__ __forceinline__ float fdiv(float a, float b)
+{
+    return __fdiv_rn(a, b);
+}
 
 // cosine / sine polynomial coefficients for quadrant parity 0 (the parity-1 table is the
 // same with the cosine coefficients negated)

@@ -79,6 +79,21 @@ def _pose_arrays(x, y, rot, track_id=None):
     return x, y, rot
 
 
+def _bev_shape(height, width, scale, ahead):
+    """the image arguments of a bird's-eye-view query, checked as the library checks them; raises ValueError otherwise"""
+    height, width = int(height), int(width)
+    with np.errstate(over="ignore"):  # the library sees binary32: 1e39 is inf there
+        scale, ahead = np.float32(scale), np.float32(ahead)
+    if not (1 <= height <= 1024 and 1 <= width <= 1024):
+        raise ValueError("height and width must be in 1..1024")
+    if not (np.isfinite(scale) and scale > 0):
+        raise ValueError("scale must be finite and > 0")
+    if not np.isfinite(ahead):
+        raise ValueError("ahead must be finite")
+    scale, ahead = float(scale), float(ahead)
+    return height, width, scale, ahead
+
+
 class Env:
     """Owns one ``OkEnv``.  ``device=-1`` builds a host-only env (tracks can be built and inspected)."""
 
@@ -303,6 +318,36 @@ class Env:
         q = _capi.OkLidarQuery(x=d_x, y=d_y, rot=d_rot, track_id=d_track_id, n=n, ray_deg=d_ray_deg,
                                rays=self.rays if rays is None else rays, **d_out)
         check(self.lib.ok_lidar_query(self.h, C.byref(q), stream))
+
+    def bev_query(self, x, y, rot, height: int, width: int, scale: float, ahead: float = 0.0, track_id=None,
+                  stream=None) -> np.ndarray:
+        """Bird's-eye-view rasters at arbitrary poses (host arrays), with no agent state read or written: u8[n, height,
+        width] of BEV_OFF / BEV_WALL / BEV_LANE, row 0 ahead, column 0 on the left; `scale` track px per image pixel,
+        `ahead` px forward (ok_bev_query_host; the header states the exact definition).  Synchronises `stream`."""
+        x, y, rot = _pose_arrays(x, y, rot, track_id)
+        height, width, scale, ahead = _bev_shape(height, width, scale, ahead)
+        if self.num_tracks() == 0:
+            raise ValueError("no track has been added")
+        t = None if track_id is None else np.ascontiguousarray(track_id, dtype=np.int32)
+        out = np.empty((len(x), height, width), dtype=np.uint8)
+        q = _capi.OkBevQuery(x=_vp(x), y=_vp(y), rot=_vp(rot), track_id=_vp(t), n=len(x), height=height, width=width,
+                             scale=scale, ahead=ahead, out=_vp(out))
+        check(self.lib.ok_bev_query_host(self.h, C.byref(q), stream))
+        return out
+
+    def bev_query_device(self, d_x, d_y, d_rot, n: int, height: int, width: int, scale: float, d_out, ahead: float = 0.0,
+                         d_track_id=None, stream=None):
+        """device-pointer form of bev_query (asynchronous on `stream`): d_out is u8[n, height, width]"""
+        height, width, scale, ahead = _bev_shape(height, width, scale, ahead)
+        if n < 0:
+            raise ValueError("n < 0")
+        if n > 0 and not (d_x and d_y and d_rot and d_out):
+            raise ValueError("pose and output pointers must not be NULL")
+        if self.num_tracks() == 0:
+            raise ValueError("no track has been added")
+        q = _capi.OkBevQuery(x=d_x, y=d_y, rot=d_rot, track_id=d_track_id, n=n, height=height, width=width, scale=scale,
+                             ahead=ahead, out=d_out)
+        check(self.lib.ok_bev_query(self.h, C.byref(q), stream))
 
     def sync(self, stream=None):
         check(self.lib.ok_sync(self.h, stream))
