@@ -186,7 +186,8 @@ int32_t ok_num_rays(const OkEnv *env);
  * = the heading offset of Environment.cpp:88-101.  Device pointers, asynchronous on `stream`. */
 int ok_reset_agents(OkEnv *env, const int64_t *d_agent_idx, const int32_t *d_pt_idx, const float *d_lane_alpha,
                     const float *d_heading_off, int64_t n, void *stream);
-/* same with HOST arrays (staged through an internal buffer; synchronises `stream`) */
+/* same with HOST arrays, staged through the env's staging buffer (kept at its largest size until ok_destroy);
+ * synchronises `stream` before it returns, on error too */
 int ok_reset_agents_host(OkEnv *env, const int64_t *h_agent_idx, const int32_t *h_pt_idx, const float *h_lane_alpha,
                          const float *h_heading_off, int64_t n, void *stream);
 
@@ -210,7 +211,8 @@ int ok_fill_random_actions(OkEnv *env, uint64_t step, uint32_t seed, void *strea
  * d_track_id i32[n] or NULL (track 0); each output is nullable.  One warp per query; asynchronous on `stream`. */
 int ok_track_query(OkEnv *env, const float *d_x, const float *d_y, const int32_t *d_track_id, int64_t n,
                    int32_t *d_nearest_idx, float *d_dist_lane_center, float *d_dist_boundary, void *stream);
-/* same with HOST arrays (staged; synchronises `stream`) */
+/* same with HOST arrays, staged through the env's staging buffer (kept at its largest size until ok_destroy);
+ * synchronises `stream` before it returns, on error too */
 int ok_track_query_host(OkEnv *env, const float *h_x, const float *h_y, const int32_t *h_track_id, int64_t n,
                         int32_t *h_nearest_idx, float *h_dist_lane_center, float *h_dist_boundary, void *stream);
 
@@ -238,7 +240,8 @@ typedef struct OkLidarQuery {
 } OkLidarQuery;
 /* device pointers; asynchronous on `stream` */
 int ok_lidar_query(OkEnv *env, const OkLidarQuery *q, void *stream);
-/* the same with HOST pointers (ray_deg included), staged through the env's staging buffer; synchronises `stream` */
+/* the same with HOST pointers (ray_deg included), staged through the env's staging buffer (kept at its largest size
+ * until ok_destroy); synchronises `stream` before it returns, on error too */
 int ok_lidar_query_host(OkEnv *env, const OkLidarQuery *q, void *stream);
 
 /* Bird's-eye-view rasters at arbitrary poses, with no agent state read or written: the observation of the apps that read
@@ -274,7 +277,8 @@ typedef struct OkBevQuery {
 } OkBevQuery;
 /* device pointers; asynchronous on `stream` */
 int ok_bev_query(OkEnv *env, const OkBevQuery *q, void *stream);
-/* the same with HOST pointers, staged through the env's staging buffer; synchronises `stream` */
+/* the same with HOST pointers, staged through the env's staging buffer (kept at its largest size until ok_destroy);
+ * synchronises `stream` before it returns, on error too */
 int ok_bev_query_host(OkEnv *env, const OkBevQuery *q, void *stream);
 
 /* The EvolutionaryRacer policy for the whole population (SURVEY.md 8f, N2): GeneticAgent::updateAction +
@@ -405,7 +409,9 @@ int ok_balance_schedule(OkEnv *env, void *stream, float out[2]);
  * tiles as {track, count, first agent} to h_out[capacity][3] and returns the number of tiles. */
 int64_t ok_debug_tiles(OkEnv *env, int64_t *h_out, int64_t capacity);
 /* evaluates the kernels' sincosf (the glibc-2.39 restatement, ok_math.cuh) on `n` host floats: lets a test
- * compare the DEVICE function with libm / the oracle directly (tests/test_gpu_math.py) */
+ * compare the DEVICE function with libm / the oracle directly (tests/test_gpu_math.py).  The arrays are staged through
+ * the env's staging buffer (kept at its largest size until ok_destroy) on the legacy default stream, which the call
+ * synchronises before it returns, on error too. */
 int ok_eval_sincosf(OkEnv *env, const float *h_in, float *h_sin, float *h_cos, int64_t n);
 
 /* Host-link probe (measurement only, no env needed): moves `bytes` between a pinned host buffer and device memory

@@ -332,6 +332,112 @@ int ensure_arena(OkEnv *e)
     return OK_SUCCESS;
 }
 
+// the bird's-eye-view band table (ok_bev_query) for the tracks added so far: its own allocation, uploaded synchronously
+int ensure_bev_table(OkEnv *e)
+{
+    if (e->bev_tracks == e->tracks.size())
+        return OK_SUCCESS;
+    ok::BevTableHost h;
+    ok::build_bev_table(e->tracks, h);
+    e->bev_tracks = 0;
+    OK_CUDA(dev_alloc(e->d_bev, h.bytes.size()));
+    OK_CUDA(cudaMemcpy(e->d_bev.get(), h.bytes.data(), h.bytes.size(), cudaMemcpyHostToDevice));
+    const uint8_t *base = e->d_bev.get();
+    e->bev_view.tracks    = reinterpret_cast<const ok::BevTrack *>(base);
+    e->bev_view.starts    = reinterpret_cast<const uint32_t *>(base + h.off_starts);
+    e->bev_view.a         = reinterpret_cast<const float4 *>(base + h.off_a);
+    e->bev_view.b         = reinterpret_cast<const float2 *>(base + h.off_b);
+    e->bev_view.n_starts  = static_cast<uint32_t>((h.off_a - h.off_starts) / sizeof(uint32_t));
+    e->bev_view.n_entries = static_cast<uint32_t>(h.entries);
+    e->bev_tracks         = e->tracks.size();
+    return OK_SUCCESS;
+}
+
+// Whether work that synchronises `s` or uploads synchronously must wait for a call outside a capture: true when `s` is
+// capturing, and when its capture status cannot be read (that query's error is cleared, so no later call reports it).
+bool stream_capturing(cudaStream_t s)
+{
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    if (cudaStreamIsCapturing(s, &cap) == cudaSuccess)
+        return cap != cudaStreamCaptureStatusNone;
+    cudaGetLastError();
+    return true;
+}
+
+// The device copies of a *_host entry point's arrays, in the env's staging buffer (grown here, never shrunk or freed
+// before ok_destroy).  A region {h_in, h_out, bytes} with either host pointer set gets a 256-byte aligned slice, d; one
+// with both NULL gets d = NULL, the device call's "absent".  upload() copies every h_in in, finish() every h_out back
+// after a successful device call and synchronises.  On any other way out, the destructor synchronises `s`: no copy may
+// still read or write the caller's arrays once the call has returned.
+struct HostStage
+{
+    struct Region
+    {
+        const void *h_in;
+        void       *h_out;
+        size_t      bytes;
+        void       *d;
+    };
+    OkEnv              *e;
+    cudaStream_t        s;
+    std::vector<Region> regions;
+    bool                pending{false};
+
+    HostStage(OkEnv *env, void *stream, std::initializer_list<Region> r) : e(env), s(static_cast<cudaStream_t>(stream)), regions(r) {}
+    ~HostStage()
+    {
+        if (pending)
+        { // an error return: the caller has the first error already, and a later call must not report this one
+            cudaStreamSynchronize(s);
+            cudaGetLastError();
+        }
+    }
+
+    int upload()
+    {
+        size_t need = 0;
+        for (const Region &r : regions)
+            if (r.h_in || r.h_out)
+                need += (r.bytes + 255) / 256 * 256;
+        if (need > e->stage_bytes)
+        {
+            e->stage_bytes = 0;
+            OK_CUDA(dev_alloc(e->d_stage, need));
+            e->stage_bytes = need;
+        }
+        pending     = true;
+        uint8_t *at = e->d_stage.get();
+        for (Region &r : regions)
+        {
+            r.d = (r.h_in || r.h_out) ? at : nullptr;
+            if (r.d)
+                at += (r.bytes + 255) / 256 * 256;
+            if (r.h_in)
+                OK_CUDA(cudaMemcpyAsync(r.d, r.h_in, r.bytes, cudaMemcpyHostToDevice, s));
+        }
+        return OK_SUCCESS;
+    }
+
+    // the device pointer of region i, typed as the device call takes it
+    template <typename T> T *d(size_t i) const
+    {
+        return static_cast<T *>(regions[i].d);
+    }
+
+    // rc: what the device call returned
+    int finish(int rc)
+    {
+        if (rc)
+            return rc;
+        for (const Region &r : regions)
+            if (r.h_out)
+                OK_CUDA(cudaMemcpyAsync(r.h_out, r.d, r.bytes, cudaMemcpyDeviceToHost, s));
+        pending = false;
+        OK_CUDA(cudaStreamSynchronize(s));
+        return OK_SUCCESS;
+    }
+};
+
 ok::StepParams base_params(OkEnv *e)
 {
     ok::StepParams p{};
@@ -409,6 +515,20 @@ int check_ready(OkEnv *e)
         return rc;
     if (e->n_agents <= 0)
         return fail(OK_ERR_STATE, "ok_alloc_agents has not been called");
+    return OK_SUCCESS;
+}
+
+// the argument checks both track-query entry points make before touching the device
+int check_track_query(OkEnv *e, const float *x, const float *y, int64_t n)
+{
+    if (int rc = check_device(e))
+        return rc;
+    if (e->tracks.empty())
+        return fail(OK_ERR_STATE, "no track has been added");
+    if (n > 0 && (!x || !y))
+        return fail(OK_ERR_INVALID_ARG, "query coordinates are NULL");
+    if (n > (int64_t{1} << 31) / 32 * 255)
+        return fail(OK_ERR_INVALID_ARG, "too many queries for one launch");
     return OK_SUCCESS;
 }
 
@@ -519,13 +639,9 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
         if (!e2e && ag.sizing.auto_balance && ag.feedback.d_tile_ns)
         { // feedback tiling: re-cut the tiles from the measured tile times, a few times early on, then now and then
             const uint64_t k = ag.feedback.launches++;
-            if (k == 16 || k == 64 || k == 256 || (k & 4095) == 4095)
-            {
-                cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-                if (cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap == cudaStreamCaptureStatusNone)
-                    if (int rc2 = rebalance_beam_tiles(e, s))
-                        return rc2;
-            }
+            if ((k == 16 || k == 64 || k == 256 || (k & 4095) == 4095) && !stream_capturing(s))
+                if (int rc2 = rebalance_beam_tiles(e, s))
+                    return rc2;
         }
         p.tiles        = ag.beam.d.get();
         p.n_tiles      = ag.beam.n;
@@ -535,13 +651,9 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
         p.first        = nullptr;
         if (!e2e && !ag.feedback.tiles.empty())
         { // the CTAs' first tiles with their track records side by side (rebuilt when the tiling or the arena changed)
-            if (ag.first_dirty)
-            {
-                cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-                if (cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap == cudaStreamCaptureStatusNone)
-                    if (int rc2 = upload_first_tiles(e, s))
-                        return rc2;
-            }
+            if (ag.first_dirty && !stream_capturing(s))
+                if (int rc2 = upload_first_tiles(e, s))
+                    return rc2;
             if (!ag.first_dirty)
                 p.first = ag.first_beam.get();
         }
@@ -1058,31 +1170,13 @@ int ok_reset_agents_host(OkEnv *e, const int64_t *h_agent_idx, const int32_t *h_
     if (!h_pt_idx)
         return fail(OK_ERR_INVALID_ARG, "pt_idx is NULL");
     DeviceGuard  g(e->cfg.device);
-    cudaStream_t s    = static_cast<cudaStream_t>(stream);
-    const size_t need = static_cast<size_t>(n) * (8 + 4 + 4 + 4) + 64;
-    if (need > e->stage_bytes)
-    {
-        e->stage_bytes = 0;
-        OK_CUDA(dev_alloc(e->d_stage, need));
-        e->stage_bytes = need;
-    }
-    int64_t *d_ai = reinterpret_cast<int64_t *>(e->d_stage.get());
-    int32_t *d_pt = reinterpret_cast<int32_t *>(e->d_stage.get() + 8 * static_cast<size_t>(n));
-    float   *d_la = reinterpret_cast<float *>(e->d_stage.get() + 12 * static_cast<size_t>(n));
-    float   *d_ho = reinterpret_cast<float *>(e->d_stage.get() + 16 * static_cast<size_t>(n));
-    if (h_agent_idx)
-        OK_CUDA(cudaMemcpyAsync(d_ai, h_agent_idx, 8 * static_cast<size_t>(n), cudaMemcpyHostToDevice, s));
-    OK_CUDA(cudaMemcpyAsync(d_pt, h_pt_idx, 4 * static_cast<size_t>(n), cudaMemcpyHostToDevice, s));
-    if (h_lane_alpha)
-        OK_CUDA(cudaMemcpyAsync(d_la, h_lane_alpha, 4 * static_cast<size_t>(n), cudaMemcpyHostToDevice, s));
-    if (h_heading_off)
-        OK_CUDA(cudaMemcpyAsync(d_ho, h_heading_off, 4 * static_cast<size_t>(n), cudaMemcpyHostToDevice, s));
-    rc = ok_reset_agents(e, h_agent_idx ? d_ai : nullptr, d_pt, h_lane_alpha ? d_la : nullptr,
-                         h_heading_off ? d_ho : nullptr, n, stream);
-    if (rc)
+    const size_t k = static_cast<size_t>(n);
+    HostStage    st(e, stream, {{h_agent_idx, nullptr, 8 * k}, {h_pt_idx, nullptr, 4 * k}, {h_lane_alpha, nullptr, 4 * k},
+                                {h_heading_off, nullptr, 4 * k}});
+    if ((rc = st.upload()))
         return rc;
-    OK_CUDA(cudaStreamSynchronize(s));
-    return OK_SUCCESS;
+    return st.finish(ok_reset_agents(e, st.d<const int64_t>(0), st.d<const int32_t>(1), st.d<const float>(2),
+                                     st.d<const float>(3), n, stream));
 }
 
 int ok_cast_rays(OkEnv *e, void *stream)
@@ -1301,16 +1395,10 @@ int ok_discounted_returns(OkEnv *e, const float *d_rewards, const uint8_t *d_don
 int ok_track_query(OkEnv *e, const float *d_x, const float *d_y, const int32_t *d_track, int64_t n, int32_t *d_idx,
                    float *d_lane, float *d_bound, void *stream)
 {
-    if (int rc = check_device(e))
+    if (int rc = check_track_query(e, d_x, d_y, n))
         return rc;
-    if (e->tracks.empty())
-        return fail(OK_ERR_STATE, "no track has been added");
     if (n <= 0)
         return OK_SUCCESS;
-    if (!d_x || !d_y)
-        return fail(OK_ERR_INVALID_ARG, "query coordinates are NULL");
-    if (n > (int64_t{1} << 31) / 32 * 255)
-        return fail(OK_ERR_INVALID_ARG, "too many queries for one launch");
     DeviceGuard g(e->cfg.device);
     int         rc = ensure_arena(e);
     if (rc)
@@ -1330,43 +1418,18 @@ int ok_track_query(OkEnv *e, const float *d_x, const float *d_y, const int32_t *
 int ok_track_query_host(OkEnv *e, const float *h_x, const float *h_y, const int32_t *h_track, int64_t n, int32_t *h_idx,
                         float *h_lane, float *h_bound, void *stream)
 {
-    if (int rc = check_device(e))
+    if (int rc = check_track_query(e, h_x, h_y, n))
         return rc;
     if (n <= 0)
         return OK_SUCCESS;
-    if (!h_x || !h_y)
-        return fail(OK_ERR_INVALID_ARG, "query coordinates are NULL");
     DeviceGuard  g(e->cfg.device);
-    cudaStream_t s     = static_cast<cudaStream_t>(stream);
     const size_t bytes = 4 * static_cast<size_t>(n);
-    uint8_t     *d     = nullptr;
-    OK_CUDA(cudaMalloc(&d, 6 * bytes));
-    float   *d_x = reinterpret_cast<float *>(d), *d_y = reinterpret_cast<float *>(d + bytes);
-    int32_t *d_t = reinterpret_cast<int32_t *>(d + 2 * bytes), *d_i = reinterpret_cast<int32_t *>(d + 3 * bytes);
-    float   *d_l = reinterpret_cast<float *>(d + 4 * bytes), *d_b = reinterpret_cast<float *>(d + 5 * bytes);
-    cudaError_t err = cudaMemcpyAsync(d_x, h_x, bytes, cudaMemcpyHostToDevice, s);
-    if (err == cudaSuccess)
-        err = cudaMemcpyAsync(d_y, h_y, bytes, cudaMemcpyHostToDevice, s);
-    if (err == cudaSuccess && h_track)
-        err = cudaMemcpyAsync(d_t, h_track, bytes, cudaMemcpyHostToDevice, s);
-    int rc = OK_SUCCESS;
-    if (err == cudaSuccess)
-        rc = ok_track_query(e, d_x, d_y, h_track ? d_t : nullptr, n, h_idx ? d_i : nullptr, h_lane ? d_l : nullptr,
-                            h_bound ? d_b : nullptr, stream);
-    if (err == cudaSuccess && rc == OK_SUCCESS && h_idx)
-        err = cudaMemcpyAsync(h_idx, d_i, bytes, cudaMemcpyDeviceToHost, s);
-    if (err == cudaSuccess && rc == OK_SUCCESS && h_lane)
-        err = cudaMemcpyAsync(h_lane, d_l, bytes, cudaMemcpyDeviceToHost, s);
-    if (err == cudaSuccess && rc == OK_SUCCESS && h_bound)
-        err = cudaMemcpyAsync(h_bound, d_b, bytes, cudaMemcpyDeviceToHost, s);
-    if (err == cudaSuccess)
-        err = cudaStreamSynchronize(s);
-    cudaFree(d);
-    if (rc)
+    HostStage    st(e, stream, {{h_x, nullptr, bytes}, {h_y, nullptr, bytes}, {h_track, nullptr, bytes}, {nullptr, h_idx, bytes},
+                                {nullptr, h_lane, bytes}, {nullptr, h_bound, bytes}});
+    if (int rc = st.upload())
         return rc;
-    if (err != cudaSuccess)
-        return fail(OK_ERR_CUDA, std::string("ok_track_query_host: ") + cudaGetErrorString(err));
-    return OK_SUCCESS;
+    return st.finish(ok_track_query(e, st.d<const float>(0), st.d<const float>(1), st.d<const int32_t>(2), n, st.d<int32_t>(3),
+                                    st.d<float>(4), st.d<float>(5), stream));
 }
 
 } // extern "C"
@@ -1409,17 +1472,10 @@ int ok_lidar_query(OkEnv *e, const OkLidarQuery *q, void *stream)
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     // the arena (and in beam mode the device tables) may still have to be built, with synchronous copies: never inside a
     // stream capture
-    if (e->arena_dirty || (e->cfg.raycast_mode == OK_RAYCAST_BEAM && !e->arena_has_beams))
-    {
-        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-        const cudaError_t       err = cudaStreamIsCapturing(s, &cap);
-        if (err != cudaSuccess)
-            cudaGetLastError();
-        if (err != cudaSuccess || cap != cudaStreamCaptureStatusNone)
-            return fail(OK_ERR_STATE, "ok_lidar_query: the track arena is not built yet and the stream is capturing; call once outside the capture");
-        if (int rc = ensure_arena(e))
-            return rc;
-    }
+    if ((e->arena_dirty || (e->cfg.raycast_mode == OK_RAYCAST_BEAM && !e->arena_has_beams)) && stream_capturing(s))
+        return fail(OK_ERR_STATE, "ok_lidar_query: the track arena is not built yet and the stream is capturing; call once outside the capture");
+    if (int rc = ensure_arena(e))
+        return rc;
     ok::LidarQueryParams p{};
     p.x = q->x, p.y = q->y, p.rot = q->rot, p.track = q->track_id, p.n = q->n;
     p.ray_deg  = q->ray_deg ? q->ray_deg : e->ag.ray_deg.get();
@@ -1445,58 +1501,20 @@ int ok_lidar_query_host(OkEnv *e, const OkLidarQuery *hq, void *stream)
     if (hq->n == 0)
         return OK_SUCCESS;
     DeviceGuard  g(e->cfg.device);
-    cudaStream_t s  = static_cast<cudaStream_t>(stream);
-    const size_t n  = static_cast<size_t>(hq->n), nr = n * static_cast<size_t>(hq->rays);
-    // one region of the env's staging buffer per array the call moves, 256-byte aligned
-    struct Region
-    {
-        const void *h_in;
-        void       *h_out;
-        size_t      bytes, off;
-    };
-    Region regions[] = {
-        {hq->x, nullptr, 4 * n, 0},           {hq->y, nullptr, 4 * n, 0},         {hq->rot, nullptr, 4 * n, 0},
-        {hq->track_id, nullptr, 4 * n, 0},    {hq->ray_deg, nullptr, 4 * static_cast<size_t>(hq->rays), 0},
-        {nullptr, hq->hit_abs, 8 * nr, 0},    {nullptr, hq->hit_rel, 8 * nr, 0},  {nullptr, hq->obs, 4 * nr, 0},
-        {nullptr, hq->hit_t, 4 * nr, 0},      {nullptr, hq->hit_seg, 4 * nr, 0},  {nullptr, hq->min_dist2, 4 * n, 0},
-        {nullptr, hq->crashed, n, 0},
-    };
-    size_t need = 0;
-    for (Region &r : regions)
-        if (r.h_in || r.h_out)
-        {
-            r.off = need;
-            need += (r.bytes + 255) / 256 * 256;
-        }
-    if (need > e->stage_bytes)
-    {
-        e->stage_bytes = 0;
-        OK_CUDA(dev_alloc(e->d_stage, need));
-        e->stage_bytes = need;
-    }
-    void *d[sizeof regions / sizeof regions[0]];
-    for (size_t i = 0; i < sizeof regions / sizeof regions[0]; ++i)
-    {
-        d[i] = (regions[i].h_in || regions[i].h_out) ? e->d_stage.get() + regions[i].off : nullptr;
-        if (regions[i].h_in)
-            OK_CUDA(cudaMemcpyAsync(d[i], regions[i].h_in, regions[i].bytes, cudaMemcpyHostToDevice, s));
-    }
-    OkLidarQuery dq = *hq;
-    dq.x = static_cast<const float *>(d[0]), dq.y = static_cast<const float *>(d[1]), dq.rot = static_cast<const float *>(d[2]);
-    dq.track_id = static_cast<const int32_t *>(d[3]), dq.ray_deg = static_cast<const float *>(d[4]);
-    dq.hit_abs = static_cast<float *>(d[5]), dq.hit_rel = static_cast<float *>(d[6]), dq.obs = static_cast<float *>(d[7]);
-    dq.hit_t = static_cast<float *>(d[8]), dq.hit_seg = static_cast<int32_t *>(d[9]), dq.min_dist2 = static_cast<float *>(d[10]);
-    dq.crashed = static_cast<uint8_t *>(d[11]);
-    if (int rc = ok_lidar_query(e, &dq, stream))
-    {
-        cudaStreamSynchronize(s); // the uploads above still read the caller's arrays
+    const size_t n = static_cast<size_t>(hq->n), nr = n * static_cast<size_t>(hq->rays);
+    HostStage    st(e, stream,
+                    {{hq->x, nullptr, 4 * n}, {hq->y, nullptr, 4 * n}, {hq->rot, nullptr, 4 * n}, {hq->track_id, nullptr, 4 * n},
+                     {hq->ray_deg, nullptr, 4 * static_cast<size_t>(hq->rays)}, {nullptr, hq->hit_abs, 8 * nr},
+                     {nullptr, hq->hit_rel, 8 * nr}, {nullptr, hq->obs, 4 * nr}, {nullptr, hq->hit_t, 4 * nr},
+                     {nullptr, hq->hit_seg, 4 * nr}, {nullptr, hq->min_dist2, 4 * n}, {nullptr, hq->crashed, n}});
+    if (int rc = st.upload())
         return rc;
-    }
-    for (size_t i = 0; i < sizeof regions / sizeof regions[0]; ++i)
-        if (regions[i].h_out)
-            OK_CUDA(cudaMemcpyAsync(regions[i].h_out, d[i], regions[i].bytes, cudaMemcpyDeviceToHost, s));
-    OK_CUDA(cudaStreamSynchronize(s));
-    return OK_SUCCESS;
+    OkLidarQuery dq = *hq;
+    dq.x = st.d<const float>(0), dq.y = st.d<const float>(1), dq.rot = st.d<const float>(2);
+    dq.track_id = st.d<const int32_t>(3), dq.ray_deg = st.d<const float>(4);
+    dq.hit_abs = st.d<float>(5), dq.hit_rel = st.d<float>(6), dq.obs = st.d<float>(7), dq.hit_t = st.d<float>(8);
+    dq.hit_seg = st.d<int32_t>(9), dq.min_dist2 = st.d<float>(10), dq.crashed = st.d<uint8_t>(11);
+    return st.finish(ok_lidar_query(e, &dq, stream));
 }
 
 } // extern "C"
@@ -1540,28 +1558,10 @@ int ok_bev_query(OkEnv *e, const OkBevQuery *q, void *stream)
     DeviceGuard  g(e->cfg.device);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     // the band table is built (with a synchronous upload) for the tracks added so far: never inside a stream capture
-    if (e->bev_tracks != e->tracks.size())
-    {
-        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-        const cudaError_t       err = cudaStreamIsCapturing(s, &cap);
-        if (err != cudaSuccess)
-            cudaGetLastError();
-        if (err != cudaSuccess || cap != cudaStreamCaptureStatusNone)
-            return fail(OK_ERR_STATE, "ok_bev_query: the band table is not built yet and the stream is capturing; call once outside the capture");
-        ok::BevTableHost h;
-        ok::build_bev_table(e->tracks, h);
-        e->bev_tracks = 0;
-        OK_CUDA(dev_alloc(e->d_bev, h.bytes.size()));
-        OK_CUDA(cudaMemcpy(e->d_bev.get(), h.bytes.data(), h.bytes.size(), cudaMemcpyHostToDevice));
-        const uint8_t *base = e->d_bev.get();
-        e->bev_view.tracks    = reinterpret_cast<const ok::BevTrack *>(base);
-        e->bev_view.starts    = reinterpret_cast<const uint32_t *>(base + h.off_starts);
-        e->bev_view.a         = reinterpret_cast<const float4 *>(base + h.off_a);
-        e->bev_view.b         = reinterpret_cast<const float2 *>(base + h.off_b);
-        e->bev_view.n_starts  = static_cast<uint32_t>((h.off_a - h.off_starts) / sizeof(uint32_t));
-        e->bev_view.n_entries = static_cast<uint32_t>(h.entries);
-        e->bev_tracks         = e->tracks.size();
-    }
+    if (e->bev_tracks != e->tracks.size() && stream_capturing(s))
+        return fail(OK_ERR_STATE, "ok_bev_query: the band table is not built yet and the stream is capturing; call once outside the capture");
+    if (int rc = ensure_bev_table(e))
+        return rc;
     ok::BevQueryParams p{};
     p.x = q->x, p.y = q->y, p.rot = q->rot, p.track = q->track_id, p.n = q->n;
     p.height = q->height, p.width = q->width, p.scale = q->scale, p.ahead = q->ahead, p.out = q->out;
@@ -1579,37 +1579,15 @@ int ok_bev_query_host(OkEnv *e, const OkBevQuery *hq, void *stream)
     if (hq->n == 0)
         return OK_SUCCESS;
     DeviceGuard  g(e->cfg.device);
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
     const size_t n = static_cast<size_t>(hq->n);
-    const size_t out_bytes = n * static_cast<size_t>(hq->height) * static_cast<size_t>(hq->width);
-    // x, y, rot, track_id, out: one region each of the env's staging buffer, 256-byte aligned
-    const size_t r4 = (4 * n + 255) / 256 * 256;
-    const size_t need = 4 * r4 + out_bytes;
-    if (need > e->stage_bytes)
-    {
-        e->stage_bytes = 0;
-        OK_CUDA(dev_alloc(e->d_stage, need));
-        e->stage_bytes = need;
-    }
-    uint8_t   *d  = e->d_stage.get();
-    OkBevQuery dq = *hq;
-    dq.x = reinterpret_cast<const float *>(d), dq.y = reinterpret_cast<const float *>(d + r4);
-    dq.rot      = reinterpret_cast<const float *>(d + 2 * r4);
-    dq.track_id = hq->track_id ? reinterpret_cast<const int32_t *>(d + 3 * r4) : nullptr;
-    dq.out      = d + 4 * r4;
-    OK_CUDA(cudaMemcpyAsync(d, hq->x, 4 * n, cudaMemcpyHostToDevice, s));
-    OK_CUDA(cudaMemcpyAsync(d + r4, hq->y, 4 * n, cudaMemcpyHostToDevice, s));
-    OK_CUDA(cudaMemcpyAsync(d + 2 * r4, hq->rot, 4 * n, cudaMemcpyHostToDevice, s));
-    if (hq->track_id)
-        OK_CUDA(cudaMemcpyAsync(d + 3 * r4, hq->track_id, 4 * n, cudaMemcpyHostToDevice, s));
-    if (int rc = ok_bev_query(e, &dq, stream))
-    {
-        cudaStreamSynchronize(s); // the uploads above still read the caller's arrays
+    HostStage    st(e, stream, {{hq->x, nullptr, 4 * n}, {hq->y, nullptr, 4 * n}, {hq->rot, nullptr, 4 * n}, {hq->track_id, nullptr, 4 * n},
+                                {nullptr, hq->out, n * static_cast<size_t>(hq->height) * static_cast<size_t>(hq->width)}});
+    if (int rc = st.upload())
         return rc;
-    }
-    OK_CUDA(cudaMemcpyAsync(hq->out, dq.out, out_bytes, cudaMemcpyDeviceToHost, s));
-    OK_CUDA(cudaStreamSynchronize(s));
-    return OK_SUCCESS;
+    OkBevQuery dq = *hq;
+    dq.x = st.d<const float>(0), dq.y = st.d<const float>(1), dq.rot = st.d<const float>(2);
+    dq.track_id = st.d<const int32_t>(3), dq.out = st.d<uint8_t>(4);
+    return st.finish(ok_bev_query(e, &dq, stream));
 }
 
 } // extern "C"
@@ -1829,22 +1807,15 @@ int ok_eval_sincosf(OkEnv *e, const float *h_in, float *h_sin, float *h_cos, int
         return fail(OK_ERR_NO_DEVICE, "no device");
     if (!h_in || !h_sin || !h_cos || n <= 0)
         return fail(OK_ERR_INVALID_ARG, "bad arguments");
-    DeviceGuard g(e->cfg.device);
-    float      *d = nullptr;
-    OK_CUDA(cudaMalloc(&d, sizeof(float) * 3 * static_cast<size_t>(n)));
-    cudaError_t err = cudaMemcpy(d, h_in, sizeof(float) * n, cudaMemcpyHostToDevice);
-    if (err == cudaSuccess)
-    {
-        ok::sincosf_kernel<<<static_cast<unsigned>((n + 255) / 256), 256>>>(d, d + n, d + 2 * n, n);
-        e->launches++;
-        err = cudaMemcpy(h_sin, d + n, sizeof(float) * n, cudaMemcpyDeviceToHost);
-        if (err == cudaSuccess)
-            err = cudaMemcpy(h_cos, d + 2 * n, sizeof(float) * n, cudaMemcpyDeviceToHost);
-    }
-    cudaFree(d);
-    if (err != cudaSuccess)
-        return fail(OK_ERR_CUDA, cudaGetErrorString(err));
-    return OK_SUCCESS;
+    DeviceGuard  g(e->cfg.device);
+    const size_t bytes = sizeof(float) * static_cast<size_t>(n);
+    HostStage    st(e, nullptr, {{h_in, nullptr, bytes}, {nullptr, h_sin, bytes}, {nullptr, h_cos, bytes}});
+    if (int rc = st.upload())
+        return rc;
+    ok::sincosf_kernel<<<static_cast<unsigned>((n + 255) / 256), 256>>>(st.d<const float>(0), st.d<float>(1), st.d<float>(2), n);
+    OK_CUDA(cudaGetLastError());
+    e->launches++;
+    return st.finish(OK_SUCCESS);
 }
 
 static int host_beam(OkEnv *e, int32_t id)

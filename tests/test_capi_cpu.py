@@ -29,6 +29,26 @@ def test_library_exports_every_declared_symbol():
     assert _capi.load().ok_abi_version() == 2
 
 
+def test_capi_allocates_device_memory_in_one_place():
+    """Pool, don't free (DESIGN.md §7): in ok_capi.cu, cudaMalloc and cudaFree are called only by dev_alloc and CudaFree,
+    the owners every buffer goes through, and by the measurement-only ok_pcie_probe.  The *_host entry points stage
+    through the env's pooled buffer.  One predicate answers "is this stream capturing?"."""
+    src = open(os.path.join(ROOT, "openkitchen_b200", "csrc", "ok_capi.cu")).read()
+    src = re.sub(r"//[^\n]*", "", src)
+    callers = {"cudaMalloc": set(), "cudaFree": set()}
+    owner = None
+    for line in src.splitlines():
+        # a definition at column 0 names the function or struct the lines below belong to
+        m = re.match(r"(?:template\s*<[^>]*>\s*)?(?:struct\s+(\w+)|[A-Za-z_][^(;=]*?\b(\w+)\s*\()", line)
+        if m and not line.startswith(("extern", "namespace")):
+            owner = m.group(1) or m.group(2)
+        for fn in callers:
+            if re.search(rf"\b{fn}\s*\(", line):
+                callers[fn].add(owner)
+    assert callers == {"cudaMalloc": {"dev_alloc", "ok_pcie_probe"}, "cudaFree": {"CudaFree", "ok_pcie_probe"}}, callers
+    assert len(re.findall(r"\bcudaStreamIsCapturing\s*\(", src)) == 1
+
+
 def test_config_defaults_are_the_reference_constants():
     c = _capi.OkConfig()
     _capi.load().ok_config_default(C.byref(c))
