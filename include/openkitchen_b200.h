@@ -118,7 +118,8 @@ typedef struct OkConfig {
     int32_t  raycast_mode;         /* OkRaycastMode */
     int32_t  auto_reset;           /* !=0: a crashed agent is reset at the start of the next step
                                       (GuidedCostLearning/test.cpp:102-111) to centre-line index
-                                      (last_reset + auto_reset_stride) mod P, with a zero action */
+                                      (last_reset + auto_reset_stride) mod P, with a zero action; with reset
+                                      draws on (ok_set_reset_draws) it is a drawn reset instead */
     int32_t  auto_reset_stride;    /* 97 */
     float    sensor_range;         /* Agent::kSensorRange 200        Agent.h:10 */
     float    speed_limit;          /* Agent::kSpeedLimit 100         Agent.h:11 */
@@ -190,6 +191,46 @@ int ok_reset_agents(OkEnv *env, const int64_t *d_agent_idx, const int32_t *d_pt_
  * synchronises `stream` before it returns, on error too */
 int ok_reset_agents_host(OkEnv *env, const int64_t *h_agent_idx, const int32_t *h_pt_idx, const float *h_lane_alpha,
                          const float *h_heading_off, int64_t n, void *stream);
+
+/* Reset draws: Environment::resetAgent's random point, lane and heading (Environment.cpp:76-122) from a counter-based
+ * stream keyed by device state, so that they run inside the step kernel (auto-reset), inside a CUDA graph, and come out the
+ * same whatever the tiling, the kernel shape or the sharding.
+ *
+ * Every agent a has a device counter k[a] (u32, zero after ok_alloc_agents; ok_reset_draw_counts).  A DRAWN reset of a:
+ *   1. o[0..3] = Philox4x32-10(counter = (lo32(id), hi32(id), k[a], 0), key = (seed, 0x525354 "RST")), id = agent_id_base + a
+ *      (the key's second word keeps this stream apart from the action stream, 0, and the PPO stream, 0x50504f);
+ *   2. U(o, m) = (uint32_t)(((uint64_t)o * m) >> 32): U{0..m-1}, each value's probability off by at most m / 2^32;
+ *   3. centre-line index pt = U(o[0], P) with OK_RESET_DRAW_POINT; otherwise an auto-reset keeps the stride rule of
+ *      OkConfig::auto_reset and an explicit reset uses RaceTrack::kStartingIdx (3, clamped to P - 1);
+ *   4. with OK_RESET_DRAW_LANE the lane lerp alpha = (float)(10 + U(o[1], 81)) / 100.0f, correctly rounded
+ *      (Environment.cpp:107-114); without it the agent starts on the centre line;
+ *   5. with OK_RESET_DRAW_HEADING the heading offset off = s * (float)(45 + U(o[2], 46)), s = -1 for even k[a] and +1 for
+ *      odd (the reference's alternating sign, Environment.cpp:88-101, per agent); without it off = 0;
+ *   6. the agent is reset exactly as ok_reset_agents resets it with (pt, alpha, off), and k[a] += 1.
+ * Resets that are not drawn (ok_reset_agents, the stride auto-reset with draws off) never touch k.  Draws are off by default. */
+#define OK_RESET_DRAW_POINT   1
+#define OK_RESET_DRAW_LANE    2
+#define OK_RESET_DRAW_HEADING 4
+typedef struct OkResetDraws {
+    uint32_t seed;
+    int32_t  flags; /* OK_RESET_DRAW_*; 0 = off */
+} OkResetDraws;
+/* d NULL = off; unknown flag bits: OK_ERR_INVALID_ARG.  With OkConfig::auto_reset != 0 and flags != 0, the auto-reset at the
+ * start of a tick is a drawn reset (its tick still runs with a zero action) in every step entry point.  The settings are
+ * read when a launch is enqueued: a CUDA graph keeps the settings it was captured with, and its replays continue the
+ * stream, because the counters live on the device. */
+int ok_set_reset_draws(OkEnv *env, const OkResetDraws *d);
+int ok_get_reset_draws(const OkEnv *env, OkResetDraws *out);
+/* a drawn reset of: the n agents d_agent_idx[0..n) (distinct indices) | every agent with d_mask[a] != 0 (u8[N], e.g. the
+ * OK_BUF_DONE buffer) | every agent (both NULL).  With a mask or for all agents n must be ok_num_agents; passing both is
+ * OK_ERR_INVALID_ARG.  With draws off the agents go to kStartingIdx and their counters still advance.  Device pointers;
+ * asynchronous on `stream`, no host synchronisation: it can be captured into a CUDA graph. */
+int ok_reset_agents_drawn(OkEnv *env, const int64_t *d_agent_idx, const uint8_t *d_mask, int64_t n, void *stream);
+/* same with HOST arrays, staged through the env's staging buffer; synchronises `stream` before it returns, on error too */
+int ok_reset_agents_drawn_host(OkEnv *env, const int64_t *h_agent_idx, const uint8_t *h_mask, int64_t n, void *stream);
+/* the device counters k: u32[ok_num_agents], owned by the env like the agent buffers; writable (to restart or move a
+ * stream) */
+int ok_reset_draw_counts(OkEnv *env, uint32_t **d_counts);
 
 /* ---- the tick ------------------------------------------------------------------------------ */
 /* CollisionChecker::checkCollision (CollisionChecker.cu:96-100,113-174): lidar + crash flag on the

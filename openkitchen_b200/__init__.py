@@ -23,6 +23,9 @@ from ._capi import (  # noqa: F401
     REWARD_NONE,
     REWARD_Q_PROGRESS,
     REWARD_TRACK_INDEX,
+    RESET_DRAW_HEADING,
+    RESET_DRAW_LANE,
+    RESET_DRAW_POINT,
     OkError,
 )
 from . import dlpack  # noqa: F401

@@ -19,6 +19,7 @@ REWARD_NONE, REWARD_Q_PROGRESS, REWARD_CMAES_PROGRESS, REWARD_CONSTANT = 0, 1, 2
 REWARD_DISPLACEMENT, REWARD_MIN_RAY, REWARD_TRACK_INDEX, REWARD_LANE_CENTER = 4, 5, 6, 7
 RAYCAST_GRID, RAYCAST_BRUTE, RAYCAST_BEAM = 0, 1, 2
 BEV_OFF, BEV_WALL, BEV_LANE = 0, 1, 2
+RESET_DRAW_POINT, RESET_DRAW_LANE, RESET_DRAW_HEADING = 1, 2, 4
 
 BUFFERS = [
     "pos_x", "pos_y", "rot", "speed", "accel", "act_throttle", "act_steer",
@@ -55,6 +56,10 @@ class OkConfig(C.Structure):
         ("beam_bins", C.c_int32),
         ("agent_id_base", C.c_uint64),
     ]
+
+
+class OkResetDraws(C.Structure):
+    _fields_ = [("seed", C.c_uint32), ("flags", C.c_int32)]
 
 
 class OkTrackInfo(C.Structure):
@@ -142,6 +147,11 @@ SIGNATURES = {
     "ok_num_rays": (C.c_int32, [_P]),
     "ok_reset_agents": (C.c_int, [_P, _P, _P, _P, _P, C.c_int64, _P]),
     "ok_reset_agents_host": (C.c_int, [_P, _P, _P, _P, _P, C.c_int64, _P]),
+    "ok_set_reset_draws": (C.c_int, [_P, C.POINTER(OkResetDraws)]),
+    "ok_get_reset_draws": (C.c_int, [_P, C.POINTER(OkResetDraws)]),
+    "ok_reset_agents_drawn": (C.c_int, [_P, _P, _P, C.c_int64, _P]),
+    "ok_reset_agents_drawn_host": (C.c_int, [_P, _P, _P, C.c_int64, _P]),
+    "ok_reset_draw_counts": (C.c_int, [_P, C.POINTER(_P)]),
     "ok_cast_rays": (C.c_int, [_P, _P]),
     "ok_launch_step": (C.c_int, [_P, _P, _P, _P]),
     "ok_launch_steps_random": (C.c_int, [_P, C.c_uint64, C.c_int32, C.c_uint32, _P]),

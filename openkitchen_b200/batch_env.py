@@ -58,6 +58,8 @@ class BatchEnv:
         self.nearest_idx = v["nearest_idx"]
         self.pos_x, self.pos_y, self.rot, self.speed = v["pos_x"], v["pos_y"], v["rot"], v["speed"]
         self.act_throttle, self.act_steer = v["act_throttle"], v["act_steer"]
+        # u32[N]: the reset-draw counters k (set_reset_draws); not an OkBuffer, so not in ok.BUFFERS / self[name]
+        self.reset_draw_count = torch.from_dlpack(DeviceBuffer(self.env, "reset_draw_count", self.env.reset_draw_counts_info()))
         self._step_count = 0
 
     # ---- views -----------------------------------------------------------------------------
@@ -208,10 +210,44 @@ class BatchEnv:
             ho = mag * sign
         self.reset(idx, pt, la, ho)
 
+    def set_reset_draws(self, seed: int, point: bool = True, lane: bool = False, heading: bool = False):
+        """Reset draws (include/openkitchen_b200.h, OkResetDraws): Environment::resetAgent's random centre-line point, lane
+        lerp and heading offset from a counter-based stream keyed by (seed, agent id, reset_draw_count[agent]).  With
+        auto_reset the tick's own reset of crashed agents draws, inside the step kernel, so a captured rollout starts its
+        episodes where the reference's apps would; reset_drawn draws too.  All three False turns the draws off."""
+        self.env.set_reset_draws(seed, point, lane, heading)
+
+    def reset_draws(self) -> dict:
+        return self.env.reset_draws()
+
+    def reset_drawn(self, agents=None):
+        """Drawn reset (ok_reset_agents_drawn) of agents: None (all), a bool / uint8 CUDA mask with one entry per agent (e.g.
+        ``env.done``, passed as it is: no nonzero, no host synchronisation), or an index tensor.  Runs on torch's current
+        stream; it can be captured into a CUDA graph."""
+        if agents is None:
+            self.env.reset_drawn_device(None, None, self.n_agents, self._stream())
+            return
+        agents = torch.as_tensor(agents, device=self.device)
+        if agents.dtype in (torch.bool, torch.uint8):
+            if agents.numel() != self.n_agents:
+                raise ValueError(f"the mask must have one entry per agent ({self.n_agents}), got {agents.numel()}")
+            mask = agents.contiguous()
+            if mask.dtype == torch.bool:
+                mask = mask.view(torch.uint8)  # same bytes: 0 / 1
+            self.env.reset_drawn_device(None, mask.data_ptr(), self.n_agents, self._stream())
+            self._keep_drawn = mask
+            return
+        idx = agents.to(torch.int64).contiguous().reshape(-1)
+        if idx.numel() == 0:
+            return
+        self.env.reset_drawn_device(idx.data_ptr(), None, int(idx.numel()), self._stream())
+        self._keep_drawn = idx  # alive until the kernel has run
+
     def close(self):
         """Drops this object's views and closes the env.  Tensors the caller still holds keep the device memory alive:
         the OkEnv is destroyed when the last of them is released (openkitchen_b200.dlpack)."""
         self._views.clear()
+        self.reset_draw_count = None
         for name in ("obs", "hits", "hit_points", "hit_seg", "hit_t", "reward", "fitness", "done", "crashed", "timed_out",
                      "nearest_idx", "pos_x", "pos_y", "rot", "speed", "act_throttle", "act_steer"):
             setattr(self, name, None)

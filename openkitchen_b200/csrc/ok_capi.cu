@@ -204,6 +204,7 @@ struct Agents
     DevPtr<float>    act_stage;
     DevPtr<uint32_t> act_ready;
     uint32_t         act_ready_target{0};
+    DevPtr<uint32_t>           draw_k; // the reset-draw counters k (ok_reset_draw_counts), zeroed here
     DevPtr<unsigned long long> stats; // ok_debug_stats: allocated on first use
     DevPtr<unsigned long long> trace; // ok_debug_trace
     int32_t                    trace_tiles{0};
@@ -213,6 +214,7 @@ struct Agents
 struct OkEnv
 {
     OkConfig               cfg{};
+    OkResetDraws           draws{}; // ok_set_reset_draws; flags 0 = off
     bool                   has_device{false};
     int                    num_sms{0};
     size_t                 max_blob{0};
@@ -312,6 +314,7 @@ int ensure_arena(OkEnv *e)
             const ok::TrackHeader *th = reinterpret_cast<const ok::TrackHeader *>(t.blob.data());
             r.seg_bytes = th->off_words; // header + segments
             r.n_points = th->n_points, r.off_points = th->off_points, r.off_headings = th->off_headings;
+            r.off_segments = th->off_segments;
         }
         refs.push_back(r);
         total += (t.blob.size() + 127) / 128 * 128;
@@ -495,6 +498,9 @@ ok::StepParams base_params(OkEnv *e)
     p.standstill_thr2   = e->cfg.standstill_threshold * e->cfg.standstill_threshold; // Environment.cpp:26
     p.standstill_period = e->cfg.standstill_period;
     p.id_base           = e->cfg.agent_id_base;
+    p.reset_k           = e->ag.draw_k.get();
+    p.reset_seed        = e->draws.seed;
+    p.reset_flags       = e->draws.flags; // launch_step keeps them only for a tick whose auto-reset draws
     return p;
 }
 
@@ -539,7 +545,12 @@ int arm_shared_memory_limit(OkEnv *e)
     int max_dynamic = 0;
     OK_CUDA(ok::arm_step_grid(e->smem_optin, &max_dynamic));
     OK_CUDA(ok::arm_step_staged(e->smem_optin, &max_dynamic));
+    OK_CUDA(ok::arm_step_grid_drawn(e->smem_optin, &max_dynamic));
+    OK_CUDA(ok::arm_step_staged_drawn(e->smem_optin, &max_dynamic));
+    int drawn_dyn_max = 0; // the fused kernel's limit is what both of its kernels allow
+    OK_CUDA(ok::arm_step_actor_drawn(e->smem_optin, &drawn_dyn_max));
     OK_CUDA(ok::arm_step_actor(e->smem_optin, &e->actor_dyn_max));
+    e->actor_dyn_max = std::min(e->actor_dyn_max, drawn_dyn_max);
     return OK_SUCCESS;
 }
 
@@ -630,6 +641,9 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
     int rc = ensure_arena(e);
     if (rc)
         return rc;
+    if (!(p.do_move && e->cfg.auto_reset))
+        p.reset_flags = 0;
+    const bool drawn = p.reset_flags != 0; // the tick's auto-reset draws: the step kernels' twins with the drawn reset
     p.arena      = e->d_arena.get();
     p.tracks     = e->d_track_refs.get();
     Agents &ag   = e->ag;
@@ -686,15 +700,15 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
         if (actor)
         { // the policy step as phase 0 of every tile (ok_ppo_actor_step): its weights sit behind the kernel's own shared memory
             p.actor_smem_off = static_cast<uint32_t>((ag.sizing.smem_beam + 15) & ~static_cast<size_t>(15));
-            OK_CUDA(ok::launch_step_actor(p, *actor, ag.beam.grid, p.actor_smem_off + actor_smem, s));
+            OK_CUDA((drawn ? ok::launch_step_actor_drawn : ok::launch_step_actor)(p, *actor, ag.beam.grid, p.actor_smem_off + actor_smem, s));
         }
         else if (ag.sizing.beam_staged)
-            OK_CUDA(ok::launch_step_staged(p, grid, ag.sizing.smem_beam, s));
+            OK_CUDA((drawn ? ok::launch_step_staged_drawn : ok::launch_step_staged)(p, grid, ag.sizing.smem_beam, s));
         else
-            OK_CUDA(ok::launch_step_unstaged(p, ag.beam.grid, ag.sizing.smem_beam, s));
+            OK_CUDA((drawn ? ok::launch_step_unstaged_drawn : ok::launch_step_unstaged)(p, ag.beam.grid, ag.sizing.smem_beam, s));
     }
     else
-        OK_CUDA(ok::launch_step_grid(p, ag.tiles.grid, ag.sizing.smem, s));
+        OK_CUDA((drawn ? ok::launch_step_grid_drawn : ok::launch_step_grid)(p, ag.tiles.grid, ag.sizing.smem, s));
     if (p.act_ready)
     { // enqueued AFTER the launch: the kernel is already running its first tiles while the host issues these
         const size_t bytes = sizeof(float) * static_cast<size_t>(e->n_agents);
@@ -1044,6 +1058,8 @@ int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg,
         e->d_buf[b]   = ag.slab.get() + offs[b];
         e->buf_off[b] = offs[b];
     }
+    OK_CUDA(dev_alloc(ag.draw_k, static_cast<size_t>(n)));
+    OK_CUDA(cudaMemset(ag.draw_k.get(), 0, sizeof(uint32_t) * static_cast<size_t>(n)));
     OK_CUDA(dev_alloc(ag.ray_deg, static_cast<size_t>(rays)));
     OK_CUDA(cudaMemcpy(ag.ray_deg.get(), h_ray_deg, sizeof(float) * rays, cudaMemcpyHostToDevice));
     e->h_track_id.assign(static_cast<size_t>(n), 0);
@@ -1177,6 +1193,80 @@ int ok_reset_agents_host(OkEnv *e, const int64_t *h_agent_idx, const int32_t *h_
         return rc;
     return st.finish(ok_reset_agents(e, st.d<const int64_t>(0), st.d<const int32_t>(1), st.d<const float>(2),
                                      st.d<const float>(3), n, stream));
+}
+
+int ok_set_reset_draws(OkEnv *e, const OkResetDraws *d)
+{
+    if (int rc = check_device(e))
+        return rc;
+    if (d && (d->flags & ~(OK_RESET_DRAW_POINT | OK_RESET_DRAW_LANE | OK_RESET_DRAW_HEADING)))
+        return fail(OK_ERR_INVALID_ARG, "unknown OK_RESET_DRAW_* flag bits");
+    e->draws = d ? *d : OkResetDraws{};
+    return OK_SUCCESS;
+}
+
+int ok_get_reset_draws(const OkEnv *e, OkResetDraws *out)
+{
+    if (int rc = check_device(e))
+        return rc;
+    if (!out)
+        return fail(OK_ERR_INVALID_ARG, "out is NULL");
+    *out = e->draws;
+    return OK_SUCCESS;
+}
+
+int ok_reset_agents_drawn(OkEnv *e, const int64_t *d_agent_idx, const uint8_t *d_mask, int64_t n, void *stream)
+{
+    int rc = check_ready(e);
+    if (rc)
+        return rc;
+    if (d_agent_idx && d_mask)
+        return fail(OK_ERR_INVALID_ARG, "pass agent indices or a mask, not both");
+    if (!d_agent_idx && n != e->n_agents)
+        return fail(OK_ERR_INVALID_ARG, "with a mask or for all agents, n must be ok_num_agents");
+    if (n <= 0)
+        return OK_SUCCESS;
+    DeviceGuard g(e->cfg.device);
+    rc = ensure_arena(e);
+    if (rc)
+        return rc;
+    ok::StepParams       p = base_params(e);
+    ok::DrawnResetParams r{d_agent_idx, d_mask, n, e->n_agents};
+    const int            threads = 128;
+    const int64_t        blocks  = (n + threads - 1) / threads;
+    ok::reset_drawn_kernel<<<static_cast<unsigned>(blocks), threads, 0, static_cast<cudaStream_t>(stream)>>>(p, r);
+    OK_CUDA(cudaGetLastError());
+    e->launches++;
+    return OK_SUCCESS;
+}
+
+int ok_reset_agents_drawn_host(OkEnv *e, const int64_t *h_agent_idx, const uint8_t *h_mask, int64_t n, void *stream)
+{
+    int rc = check_ready(e);
+    if (rc)
+        return rc;
+    if (h_agent_idx && h_mask)
+        return fail(OK_ERR_INVALID_ARG, "pass agent indices or a mask, not both");
+    if (!h_agent_idx && n != e->n_agents)
+        return fail(OK_ERR_INVALID_ARG, "with a mask or for all agents, n must be ok_num_agents");
+    if (n <= 0)
+        return OK_SUCCESS;
+    DeviceGuard  g(e->cfg.device);
+    const size_t k = static_cast<size_t>(n);
+    HostStage    st(e, stream, {{h_agent_idx, nullptr, 8 * k}, {h_mask, nullptr, k}});
+    if ((rc = st.upload()))
+        return rc;
+    return st.finish(ok_reset_agents_drawn(e, st.d<const int64_t>(0), st.d<const uint8_t>(1), n, stream));
+}
+
+int ok_reset_draw_counts(OkEnv *e, uint32_t **d_counts)
+{
+    if (int rc = check_ready(e))
+        return rc;
+    if (!d_counts)
+        return fail(OK_ERR_INVALID_ARG, "d_counts is NULL");
+    *d_counts = e->ag.draw_k.get();
+    return OK_SUCCESS;
 }
 
 int ok_cast_rays(OkEnv *e, void *stream)
@@ -1964,14 +2054,19 @@ int ok_debug_violations(OkEnv *e, uint64_t *count, int32_t *checks_compiled_in)
     DeviceGuard g(e->cfg.device);
     OK_CUDA(cudaDeviceSynchronize());
     unsigned long long staged = 0, unstaged = 0, actor = 0, grid = 0, lidar = 0, bev = 0;
+    unsigned long long staged_d = 0, unstaged_d = 0, actor_d = 0, grid_d = 0; // the step kernels with drawn resets
     OK_CUDA(ok::violations_step_staged(&staged));
     OK_CUDA(ok::violations_step_unstaged(&unstaged));
     OK_CUDA(ok::violations_step_actor(&actor));
     OK_CUDA(ok::violations_step_grid(&grid));
+    OK_CUDA(ok::violations_step_staged_drawn(&staged_d));
+    OK_CUDA(ok::violations_step_unstaged_drawn(&unstaged_d));
+    OK_CUDA(ok::violations_step_actor_drawn(&actor_d));
+    OK_CUDA(ok::violations_step_grid_drawn(&grid_d));
     OK_CUDA(ok::violations_lidar_query(&lidar));
     OK_CUDA(ok::violations_bev(&bev));
     if (count)
-        *count = staged + unstaged + actor + grid + lidar + bev;
+        *count = staged + unstaged + actor + grid + staged_d + unstaged_d + actor_d + grid_d + lidar + bev;
     if (checks_compiled_in)
         *checks_compiled_in = OK_CHECKED;
     return OK_SUCCESS;

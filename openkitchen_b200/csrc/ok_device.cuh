@@ -45,9 +45,10 @@ struct TrackRef
     int32_t  bnx, bny, bnb;
     uint32_t boff_rows, boff_entries, boff_items, bn_rows, bn_chunks;
     uint32_t seg_bytes;   // header + segments (+ the null segment) = the blob's prefix up to the grid words; no kernel reads it
-    // what a crashed agent's auto-reset needs of the blob's header (phase 1 reads the GLOBAL blob: one trip to memory less)
+    // what a crashed agent's auto-reset needs of the blob's header (phase 1 reads the GLOBAL blob: one trip to memory less);
+    // off_segments: the lane lerp of a drawn reset reads the LI / RI segment start points
     int32_t  n_points;
-    uint32_t off_points, off_headings, pad;
+    uint32_t off_points, off_headings, off_segments;
 };
 static_assert(sizeof(TrackRef) == 96, "TrackRef layout");
 // a CTA's FIRST tile with its track record next to it: one trip to memory instead of two before any work can start
@@ -120,6 +121,11 @@ struct StepParams
     int32_t  movement_mode, reward_mode, raycast_mode, auto_reset, auto_reset_stride;
     float    sensor_range, speed_limit, dt, collision_dist2, sensor_offset, standstill_thr2;
     uint32_t standstill_period;
+    // reset draws (ok_set_reset_draws): the per-agent stream counters k, the key and the OK_RESET_DRAW_* flags.  A step
+    // launch carries the flags only when its auto-reset draws, and then runs the kDraws instantiation of its kernel.
+    uint32_t *reset_k;
+    uint32_t  reset_seed;
+    int32_t   reset_flags;
 };
 
 // view of the staged blob
@@ -701,11 +707,67 @@ __device__ __forceinline__ float finish_ray(const StepParams &p, const float4 *s
     return sq;
 }
 
+// ---------------------------------------------------------------------------------------------
+// resets: Environment::resetAgent (Environment.cpp:79-122) + Agent::reset (Agent.cpp:123-135)
+// ---------------------------------------------------------------------------------------------
+// The draws of a drawn reset (OkResetDraws, include/openkitchen_b200.h): Philox4x32-10 keyed by (seed, "RST") at counter
+// (id, k) -> (pt, lane alpha, heading offset).  `pt_otherwise` is the point without OK_RESET_DRAW_POINT.  The one
+// definition of the mapping: the step kernels' auto-reset and reset_drawn_kernel both call it.
+constexpr uint32_t kResetStreamKey = 0x525354u; // "RST"
+constexpr int32_t  kStartingIdx    = 3;          // RaceTrack::kStartingIdx (RaceTrack.h:18): an explicit reset's point without draws
+struct ResetDraw
+{
+    int32_t pt;
+    bool    lane; // alpha is valid
+    float   alpha, off;
+};
+__device__ __forceinline__ ResetDraw reset_draw(const uint32_t seed, const int32_t flags, const uint64_t id, const uint32_t k,
+                                                const int32_t n_points, const int32_t pt_otherwise)
+{
+    uint32_t o[4];
+    philox4x32_10(static_cast<uint32_t>(id), static_cast<uint32_t>(id >> 32), k, 0u, seed, kResetStreamKey, o);
+    ResetDraw d;
+    // U(o, m) = (o * m) >> 32: U{0..m-1}
+    d.pt    = (flags & OK_RESET_DRAW_POINT) ? static_cast<int32_t>(__umulhi(o[0], static_cast<uint32_t>(n_points))) : pt_otherwise;
+    d.lane  = (flags & OK_RESET_DRAW_LANE) != 0;
+    d.alpha = __fdiv_rn(static_cast<float>(10u + __umulhi(o[1], 81u)), 100.0f);
+    const float mag = static_cast<float>(45u + __umulhi(o[2], 46u));
+    d.off   = (flags & OK_RESET_DRAW_HEADING) ? ((k & 1u) ? mag : -mag) : 0.0f;
+    return d;
+}
+
+// The pose a reset gives: centre-line point pt (Environment.cpp:103-106), or with `lane` the lerp by alpha between the LI
+// and RI points (Environment.cpp:107-114; they are the start points of the LI / RI segment chains, and the last point
+// starts the closure segments), heading headings[pt] + off (Environment.cpp:121).  Shared by every kind of reset.
+__device__ __forceinline__ float3 reset_pose(const float2 *pts, const float *headings, const float4 *seg, const int32_t n,
+                                             const int32_t pt, const bool lane, const float alpha, const float off)
+{
+    float sx, sy;
+    if (lane)
+    {
+        const float4 ls = seg[pt < n - 1 ? pt : 4 * (n - 1)];
+        const float4 rs = seg[pt < n - 1 ? 2 * (n - 1) + pt : 4 * (n - 1) + 1];
+        OK_CHECK(pt >= 0 && pt < n);
+        const float one_minus = fsub(1.0f, alpha);
+        sx = fadd(fmul(ls.x, alpha), fmul(rs.x, one_minus));
+        sy = fadd(fmul(ls.y, alpha), fmul(rs.y, one_minus));
+    }
+    else
+    {
+        const float2 c = pts[pt];
+        sx = c.x, sy = c.y;
+    }
+    return make_float3(sx, sy, fadd(headings[pt], off));
+}
+
 // Phase 1 for agent `a` (one thread): optional auto-reset, kinematics from the action, standstill timeout
 // (Environment.cpp:128-143), lidar origin (CollisionChecker.cu:121-124).  Writes the agent's state buffers and
 // returns the record the ray and reward phases work from.
 // `gblob` is the track's blob in the GLOBAL arena: only a crashed agent's auto-reset reads it (centre line, headings),
 // so phase 1 does not have to wait for the blob to be staged in shared memory.
+// kDraws: the auto-reset is a drawn reset (p.reset_flags != 0; the host launches this instantiation only then), so that the
+// kernels without draws stay what they were.
+template <bool kDraws = false>
 __device__ __forceinline__ AgentRec agent_pre(const StepParams &p, const uint8_t *gblob, const TrackRef &tr, const BeamView &bv, const int64_t a,
                                               const bool act_staged = false, const float2 *s_action = nullptr)
 {
@@ -713,6 +775,8 @@ __device__ __forceinline__ AgentRec agent_pre(const StepParams &p, const uint8_t
     bool     crashed = p.crashed[a] != 0, timed_out = p.timed_out[a] != 0;
     // (auto-reset) the reset point is requested with the rest of the state, not after the crash flag has arrived
     const int32_t reset_pt0 = (p.auto_reset && p.do_move) ? p.reset_pt[a] : 0;
+    // (drawn auto-reset) so is the agent's draw counter
+    const uint32_t k0 = kDraws ? p.reset_k[a] : 0u;
     // the standstill record is read up front with the rest of the state: a load issued only after the kinematics
     // would add a second trip to memory to the latency of this (latency-bound) phase
     const uint32_t ss_ctr0 = p.ss_ctr[a];
@@ -783,9 +847,22 @@ __device__ __forceinline__ AgentRec agent_pre(const StepParams &p, const uint8_t
         // prev / nearest / fitness are finalised in phase 4 (they need a centre-line search).
         if (p.auto_reset && crashed)
         {
-            const int32_t pt = static_cast<int32_t>((static_cast<int64_t>(reset_pt0) + p.auto_reset_stride) % tr.n_points);
-            const float2  c  = reinterpret_cast<const float2 *>(gblob + tr.off_points)[pt];
-            x = c.x, y = c.y, rot = reinterpret_cast<const float *>(gblob + tr.off_headings)[pt];
+            int32_t pt = static_cast<int32_t>((static_cast<int64_t>(reset_pt0) + p.auto_reset_stride) % tr.n_points);
+            if constexpr (kDraws)
+            { // the Philox rounds run here only, for the crashed agents
+                const ResetDraw d = reset_draw(p.reset_seed, p.reset_flags, p.id_base + static_cast<uint64_t>(a), k0, tr.n_points, pt);
+                pt                = d.pt;
+                const float3 q    = reset_pose(reinterpret_cast<const float2 *>(gblob + tr.off_points),
+                                               reinterpret_cast<const float *>(gblob + tr.off_headings),
+                                               reinterpret_cast<const float4 *>(gblob + tr.off_segments), tr.n_points, pt, d.lane, d.alpha, d.off);
+                x = q.x, y = q.y, rot = q.z;
+                p.reset_k[a] = k0 + 1u;
+            }
+            else
+            {
+                const float2 c = reinterpret_cast<const float2 *>(gblob + tr.off_points)[pt];
+                x = c.x, y = c.y, rot = reinterpret_cast<const float *>(gblob + tr.off_headings)[pt];
+            }
             accel = 0.0f, speed = 0.0f;
             crashed = false, timed_out = false;
             thr = 0.0f, steer = 0.0f; // Agent::reset zeroes current_action_

@@ -8,8 +8,34 @@
 namespace ok
 {
 
-// Environment::resetAgent (Environment.cpp:79-122) + Agent::reset (Agent.cpp:123-135), one thread
-// per request, reading the track blobs from global memory.
+// Environment::resetAgent (Environment.cpp:79-122) + Agent::reset (Agent.cpp:123-135) of agent `a` with the draws
+// (pt, alpha, off) made explicit, and the episode bookkeeping (main_eigen.cpp:121-130: prev_track_idx_ = nearest index of the
+// post-reset pose, fitness restarts); the standstill record is not touched (Environment.cpp never resets it).
+__device__ __forceinline__ void reset_agent(const StepParams &p, const TrackView &tv, const int64_t a, const int32_t pt, const bool lane,
+                                            const float alpha, const float off)
+{
+    const float3 q = reset_pose(tv.pts, tv.headings, tv.seg, tv.n_pts, pt, lane, alpha, off);
+    p.x[a] = q.x, p.y[a] = q.y;
+    p.rot[a]       = q.z;
+    p.accel[a]     = 0.0f;
+    p.speed[a]     = 0.0f;
+    p.crashed[a]   = 0;
+    p.timed_out[a] = 0;
+    p.done[a]      = 0;
+    p.act_thr[a]   = 0.0f;
+    p.act_steer[a] = 0.0f;
+    p.reset_pt[a]  = pt;
+    p.start_x[a]   = q.x;
+    p.start_y[a]   = q.y;
+    float   d2;
+    int32_t near  = nearest_index(tv, q.x, q.y, 0, 1, d2);
+    p.prev[a]     = near;
+    p.nearest[a]  = near;
+    p.fitness[a]  = 0.0f;
+    p.reward[a]   = 0.0f;
+}
+
+// ok_reset_agents: one thread per request, reading the track blobs from global memory.
 struct ResetParams
 {
     const int64_t *agent_idx; // nullable
@@ -27,54 +53,34 @@ __global__ void reset_kernel(const StepParams p, const ResetParams r)
     const int64_t a = r.agent_idx ? r.agent_idx[k] : k;
     if (a < 0 || a >= r.n_agents)
         return;
-    const uint8_t    *blob = p.arena + p.tracks[p.track_id[a]].offset;
-    const TrackView   tv   = make_view(blob);
-    int32_t           pt   = r.pt_idx[k];
-    pt                     = min(max(pt, 0), tv.n_pts - 1);
-    float sx, sy;
-    if (r.lane_alpha)
-    { // Environment.cpp:107-114; LI / RI points are the start points of the LI / RI segment chains
-        const float   alpha = r.lane_alpha[k];
-        const int32_t n     = tv.n_pts;
-        float2        l, rr;
-        if (pt < n - 1)
-        {
-            const float4 ls = tv.seg[pt], rs = tv.seg[2 * (n - 1) + pt];
-            l = make_float2(ls.x, ls.y), rr = make_float2(rs.x, rs.y);
-        }
-        else
-        { // the last point starts the closure segments
-            const float4 ls = tv.seg[4 * (n - 1)], rs = tv.seg[4 * (n - 1) + 1];
-            l = make_float2(ls.x, ls.y), rr = make_float2(rs.x, rs.y);
-        }
-        const float one_minus = fsub(1.0f, alpha);
-        sx = fadd(fmul(l.x, alpha), fmul(rr.x, one_minus));
-        sy = fadd(fmul(l.y, alpha), fmul(rr.y, one_minus));
-    }
-    else
-    {
-        const float2 c = tv.pts[pt];
-        sx = c.x, sy = c.y;
-    }
-    const float off = r.heading_off ? r.heading_off[k] : 0.0f;
-    p.x[a] = sx, p.y[a] = sy;
-    p.rot[a]       = fadd(tv.headings[pt], off);
-    p.accel[a]     = 0.0f;
-    p.speed[a]     = 0.0f;
-    p.crashed[a]   = 0;
-    p.timed_out[a] = 0;
-    p.done[a]      = 0;
-    p.act_thr[a]   = 0.0f;
-    p.act_steer[a] = 0.0f;
-    p.reset_pt[a]  = pt;
-    p.start_x[a]   = sx;
-    p.start_y[a]   = sy;
-    float   d2;
-    int32_t near  = nearest_index(tv, sx, sy, 0, 1, d2);
-    p.prev[a]     = near;
-    p.nearest[a]  = near;
-    p.fitness[a]  = 0.0f;
-    p.reward[a]   = 0.0f;
+    const TrackView tv = make_view(p.arena + p.tracks[p.track_id[a]].offset);
+    const int32_t   pt = min(max(r.pt_idx[k], 0), tv.n_pts - 1);
+    reset_agent(p, tv, a, pt, r.lane_alpha != nullptr, r.lane_alpha ? r.lane_alpha[k] : 0.0f, r.heading_off ? r.heading_off[k] : 0.0f);
+}
+
+// ok_reset_agents_drawn: a drawn reset (reset_draw) of agent agent_idx[k], or of agent k when mask is NULL or mask[k] != 0;
+// one thread per request.
+struct DrawnResetParams
+{
+    const int64_t *agent_idx; // nullable
+    const uint8_t *mask;      // nullable; not with agent_idx
+    int64_t        n, n_agents;
+};
+
+__global__ void reset_drawn_kernel(const StepParams p, const DrawnResetParams r)
+{
+    const int64_t k = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (k >= r.n)
+        return;
+    const int64_t a = r.agent_idx ? r.agent_idx[k] : k;
+    if (a < 0 || a >= r.n_agents || (r.mask && !r.mask[a]))
+        return;
+    const TrackView tv = make_view(p.arena + p.tracks[p.track_id[a]].offset);
+    const uint32_t  k0 = p.reset_k[a];
+    const ResetDraw d  = reset_draw(p.reset_seed, p.reset_flags, p.id_base + static_cast<uint64_t>(a), k0, tv.n_pts,
+                                    min(kStartingIdx, tv.n_pts - 1));
+    reset_agent(p, tv, a, d.pt, d.lane, d.alpha, d.off);
+    p.reset_k[a] = k0 + 1u;
 }
 
 // GeneticAgent::updateAction + Network::infer for every agent (EvolutionaryRacer/GeneticAgent.hpp:37-50,

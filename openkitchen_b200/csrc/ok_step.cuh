@@ -423,9 +423,11 @@ __device__ __forceinline__ void rearm_scheduler(const StepParams &p, const bool 
 // The beam kernel.  kActor (ok_ppo_actor_step): the PPO racers' policy step runs as phase 0 of every tile -- the tile's
 // agents choose their actions from last tick's observations (actor_agent) and the kinematics read them from the action
 // buffers -- so that a rollout tick is ONE launch: at a few thousand agents a tick is latency, and two kernels pay it twice.
-template <bool kStaged, bool kActor = false>
-__global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN_CTAS)
-    beam_step_kernel(const StepParams p, const typename ActorArg<kActor>::type q)
+// The body is beam_tick; beam_step_kernel and beam_step_drawn_kernel (below) are its two entry points.  kDraws: the
+// auto-reset is a drawn reset (agent_pre<true>), in a kernel of its own, so that the kernels without draws keep their
+// registers and schedule.
+template <bool kStaged, bool kActor, bool kDraws>
+__device__ __forceinline__ void beam_tick(const StepParams &p, const typename ActorArg<kActor>::type &q)
 {
     constexpr int kBlock   = beam_block(kStaged);
     constexpr int kPendCap = beam_pend_cap(kStaged);
@@ -510,7 +512,7 @@ __global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN
             __syncthreads(); // the chosen actions are in shared memory: the agents' own threads read them next
         }
         if (tid < count)
-            recs[tid] = agent_pre(p, gblob, tr, bv, tl.begin + tid, n_done > 0 && s_actdev != 0, kActor ? s_actor_act + tid : nullptr);
+            recs[tid] = agent_pre<kDraws>(p, gblob, tr, bv, tl.begin + tid, n_done > 0 && s_actdev != 0, kActor ? s_actor_act + tid : nullptr);
         if (tid == 0)
         {
             s_pool2 = 0, s_npend = 0, s_adone = 0;
@@ -865,6 +867,21 @@ __global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN
     rearm_scheduler(p, single_wave, tid);
 }
 
+template <bool kStaged, bool kActor = false>
+__global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN_CTAS)
+    beam_step_kernel(const StepParams p, const typename ActorArg<kActor>::type q)
+{
+    beam_tick<kStaged, kActor, false>(p, q);
+}
+
+// the same tick with the drawn auto-reset (OkResetDraws): launched instead of beam_step_kernel when p.reset_flags != 0
+template <bool kStaged, bool kActor = false>
+__global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN_CTAS)
+    beam_step_drawn_kernel(const StepParams p, const typename ActorArg<kActor>::type q)
+{
+    beam_tick<kStaged, kActor, true>(p, q);
+}
+
 // ---------------------------------------------------------------------------------------------
 // the host's interface to the step kernels, one translation unit each (see the top of this file):
 //   launch_step_<unit>      launches the unit's kernel on `grid` CTAs with `smem_bytes` of dynamic shared memory
@@ -873,6 +890,8 @@ __global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN
 //                           static shared memory
 //   occupancy_step_<unit>   CTAs per SM at `smem_bytes` of dynamic shared memory
 //   violations_step_<unit>  the unit's self-check counter (OK_CHECKED builds; zero otherwise)
+// Every step kernel has a twin with the drawn auto-reset (OkResetDraws) in a unit of its own, <unit>_drawn, with the same
+// functions; the host launches it for the ticks whose auto-reset draws (StepParams::reset_flags != 0).
 // ---------------------------------------------------------------------------------------------
 cudaError_t launch_step_staged(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
 cudaError_t arm_step_staged(int smem_optin, int *max_dynamic);
@@ -896,6 +915,18 @@ constexpr int kGridBlock = OK_BLOCK;
 cudaError_t launch_step_grid(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
 cudaError_t arm_step_grid(int smem_optin, int *max_dynamic);
 cudaError_t violations_step_grid(unsigned long long *count);
+
+cudaError_t launch_step_staged_drawn(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
+cudaError_t arm_step_staged_drawn(int smem_optin, int *max_dynamic);
+cudaError_t violations_step_staged_drawn(unsigned long long *count);
+cudaError_t launch_step_unstaged_drawn(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
+cudaError_t violations_step_unstaged_drawn(unsigned long long *count);
+cudaError_t launch_step_actor_drawn(const StepParams &p, const ActorParams &q, int grid, size_t smem_bytes, cudaStream_t stream);
+cudaError_t arm_step_actor_drawn(int smem_optin, int *max_dynamic);
+cudaError_t violations_step_actor_drawn(unsigned long long *count);
+cudaError_t launch_step_grid_drawn(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
+cudaError_t arm_step_grid_drawn(int smem_optin, int *max_dynamic);
+cudaError_t violations_step_grid_drawn(unsigned long long *count);
 __host__ __device__ inline size_t batch_smem_bytes(int agents, int rays)
 { // the grid kernel's batch scratch: AgentRec + per ray float2 direction
     return static_cast<size_t>(agents) * (sizeof(AgentRec) + 8u * static_cast<size_t>(rays));

@@ -99,9 +99,11 @@ def to_capsule(ptr: int, shape, dtype, device_id: int, owner):
 class DeviceBuffer:
     """``__dlpack__`` provider for one OkEnv buffer (what ``torch.from_dlpack`` expects)."""
 
-    def __init__(self, env, name: str):
+    def __init__(self, env, name: str, info=None):
+        """info: (device pointer, shape, dtype) of a device array the env owns that is not an OkBuffer (e.g. the
+        reset-draw counters); None = env.buffer_info(name)"""
         self.env, self.name = env, name
-        self.ptr, self.shape, self.dtype = env.buffer_info(name)
+        self.ptr, self.shape, self.dtype = info if info is not None else env.buffer_info(name)
 
     def __dlpack__(self, stream=None, **_):
         """`stream` (DLPack protocol: the consumer's stream; 1 = legacy default, 2 = per-thread default, -1 = no sync):

@@ -232,6 +232,68 @@ class Env:
     def reset_device(self, d_agent_idx, d_pt_idx, d_lane_alpha, d_heading_off, n, stream=None):
         check(self.lib.ok_reset_agents(self.h, d_agent_idx, d_pt_idx, d_lane_alpha, d_heading_off, n, stream))
 
+    # ---- reset draws (OkResetDraws: include/openkitchen_b200.h states the definition) -----
+    def set_reset_draws(self, seed: int, point: bool = True, lane: bool = False, heading: bool = False):
+        """Turn the reset draws on: with auto_reset the auto-reset of a crashed agent becomes a drawn reset, and
+        reset_drawn / reset_drawn_device draw.  point / lane / heading: Environment::resetAgent's random centre-line point,
+        lane lerp and +-(45..90) degree heading offset.  All three False turns the draws off."""
+        flags = (_capi.RESET_DRAW_POINT if point else 0) | (_capi.RESET_DRAW_LANE if lane else 0) | (
+            _capi.RESET_DRAW_HEADING if heading else 0)
+        self.set_reset_draw_flags(seed, flags)
+
+    def set_reset_draw_flags(self, seed: int, flags: int):
+        """the same with the OK_RESET_DRAW_* bits (0 = off)"""
+        flags = int(flags)
+        if flags & ~(_capi.RESET_DRAW_POINT | _capi.RESET_DRAW_LANE | _capi.RESET_DRAW_HEADING):
+            raise ValueError(f"unknown reset-draw flag bits in {flags:#x}")
+        d = _capi.OkResetDraws(seed=int(seed) & 0xFFFFFFFF, flags=flags)
+        check(self.lib.ok_set_reset_draws(self.h, C.byref(d)))
+
+    def reset_draws(self) -> dict:
+        """{"seed", "point", "lane", "heading"} as set; every flag False = off"""
+        d = _capi.OkResetDraws()
+        check(self.lib.ok_get_reset_draws(self.h, C.byref(d)))
+        return {"seed": int(d.seed), "point": bool(d.flags & _capi.RESET_DRAW_POINT),
+                "lane": bool(d.flags & _capi.RESET_DRAW_LANE), "heading": bool(d.flags & _capi.RESET_DRAW_HEADING)}
+
+    def _drawn_args(self, agent_idx, mask):
+        if agent_idx is not None and mask is not None:
+            raise ValueError("pass agent indices or a mask, not both")
+        if agent_idx is not None:
+            ai = np.ascontiguousarray(agent_idx, dtype=np.int64).reshape(-1)
+            return ai, None, len(ai)
+        if mask is not None:
+            m = np.ascontiguousarray(mask).reshape(-1)
+            if len(m) != self.n:
+                raise ValueError(f"the mask must have one entry per agent ({self.n}), got {len(m)}")
+            return None, m.astype(np.uint8), self.n
+        return None, None, self.n
+
+    def reset_drawn(self, agent_idx=None, mask=None, stream=None):
+        """Drawn reset (host arrays) of the agents agent_idx, of those where mask is set (one entry per agent), or of all
+        agents.  Synchronises `stream`."""
+        ai, m, n = self._drawn_args(agent_idx, mask)
+        check(self.lib.ok_reset_agents_drawn_host(self.h, _vp(ai), _vp(m), n, stream))
+
+    def reset_drawn_device(self, d_agent_idx=None, d_mask=None, n=None, stream=None):
+        """device-pointer form of reset_drawn (asynchronous on `stream`): d_agent_idx i64[n], or d_mask u8[agents], or
+        neither (all agents); n defaults to the agent count"""
+        if d_agent_idx and d_mask:
+            raise ValueError("pass agent indices or a mask, not both")
+        if n is None:
+            if d_agent_idx:
+                raise ValueError("n is required with agent indices")
+            n = self.n
+        elif not d_agent_idx and n != self.n:
+            raise ValueError(f"with a mask or for all agents, n must be the agent count ({self.n})")
+        check(self.lib.ok_reset_agents_drawn(self.h, d_agent_idx, d_mask, n, stream))
+
+    def reset_draw_counts_info(self):
+        """(device pointer, shape, dtype) of the reset-draw counters k, u32[agents]"""
+        ptr = C.c_void_p()
+        check(self.lib.ok_reset_draw_counts(self.h, C.byref(ptr)))
+        return ptr.value, (self.n,), np.uint32
+
     # ---- the tick -----------------------------------------------------------------------
     def cast_rays(self, stream=None):
         check(self.lib.ok_cast_rays(self.h, stream))

@@ -64,7 +64,9 @@ class GraphedRollout:
     its parameters may be updated in place between replays).  action_table: f32[A, 2] = (throttle, steering) per
     discrete action (kActionMap of the RL racers).  sample=False takes the argmax instead of sampling.
     After ``run()``: ``obs`` f32[T, N, R] (the state each action was chosen from), ``actions`` i64[T, N], ``log_prob``
-    f32[T, N], ``rewards`` f32[T, N], ``dones`` u8[T, N] (after the tick)."""
+    f32[T, N], ``rewards`` f32[T, N], ``dones`` u8[T, N] (after the tick).  With auto_reset and reset draws on
+    (BatchEnv.set_reset_draws) the crashed agents restart at drawn points inside the graph, and each replay continues the
+    reset stream."""
 
     def __init__(self, env: BatchEnv, policy: Callable[[torch.Tensor], torch.Tensor], action_table: torch.Tensor, steps: int,
                  sample: bool = True):
@@ -214,7 +216,9 @@ class FusedActorRollout:
 
     def run(self):
         """one rollout of ``steps`` ticks from the env's current state (captures the graph on first use; a replay draws
-        the same Philox stream again unless ``uniform`` is refreshed by the caller)"""
+        the same Philox action stream again unless ``uniform`` is refreshed by the caller).  Episode starts are another
+        matter: with auto_reset and reset draws on (BatchEnv.set_reset_draws), each replay continues the reset stream,
+        whose counters live on the device, so consecutive rollouts start their episodes at new draws"""
         if self.graph is None:
             self.capture()
         self.graph.replay()
