@@ -119,7 +119,8 @@ typedef struct OkConfig {
     int32_t  auto_reset;           /* !=0: a crashed agent is reset at the start of the next step
                                       (GuidedCostLearning/test.cpp:102-111) to centre-line index
                                       (last_reset + auto_reset_stride) mod P, with a zero action; with reset
-                                      draws on (ok_set_reset_draws) it is a drawn reset instead */
+                                      draws on (ok_set_reset_draws) it is a drawn reset instead; with lap
+                                      accounting on (ok_set_laps) a completed agent is reset too */
     int32_t  auto_reset_stride;    /* 97 */
     float    sensor_range;         /* Agent::kSensorRange 200        Agent.h:10 */
     float    speed_limit;          /* Agent::kSpeedLimit 100         Agent.h:11 */
@@ -231,6 +232,59 @@ int ok_reset_agents_drawn_host(OkEnv *env, const int64_t *h_agent_idx, const uin
 /* the device counters k: u32[ok_num_agents], owned by the env like the agent buffers; writable (to restart or move a
  * stream) */
 int ok_reset_draw_counts(OkEnv *env, uint32_t **d_counts);
+
+/* Lap accounting: centre-line progress, laps and lap times per agent, and Agent::completed_ (Agent.h:73, ORed into
+ * Agent::isDone, Agent.cpp:138-144) at a target lap count, inside the step.  A lap is P centre-line points (P = the
+ * agent's track's point count) travelled from wherever the episode started, not a crossing of index 0.
+ *
+ * Every agent a has device state (zero after ok_alloc_agents allocates it, then restarted by its initial reset):
+ *   lap_idx[a]   i32  the centre-line index at which progress was last measured
+ *   progress[a]  i32  signed centre-line points travelled since the last restart
+ *   laps[a]      i32  laps completed
+ *   ticks[a]     u32  ticks the agent moved since the last restart
+ *   lap_start[a] u32  the value of ticks when the current lap began
+ *   last_lap[a]  u32  ticks of the last completed lap; 0 = none yet
+ *   completed[a] u8   Agent::completed_
+ * 1. RESTART of a: lap_idx = the nearest centre-line index of the agent's pose (RaceTrack::findNearestTrackIndexBruteForce,
+ *    the value a reset writes to OK_BUF_PREV_IDX), every other field 0.  It happens at every reset of a by ok_reset_agents[_host],
+ *    ok_reset_agents_drawn[_host] and ok_alloc_agents (with accounting on or off), at the auto-reset inside a tick with
+ *    accounting on, and for every agent when ok_set_laps switches accounting from off to on.
+ * 2. A TICK with accounting on, for every agent that moves in it (not crashed at the start of the tick, after the tick's
+ *    auto-reset: the agents Environment.cpp:128-143 moves, one that crashes in this tick included), after the move:
+ *    n = the nearest index of the new pose (written to OK_BUF_NEAREST_IDX, which is then updated every tick in every
+ *    reward mode); d = n - lap_idx; if 2d > P then d -= P, else if 2d <= -P then d += P (so d lies in (-P/2, P/2]);
+ *    progress += d; lap_idx = n; ticks += 1;
+ *    if (int64)progress >= ((int64)laps + 1) * P: laps += 1, last_lap = ticks - lap_start, lap_start = ticks;
+ *    if target > 0 and laps >= target: completed = 1.
+ *    (Arithmetic on the 32-bit fields wraps in two's complement.)  At most one lap completes per tick; driving backwards
+ *    lowers progress but never laps, and a lap regained after a reversal counts once progress passes the next multiple of P.
+ *    OK_BUF_DONE = crashed || completed for every agent, and so is ok_step_host[_q16]'s host done mirror.
+ * 3. A completed agent keeps driving and sensing (Environment::step moves every agent whose crashed_ is clear); completed
+ *    stays set until the next restart.
+ * 4. With OkConfig::auto_reset and accounting on, the auto-reset at the start of a tick resets every agent with crashed ||
+ *    completed, by the same rule as for a crashed agent (the stride rule, or a drawn reset with reset draws on), and
+ *    restarts its lap state.
+ * 5. With accounting off, the tick neither reads nor writes lap state (its auto-reset does not restart it either: the
+ *    switch to on restarts every agent); OK_BUF_DONE = crashed as before.  ok_cast_rays, which moves nothing, never
+ *    touches it, and writes OK_BUF_DONE = crashed as it always has.
+ * Accounting is off by default. */
+typedef struct OkLaps {
+    int32_t enabled; /* != 0: on */
+    int32_t target;  /* laps at which completed is set; 0 = never */
+} OkLaps;
+/* l NULL = off; a negative target is OK_ERR_INVALID_ARG.  A switch from off to on enqueues the restart of every agent on
+ * `stream` (asynchronous, no host synchronisation).  The settings are read when a step launch is enqueued: a CUDA graph
+ * keeps the settings it was captured with, and its replays continue the lap state, which lives on the device. */
+int ok_set_laps(OkEnv *env, const OkLaps *l, void *stream);
+int ok_get_laps(const OkEnv *env, OkLaps *out);
+typedef struct OkLapBuffers {
+    int32_t  *lap_idx, *progress, *laps;
+    uint32_t *ticks, *lap_start, *last_lap;
+    uint8_t  *completed;
+} OkLapBuffers;
+/* device pointers to the seven arrays, [ok_num_agents] each, owned by the env like the agent buffers; writable (to plant
+ * state) */
+int ok_lap_buffers(OkEnv *env, OkLapBuffers *out);
 
 /* ---- the tick ------------------------------------------------------------------------------ */
 /* CollisionChecker::checkCollision (CollisionChecker.cu:96-100,113-174): lidar + crash flag on the

@@ -62,6 +62,20 @@ class OkResetDraws(C.Structure):
     _fields_ = [("seed", C.c_uint32), ("flags", C.c_int32)]
 
 
+class OkLaps(C.Structure):
+    _fields_ = [("enabled", C.c_int32), ("target", C.c_int32)]
+
+
+class OkLapBuffers(C.Structure):
+    _fields_ = [("lap_idx", C.c_void_p), ("progress", C.c_void_p), ("laps", C.c_void_p), ("ticks", C.c_void_p),
+                ("lap_start", C.c_void_p), ("last_lap", C.c_void_p), ("completed", C.c_void_p)]
+
+
+# the lap arrays of OkLapBuffers: field -> numpy dtype
+LAP_ARRAYS = {"lap_idx": "int32", "progress": "int32", "laps": "int32", "ticks": "uint32", "lap_start": "uint32",
+              "last_lap": "uint32", "completed": "uint8"}
+
+
 class OkTrackInfo(C.Structure):
     _fields_ = [
         ("n_points", C.c_int32),
@@ -152,6 +166,9 @@ SIGNATURES = {
     "ok_reset_agents_drawn": (C.c_int, [_P, _P, _P, C.c_int64, _P]),
     "ok_reset_agents_drawn_host": (C.c_int, [_P, _P, _P, C.c_int64, _P]),
     "ok_reset_draw_counts": (C.c_int, [_P, C.POINTER(_P)]),
+    "ok_set_laps": (C.c_int, [_P, C.POINTER(OkLaps), _P]),
+    "ok_get_laps": (C.c_int, [_P, C.POINTER(OkLaps)]),
+    "ok_lap_buffers": (C.c_int, [_P, C.POINTER(OkLapBuffers)]),
     "ok_cast_rays": (C.c_int, [_P, _P]),
     "ok_launch_step": (C.c_int, [_P, _P, _P, _P]),
     "ok_launch_steps_random": (C.c_int, [_P, C.c_uint64, C.c_int32, C.c_uint32, _P]),

@@ -60,6 +60,15 @@ class BatchEnv:
         self.act_throttle, self.act_steer = v["act_throttle"], v["act_steer"]
         # u32[N]: the reset-draw counters k (set_reset_draws); not an OkBuffer, so not in ok.BUFFERS / self[name]
         self.reset_draw_count = torch.from_dlpack(DeviceBuffer(self.env, "reset_draw_count", self.env.reset_draw_counts_info()))
+        # [N] each: the lap-accounting state (set_laps; OkLaps in include/openkitchen_b200.h), also not OkBuffers
+        lap = {f: torch.from_dlpack(DeviceBuffer(self.env, f, info)) for f, info in self.env.lap_buffers_info().items()}
+        self.lap_idx = lap["lap_idx"]            # i32: centre-line index at which progress was last measured
+        self.lap_progress = lap["progress"]      # i32: signed centre-line points since the episode started
+        self.laps = lap["laps"]                  # i32: laps completed
+        self.lap_ticks = lap["ticks"]            # u32: ticks moved since the episode started
+        self.lap_start_ticks = lap["lap_start"]  # u32: lap_ticks when the current lap began
+        self.last_lap_ticks = lap["last_lap"]    # u32: ticks of the last completed lap, 0 = none yet
+        self.completed = lap["completed"]        # u8: Agent::completed_ (laps >= target)
         self._step_count = 0
 
     # ---- views -----------------------------------------------------------------------------
@@ -220,6 +229,18 @@ class BatchEnv:
     def reset_draws(self) -> dict:
         return self.env.reset_draws()
 
+    def set_laps(self, target: int = 0, enabled: bool = True):
+        """Lap accounting (include/openkitchen_b200.h, OkLaps): every moving tick adds the agent's signed centre-line
+        progress to lap_progress, counts laps of P centre-line points from where its episode started (laps) and their
+        lengths in ticks (last_lap_ticks); with target > 0 an agent's completed flag, and so done, is set at `target` laps,
+        and auto_reset resets it like a crashed agent.  All inside the step kernel.  Switching it on restarts every agent's
+        lap state on torch's current stream; enabled=False turns it off (the tick then leaves the arrays alone)."""
+        self.env.set_laps(target, enabled, self._stream())
+
+    def lap_settings(self) -> dict:
+        """{"enabled", "target"} as set"""
+        return self.env.laps()
+
     def reset_drawn(self, agents=None):
         """Drawn reset (ok_reset_agents_drawn) of agents: None (all), a bool / uint8 CUDA mask with one entry per agent (e.g.
         ``env.done``, passed as it is: no nonzero, no host synchronisation), or an index tensor.  Runs on torch's current
@@ -248,6 +269,8 @@ class BatchEnv:
         the OkEnv is destroyed when the last of them is released (openkitchen_b200.dlpack)."""
         self._views.clear()
         self.reset_draw_count = None
+        for name in ("lap_idx", "lap_progress", "laps", "lap_ticks", "lap_start_ticks", "last_lap_ticks", "completed"):
+            setattr(self, name, None)
         for name in ("obs", "hits", "hit_points", "hit_seg", "hit_t", "reward", "fitness", "done", "crashed", "timed_out",
                      "nearest_idx", "pos_x", "pos_y", "rot", "speed", "act_throttle", "act_steer"):
             setattr(self, name, None)

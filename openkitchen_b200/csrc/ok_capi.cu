@@ -205,6 +205,8 @@ struct Agents
     DevPtr<uint32_t> act_ready;
     uint32_t         act_ready_target{0};
     DevPtr<uint32_t>           draw_k; // the reset-draw counters k (ok_reset_draw_counts), zeroed here
+    DevPtr<uint8_t>            lap_slab; // the seven lap-accounting arrays (ok_lap_buffers), zeroed here
+    OkLapBuffers               lap{};
     DevPtr<unsigned long long> stats; // ok_debug_stats: allocated on first use
     DevPtr<unsigned long long> trace; // ok_debug_trace
     int32_t                    trace_tiles{0};
@@ -215,6 +217,7 @@ struct OkEnv
 {
     OkConfig               cfg{};
     OkResetDraws           draws{}; // ok_set_reset_draws; flags 0 = off
+    OkLaps                 laps{};  // ok_set_laps; enabled 0 = off
     bool                   has_device{false};
     int                    num_sms{0};
     size_t                 max_blob{0};
@@ -501,6 +504,8 @@ ok::StepParams base_params(OkEnv *e)
     p.reset_k           = e->ag.draw_k.get();
     p.reset_seed        = e->draws.seed;
     p.reset_flags       = e->draws.flags; // launch_step keeps them only for a tick whose auto-reset draws
+    p.lap               = e->ag.lap;
+    p.lap_target        = e->laps.target;
     return p;
 }
 
@@ -547,10 +552,13 @@ int arm_shared_memory_limit(OkEnv *e)
     OK_CUDA(ok::arm_step_staged(e->smem_optin, &max_dynamic));
     OK_CUDA(ok::arm_step_grid_drawn(e->smem_optin, &max_dynamic));
     OK_CUDA(ok::arm_step_staged_drawn(e->smem_optin, &max_dynamic));
-    int drawn_dyn_max = 0; // the fused kernel's limit is what both of its kernels allow
+    OK_CUDA(ok::arm_step_grid_laps(e->smem_optin, &max_dynamic));
+    OK_CUDA(ok::arm_step_staged_laps(e->smem_optin, &max_dynamic));
+    int drawn_dyn_max = 0, laps_dyn_max = 0; // the fused kernel's limit is what all three of its kernels allow
     OK_CUDA(ok::arm_step_actor_drawn(e->smem_optin, &drawn_dyn_max));
+    OK_CUDA(ok::arm_step_actor_laps(e->smem_optin, &laps_dyn_max));
     OK_CUDA(ok::arm_step_actor(e->smem_optin, &e->actor_dyn_max));
-    e->actor_dyn_max = std::min(e->actor_dyn_max, drawn_dyn_max);
+    e->actor_dyn_max = std::min({e->actor_dyn_max, drawn_dyn_max, laps_dyn_max});
     return OK_SUCCESS;
 }
 
@@ -644,6 +652,8 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
     if (!(p.do_move && e->cfg.auto_reset))
         p.reset_flags = 0;
     const bool drawn = p.reset_flags != 0; // the tick's auto-reset draws: the step kernels' twins with the drawn reset
+    // lap accounting on: the laps twins, which decide at run time whether the auto-reset draws (p.reset_flags)
+    const bool laps = p.do_move && e->laps.enabled;
     p.arena      = e->d_arena.get();
     p.tracks     = e->d_track_refs.get();
     Agents &ag   = e->ag;
@@ -700,15 +710,15 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
         if (actor)
         { // the policy step as phase 0 of every tile (ok_ppo_actor_step): its weights sit behind the kernel's own shared memory
             p.actor_smem_off = static_cast<uint32_t>((ag.sizing.smem_beam + 15) & ~static_cast<size_t>(15));
-            OK_CUDA((drawn ? ok::launch_step_actor_drawn : ok::launch_step_actor)(p, *actor, ag.beam.grid, p.actor_smem_off + actor_smem, s));
+            OK_CUDA((laps ? ok::launch_step_actor_laps : drawn ? ok::launch_step_actor_drawn : ok::launch_step_actor)(p, *actor, ag.beam.grid, p.actor_smem_off + actor_smem, s));
         }
         else if (ag.sizing.beam_staged)
-            OK_CUDA((drawn ? ok::launch_step_staged_drawn : ok::launch_step_staged)(p, grid, ag.sizing.smem_beam, s));
+            OK_CUDA((laps ? ok::launch_step_staged_laps : drawn ? ok::launch_step_staged_drawn : ok::launch_step_staged)(p, grid, ag.sizing.smem_beam, s));
         else
-            OK_CUDA((drawn ? ok::launch_step_unstaged_drawn : ok::launch_step_unstaged)(p, ag.beam.grid, ag.sizing.smem_beam, s));
+            OK_CUDA((laps ? ok::launch_step_unstaged_laps : drawn ? ok::launch_step_unstaged_drawn : ok::launch_step_unstaged)(p, ag.beam.grid, ag.sizing.smem_beam, s));
     }
     else
-        OK_CUDA((drawn ? ok::launch_step_grid_drawn : ok::launch_step_grid)(p, ag.tiles.grid, ag.sizing.smem, s));
+        OK_CUDA((laps ? ok::launch_step_grid_laps : drawn ? ok::launch_step_grid_drawn : ok::launch_step_grid)(p, ag.tiles.grid, ag.sizing.smem, s));
     if (p.act_ready)
     { // enqueued AFTER the launch: the kernel is already running its first tiles while the host issues these
         const size_t bytes = sizeof(float) * static_cast<size_t>(e->n_agents);
@@ -1060,6 +1070,19 @@ int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg,
     }
     OK_CUDA(dev_alloc(ag.draw_k, static_cast<size_t>(n)));
     OK_CUDA(cudaMemset(ag.draw_k.get(), 0, sizeof(uint32_t) * static_cast<size_t>(n)));
+    { // the lap arrays: six 4-byte arrays and the u8 completed flags, 256-byte aligned, zero until the initial reset below
+        const size_t a4 = (4 * static_cast<size_t>(n) + 255) / 256 * 256;
+        OK_CUDA(dev_alloc(ag.lap_slab, 6 * a4 + static_cast<size_t>(n)));
+        OK_CUDA(cudaMemset(ag.lap_slab.get(), 0, 6 * a4 + static_cast<size_t>(n)));
+        uint8_t *b       = ag.lap_slab.get();
+        ag.lap.lap_idx   = reinterpret_cast<int32_t *>(b);
+        ag.lap.progress  = reinterpret_cast<int32_t *>(b + a4);
+        ag.lap.laps      = reinterpret_cast<int32_t *>(b + 2 * a4);
+        ag.lap.ticks     = reinterpret_cast<uint32_t *>(b + 3 * a4);
+        ag.lap.lap_start = reinterpret_cast<uint32_t *>(b + 4 * a4);
+        ag.lap.last_lap  = reinterpret_cast<uint32_t *>(b + 5 * a4);
+        ag.lap.completed = b + 6 * a4;
+    }
     OK_CUDA(dev_alloc(ag.ray_deg, static_cast<size_t>(rays)));
     OK_CUDA(cudaMemcpy(ag.ray_deg.get(), h_ray_deg, sizeof(float) * rays, cudaMemcpyHostToDevice));
     e->h_track_id.assign(static_cast<size_t>(n), 0);
@@ -1266,6 +1289,50 @@ int ok_reset_draw_counts(OkEnv *e, uint32_t **d_counts)
     if (!d_counts)
         return fail(OK_ERR_INVALID_ARG, "d_counts is NULL");
     *d_counts = e->ag.draw_k.get();
+    return OK_SUCCESS;
+}
+
+int ok_set_laps(OkEnv *e, const OkLaps *l, void *stream)
+{
+    if (int rc = check_device(e))
+        return rc;
+    if (l && l->target < 0)
+        return fail(OK_ERR_INVALID_ARG, "the lap target must be >= 0");
+    const OkLaps next      = l ? *l : OkLaps{};
+    const bool   switch_on = next.enabled && !e->laps.enabled;
+    if (switch_on && e->n_agents > 0)
+    { // rule 1: every agent restarts at its current pose
+        DeviceGuard g(e->cfg.device);
+        if (int rc = ensure_arena(e))
+            return rc;
+        ok::StepParams p       = base_params(e);
+        const int      threads = 128;
+        const int64_t  blocks  = (e->n_agents + threads - 1) / threads;
+        ok::laps_restart_kernel<<<static_cast<unsigned>(blocks), threads, 0, static_cast<cudaStream_t>(stream)>>>(p);
+        OK_CUDA(cudaGetLastError());
+        e->launches++;
+    }
+    e->laps = next;
+    return OK_SUCCESS;
+}
+
+int ok_get_laps(const OkEnv *e, OkLaps *out)
+{
+    if (int rc = check_device(e))
+        return rc;
+    if (!out)
+        return fail(OK_ERR_INVALID_ARG, "out is NULL");
+    *out = e->laps;
+    return OK_SUCCESS;
+}
+
+int ok_lap_buffers(OkEnv *e, OkLapBuffers *out)
+{
+    if (int rc = check_ready(e))
+        return rc;
+    if (!out)
+        return fail(OK_ERR_INVALID_ARG, "out is NULL");
+    *out = e->ag.lap;
     return OK_SUCCESS;
 }
 
@@ -2055,6 +2122,7 @@ int ok_debug_violations(OkEnv *e, uint64_t *count, int32_t *checks_compiled_in)
     OK_CUDA(cudaDeviceSynchronize());
     unsigned long long staged = 0, unstaged = 0, actor = 0, grid = 0, lidar = 0, bev = 0;
     unsigned long long staged_d = 0, unstaged_d = 0, actor_d = 0, grid_d = 0; // the step kernels with drawn resets
+    unsigned long long staged_l = 0, unstaged_l = 0, actor_l = 0, grid_l = 0; // ... with lap accounting
     OK_CUDA(ok::violations_step_staged(&staged));
     OK_CUDA(ok::violations_step_unstaged(&unstaged));
     OK_CUDA(ok::violations_step_actor(&actor));
@@ -2063,10 +2131,15 @@ int ok_debug_violations(OkEnv *e, uint64_t *count, int32_t *checks_compiled_in)
     OK_CUDA(ok::violations_step_unstaged_drawn(&unstaged_d));
     OK_CUDA(ok::violations_step_actor_drawn(&actor_d));
     OK_CUDA(ok::violations_step_grid_drawn(&grid_d));
+    OK_CUDA(ok::violations_step_staged_laps(&staged_l));
+    OK_CUDA(ok::violations_step_unstaged_laps(&unstaged_l));
+    OK_CUDA(ok::violations_step_actor_laps(&actor_l));
+    OK_CUDA(ok::violations_step_grid_laps(&grid_l));
     OK_CUDA(ok::violations_lidar_query(&lidar));
     OK_CUDA(ok::violations_bev(&bev));
     if (count)
-        *count = staged + unstaged + actor + grid + staged_d + unstaged_d + actor_d + grid_d + lidar + bev;
+        *count = staged + unstaged + actor + grid + staged_d + unstaged_d + actor_d + grid_d + staged_l + unstaged_l + actor_l + grid_l +
+                 lidar + bev;
     if (checks_compiled_in)
         *checks_compiled_in = OK_CHECKED;
     return OK_SUCCESS;

@@ -126,6 +126,10 @@ struct StepParams
     uint32_t *reset_k;
     uint32_t  reset_seed;
     int32_t   reset_flags;
+    // lap accounting (ok_set_laps): the seven per-agent arrays, written by every explicit reset; the tick reads them only
+    // in the kLaps instantiation of its kernel, which the host launches when accounting is on.  lap_target 0 = never.
+    OkLapBuffers lap;
+    int32_t      lap_target;
 };
 
 // view of the staged blob
@@ -603,7 +607,9 @@ enum : uint32_t
 {
     kFlagCrashed = 1u,
     kFlagTimedOut = 2u,
-    kFlagReset = 4u
+    kFlagReset = 4u,
+    kFlagMoved = 8u,     // (kLaps kernels only) the agent moved in this tick
+    kFlagCompleted = 16u // (kLaps kernels only) completed[a] was set at the start of the tick and no reset cleared it
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -760,6 +766,49 @@ __device__ __forceinline__ float3 reset_pose(const float2 *pts, const float *hea
     return make_float3(sx, sy, fadd(headings[pt], off));
 }
 
+// ---------------------------------------------------------------------------------------------
+// lap accounting (OkLaps, include/openkitchen_b200.h states the definition)
+// ---------------------------------------------------------------------------------------------
+// rule 1: the restart of agent a's lap state at centre-line index `near`
+__device__ __forceinline__ void lap_restart(const OkLapBuffers &l, const int64_t a, const int32_t near)
+{
+    l.lap_idx[a]   = near;
+    l.progress[a]  = 0;
+    l.laps[a]      = 0;
+    l.ticks[a]     = 0;
+    l.lap_start[a] = 0;
+    l.last_lap[a]  = 0;
+    l.completed[a] = 0;
+}
+
+struct LapState
+{
+    int32_t  idx, progress, laps;
+    uint32_t ticks, lap_start, last_lap;
+    bool     completed;
+};
+
+// rule 2: the tick of an agent that moved to nearest index n on a track of P points (32-bit fields wrap)
+__device__ __forceinline__ void lap_advance(LapState &s, const int32_t n, const int32_t P, const int32_t target)
+{
+    int32_t d = static_cast<int32_t>(static_cast<uint32_t>(n) - static_cast<uint32_t>(s.idx));
+    if (2 * static_cast<int64_t>(d) > P)
+        d -= P;
+    else if (2 * static_cast<int64_t>(d) <= -static_cast<int64_t>(P))
+        d += P;
+    s.progress = static_cast<int32_t>(static_cast<uint32_t>(s.progress) + static_cast<uint32_t>(d));
+    s.idx      = n;
+    s.ticks += 1u;
+    if (static_cast<int64_t>(s.progress) >= (static_cast<int64_t>(s.laps) + 1) * P)
+    { // |d| <= P/2: at most one lap per tick
+        s.laps      = static_cast<int32_t>(static_cast<uint32_t>(s.laps) + 1u);
+        s.last_lap  = s.ticks - s.lap_start;
+        s.lap_start = s.ticks;
+    }
+    if (target > 0 && s.laps >= target)
+        s.completed = true;
+}
+
 // Phase 1 for agent `a` (one thread): optional auto-reset, kinematics from the action, standstill timeout
 // (Environment.cpp:128-143), lidar origin (CollisionChecker.cu:121-124).  Writes the agent's state buffers and
 // returns the record the ray and reward phases work from.
@@ -767,7 +816,10 @@ __device__ __forceinline__ float3 reset_pose(const float2 *pts, const float *hea
 // so phase 1 does not have to wait for the blob to be staged in shared memory.
 // kDraws: the auto-reset is a drawn reset (p.reset_flags != 0; the host launches this instantiation only then), so that the
 // kernels without draws stay what they were.
-template <bool kDraws = false>
+// kLaps: lap accounting is on (OkLaps): a completed agent is auto-reset too, and the record says whether the agent moves
+// (kFlagMoved) and whether it is still completed (kFlagCompleted).  Whether its auto-reset draws is decided here at run time
+// (p.reset_flags), so that one laps twin serves both kinds of tick.
+template <bool kDraws = false, bool kLaps = false>
 __device__ __forceinline__ AgentRec agent_pre(const StepParams &p, const uint8_t *gblob, const TrackRef &tr, const BeamView &bv, const int64_t a,
                                               const bool act_staged = false, const float2 *s_action = nullptr)
 {
@@ -776,7 +828,15 @@ __device__ __forceinline__ AgentRec agent_pre(const StepParams &p, const uint8_t
     // (auto-reset) the reset point is requested with the rest of the state, not after the crash flag has arrived
     const int32_t reset_pt0 = (p.auto_reset && p.do_move) ? p.reset_pt[a] : 0;
     // (drawn auto-reset) so is the agent's draw counter
-    const uint32_t k0 = kDraws ? p.reset_k[a] : 0u;
+    uint32_t k0 = kDraws ? p.reset_k[a] : 0u;
+    // (laps) and its completed flag, and the counter if this tick's auto-reset draws
+    bool completed = false;
+    if constexpr (kLaps)
+    {
+        completed = p.lap.completed[a] != 0;
+        if (p.reset_flags != 0)
+            k0 = p.reset_k[a];
+    }
     // the standstill record is read up front with the rest of the state: a load issued only after the kinematics
     // would add a second trip to memory to the latency of this (latency-bound) phase
     const uint32_t ss_ctr0 = p.ss_ctr[a];
@@ -845,11 +905,14 @@ __device__ __forceinline__ AgentRec agent_pre(const StepParams &p, const uint8_t
         // app-side reset of a crashed agent before the tick (GuidedCostLearning/test.cpp:102-111):
         // Environment::resetAgent + Agent::reset, Environment.cpp:103-121 / Agent.cpp:123-135.
         // prev / nearest / fitness are finalised in phase 4 (they need a centre-line search).
-        if (p.auto_reset && crashed)
+        bool reset = crashed;
+        if constexpr (kLaps)
+            reset = crashed || completed;
+        if (p.auto_reset && reset)
         {
             int32_t pt = static_cast<int32_t>((static_cast<int64_t>(reset_pt0) + p.auto_reset_stride) % tr.n_points);
-            if constexpr (kDraws)
-            { // the Philox rounds run here only, for the crashed agents
+            if (kDraws || (kLaps && p.reset_flags != 0))
+            { // the Philox rounds run here only, for the agents being reset
                 const ResetDraw d = reset_draw(p.reset_seed, p.reset_flags, p.id_base + static_cast<uint64_t>(a), k0, tr.n_points, pt);
                 pt                = d.pt;
                 const float3 q    = reset_pose(reinterpret_cast<const float2 *>(gblob + tr.off_points),
@@ -865,6 +928,8 @@ __device__ __forceinline__ AgentRec agent_pre(const StepParams &p, const uint8_t
             }
             accel = 0.0f, speed = 0.0f;
             crashed = false, timed_out = false;
+            if constexpr (kLaps)
+                completed = false;
             thr = 0.0f, steer = 0.0f; // Agent::reset zeroes current_action_
             rx = x, ry = y;
             flags |= kFlagReset;
@@ -879,6 +944,8 @@ __device__ __forceinline__ AgentRec agent_pre(const StepParams &p, const uint8_t
         p.act_steer[a] = steer;
         if (!crashed)
         {
+            if constexpr (kLaps)
+                flags |= kFlagMoved;
             rot = fadd(rot, steer);
             if (p.movement_mode == 1)
             { // moveViaAcceleration, Agent.cpp:82-98
@@ -931,6 +998,8 @@ __device__ __forceinline__ AgentRec agent_pre(const StepParams &p, const uint8_t
     rec.ox = o.x, rec.oy = o.y;
     rec.rc = rc, rec.rs = rs, rec.rot = rot, rec.x = x, rec.y = y, rec.rx = rx, rec.ry = ry;
     rec.min_d2_bits = __float_as_int(fmul(p.sensor_range, p.sensor_range));
+    if constexpr (kLaps)
+        flags |= completed ? kFlagCompleted : 0u;
     rec.flags       = flags | (crashed ? kFlagCrashed : 0u) | (timed_out ? kFlagTimedOut : 0u);
     OK_PROBE(4, rec.ox + rec.oy)
     rec.row         = beam_row(bv, rec.ox, rec.oy); // -1 when bv is not valid
@@ -942,12 +1011,13 @@ __device__ __forceinline__ AgentRec agent_pre(const StepParams &p, const uint8_t
 // Phase 4 for agent `a` (kPostLanes consecutive lanes per agent, they split the centre-line window; the WHOLE warp must
 // call this, lanes without an agent with valid = false):
 // crash flag (CollisionChecker.cu:167-171), nearest centre-line index, progress / reward / done.
-template <int kPostLanes>
+// kLaps: lap accounting (rule 2 of OkLaps) from the nearest index, which every reward mode then searches.
+template <int kPostLanes, bool kLaps = false>
 __device__ __forceinline__ void agent_post(const StepParams &p, const TrackView &tv, const AgentRec &rec, const int64_t a,
                                            const bool valid, const int lane)
 {
     const int  mode     = p.reward_mode;
-    const bool need_idx = p.do_move && (mode == 1 || mode == 2 || mode == 6 || mode == 7);
+    const bool need_idx = p.do_move && (kLaps || mode == 1 || mode == 2 || mode == 6 || mode == 7);
             const float    min_d2 = __int_as_float(rec.min_d2_bits);
     bool           crashed = (rec.flags & kFlagCrashed) != 0;
     const bool     timed_out = (rec.flags & kFlagTimedOut) != 0;
@@ -982,6 +1052,7 @@ __device__ __forceinline__ void agent_post(const StepParams &p, const TrackView 
     }
     if (want_reset)
         near = prev;
+    const int32_t reset_near = prev; // (laps) a reset's restart index; the reward modes below move prev on
     const bool want_near = valid && need_idx;
     bool       ok_near   = true;
     if (__any_sync(0xffffffffu, want_near))
@@ -1069,10 +1140,33 @@ __device__ __forceinline__ void agent_post(const StepParams &p, const TrackView 
             if (need_idx || (rec.flags & kFlagReset))
                 p.nearest[a] = near;
         }
+        bool done = crashed; // Agent::isDone, Agent.cpp:138-144 (without lap accounting completed_ is never set)
+        if constexpr (kLaps)
+        {
+            const OkLapBuffers &l = p.lap;
+            LapState            s;
+            s.completed = (rec.flags & kFlagCompleted) != 0;
+            if (rec.flags & kFlagReset)
+                s = LapState{reset_near, 0, 0, 0u, 0u, 0u, false}; // rule 1 (the auto-reset of this tick)
+            else if (rec.flags & kFlagMoved)
+                s = LapState{l.lap_idx[a], l.progress[a], l.laps[a], l.ticks[a], l.lap_start[a], l.last_lap[a], s.completed};
+            if (rec.flags & kFlagMoved) // a reset agent always moves
+            {
+                lap_advance(s, near, tv.n_pts, p.lap_target);
+                l.lap_idx[a]   = s.idx;
+                l.progress[a]  = s.progress;
+                l.laps[a]      = s.laps;
+                l.ticks[a]     = s.ticks;
+                l.lap_start[a] = s.lap_start;
+                l.last_lap[a]  = s.last_lap;
+                l.completed[a] = s.completed;
+            }
+            done = crashed || s.completed;
+        }
         p.crashed[a]   = crashed;
-        p.done[a]      = crashed; // Agent::isDone, Agent.cpp:138-144 (completed_ is never set)
+        p.done[a]      = done;
         if (p.host_done)
-            p.host_done[a] = crashed;
+            p.host_done[a] = done;
         p.min_dist2[a] = min_d2;
     }
 }

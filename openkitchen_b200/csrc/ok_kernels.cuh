@@ -10,7 +10,8 @@ namespace ok
 
 // Environment::resetAgent (Environment.cpp:79-122) + Agent::reset (Agent.cpp:123-135) of agent `a` with the draws
 // (pt, alpha, off) made explicit, and the episode bookkeeping (main_eigen.cpp:121-130: prev_track_idx_ = nearest index of the
-// post-reset pose, fitness restarts); the standstill record is not touched (Environment.cpp never resets it).
+// post-reset pose, fitness restarts) and the restart of the lap state (OkLaps, with accounting on or off); the standstill
+// record is not touched (Environment.cpp never resets it).
 __device__ __forceinline__ void reset_agent(const StepParams &p, const TrackView &tv, const int64_t a, const int32_t pt, const bool lane,
                                             const float alpha, const float off)
 {
@@ -33,6 +34,7 @@ __device__ __forceinline__ void reset_agent(const StepParams &p, const TrackView
     p.nearest[a]  = near;
     p.fitness[a]  = 0.0f;
     p.reward[a]   = 0.0f;
+    lap_restart(p.lap, a, near);
 }
 
 // ok_reset_agents: one thread per request, reading the track blobs from global memory.
@@ -81,6 +83,17 @@ __global__ void reset_drawn_kernel(const StepParams p, const DrawnResetParams r)
                                     min(kStartingIdx, tv.n_pts - 1));
     reset_agent(p, tv, a, d.pt, d.lane, d.alpha, d.off);
     p.reset_k[a] = k0 + 1u;
+}
+
+// ok_set_laps switching accounting on: the restart of every agent's lap state at its current pose, one thread per agent.
+__global__ void laps_restart_kernel(const StepParams p)
+{
+    const int64_t a = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (a >= p.n_agents)
+        return;
+    const TrackView tv = make_view(p.arena + p.tracks[p.track_id[a]].offset);
+    float           d2;
+    lap_restart(p.lap, a, nearest_index(tv, p.x[a], p.y[a], 0, 1, d2));
 }
 
 // GeneticAgent::updateAction + Network::infer for every agent (EvolutionaryRacer/GeneticAgent.hpp:37-50,

@@ -379,7 +379,7 @@ __device__ __forceinline__ int claim_tile(const StepParams &p, const bool single
 // =====================================================================================
 // phase 4 -- four lanes (small batches) or one thread per agent: crash flag, centre-line search, reward, done
 // =====================================================================================
-template <int kBlock>
+template <int kBlock, bool kLaps = false>
 __device__ __forceinline__ void post_tile(const StepParams &p, const TrackView &tv, const AgentRec *recs, const Tile &tl, const int tid)
 {
     const int lane = tid & 31, warp = tid >> 5;
@@ -389,19 +389,19 @@ __device__ __forceinline__ void post_tile(const StepParams &p, const TrackView &
         const int  al    = tid >> 2;
         const bool valid = al < count;
         if ((warp << 3) < count) // warp-uniform: this warp has at least one agent
-            agent_post<4>(p, tv, recs[valid ? al : 0], tl.begin + (valid ? al : 0), valid, lane);
+            agent_post<4, kLaps>(p, tv, recs[valid ? al : 0], tl.begin + (valid ? al : 0), valid, lane);
     }
     else if (count <= kBlock / 2)
     { // the balanced tiling's large tiles (about 450 agents at the bench workload): two lanes per agent
         const int  al    = tid >> 1;
         const bool valid = al < count;
         if ((warp << 4) < count)
-            agent_post<2>(p, tv, recs[valid ? al : 0], tl.begin + (valid ? al : 0), valid, lane);
+            agent_post<2, kLaps>(p, tv, recs[valid ? al : 0], tl.begin + (valid ? al : 0), valid, lane);
     }
     else if ((warp << 5) < count)
     {
         const bool valid = tid < count;
-        agent_post<1>(p, tv, recs[valid ? tid : 0], tl.begin + (valid ? tid : 0), valid, lane);
+        agent_post<1, kLaps>(p, tv, recs[valid ? tid : 0], tl.begin + (valid ? tid : 0), valid, lane);
     }
 }
 
@@ -423,10 +423,11 @@ __device__ __forceinline__ void rearm_scheduler(const StepParams &p, const bool 
 // The beam kernel.  kActor (ok_ppo_actor_step): the PPO racers' policy step runs as phase 0 of every tile -- the tile's
 // agents choose their actions from last tick's observations (actor_agent) and the kinematics read them from the action
 // buffers -- so that a rollout tick is ONE launch: at a few thousand agents a tick is latency, and two kernels pay it twice.
-// The body is beam_tick; beam_step_kernel and beam_step_drawn_kernel (below) are its two entry points.  kDraws: the
-// auto-reset is a drawn reset (agent_pre<true>), in a kernel of its own, so that the kernels without draws keep their
-// registers and schedule.
-template <bool kStaged, bool kActor, bool kDraws>
+// The body is beam_tick; beam_step_kernel, beam_step_drawn_kernel and beam_step_laps_kernel (below) are its entry points.
+// kDraws: the auto-reset is a drawn reset (agent_pre<true>), in a kernel of its own, so that the kernels without draws keep
+// their registers and schedule.  kLaps: lap accounting (OkLaps; agent_pre / agent_post with kLaps), likewise in a kernel
+// of its own.
+template <bool kStaged, bool kActor, bool kDraws, bool kLaps = false>
 __device__ __forceinline__ void beam_tick(const StepParams &p, const typename ActorArg<kActor>::type &q)
 {
     constexpr int kBlock   = beam_block(kStaged);
@@ -512,7 +513,7 @@ __device__ __forceinline__ void beam_tick(const StepParams &p, const typename Ac
             __syncthreads(); // the chosen actions are in shared memory: the agents' own threads read them next
         }
         if (tid < count)
-            recs[tid] = agent_pre<kDraws>(p, gblob, tr, bv, tl.begin + tid, n_done > 0 && s_actdev != 0, kActor ? s_actor_act + tid : nullptr);
+            recs[tid] = agent_pre<kDraws, kLaps>(p, gblob, tr, bv, tl.begin + tid, n_done > 0 && s_actdev != 0, kActor ? s_actor_act + tid : nullptr);
         if (tid == 0)
         {
             s_pool2 = 0, s_npend = 0, s_adone = 0;
@@ -854,7 +855,7 @@ __device__ __forceinline__ void beam_tick(const StepParams &p, const typename Ac
             atomicAdd(p.stats, static_cast<unsigned long long>(n_rays));
             atomicAdd(p.stats + 1, static_cast<unsigned long long>(s_npend));
         }
-        post_tile<kBlock>(p, tv, recs, tl, tid);
+        post_tile<kBlock, kLaps>(p, tv, recs, tl, tid);
         OK_TRACE(5); // thread 0's own phase 4 (the CTA-wide end is the next tile's start)
         if (p.tile_ns && tid == 0)
         {
@@ -882,6 +883,15 @@ __global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN
     beam_tick<kStaged, kActor, true>(p, q);
 }
 
+// the same tick with lap accounting (OkLaps): launched instead of the two above when accounting is on; its auto-reset
+// draws or not as p.reset_flags says
+template <bool kStaged, bool kActor = false>
+__global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN_CTAS)
+    beam_step_laps_kernel(const StepParams p, const typename ActorArg<kActor>::type q)
+{
+    beam_tick<kStaged, kActor, false, true>(p, q);
+}
+
 // ---------------------------------------------------------------------------------------------
 // the host's interface to the step kernels, one translation unit each (see the top of this file):
 //   launch_step_<unit>      launches the unit's kernel on `grid` CTAs with `smem_bytes` of dynamic shared memory
@@ -891,7 +901,9 @@ __global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN
 //   occupancy_step_<unit>   CTAs per SM at `smem_bytes` of dynamic shared memory
 //   violations_step_<unit>  the unit's self-check counter (OK_CHECKED builds; zero otherwise)
 // Every step kernel has a twin with the drawn auto-reset (OkResetDraws) in a unit of its own, <unit>_drawn, with the same
-// functions; the host launches it for the ticks whose auto-reset draws (StepParams::reset_flags != 0).
+// functions; the host launches it for the ticks whose auto-reset draws (StepParams::reset_flags != 0).  And every step
+// kernel has a twin with lap accounting (OkLaps), <unit>_laps, which the host launches for every moving tick while
+// accounting is on, whether its auto-reset draws or not.
 // ---------------------------------------------------------------------------------------------
 cudaError_t launch_step_staged(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
 cudaError_t arm_step_staged(int smem_optin, int *max_dynamic);
@@ -927,6 +939,18 @@ cudaError_t violations_step_actor_drawn(unsigned long long *count);
 cudaError_t launch_step_grid_drawn(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
 cudaError_t arm_step_grid_drawn(int smem_optin, int *max_dynamic);
 cudaError_t violations_step_grid_drawn(unsigned long long *count);
+
+cudaError_t launch_step_staged_laps(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
+cudaError_t arm_step_staged_laps(int smem_optin, int *max_dynamic);
+cudaError_t violations_step_staged_laps(unsigned long long *count);
+cudaError_t launch_step_unstaged_laps(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
+cudaError_t violations_step_unstaged_laps(unsigned long long *count);
+cudaError_t launch_step_actor_laps(const StepParams &p, const ActorParams &q, int grid, size_t smem_bytes, cudaStream_t stream);
+cudaError_t arm_step_actor_laps(int smem_optin, int *max_dynamic);
+cudaError_t violations_step_actor_laps(unsigned long long *count);
+cudaError_t launch_step_grid_laps(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
+cudaError_t arm_step_grid_laps(int smem_optin, int *max_dynamic);
+cudaError_t violations_step_grid_laps(unsigned long long *count);
 __host__ __device__ inline size_t batch_smem_bytes(int agents, int rays)
 { // the grid kernel's batch scratch: AgentRec + per ray float2 direction
     return static_cast<size_t>(agents) * (sizeof(AgentRec) + 8u * static_cast<size_t>(rays));

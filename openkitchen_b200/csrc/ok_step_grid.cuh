@@ -1,8 +1,8 @@
 // ok_step_grid.cuh -- the grid / brute-force step kernel's body (OK_RAYCAST_GRID, OK_RAYCAST_BRUTE): per-ray directions in
 // shared memory, rays pulled one by one from a CTA-wide pool and walked through the uniform grid (or tested against every
-// segment, the reference's loop), then one thread per ray for the outputs.  Its two kernels, grid_step_kernel and
-// grid_step_drawn_kernel (the auto-reset is a drawn reset), are in translation units of their own (ok_step_grid.cu,
-// ok_step_grid_drawn.cu).
+// segment, the reference's loop), then one thread per ray for the outputs.  Its three kernels, grid_step_kernel,
+// grid_step_drawn_kernel (the auto-reset is a drawn reset) and grid_step_laps_kernel (lap accounting), are in translation
+// units of their own (ok_step_grid.cu, ok_step_grid_drawn.cu, ok_step_grid_laps.cu).
 #pragma once
 
 #include "ok_step.cuh"
@@ -14,7 +14,7 @@ namespace ok
 #endif
 constexpr int kUnitsPerRefill = OK_UNITS; // units of work a lane does between two looks at the pool
 
-template <bool kDraws>
+template <bool kDraws, bool kLaps = false>
 __device__ __forceinline__ void grid_tick(const StepParams &p)
 {
     extern __shared__ __align__(128) uint8_t smem[];
@@ -67,7 +67,7 @@ __device__ __forceinline__ void grid_tick(const StepParams &p)
         // phase 1 -- one thread per agent: optional reset, kinematics, standstill (Environment.cpp:128-143)
         // =====================================================================================
         if (tid < count)
-            recs[tid] = agent_pre<kDraws>(p, gblob, tr, bv, tl.begin + tid);
+            recs[tid] = agent_pre<kDraws, kLaps>(p, gblob, tr, bv, tl.begin + tid);
         if (tid == 0)
             s_pool = 0;
         if (restage)
@@ -200,7 +200,7 @@ __device__ __forceinline__ void grid_tick(const StepParams &p)
         __syncthreads();
         if (tid == 0)
             s_tile = claim_tile(p, single_wave); // every thread read the old value long ago; visible after the loop-top barrier
-        post_tile<kGridBlock>(p, tv, recs, tl, tid);
+        post_tile<kGridBlock, kLaps>(p, tv, recs, tl, tid);
         ++n_done;
     }
     rearm_scheduler(p, single_wave, tid);

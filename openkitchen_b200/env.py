@@ -294,6 +294,29 @@ class Env:
         check(self.lib.ok_reset_draw_counts(self.h, C.byref(ptr)))
         return ptr.value, (self.n,), np.uint32
 
+    # ---- lap accounting (OkLaps: include/openkitchen_b200.h states the definition) -------
+    def set_laps(self, target: int = 0, enabled: bool = True, stream=None):
+        """Lap accounting on (or off with enabled=False): every moving tick adds the agent's signed centre-line progress,
+        counts laps of P points from where its episode started and their lengths in ticks, and with target > 0 sets the
+        agent's completed flag (and so done) at `target` laps; with auto_reset a completed agent is reset.  target 0 =
+        never complete.  Switching it on restarts every agent's lap state (asynchronous on `stream`)."""
+        target = int(target)
+        if target < 0:
+            raise ValueError("the lap target must be >= 0")
+        check(self.lib.ok_set_laps(self.h, C.byref(_capi.OkLaps(enabled=1 if enabled else 0, target=target)), stream))
+
+    def laps(self) -> dict:
+        """{"enabled", "target"} as set"""
+        l = _capi.OkLaps()
+        check(self.lib.ok_get_laps(self.h, C.byref(l)))
+        return {"enabled": bool(l.enabled), "target": int(l.target)}
+
+    def lap_buffers_info(self) -> dict:
+        """{field: (device pointer, shape, dtype)} of the seven lap arrays (OkLapBuffers), [agents] each"""
+        b = _capi.OkLapBuffers()
+        check(self.lib.ok_lap_buffers(self.h, C.byref(b)))
+        return {f: (getattr(b, f), (self.n,), np.dtype(dt).type) for f, dt in _capi.LAP_ARRAYS.items()}
+
     # ---- the tick -----------------------------------------------------------------------
     def cast_rays(self, stream=None):
         check(self.lib.ok_cast_rays(self.h, stream))

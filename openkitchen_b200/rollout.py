@@ -66,7 +66,8 @@ class GraphedRollout:
     After ``run()``: ``obs`` f32[T, N, R] (the state each action was chosen from), ``actions`` i64[T, N], ``log_prob``
     f32[T, N], ``rewards`` f32[T, N], ``dones`` u8[T, N] (after the tick).  With auto_reset and reset draws on
     (BatchEnv.set_reset_draws) the crashed agents restart at drawn points inside the graph, and each replay continues the
-    reset stream."""
+    reset stream.  With lap accounting on (BatchEnv.set_laps with a target) ``dones`` also marks the agents that completed
+    their laps in that tick, and auto_reset restarts them too."""
 
     def __init__(self, env: BatchEnv, policy: Callable[[torch.Tensor], torch.Tensor], action_table: torch.Tensor, steps: int,
                  sample: bool = True):
@@ -136,7 +137,8 @@ class FusedActorRollout:
 
     l1, l2: ``torch.nn.Linear`` modules (the reference's ``Actor::l1`` / ``l2``); their parameters are read in place,
     so an optimizer step between rollouts is picked up by the next replay.  After ``run()``: ``obs`` f32[T, N, R],
-    ``actions`` i32[T, N], ``log_prob`` f32[T, N], ``rewards`` f32[T, N], ``dones`` u8[T, N]."""
+    ``actions`` i32[T, N], ``log_prob`` f32[T, N], ``rewards`` f32[T, N], ``dones`` u8[T, N] (crashed, or with lap
+    accounting on (BatchEnv.set_laps) completed)."""
 
     def __init__(self, env: BatchEnv, l1: torch.nn.Linear, l2: torch.nn.Linear, action_table: torch.Tensor, steps: int,
                  sample: bool = True, seed: int = 0x0C17C4E2, one_launch: bool = True):
