@@ -543,22 +543,38 @@ int check_track_query(OkEnv *e, const float *x, const float *y, int64_t n)
     return OK_SUCCESS;
 }
 
-// cudaFuncAttributeMaxDynamicSharedMemorySize of the grid, staged and actor step kernels = everything the device allows.
-// Idempotent.
+// the step units (ok_step.cuh) by shape and variant, in the order of the two enums
+using ok::StepShape;
+using ok::StepUnitOf;
+using ok::StepVariant;
+constexpr const ok::StepUnit *kStepUnits[4][3] = {
+    {&StepUnitOf<StepShape::staged, StepVariant::plain>::unit, &StepUnitOf<StepShape::staged, StepVariant::drawn>::unit,
+     &StepUnitOf<StepShape::staged, StepVariant::laps>::unit},
+    {&StepUnitOf<StepShape::unstaged, StepVariant::plain>::unit, &StepUnitOf<StepShape::unstaged, StepVariant::drawn>::unit,
+     &StepUnitOf<StepShape::unstaged, StepVariant::laps>::unit},
+    {&StepUnitOf<StepShape::actor, StepVariant::plain>::unit, &StepUnitOf<StepShape::actor, StepVariant::drawn>::unit,
+     &StepUnitOf<StepShape::actor, StepVariant::laps>::unit},
+    {&StepUnitOf<StepShape::grid, StepVariant::plain>::unit, &StepUnitOf<StepShape::grid, StepVariant::drawn>::unit,
+     &StepUnitOf<StepShape::grid, StepVariant::laps>::unit},
+};
+const ok::StepUnit &step_unit_of(StepShape shape, StepVariant variant)
+{
+    return *kStepUnits[static_cast<int>(shape)][static_cast<int>(variant)];
+}
+
+// cudaFuncAttributeMaxDynamicSharedMemorySize of the grid, staged and actor step kernels = everything the device allows
+// (the unstaged kernels' few kilobytes of agent records need no opt-in).  Idempotent.
 int arm_shared_memory_limit(OkEnv *e)
 {
-    int max_dynamic = 0;
-    OK_CUDA(ok::arm_step_grid(e->smem_optin, &max_dynamic));
-    OK_CUDA(ok::arm_step_staged(e->smem_optin, &max_dynamic));
-    OK_CUDA(ok::arm_step_grid_drawn(e->smem_optin, &max_dynamic));
-    OK_CUDA(ok::arm_step_staged_drawn(e->smem_optin, &max_dynamic));
-    OK_CUDA(ok::arm_step_grid_laps(e->smem_optin, &max_dynamic));
-    OK_CUDA(ok::arm_step_staged_laps(e->smem_optin, &max_dynamic));
-    int drawn_dyn_max = 0, laps_dyn_max = 0; // the fused kernel's limit is what all three of its kernels allow
-    OK_CUDA(ok::arm_step_actor_drawn(e->smem_optin, &drawn_dyn_max));
-    OK_CUDA(ok::arm_step_actor_laps(e->smem_optin, &laps_dyn_max));
-    OK_CUDA(ok::arm_step_actor(e->smem_optin, &e->actor_dyn_max));
-    e->actor_dyn_max = std::min({e->actor_dyn_max, drawn_dyn_max, laps_dyn_max});
+    e->actor_dyn_max = e->smem_optin;
+    for (const StepShape shape : {StepShape::grid, StepShape::staged, StepShape::actor})
+        for (const ok::StepUnit *unit : kStepUnits[static_cast<int>(shape)])
+        {
+            int max_dynamic = 0;
+            OK_CUDA(ok::arm_dynamic_smem(unit->kernel, e->smem_optin, &max_dynamic));
+            if (shape == StepShape::actor) // the fused kernel's limit is what all three of its kernels allow
+                e->actor_dyn_max = std::min(e->actor_dyn_max, max_dynamic);
+        }
     return OK_SUCCESS;
 }
 
@@ -651,12 +667,17 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
         return rc;
     if (!(p.do_move && e->cfg.auto_reset))
         p.reset_flags = 0;
-    const bool drawn = p.reset_flags != 0; // the tick's auto-reset draws: the step kernels' twins with the drawn reset
-    // lap accounting on: the laps twins, which decide at run time whether the auto-reset draws (p.reset_flags)
-    const bool laps = p.do_move && e->laps.enabled;
+    // lap accounting on: the laps kernels, which decide at run time whether the auto-reset draws (p.reset_flags); else the
+    // drawn kernels when the tick's auto-reset draws
+    const StepVariant variant = p.do_move && e->laps.enabled ? StepVariant::laps
+                                : p.reset_flags != 0         ? StepVariant::drawn
+                                                             : StepVariant::plain;
     p.arena      = e->d_arena.get();
     p.tracks     = e->d_track_refs.get();
     Agents &ag   = e->ag;
+    StepShape shape      = StepShape::grid;
+    int       ctas       = ag.tiles.grid;
+    size_t    smem_bytes = ag.sizing.smem;
     if (e->cfg.raycast_mode == OK_RAYCAST_BEAM)
     {
         const bool e2e = (p.host_obs || p.host_obs_q16) && ag.e2e.d;
@@ -710,15 +731,14 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
         if (actor)
         { // the policy step as phase 0 of every tile (ok_ppo_actor_step): its weights sit behind the kernel's own shared memory
             p.actor_smem_off = static_cast<uint32_t>((ag.sizing.smem_beam + 15) & ~static_cast<size_t>(15));
-            OK_CUDA((laps ? ok::launch_step_actor_laps : drawn ? ok::launch_step_actor_drawn : ok::launch_step_actor)(p, *actor, ag.beam.grid, p.actor_smem_off + actor_smem, s));
+            shape = StepShape::actor, ctas = ag.beam.grid, smem_bytes = p.actor_smem_off + actor_smem;
         }
         else if (ag.sizing.beam_staged)
-            OK_CUDA((laps ? ok::launch_step_staged_laps : drawn ? ok::launch_step_staged_drawn : ok::launch_step_staged)(p, grid, ag.sizing.smem_beam, s));
+            shape = StepShape::staged, ctas = grid, smem_bytes = ag.sizing.smem_beam;
         else
-            OK_CUDA((laps ? ok::launch_step_unstaged_laps : drawn ? ok::launch_step_unstaged_drawn : ok::launch_step_unstaged)(p, ag.beam.grid, ag.sizing.smem_beam, s));
+            shape = StepShape::unstaged, ctas = ag.beam.grid, smem_bytes = ag.sizing.smem_beam;
     }
-    else
-        OK_CUDA((laps ? ok::launch_step_grid_laps : drawn ? ok::launch_step_grid_drawn : ok::launch_step_grid)(p, ag.tiles.grid, ag.sizing.smem, s));
+    OK_CUDA(step_unit_of(shape, variant).launch(p, actor, ctas, smem_bytes, s));
     if (p.act_ready)
     { // enqueued AFTER the launch: the kernel is already running its first tiles while the host issues these
         const size_t bytes = sizeof(float) * static_cast<size_t>(e->n_agents);
@@ -1108,7 +1128,8 @@ int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg,
     {
         int per_sm = 1;
         if (!ag.sizing.beam_staged)
-            OK_CUDA(ok::occupancy_step_unstaged(ag.sizing.smem_beam, &per_sm));
+            OK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, step_unit_of(StepShape::unstaged, StepVariant::plain).kernel,
+                                                                  ok::kBeamBlockUnstaged, ag.sizing.smem_beam));
         ag.sizing.ctas_per_sm_beam = std::max(1, per_sm);
     }
     ok::PopulationTilings tilings = ok::tile_population(e->h_track_id.data(), n, ag.sizing, e->num_sms, knobs);
@@ -2120,26 +2141,19 @@ int ok_debug_violations(OkEnv *e, uint64_t *count, int32_t *checks_compiled_in)
         return fail(OK_ERR_NO_DEVICE, "no device");
     DeviceGuard g(e->cfg.device);
     OK_CUDA(cudaDeviceSynchronize());
-    unsigned long long staged = 0, unstaged = 0, actor = 0, grid = 0, lidar = 0, bev = 0;
-    unsigned long long staged_d = 0, unstaged_d = 0, actor_d = 0, grid_d = 0; // the step kernels with drawn resets
-    unsigned long long staged_l = 0, unstaged_l = 0, actor_l = 0, grid_l = 0; // ... with lap accounting
-    OK_CUDA(ok::violations_step_staged(&staged));
-    OK_CUDA(ok::violations_step_unstaged(&unstaged));
-    OK_CUDA(ok::violations_step_actor(&actor));
-    OK_CUDA(ok::violations_step_grid(&grid));
-    OK_CUDA(ok::violations_step_staged_drawn(&staged_d));
-    OK_CUDA(ok::violations_step_unstaged_drawn(&unstaged_d));
-    OK_CUDA(ok::violations_step_actor_drawn(&actor_d));
-    OK_CUDA(ok::violations_step_grid_drawn(&grid_d));
-    OK_CUDA(ok::violations_step_staged_laps(&staged_l));
-    OK_CUDA(ok::violations_step_unstaged_laps(&unstaged_l));
-    OK_CUDA(ok::violations_step_actor_laps(&actor_l));
-    OK_CUDA(ok::violations_step_grid_laps(&grid_l));
-    OK_CUDA(ok::violations_lidar_query(&lidar));
-    OK_CUDA(ok::violations_bev(&bev));
+    unsigned long long total = 0, n = 0;
+    for (const auto &units : kStepUnits)
+        for (const ok::StepUnit *unit : units)
+        {
+            OK_CUDA(unit->violations(&n));
+            total += n;
+        }
+    OK_CUDA(ok::violations_lidar_query(&n));
+    total += n;
+    OK_CUDA(ok::violations_bev(&n));
+    total += n;
     if (count)
-        *count = staged + unstaged + actor + grid + staged_d + unstaged_d + actor_d + grid_d + staged_l + unstaged_l + actor_l + grid_l +
-                 lidar + bev;
+        *count = total;
     if (checks_compiled_in)
         *checks_compiled_in = OK_CHECKED;
     return OK_SUCCESS;

@@ -18,13 +18,13 @@
 //     shared memory;
 //   * the rays: beam_step_kernel reads precomputed candidate lists (ok_beam.hpp) -- warps pull groups of 32 rays, a ray's
 //     first chunk of candidates is tested by its own lane, the rest is dealt evenly over the warp, results meet in a
-//     64-bit atomicMin key per ray; grid_step_kernel (ok_step_grid.cu) walks a uniform grid ray by ray from a CTA-wide
+//     64-bit atomicMin key per ray; grid_step_kernel (ok_step_grid.cuh) walks a uniform grid ray by ray from a CTA-wide
 //     pool (or tests every segment: the reference's loop);
 //   * state is structure-of-arrays; per-ray outputs are written coalesced (lane = ray).
 // The path is warp-issue bound, not HBM bound, and is not a contraction: no tensor cores (DESIGN.md section 4).
 //
-// Every step kernel is compiled in a translation unit of its own (ok_step_staged.cu, ok_step_unstaged.cu,
-// ok_step_actor.cu, ok_step_grid.cu; tests/test_step_units_cpu.py checks it): with two of them in one unit ptxas shares
+// Every step kernel, one per shape (StepShape) and variant (StepVariant), is compiled in a translation unit of its own,
+// ok_step_<shape>[_<variant>].cu (tests/test_step_units_cpu.py checks it): with two of them in one unit ptxas shares
 // the out-of-line device functions (beam_literal_key, beam_walk_fallback) between kernels with different launch bounds
 // and address spaces, and the staged kernel lost a third of its speed (0.139 vs 0.095 ms per tick, DESIGN.md section 7).
 #pragma once
@@ -317,6 +317,19 @@ __device__ __forceinline__ unsigned long long global_timer()
             p.trace[(static_cast<size_t>(blockIdx.x) * p.trace_tiles + n_done) * 6 + (slot)] = global_timer();         \
     } while (0)
 
+// What a step kernel does besides the plain tick; every variant is a kernel of its own, so that the plain kernels keep
+// their registers and schedule:
+//   drawn  the auto-reset is a drawn reset (OkResetDraws; agent_pre with kDraws), launched for a tick whose auto-reset
+//          draws (StepParams::reset_flags != 0);
+//   laps   lap accounting (OkLaps; agent_pre / agent_post with kLaps), launched for every moving tick while accounting is
+//          on; its auto-reset draws or not as p.reset_flags says.
+enum class StepVariant
+{
+    plain,
+    drawn,
+    laps
+};
+
 // the second kernel argument of beam_step_kernel: the actor's parameters in the fused instantiation (kActor), nothing otherwise
 struct NoActor
 {
@@ -423,13 +436,13 @@ __device__ __forceinline__ void rearm_scheduler(const StepParams &p, const bool 
 // The beam kernel.  kActor (ok_ppo_actor_step): the PPO racers' policy step runs as phase 0 of every tile -- the tile's
 // agents choose their actions from last tick's observations (actor_agent) and the kinematics read them from the action
 // buffers -- so that a rollout tick is ONE launch: at a few thousand agents a tick is latency, and two kernels pay it twice.
-// The body is beam_tick; beam_step_kernel, beam_step_drawn_kernel and beam_step_laps_kernel (below) are its entry points.
-// kDraws: the auto-reset is a drawn reset (agent_pre<true>), in a kernel of its own, so that the kernels without draws keep
-// their registers and schedule.  kLaps: lap accounting (OkLaps; agent_pre / agent_post with kLaps), likewise in a kernel
-// of its own.
-template <bool kStaged, bool kActor, bool kDraws, bool kLaps = false>
+// The body is beam_tick; beam_step_kernel (below) is its entry point.  kVariant (StepVariant) selects what agent_pre /
+// agent_post do besides the plain tick.
+template <bool kStaged, bool kActor, StepVariant kVariant>
 __device__ __forceinline__ void beam_tick(const StepParams &p, const typename ActorArg<kActor>::type &q)
 {
+    constexpr bool kDraws  = kVariant == StepVariant::drawn;
+    constexpr bool kLaps   = kVariant == StepVariant::laps;
     constexpr int kBlock   = beam_block(kStaged);
     constexpr int kPendCap = beam_pend_cap(kStaged);
     extern __shared__ __align__(128) uint8_t smem[];
@@ -868,94 +881,71 @@ __device__ __forceinline__ void beam_tick(const StepParams &p, const typename Ac
     rearm_scheduler(p, single_wave, tid);
 }
 
-template <bool kStaged, bool kActor = false>
+template <bool kStaged, bool kActor, StepVariant kVariant>
 __global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN_CTAS)
     beam_step_kernel(const StepParams p, const typename ActorArg<kActor>::type q)
 {
-    beam_tick<kStaged, kActor, false>(p, q);
+    beam_tick<kStaged, kActor, kVariant>(p, q);
 }
 
-// the same tick with the drawn auto-reset (OkResetDraws): launched instead of beam_step_kernel when p.reset_flags != 0
-template <bool kStaged, bool kActor = false>
-__global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN_CTAS)
-    beam_step_drawn_kernel(const StepParams p, const typename ActorArg<kActor>::type q)
-{
-    beam_tick<kStaged, kActor, true>(p, q);
-}
-
-// the same tick with lap accounting (OkLaps): launched instead of the two above when accounting is on; its auto-reset
-// draws or not as p.reset_flags says
-template <bool kStaged, bool kActor = false>
-__global__ void __launch_bounds__(beam_block(kStaged), kStaged ? 1 : OK_BEAM_MIN_CTAS)
-    beam_step_laps_kernel(const StepParams p, const typename ActorArg<kActor>::type q)
-{
-    beam_tick<kStaged, kActor, false, true>(p, q);
-}
-
-// ---------------------------------------------------------------------------------------------
-// the host's interface to the step kernels, one translation unit each (see the top of this file):
-//   launch_step_<unit>      launches the unit's kernel on `grid` CTAs with `smem_bytes` of dynamic shared memory
-//   arm_step_<unit>         sets the kernel's cudaFuncAttributeMaxDynamicSharedMemorySize to everything the device allows
-//                           (an attribute of the function, not of the env); *max_dynamic = smem_optin less the kernel's
-//                           static shared memory
-//   occupancy_step_<unit>   CTAs per SM at `smem_bytes` of dynamic shared memory
-//   violations_step_<unit>  the unit's self-check counter (OK_CHECKED builds; zero otherwise)
-// Every step kernel has a twin with the drawn auto-reset (OkResetDraws) in a unit of its own, <unit>_drawn, with the same
-// functions; the host launches it for the ticks whose auto-reset draws (StepParams::reset_flags != 0).  And every step
-// kernel has a twin with lap accounting (OkLaps), <unit>_laps, which the host launches for every moving tick while
-// accounting is on, whether its auto-reset draws or not.
-// ---------------------------------------------------------------------------------------------
-cudaError_t launch_step_staged(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
-cudaError_t arm_step_staged(int smem_optin, int *max_dynamic);
-cudaError_t violations_step_staged(unsigned long long *count);
-
-cudaError_t launch_step_unstaged(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
-cudaError_t occupancy_step_unstaged(size_t smem_bytes, int *ctas_per_sm);
-cudaError_t violations_step_unstaged(unsigned long long *count);
-
-// the unstaged beam kernel with the policy step fused in
-cudaError_t launch_step_actor(const StepParams &p, const ActorParams &q, int grid, size_t smem_bytes, cudaStream_t stream);
-cudaError_t arm_step_actor(int smem_optin, int *max_dynamic);
-cudaError_t violations_step_actor(unsigned long long *count);
-
-// the grid / brute-force kernel (OK_RAYCAST_GRID, OK_RAYCAST_BRUTE), kGridBlock threads per CTA; its dynamic shared
-// memory is the staged track and batch_smem_bytes
+// the grid / brute-force kernel (OK_RAYCAST_GRID, OK_RAYCAST_BRUTE; ok_step_grid.cuh), kGridBlock threads per CTA; its
+// dynamic shared memory is the staged track and batch_smem_bytes
 #ifndef OK_BLOCK
 #define OK_BLOCK 1024
 #endif
 constexpr int kGridBlock = OK_BLOCK;
-cudaError_t launch_step_grid(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
-cudaError_t arm_step_grid(int smem_optin, int *max_dynamic);
-cudaError_t violations_step_grid(unsigned long long *count);
-
-cudaError_t launch_step_staged_drawn(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
-cudaError_t arm_step_staged_drawn(int smem_optin, int *max_dynamic);
-cudaError_t violations_step_staged_drawn(unsigned long long *count);
-cudaError_t launch_step_unstaged_drawn(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
-cudaError_t violations_step_unstaged_drawn(unsigned long long *count);
-cudaError_t launch_step_actor_drawn(const StepParams &p, const ActorParams &q, int grid, size_t smem_bytes, cudaStream_t stream);
-cudaError_t arm_step_actor_drawn(int smem_optin, int *max_dynamic);
-cudaError_t violations_step_actor_drawn(unsigned long long *count);
-cudaError_t launch_step_grid_drawn(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
-cudaError_t arm_step_grid_drawn(int smem_optin, int *max_dynamic);
-cudaError_t violations_step_grid_drawn(unsigned long long *count);
-
-cudaError_t launch_step_staged_laps(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
-cudaError_t arm_step_staged_laps(int smem_optin, int *max_dynamic);
-cudaError_t violations_step_staged_laps(unsigned long long *count);
-cudaError_t launch_step_unstaged_laps(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
-cudaError_t violations_step_unstaged_laps(unsigned long long *count);
-cudaError_t launch_step_actor_laps(const StepParams &p, const ActorParams &q, int grid, size_t smem_bytes, cudaStream_t stream);
-cudaError_t arm_step_actor_laps(int smem_optin, int *max_dynamic);
-cudaError_t violations_step_actor_laps(unsigned long long *count);
-cudaError_t launch_step_grid_laps(const StepParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
-cudaError_t arm_step_grid_laps(int smem_optin, int *max_dynamic);
-cudaError_t violations_step_grid_laps(unsigned long long *count);
 __host__ __device__ inline size_t batch_smem_bytes(int agents, int rays)
 { // the grid kernel's batch scratch: AgentRec + per ray float2 direction
     return static_cast<size_t>(agents) * (sizeof(AgentRec) + 8u * static_cast<size_t>(rays));
 }
-// what arm_step_<unit> does for `kernel`
+
+// ---------------------------------------------------------------------------------------------
+// the host's interface to the step kernels: one StepUnit record per translation unit (see the top of this file), which
+// defines StepUnitOf<shape, variant>::unit with beam_step_unit or grid_step_unit
+// ---------------------------------------------------------------------------------------------
+enum class StepShape
+{
+    staged,   // the staged beam kernel
+    unstaged, // the unstaged beam kernel
+    actor,    // the unstaged beam kernel with the policy step fused in
+    grid      // the grid / brute-force kernel
+};
+struct StepUnit
+{
+    // launches the unit's kernel on `grid` CTAs with `smem_bytes` of dynamic shared memory; `q` is read by the actor shape only
+    cudaError_t (*launch)(const StepParams &p, const ActorParams *q, int grid, size_t smem_bytes, cudaStream_t stream);
+    const void *kernel; // the kernel's host stub: arm_dynamic_smem, occupancy queries
+    cudaError_t (*violations)(unsigned long long *count); // the unit's self-check counter (OK_CHECKED builds; zero otherwise)
+};
+template <StepShape kShape, StepVariant kVariant> struct StepUnitOf
+{
+    static const StepUnit unit;
+};
+
+// the self-check counter of the translation unit that takes this function's address (g_violations is static: one per unit)
+static inline cudaError_t unit_violations(unsigned long long *count)
+{
+    return cudaMemcpyFromSymbol(count, g_violations, sizeof *count);
+}
+
+template <bool kStaged, bool kActor, StepVariant kVariant>
+cudaError_t launch_beam_step(const StepParams &p, const ActorParams *q, int grid, size_t smem_bytes, cudaStream_t stream)
+{
+    if constexpr (kActor)
+        beam_step_kernel<kStaged, kActor, kVariant><<<grid, beam_block(kStaged), smem_bytes, stream>>>(p, *q);
+    else
+        beam_step_kernel<kStaged, kActor, kVariant><<<grid, beam_block(kStaged), smem_bytes, stream>>>(p, NoActor{});
+    return cudaGetLastError();
+}
+// the record of a beam unit; static, so that it takes the address of its own unit's unit_violations
+template <bool kStaged, bool kActor, StepVariant kVariant> static StepUnit beam_step_unit()
+{
+    return {launch_beam_step<kStaged, kActor, kVariant>, reinterpret_cast<const void *>(beam_step_kernel<kStaged, kActor, kVariant>),
+            unit_violations};
+}
+
+// sets `kernel`'s cudaFuncAttributeMaxDynamicSharedMemorySize to everything the device allows (an attribute of the
+// function, not of the env); *max_dynamic = smem_optin less the kernel's static shared memory
 inline cudaError_t arm_dynamic_smem(const void *kernel, int smem_optin, int *max_dynamic)
 {
     cudaFuncAttributes fa{};

@@ -6,19 +6,5 @@
 
 namespace ok
 {
-cudaError_t launch_step_actor(const StepParams &p, const ActorParams &q, int grid, size_t smem_bytes, cudaStream_t stream)
-{
-    beam_step_kernel<false, true><<<grid, kBeamBlockUnstaged, smem_bytes, stream>>>(p, q);
-    return cudaGetLastError();
-}
-
-cudaError_t arm_step_actor(int smem_optin, int *max_dynamic)
-{
-    return arm_dynamic_smem(reinterpret_cast<const void *>(beam_step_kernel<false, true>), smem_optin, max_dynamic);
-}
-
-cudaError_t violations_step_actor(unsigned long long *count)
-{
-    return cudaMemcpyFromSymbol(count, g_violations, sizeof *count);
-}
+template <> const StepUnit StepUnitOf<StepShape::actor, StepVariant::plain>::unit = beam_step_unit<false, true, StepVariant::plain>();
 } // namespace ok

@@ -1,23 +1,7 @@
-// ok_step_actor_drawn.cu -- the unstaged beam kernel with the policy step fused in (ok_step_actor.cu) with the drawn
-// auto-reset (OkResetDraws; agent_pre<true>), in a translation unit of its own like every step kernel.  The host
-// launches it instead of the kernel without draws for a tick whose auto-reset draws.
+// ok_step_actor_drawn.cu -- the kernel of ok_step_actor.cu with the drawn auto-reset (StepVariant::drawn).
 #include "ok_step.cuh"
 
 namespace ok
 {
-cudaError_t launch_step_actor_drawn(const StepParams &p, const ActorParams &q, int grid, size_t smem_bytes, cudaStream_t stream)
-{
-    beam_step_drawn_kernel<false, true><<<grid, kBeamBlockUnstaged, smem_bytes, stream>>>(p, q);
-    return cudaGetLastError();
-}
-
-cudaError_t arm_step_actor_drawn(int smem_optin, int *max_dynamic)
-{
-    return arm_dynamic_smem(reinterpret_cast<const void *>(beam_step_drawn_kernel<false, true>), smem_optin, max_dynamic);
-}
-
-cudaError_t violations_step_actor_drawn(unsigned long long *count)
-{
-    return cudaMemcpyFromSymbol(count, g_violations, sizeof *count);
-}
+template <> const StepUnit StepUnitOf<StepShape::actor, StepVariant::drawn>::unit = beam_step_unit<false, true, StepVariant::drawn>();
 } // namespace ok

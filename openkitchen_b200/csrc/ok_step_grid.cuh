@@ -1,8 +1,8 @@
 // ok_step_grid.cuh -- the grid / brute-force step kernel's body (OK_RAYCAST_GRID, OK_RAYCAST_BRUTE): per-ray directions in
 // shared memory, rays pulled one by one from a CTA-wide pool and walked through the uniform grid (or tested against every
-// segment, the reference's loop), then one thread per ray for the outputs.  Its three kernels, grid_step_kernel,
-// grid_step_drawn_kernel (the auto-reset is a drawn reset) and grid_step_laps_kernel (lap accounting), are in translation
-// units of their own (ok_step_grid.cu, ok_step_grid_drawn.cu, ok_step_grid_laps.cu).
+// segment, the reference's loop), then one thread per ray for the outputs.  Its kernel, grid_step_kernel<StepVariant>, is
+// instantiated once per variant, each in a translation unit of its own (ok_step_grid.cu, ok_step_grid_drawn.cu,
+// ok_step_grid_laps.cu).
 #pragma once
 
 #include "ok_step.cuh"
@@ -14,9 +14,11 @@ namespace ok
 #endif
 constexpr int kUnitsPerRefill = OK_UNITS; // units of work a lane does between two looks at the pool
 
-template <bool kDraws, bool kLaps = false>
+template <StepVariant kVariant>
 __device__ __forceinline__ void grid_tick(const StepParams &p)
 {
+    constexpr bool kDraws = kVariant == StepVariant::drawn;
+    constexpr bool kLaps  = kVariant == StepVariant::laps;
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ uint16_t                      s_order[1024]; // pool order of the rays (p.ray_order)
     __shared__ __align__(8) uint64_t         bar;
@@ -204,5 +206,22 @@ __device__ __forceinline__ void grid_tick(const StepParams &p)
         ++n_done;
     }
     rearm_scheduler(p, single_wave, tid);
+}
+
+template <StepVariant kVariant> __global__ void __launch_bounds__(kGridBlock, 1) grid_step_kernel(const StepParams p)
+{
+    grid_tick<kVariant>(p);
+}
+
+template <StepVariant kVariant>
+cudaError_t launch_grid_step(const StepParams &p, const ActorParams *, int grid, size_t smem_bytes, cudaStream_t stream)
+{
+    grid_step_kernel<kVariant><<<grid, kGridBlock, smem_bytes, stream>>>(p);
+    return cudaGetLastError();
+}
+// the record of a grid unit; static, so that it takes the address of its own unit's unit_violations
+template <StepVariant kVariant> static StepUnit grid_step_unit()
+{
+    return {launch_grid_step<kVariant>, reinterpret_cast<const void *>(grid_step_kernel<kVariant>), unit_violations};
 }
 } // namespace ok

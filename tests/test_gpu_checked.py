@@ -6,18 +6,30 @@ import pytest
 import torch
 
 import openkitchen_b200 as ok
+from openkitchen_b200.dlpack import DeviceBuffer
 from openkitchen_b200.rollout import FusedActorRollout
 
 pytestmark = pytest.mark.gpu
 
 
+def _sum_u32(env, name, info) -> int:
+    return int(torch.from_dlpack(DeviceBuffer(env, name, info)).view(torch.int32).to(torch.int64).sum())
+
+
 def test_no_index_leaves_its_array():
     names = ["Spa", "Monza", "Sepang", "Austin", "Oschersleben"]
-    for n, offset in ((2560, 0.0), (2304, 4.0), (160, -3.0)):  # staged kernel, with sensor offset, unstaged kernel
+    # staged kernel, with sensor offset, unstaged kernel; the unstaged kernel with drawn resets and the staged kernel with
+    # lap accounting (each variant is a kernel of its own, with its own counter)
+    for n, offset, variant in ((2560, 0.0, "plain"), (2304, 4.0, "plain"), (160, -3.0, "plain"), (160, 0.0, "drawn"),
+                               (2560, 0.0, "laps")):
         env = ok.Env(device=0, reward_mode=ok.REWARD_CMAES_PROGRESS, auto_reset=1, sensor_offset=offset)
         for nm in names:
             env.add_named_track(nm)
         env.alloc_agents(n, ok.ray_fan(32), (np.arange(n) * len(names) // n).astype(np.int32))
+        if variant == "drawn":
+            env.set_reset_draws(0x5EED, point=True, lane=True, heading=True)
+        elif variant == "laps":
+            env.set_laps(1)
         env.launch_steps_random(0, 60)
         # poses far outside the lane and non-finite ones take the uncovered / grid-walk paths
         x = env.read("pos_x")
@@ -26,6 +38,11 @@ def test_no_index_leaves_its_array():
         env.write("pos_x", x)
         env.write("crashed", np.zeros(n, dtype=np.uint8))
         env.launch_steps_random(60, 5)
+        env.sync()
+        if variant == "drawn":  # the drawn auto-reset ran
+            assert _sum_u32(env, "k", env.reset_draw_counts_info()) > 0
+        elif variant == "laps":  # the accounting ran
+            assert _sum_u32(env, "ticks", env.lap_buffers_info()["ticks"]) > 0
         count, compiled_in = env.debug_violations()
         assert count == 0, f"{count} out-of-range indices"
         env.close()

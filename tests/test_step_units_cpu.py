@@ -14,19 +14,30 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "openkitchen_b200", "lib", "libopenkitchen_b200.so")
 CUOBJDUMP = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
 
-# mangled name -> (unit, stack frame limit in bytes or None).  The limits are the stack frames of the beam kernels when
-# they were split into these units (CUDA 12.9): a kernel change that moves them is to update them on purpose.
+# mangled name -> (unit, stack frame limit in bytes).  The limits are the stack frames the kernels are built with (CUDA
+# 12.9): a kernel change that moves them is to update them on purpose.  The last template argument is the StepVariant:
+# 0 plain, 1 drawn, 2 laps.
 EXPECTED = {
-    "_ZN2ok16beam_step_kernelILb1ELb0EEEvNS_10StepParamsENS_8ActorArgIXT0_EE4typeE": ("ok_step_staged.cu", 56),
-    "_ZN2ok16beam_step_kernelILb0ELb0EEEvNS_10StepParamsENS_8ActorArgIXT0_EE4typeE": ("ok_step_unstaged.cu", 56),
-    "_ZN2ok16beam_step_kernelILb0ELb1EEEvNS_10StepParamsENS_8ActorArgIXT0_EE4typeE": ("ok_step_actor.cu", 80),
-    "_ZN2ok16grid_step_kernelENS_10StepParamsE": ("ok_step_grid.cu", None),
+    "_ZN2ok16beam_step_kernelILb1ELb0ELNS_11StepVariantE0EEEvNS_10StepParamsENS_8ActorArgIXT0_EE4typeE": ("ok_step_staged.cu", 56),
+    "_ZN2ok16beam_step_kernelILb0ELb0ELNS_11StepVariantE0EEEvNS_10StepParamsENS_8ActorArgIXT0_EE4typeE": ("ok_step_unstaged.cu", 56),
+    "_ZN2ok16beam_step_kernelILb0ELb1ELNS_11StepVariantE0EEEvNS_10StepParamsENS_8ActorArgIXT0_EE4typeE": ("ok_step_actor.cu", 80),
+    "_ZN2ok16grid_step_kernelILNS_11StepVariantE0EEEvNS_10StepParamsE": ("ok_step_grid.cu", 0),
+    "_ZN2ok16beam_step_kernelILb1ELb0ELNS_11StepVariantE1EEEvNS_10StepParamsENS_8ActorArgIXT0_EE4typeE": ("ok_step_staged_drawn.cu", 56),
+    "_ZN2ok16beam_step_kernelILb0ELb0ELNS_11StepVariantE1EEEvNS_10StepParamsENS_8ActorArgIXT0_EE4typeE": ("ok_step_unstaged_drawn.cu", 56),
+    "_ZN2ok16beam_step_kernelILb0ELb1ELNS_11StepVariantE1EEEvNS_10StepParamsENS_8ActorArgIXT0_EE4typeE": ("ok_step_actor_drawn.cu", 80),
+    "_ZN2ok16grid_step_kernelILNS_11StepVariantE1EEEvNS_10StepParamsE": ("ok_step_grid_drawn.cu", 0),
+    "_ZN2ok16beam_step_kernelILb1ELb0ELNS_11StepVariantE2EEEvNS_10StepParamsENS_8ActorArgIXT0_EE4typeE": ("ok_step_staged_laps.cu", 136),
+    "_ZN2ok16beam_step_kernelILb0ELb0ELNS_11StepVariantE2EEEvNS_10StepParamsENS_8ActorArgIXT0_EE4typeE": ("ok_step_unstaged_laps.cu", 120),
+    "_ZN2ok16beam_step_kernelILb0ELb1ELNS_11StepVariantE2EEEvNS_10StepParamsENS_8ActorArgIXT0_EE4typeE": ("ok_step_actor_laps.cu", 160),
+    "_ZN2ok16grid_step_kernelILNS_11StepVariantE2EEEvNS_10StepParamsE": ("ok_step_grid_laps.cu", 40),
 }
+# demangled: ok::beam_step_kernel<...> and ok::grid_step_kernel<...>, every __global__ step kernel
+STEP_KERNEL_PREFIXES = ("_ZN2ok16beam_step_kernelI", "_ZN2ok16grid_step_kernelI")
 
 
 @functools.cache
 def _step_kernels():
-    """{unit: {function: (registers, stack bytes)}} of every function whose name contains step_kernel"""
+    """{unit: {function: (registers, stack bytes)}} of every step kernel"""
     if not os.path.exists(CUOBJDUMP):
         pytest.skip("cuobjdump not found")
     if not os.path.exists(LIB):
@@ -39,7 +50,7 @@ def _step_kernels():
         elif m := re.match(r"Function (\S+):$", line.strip()):
             fn = m.group(1)
         elif fn and (m := re.search(r"REG:(\d+) STACK:(\d+)", line)):
-            if "step_kernel" in fn:
+            if fn.startswith(STEP_KERNEL_PREFIXES):
                 units.setdefault(unit, {})[fn] = (int(m.group(1)), int(m.group(2)))
             fn = None
     return units
@@ -53,11 +64,9 @@ def test_one_step_kernel_per_unit():
     assert found == {fn: unit for fn, (unit, _) in EXPECTED.items()}
 
 
-def test_beam_kernels_keep_their_registers_and_stack():
+def test_step_kernels_keep_their_registers_and_stack():
     units = _step_kernels()
     for fn, (unit, stack_limit) in EXPECTED.items():
-        if stack_limit is None:
-            continue
         regs, stack = units[unit][fn]
         assert regs <= 64, f"{unit}: {regs} registers"
         assert stack <= stack_limit, f"{unit}: {stack}-byte stack frame, was {stack_limit}"
