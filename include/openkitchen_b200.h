@@ -286,6 +286,59 @@ typedef struct OkLapBuffers {
  * state) */
 int ok_lap_buffers(OkEnv *env, OkLapBuffers *out);
 
+/* Races: the cars of a group see each other in the lidar and crash on contact, in a pass after the tick.  The reference's
+ * co-located agents never see each other; races depart from it on purpose, and only while they are on.
+ *   - GROUPS.  Agent a (local index) belongs to race a / group: consecutive agents, the last race may be short.  Every agent
+ *     is a car body, a disc of radius `radius` around (pos_x, pos_y), crashed or not.  Agent j is an OPPONENT of agent i when
+ *     they are in the same race, on the same track_id, and j != i: cars on different tracks never meet.  For a sharded
+ *     population, a shard's races equal the unsharded ones when its first agent (OkConfig::agent_id_base) is a multiple of
+ *     `group`.
+ *   - THE PASS runs after the step kernel of every call that casts the agents' rays: ok_cast_rays, ok_launch_step, every tick
+ *     of ok_launch_steps_random and ok_ppo_actor_step (fused or as two launches), on the same stream.  It reads the tick's
+ *     outputs and the poses.  Every agent i whose crashed flag is clear when the pass starts is processed; the others are
+ *     left as they are.
+ *   - SENSING (OK_RACE_SENSE).  For each ray r of i, (ox, oy) = the lidar origin and (dx, dy) = the ray's direction exactly
+ *     as the tick computed them (the sensor-offset origin; the device sincosf of kDeg2Rad * (rot + ray_deg[r])).  For each
+ *     opponent j, in binary32, every operation correctly rounded in this order, no contraction:
+ *       wx = x_j - ox;  wy = y_j - oy;  b = wx*dx + wy*dy;  c = (wx*wx + wy*wy) - radius*radius;
+ *     if c <= 0 then t = 0; else if b > 0 and q = b*b - c >= 0 then t = max(b - sqrt(q), 0); else j is missed.  j is hit
+ *     when t <= sensor_range (a comparison with NaN is false: a NaN pose neither hits nor is hit).  The nearest car is the
+ *     smallest t, the lowest j among ties.  It replaces the track hit only if t < hit_t[i,r] (strictly); then hit_t = t,
+ *     hit_abs = (ox + t*dx, oy + t*dy), hit_seg = -1, hit_car[i,r] = j, and hit_rel and obs follow the unpack
+ *     (CollisionChecker.cu:152-165) exactly as the tick writes them.  Rays whose track hit stands get hit_car = -1.  If a ray
+ *     was replaced, min_dist2 is the unpack's minimum over all R rays again, and the agent crashes if it is < collision_dist2:
+ *     the reference's lidar-derived crash rule applied to what the lidar now sees.
+ *   - CONTACT (OK_RACE_CONTACT).  i crashes if some opponent j has (x_i - x_j)^2 + (y_i - y_j)^2 < (radius + radius)^2, in
+ *     binary32 in that order (pos_, not the sensor origin).  The rule is symmetric.
+ *   - A CRASH BY THE PASS writes crashed = 1, done = 1 and contact[i] = 1.  contact is 0 for every other agent and is
+ *     rewritten by every pass.  timed_out, reward, fitness, prev_idx, nearest_idx and the lap state are never touched: the
+ *     tick's reward stays the track-only reward.  The crash takes effect from the next tick: the car does not move, the
+ *     auto-reset (stride or drawn) resets it, lap accounting restarts it.  A trainer that wants a penalty writes
+ *     reward[contact] = ... itself.
+ *   - ok_step_host, ok_step_host_q16 and ok_step_packed deliver their results from inside the step kernel and return
+ *     OK_ERR_STATE while races are on.  ok_lidar_query, ok_bev_query and the resets do not see cars.  The settings are read
+ *     when a launch is enqueued: a CUDA graph keeps the settings it was captured with.
+ * Races are off by default. */
+#define OK_RACE_SENSE   1
+#define OK_RACE_CONTACT 2
+typedef struct OkRaces {
+    int32_t group;  /* agents per race, 2..1024; 0 = off */
+    int32_t flags;  /* a non-empty set of OK_RACE_SENSE | OK_RACE_CONTACT */
+    float   radius; /* car body radius in px, finite and > 0 */
+} OkRaces;
+/* r NULL or r->group == 0: off.  Otherwise a group outside 2..1024, a radius that is not finite and > 0, or flags that are
+ * not a non-empty subset of the two: OK_ERR_INVALID_ARG.  Switching races on with agents allocated allocates the race
+ * buffers (synchronously) if they do not exist yet. */
+int ok_set_races(OkEnv *env, const OkRaces *r);
+int ok_get_races(const OkEnv *env, OkRaces *out);
+typedef struct OkRaceBuffers {
+    int32_t *hit_car; /* i32[N,R]: the opponent a ray hit, -1 = none (also right after allocation) */
+    uint8_t *contact; /* u8[N]: 1 = crashed by the last pass */
+} OkRaceBuffers;
+/* device pointers, owned by the env like the agent buffers: allocated when races are first switched on, or by
+ * ok_alloc_agents while races are on.  Before that: OK_ERR_STATE. */
+int ok_race_buffers(OkEnv *env, OkRaceBuffers *out);
+
 /* ---- the tick ------------------------------------------------------------------------------ */
 /* CollisionChecker::checkCollision (CollisionChecker.cu:96-100,113-174): lidar + crash flag on the
  * current poses, no movement. */

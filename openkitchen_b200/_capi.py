@@ -71,6 +71,17 @@ class OkLapBuffers(C.Structure):
                 ("lap_start", C.c_void_p), ("last_lap", C.c_void_p), ("completed", C.c_void_p)]
 
 
+class OkRaces(C.Structure):
+    _fields_ = [("group", C.c_int32), ("flags", C.c_int32), ("radius", C.c_float)]
+
+
+class OkRaceBuffers(C.Structure):
+    _fields_ = [("hit_car", C.c_void_p), ("contact", C.c_void_p)]
+
+
+RACE_SENSE, RACE_CONTACT = 1, 2  # OK_RACE_SENSE, OK_RACE_CONTACT
+
+
 # the lap arrays of OkLapBuffers: field -> numpy dtype
 LAP_ARRAYS = {"lap_idx": "int32", "progress": "int32", "laps": "int32", "ticks": "uint32", "lap_start": "uint32",
               "last_lap": "uint32", "completed": "uint8"}
@@ -169,6 +180,9 @@ SIGNATURES = {
     "ok_set_laps": (C.c_int, [_P, C.POINTER(OkLaps), _P]),
     "ok_get_laps": (C.c_int, [_P, C.POINTER(OkLaps)]),
     "ok_lap_buffers": (C.c_int, [_P, C.POINTER(OkLapBuffers)]),
+    "ok_set_races": (C.c_int, [_P, C.POINTER(OkRaces)]),
+    "ok_get_races": (C.c_int, [_P, C.POINTER(OkRaces)]),
+    "ok_race_buffers": (C.c_int, [_P, C.POINTER(OkRaceBuffers)]),
     "ok_cast_rays": (C.c_int, [_P, _P]),
     "ok_launch_step": (C.c_int, [_P, _P, _P, _P]),
     "ok_launch_steps_random": (C.c_int, [_P, C.c_uint64, C.c_int32, C.c_uint32, _P]),

@@ -69,6 +69,10 @@ class BatchEnv:
         self.lap_start_ticks = lap["lap_start"]  # u32: lap_ticks when the current lap began
         self.last_lap_ticks = lap["last_lap"]    # u32: ticks of the last completed lap, 0 = none yet
         self.completed = lap["completed"]        # u8: Agent::completed_ (laps >= target)
+        # the race pass's outputs (set_races; OkRaces in include/openkitchen_b200.h), not OkBuffers either: they exist once
+        # races have been switched on, and are None until then
+        self.hit_car = None  # i32[N,R]: the opponent a ray hit, -1 = none
+        self.contact = None  # u8[N]: crashed by the last race pass
         self._step_count = 0
 
     # ---- views -----------------------------------------------------------------------------
@@ -241,6 +245,22 @@ class BatchEnv:
         """{"enabled", "target"} as set"""
         return self.env.laps()
 
+    def set_races(self, group: int, radius: float = 0.0, sense: bool = True, contact: bool = True):
+        """Races (include/openkitchen_b200.h, OkRaces): agents a // group race each other, as discs of `radius` px on the
+        same track.  After every tick a pass on torch's current stream lets the lidar see the opponents (sense: a nearer car
+        replaces the track hit, hit_car names it, and min_dist2's crash rule applies to it) and crashes overlapping cars
+        (contact).  A car the pass crashes has crashed, done and contact set; reward is the track-only reward, so a penalty
+        is one op: ``env.reward[env.contact.bool()] -= p``.  group 0 turns races off."""
+        self.env.set_races(group, radius, sense, contact)
+        if self.hit_car is None and int(group):
+            bufs = self.env.race_buffers_info()
+            self.hit_car = torch.from_dlpack(DeviceBuffer(self.env, "hit_car", bufs["hit_car"]))
+            self.contact = torch.from_dlpack(DeviceBuffer(self.env, "contact", bufs["contact"]))
+
+    def race_settings(self) -> dict:
+        """{"group", "radius", "sense", "contact"} as set; group 0 = off"""
+        return self.env.races()
+
     def reset_drawn(self, agents=None):
         """Drawn reset (ok_reset_agents_drawn) of agents: None (all), a bool / uint8 CUDA mask with one entry per agent (e.g.
         ``env.done``, passed as it is: no nonzero, no host synchronisation), or an index tensor.  Runs on torch's current
@@ -269,7 +289,8 @@ class BatchEnv:
         the OkEnv is destroyed when the last of them is released (openkitchen_b200.dlpack)."""
         self._views.clear()
         self.reset_draw_count = None
-        for name in ("lap_idx", "lap_progress", "laps", "lap_ticks", "lap_start_ticks", "last_lap_ticks", "completed"):
+        for name in ("lap_idx", "lap_progress", "laps", "lap_ticks", "lap_start_ticks", "last_lap_ticks", "completed",
+                     "hit_car", "contact"):
             setattr(self, name, None)
         for name in ("obs", "hits", "hit_points", "hit_seg", "hit_t", "reward", "fitness", "done", "crashed", "timed_out",
                      "nearest_idx", "pos_x", "pos_y", "rot", "speed", "act_throttle", "act_steer"):

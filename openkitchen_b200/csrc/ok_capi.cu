@@ -8,6 +8,7 @@
 #include "ok_bev.cuh"
 #include "ok_kernels.cuh"
 #include "ok_lidar_query.cuh"
+#include "ok_race.cuh"
 #include "ok_step.cuh"
 #include "ok_track.hpp"
 
@@ -207,6 +208,8 @@ struct Agents
     DevPtr<uint32_t>           draw_k; // the reset-draw counters k (ok_reset_draw_counts), zeroed here
     DevPtr<uint8_t>            lap_slab; // the seven lap-accounting arrays (ok_lap_buffers), zeroed here
     OkLapBuffers               lap{};
+    DevPtr<int32_t>            hit_car; // the race buffers (ok_race_buffers): allocated while races are on
+    DevPtr<uint8_t>            contact;
     DevPtr<unsigned long long> stats; // ok_debug_stats: allocated on first use
     DevPtr<unsigned long long> trace; // ok_debug_trace
     int32_t                    trace_tiles{0};
@@ -218,6 +221,7 @@ struct OkEnv
     OkConfig               cfg{};
     OkResetDraws           draws{}; // ok_set_reset_draws; flags 0 = off
     OkLaps                 laps{};  // ok_set_laps; enabled 0 = off
+    OkRaces                races{}; // ok_set_races; group 0 = off
     bool                   has_device{false};
     int                    num_sms{0};
     size_t                 max_blob{0};
@@ -659,6 +663,47 @@ StreamWriteValue32Fn stream_write_value32()
     return fn;
 }
 
+// hit_car (-1) and contact (0) of the current population, if it has none yet
+int ensure_race_buffers(OkEnv *e)
+{
+    if (e->ag.hit_car || e->n_agents <= 0)
+        return OK_SUCCESS;
+    const size_t rays = static_cast<size_t>(e->n_agents) * static_cast<size_t>(e->rays);
+    OK_CUDA(dev_alloc(e->ag.contact, static_cast<size_t>(e->n_agents)));
+    OK_CUDA(cudaMemset(e->ag.contact.get(), 0, static_cast<size_t>(e->n_agents)));
+    DevPtr<int32_t> hit_car;
+    OK_CUDA(dev_alloc(hit_car, rays));
+    OK_CUDA(cudaMemset(hit_car.get(), 0xff, sizeof(int32_t) * rays));
+    e->ag.hit_car = std::move(hit_car);
+    return OK_SUCCESS;
+}
+
+// the race pass (OkRaces) after the tick of `p`, on the tick's stream
+int launch_race_pass(OkEnv *e, const ok::StepParams &p, cudaStream_t s)
+{
+    const OkRaces &r = e->races;
+    ok::RaceParams q{};
+    q.x = p.x, q.y = p.y, q.rot = p.rot, q.track_id = p.track_id;
+    q.crashed = p.crashed, q.done = p.done;
+    q.hit_abs = p.hit_abs, q.hit_rel = p.hit_rel, q.obs = p.obs, q.hit_t = p.hit_t, q.hit_seg = p.hit_seg;
+    q.min_dist2 = p.min_dist2;
+    q.hit_car = e->ag.hit_car.get(), q.contact = e->ag.contact.get();
+    q.ray_deg = p.ray_deg;
+    q.n = e->n_agents, q.rays = e->rays, q.group = r.group, q.flags = r.flags;
+    q.n_tracks = static_cast<int32_t>(e->tracks.size());
+    q.radius = r.radius, q.sensor_range = e->cfg.sensor_range, q.sensor_offset = e->cfg.sensor_offset;
+    q.collision_dist2 = e->cfg.collision_dist2;
+    // no body farther than sensor_range + radius from the origin can be hit; the 1 % (plus 1 px^2) margin on the square is
+    // far above the rounding error of the binary32 test (about 2^-11 of the distance where a ray grazes a body)
+    const double reach = static_cast<double>(q.sensor_range) + static_cast<double>(q.radius);
+    q.cull_d2          = static_cast<float>(std::min(reach * reach * 1.01 + 1.0, 3.0e38));
+    if (!(q.cull_d2 >= 0.0f))
+        q.cull_d2 = 3.0e38f; // a NaN range: every body is tested, and the test itself then hits nothing
+    OK_CUDA(ok::launch_race_pass(q, s));
+    e->launches++;
+    return OK_SUCCESS;
+}
+
 int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorParams *actor = nullptr, size_t actor_smem = 0)
 {
     NvtxRange range(actor ? "ok::step (actor + tick)" : "ok::step");
@@ -752,6 +797,8 @@ int launch_step(OkEnv *e, ok::StepParams &p, cudaStream_t s, const ok::ActorPara
     if (p.tile_flag) // join: the tick is complete when the last tile has reached the host
         OK_CUDA(cudaStreamWaitEvent(s, e->ev_join.get(), 0));
     e->launches++;
+    if (e->races.group)
+        return launch_race_pass(e, p, s);
     return OK_SUCCESS;
 }
 } // namespace
@@ -1103,6 +1150,9 @@ int alloc_agents_impl(OkEnv *e, int64_t n, int32_t rays, const float *h_ray_deg,
         ag.lap.last_lap  = reinterpret_cast<uint32_t *>(b + 5 * a4);
         ag.lap.completed = b + 6 * a4;
     }
+    if (e->races.group)
+        if (int rc = ensure_race_buffers(e))
+            return rc;
     OK_CUDA(dev_alloc(ag.ray_deg, static_cast<size_t>(rays)));
     OK_CUDA(cudaMemcpy(ag.ray_deg.get(), h_ray_deg, sizeof(float) * rays, cudaMemcpyHostToDevice));
     e->h_track_id.assign(static_cast<size_t>(n), 0);
@@ -1354,6 +1404,55 @@ int ok_lap_buffers(OkEnv *e, OkLapBuffers *out)
     if (!out)
         return fail(OK_ERR_INVALID_ARG, "out is NULL");
     *out = e->ag.lap;
+    return OK_SUCCESS;
+}
+
+int ok_set_races(OkEnv *e, const OkRaces *r)
+{
+    if (!e)
+        return fail(OK_ERR_INVALID_ARG, "env is NULL");
+    const OkRaces next = r && r->group ? *r : OkRaces{};
+    if (next.group)
+    {
+        if (next.group < 2 || next.group > 1024)
+            return fail(OK_ERR_INVALID_ARG, "the race group must be 0 (off) or in 2..1024");
+        if (!(std::isfinite(next.radius) && next.radius > 0.0f))
+            return fail(OK_ERR_INVALID_ARG, "the car radius must be finite and > 0");
+        if (next.flags <= 0 || (next.flags & ~(OK_RACE_SENSE | OK_RACE_CONTACT)))
+            return fail(OK_ERR_INVALID_ARG, "race flags must be a non-empty set of OK_RACE_SENSE | OK_RACE_CONTACT");
+    }
+    if (int rc = check_device(e))
+        return rc;
+    if (next.group)
+    {
+        DeviceGuard g(e->cfg.device);
+        if (int rc = ensure_race_buffers(e))
+            return rc;
+    }
+    e->races = next;
+    return OK_SUCCESS;
+}
+
+int ok_get_races(const OkEnv *e, OkRaces *out)
+{
+    if (int rc = check_device(e))
+        return rc;
+    if (!out)
+        return fail(OK_ERR_INVALID_ARG, "out is NULL");
+    *out = e->races;
+    return OK_SUCCESS;
+}
+
+int ok_race_buffers(OkEnv *e, OkRaceBuffers *out)
+{
+    if (int rc = check_ready(e))
+        return rc;
+    if (!out)
+        return fail(OK_ERR_INVALID_ARG, "out is NULL");
+    if (!e->ag.hit_car)
+        return fail(OK_ERR_STATE, "races have not been switched on for this population: there are no race buffers");
+    out->hit_car = e->ag.hit_car.get();
+    out->contact = e->ag.contact.get();
     return OK_SUCCESS;
 }
 
@@ -1782,6 +1881,8 @@ int step_host_impl(OkEnv *e, const float *h_thr, const float *h_steer, void *h_o
         return rc;
     if ((h_thr == nullptr) != (h_steer == nullptr))
         return fail(OK_ERR_INVALID_ARG, "pass both action arrays or neither");
+    if (e->races.group)
+        return fail(OK_ERR_STATE, "races are on: the race pass would leave the host copies of this call stale; use ok_launch_step");
     DeviceGuard  g(e->cfg.device);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const size_t n = static_cast<size_t>(e->n_agents);
@@ -1882,6 +1983,8 @@ int ok_step_packed(OkEnv *e, void *h_state, void *h_hits, int32_t move, void *st
         return rc;
     if (!h_state)
         return fail(OK_ERR_INVALID_ARG, "h_state is NULL");
+    if (e->races.group)
+        return fail(OK_ERR_STATE, "races are on: the race pass would leave the host copies of this call stale; use ok_launch_step");
     OkPackedLayout lay;
     rc = ok_packed_layout(e, &lay);
     if (rc)
@@ -2151,6 +2254,8 @@ int ok_debug_violations(OkEnv *e, uint64_t *count, int32_t *checks_compiled_in)
     OK_CUDA(ok::violations_lidar_query(&n));
     total += n;
     OK_CUDA(ok::violations_bev(&n));
+    total += n;
+    OK_CUDA(ok::violations_race(&n));
     total += n;
     if (count)
         *count = total;

@@ -317,6 +317,35 @@ class Env:
         check(self.lib.ok_lap_buffers(self.h, C.byref(b)))
         return {f: (getattr(b, f), (self.n,), np.dtype(dt).type) for f, dt in _capi.LAP_ARRAYS.items()}
 
+    # ---- races (OkRaces: include/openkitchen_b200.h states the definition) ---------------
+    def set_races(self, group: int, radius: float = 0.0, sense: bool = True, contact: bool = True):
+        """Races on: agents a // group race each other.  A car is a disc of `radius` px around its position; with `sense`
+        the lidar sees the opponents on its track, with `contact` overlapping cars crash.  A pass after every tick that
+        casts rays does both; a car it crashes has crashed, done and contact set.  group 0 turns races off."""
+        group = int(group)
+        flags = (_capi.RACE_SENSE if sense else 0) | (_capi.RACE_CONTACT if contact else 0)
+        if group and not (2 <= group <= 1024):
+            raise ValueError("the race group must be 0 (off) or in 2..1024")
+        if group and not (np.isfinite(radius) and radius > 0):
+            raise ValueError("the car radius must be finite and > 0")
+        if group and not flags:
+            raise ValueError("a race needs sense, contact or both")
+        check(self.lib.ok_set_races(self.h, C.byref(_capi.OkRaces(group=group, flags=flags, radius=float(radius)))))
+
+    def races(self) -> dict:
+        """{"group", "radius", "sense", "contact"} as set; group 0 = off"""
+        r = _capi.OkRaces()
+        check(self.lib.ok_get_races(self.h, C.byref(r)))
+        return {"group": int(r.group), "radius": float(r.radius), "sense": bool(r.flags & _capi.RACE_SENSE),
+                "contact": bool(r.flags & _capi.RACE_CONTACT)}
+
+    def race_buffers_info(self) -> dict:
+        """{"hit_car": (device pointer, (agents, rays), int32), "contact": (pointer, (agents,), uint8)} (OkRaceBuffers);
+        they exist once races have been switched on for this population"""
+        b = _capi.OkRaceBuffers()
+        check(self.lib.ok_race_buffers(self.h, C.byref(b)))
+        return {"hit_car": (b.hit_car, (self.n, self.rays), np.int32), "contact": (b.contact, (self.n,), np.uint8)}
+
     # ---- the tick -----------------------------------------------------------------------
     def cast_rays(self, stream=None):
         check(self.lib.ok_cast_rays(self.h, stream))

@@ -67,7 +67,8 @@ class GraphedRollout:
     f32[T, N], ``rewards`` f32[T, N], ``dones`` u8[T, N] (after the tick).  With auto_reset and reset draws on
     (BatchEnv.set_reset_draws) the crashed agents restart at drawn points inside the graph, and each replay continues the
     reset stream.  With lap accounting on (BatchEnv.set_laps with a target) ``dones`` also marks the agents that completed
-    their laps in that tick, and auto_reset restarts them too."""
+    their laps in that tick, and auto_reset restarts them too.  With races on (BatchEnv.set_races) every tick's race pass
+    is captured with it: ``obs`` includes the other cars and ``dones`` the contact crashes."""
 
     def __init__(self, env: BatchEnv, policy: Callable[[torch.Tensor], torch.Tensor], action_table: torch.Tensor, steps: int,
                  sample: bool = True):
@@ -138,7 +139,8 @@ class FusedActorRollout:
     l1, l2: ``torch.nn.Linear`` modules (the reference's ``Actor::l1`` / ``l2``); their parameters are read in place,
     so an optimizer step between rollouts is picked up by the next replay.  After ``run()``: ``obs`` f32[T, N, R],
     ``actions`` i32[T, N], ``log_prob`` f32[T, N], ``rewards`` f32[T, N], ``dones`` u8[T, N] (crashed, or with lap
-    accounting on (BatchEnv.set_laps) completed)."""
+    accounting on (BatchEnv.set_laps) completed).  With races on (BatchEnv.set_races) ok_ppo_actor_step enqueues the race
+    pass after each tick, so the graph holds it: ``obs`` includes the other cars and ``dones`` the contact crashes."""
 
     def __init__(self, env: BatchEnv, l1: torch.nn.Linear, l2: torch.nn.Linear, action_table: torch.Tensor, steps: int,
                  sample: bool = True, seed: int = 0x0C17C4E2, one_launch: bool = True):
