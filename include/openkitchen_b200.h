@@ -131,7 +131,9 @@ typedef struct OkConfig {
     float    standstill_threshold; /* kDisplamentThreshold 20        Environment.h:20 */
     float    grid_cell;            /* broadphase cell size in px (8) */
     float    beam_cell;            /* OK_RAYCAST_BEAM: start-cell size in px (2); 0 = default */
-    int32_t  beam_bins;            /* OK_RAYCAST_BEAM: direction bins, a power of two (256); 0 = default */
+    int32_t  beam_bins;            /* OK_RAYCAST_BEAM: direction bins, a power of two (256); 0 = default.  A track
+                                      whose table would pass 4 GB (1 px x 1,024 bins on some tracks) fails at table
+                                      time (ok_alloc_agents, ok_beam_lookup) with OK_ERR_INVALID_ARG */
     uint64_t agent_id_base;        /* global id of this env's agent 0 (multi-GPU: the first agent of the rank's slice).
                                       The synthetic Philox action stream is keyed by (agent_id_base + a, step), so a
                                       shard reproduces, bit for bit, its slice of the unsharded population */

@@ -265,6 +265,12 @@ bool beam_plan(const Track &t, const BeamConfig &cfg, BeamPlan &pl, std::string 
             pl.rows[c] = static_cast<uint32_t>(pl.covered.size());
             pl.covered.push_back(static_cast<uint32_t>(c));
         }
+    // the rows and entries alone already pass the 32-bit offsets of beam_layout: fail before any list is built
+    if (sizeof(BeamHeader) + pl.rows.size() * 4 + pl.covered.size() * static_cast<size_t>(pl.nb) * 16 >= 0xffffffffull)
+    {
+        err = "beam table too large";
+        return false;
+    }
     return true;
 }
 
